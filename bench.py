@@ -3,7 +3,7 @@
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
                     [--workload mica_ompa|synthetic] [--num-shuffling 1000] [--scaling strong|weak]
-                    [--no-config4] [--no-cpu-baseline]
+                    [--no-config4] [--no-cpu-baseline] [--dump-outputs DIR]
 
 Metric (BASELINE.json): shuffled pairs / second of the probability stage of
 `ractip --zscore=12 --num-shuffling=1000` (per shuffled pair: 2 single-strand
@@ -19,6 +19,13 @@ clocks, e2e and cpu_baseline (--workload synthetic makes it the headline instead
 --impl reference: the reference's probability stage cannot be built here (ViennaRNA absent,
 DESIGN.md section 5), so the timed CPU implementation is the oracle port (oracle/) on all host
 threads; it does not load the product library.
+
+--dump-outputs DIR: after the timed steps, the thresholded lists x, y, z, v, w of the last step (what a
+caller of the timed path receives) go to DIR/<list>.npy, and those of the configs[4] leg to
+DIR/config4_<list>.npy: float32 rows (pair index in the batch, i, j, p).  On N GPUs rank 0 writes the lists of
+all ranks; with weak scaling the pair index runs over the ranks' batches in rank order.  The inputs depend only
+on the arguments, so two builds can be compared output for output.  The legs share 64 MB equally; a leg whose
+lists exceed its share is cut to a seeded sample of its pairs.
 """
 from __future__ import annotations
 
@@ -42,6 +49,7 @@ METRIC = "shuffled pairs/sec, probability stage of --zscore=12 (McCaskill in/out
 UNIT = "pairs/s"
 CONFIG4_PAIRS_PER_GPU = 148      # bounded batch of the configs[4] leg: one two-strand problem per SM
 CONFIG4_REF_PAIRS = 8            # ... and of its CPU arm (the port does ~0.5 pairs/s on 16 cores)
+DUMP_BYTES = 64 << 20            # --dump-outputs: all legs together
 
 
 # --------------------------------------------------------------------------- workload
@@ -224,7 +232,7 @@ def run_reference(args, rank: int, world: int):
     if args.workload == "mica_ompa":
         line = arm("mica_ompa", args.num_shuffling, args.steps, args.warmup)
         if not args.no_config4:
-            c4 = arm("synthetic", CONFIG4_REF_PAIRS, 2, 0)
+            c4 = arm("synthetic", CONFIG4_REF_PAIRS, args.steps, args.warmup)
             line["config4"] = {k: c4[k] for k in ("value", "unit", "steps", "ms_per_step", "config", "cpu_baseline", "e2e", "data")}
     else:
         line = arm("synthetic", max(2, cores // 4), args.steps, args.warmup)
@@ -246,10 +254,41 @@ def traffic_record(workload: str):
     return rec, None
 
 
+def step_lists(plan, pairs_all, opts, buf, world: int, weak: bool):
+    """PairRecords of every pair of a step from the host copy of the gathered buffer (of `local` when N = 1), in batch
+    order.  With weak scaling each rank ran a batch of its own, laid out by its own plan at the start of its
+    equally sized slot; the batches follow one another in rank order."""
+    if not weak:
+        return plan.unpack(buf)
+    from ractip_b200.dist import ShardPlan
+    slots = buf.reshape(world, -1)
+    out = []
+    for r in range(world):
+        own = ShardPlan(pairs_all[r], opts, 0, 1)
+        out += own.unpack(slots[r][:own.nbytes])
+    return out
+
+
+def dump_outputs(out_dir: Path, legs):
+    """--dump-outputs: legs = [(file prefix, PairRecords of every pair in batch order)]."""
+    out_dir.mkdir(parents=True, exist_ok=True)
+    for prefix, recs in legs:
+        assert len(recs) < 1 << 24, "pair indices must stay exact in float32"
+        nbytes = np.array([sum(len(getattr(r, name)) for name in "xyzvw") * 16 for r in recs])
+        order = np.random.default_rng(0).permutation(len(recs))
+        keep = np.sort(order[:np.searchsorted(np.cumsum(nbytes[order]), DUMP_BYTES // len(legs), side="right")])
+        for name in "xyzvw":
+            lists = [getattr(recs[k], name) for k in keep]
+            rows = [np.column_stack([np.full(len(a), k), a["i"], a["j"], a["p"]]) for k, a in zip(keep, lists)]
+            np.save(out_dir / f"{prefix}{name}.npy",
+                    np.concatenate(rows).astype(np.float32) if rows else np.zeros((0, 4), dtype=np.float32))
+
+
 def measure(args, stage, workload, pairs_all, desc, data, rank, world, local_rank, steps, warmup, scaling, dev, stream,
-            cpu_sample, with_cpu):
+            cpu_sample, with_cpu, dump=False):
     """One workload through the three measurements: device-resident step ("value"), end to end through the C ABI
-    with host buffers ("e2e"), roofline of the kernels and the CPU port beside it (rank 0, N = 1)."""
+    with host buffers ("e2e"), roofline of the kernels and the CPU port beside it (rank 0, N = 1).  dump: rank 0 also
+    returns the lists of the last timed step under "outputs"."""
     import torch
     import torch.distributed as dist
 
@@ -342,6 +381,10 @@ def measure(args, stage, workload, pairs_all, desc, data, rank, world, local_ran
         for r in range(world):
             cr = g[r][plan.rec_bytes:plan.rec_bytes + 24 * len(plan.shards[r])].view(np.int32).reshape(-1, 6)
             assert cr[:, :3].sum() > 0, f"rank {r} gathered nothing"
+    outputs = None
+    if dump and rank == 0:
+        outputs = step_lists(plan, pairs_all, opts, (gathered if world > 1 else local).cpu().numpy(), world,
+                             scaling == "weak" and world > 1)
 
     # ---------------- end to end through the C ABI with host buffers
     n = len(mine)
@@ -450,6 +493,8 @@ def measure(args, stage, workload, pairs_all, desc, data, rank, world, local_ran
         res["roofline"] = roofline
     if cpu:
         res["cpu_baseline"] = cpu
+    if outputs is not None:
+        res["outputs"] = outputs
     lib.rp_host_free(C.c_void_p(pin)); lib.rp_host_free(C.c_void_p(pin_recs)); lib.rp_host_free(C.c_void_p(pin_cnt))
     batch.close()
     return res
@@ -486,8 +531,9 @@ def run_ours(args, rank: int, world: int, local_rank: int):
     pairs, desc, data = workload_pairs(args.workload, args.num_shuffling, args.scaling)
     cpu_n = (min(args.num_shuffling, 1000), max(1, min(64, args.num_shuffling // 4))) if args.workload == "mica_ompa" \
         else (max(2, (os.cpu_count() or 1) // 4), 1)
+    dump = args.dump_outputs is not None
     head = measure(args, stage, args.workload, pairs, desc, data, rank, world, local_rank, args.steps, args.warmup,
-                   args.scaling, dev, stream, cpu_n, not args.no_cpu_baseline)
+                   args.scaling, dev, stream, cpu_n, not args.no_cpu_baseline, dump)
     c4 = None
     if args.workload == "mica_ompa" and not args.no_config4:
         # BASELINE configs[4] in the same run: a bounded batch, fixed work per GPU ("weak")
@@ -495,10 +541,12 @@ def run_ours(args, rank: int, world: int, local_rank: int):
         p4 = [p[0] for p in per_rank] if world > 1 else per_rank[0][0]
         c4 = measure(args, stage, "synthetic", p4, per_rank[0][1].replace(f"--num-shuffling={CONFIG4_PAIRS_PER_GPU}",
                      f"{CONFIG4_PAIRS_PER_GPU} of the --num-shuffling=1000 shuffles per GPU"), per_rank[0][2], rank, world,
-                     local_rank, 2, 3, "weak" if world > 1 else "strong", dev, stream, (CONFIG4_REF_PAIRS, 1),
-                     not args.no_cpu_baseline)
+                     local_rank, args.steps, args.warmup, "weak" if world > 1 else "strong", dev, stream,
+                     (CONFIG4_REF_PAIRS, 1), not args.no_cpu_baseline, dump)
         if world == 1:
             c4["scaling"] = "weak"
+    if dump and rank == 0:
+        dump_outputs(Path(args.dump_outputs), [("", head.pop("outputs"))] + ([("config4_", c4.pop("outputs"))] if c4 else []))
     if rank == 0:
         line = {"metric": METRIC, "value": head["value"], "unit": UNIT, "n_gpus": world, "steps": head["steps"],
                 "warmup": head["warmup"], "ms_per_step": head["ms_per_step"], "higher_is_better": True,
@@ -540,7 +588,13 @@ def main():
     ap.add_argument("--scaling", default="strong", choices=["strong", "weak"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-config4", action="store_true", help="skip the BASELINE configs[4] leg of the default run")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the thresholded lists of the last timed step to DIR/*.npy (see the module docstring)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs is not None and args.impl != "ours":
+        ap.error("--dump-outputs writes what the GPU path computed: it needs --impl ours")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))

@@ -1,13 +1,15 @@
 """Energy-model layer: BL* copy semantics (reference src/boltzmann_param.c:5908-6026),
 the embedded Turner-2004 residual tables and the -P reader."""
 import ctypes as C
-import re
+import struct
 from pathlib import Path
 
 import numpy as np
-import pytest
 
-REF = Path("/root/reference/src/boltzmann_param.c")
+# The reference's BL* initialisers (src/boltzmann_param.c:21-5906, macros expanded), frozen: a byte copy of
+# params/blstar.bin as tools/gen_blstar_bin.py wrote it from that source, which this test had checked it against.
+# Kept apart from params/ so that an edit of the product's tables cannot move the expectation with it.
+BLSTAR_REF = Path(__file__).resolve().parent / "golden" / "blstar_reference.bin"
 INF = 10000000
 
 
@@ -42,14 +44,27 @@ def test_default_model_digest_is_stable(lib, model):
     assert int(golden.read_text().strip()) == d1
 
 
-@pytest.mark.skipif(not REF.exists(), reason="reference tree only exists in the build container")
+def _blstar_arrays():
+    """name -> values of the frozen reference arrays (the packed layout of tools/gen_blstar_bin.py)."""
+    blob = BLSTAR_REF.read_bytes()
+    assert blob[:8] == b"RPBLSTR1"
+    (n,), p = struct.unpack_from("<i", blob, 8), 12
+    arrays = {}
+    for _ in range(n):
+        name = blob[p:p + 24].rstrip(b"\0").decode()
+        (cnt,) = struct.unpack_from("<i", blob, p + 24)
+        arrays[name] = list(struct.unpack_from("<%di" % cnt, blob, p + 28))
+        p += 28 + 4 * cnt
+    return arrays
+
+
 def test_blstar_matches_reference_source(model):
     """Every BL* array against the reference's own initialisers, with the reference's index ranges."""
-    text = re.sub(r"/\*.*?\*/", " ", REF.read_text(), flags=re.S)
-    mac = {"INF": INF, "NST": 0, "DEF": -50}
-    arrays = {}
-    for mm in re.finditer(r"static\s+int\s+(\w+)\s*\[\]\s*=\s*\{(.*?)\};", text, flags=re.S):
-        arrays[mm.group(1)] = [mac[t.strip()] if t.strip() in mac else int(t) for t in mm.group(2).split(",") if t.strip()]
+    arrays = _blstar_arrays()
+    assert {k: len(v) for k, v in arrays.items()} == {
+        "stack37a": 49, "mismatchH37a": 175, "mismatchI37a": 175, "dangle5_37a": 40, "dangle3_37a": 40,
+        "int11_37a": 1225, "int21_37a": 6125, "int22_37a": 12544, "hairpin37a": 31, "bulge37a": 31,
+        "internal_loop37a": 31, "MLparams_a": 4, "ninio_a": 2}
     m = model
     a = arrays["stack37a"]; p = 0
     for i in range(1, 8):
