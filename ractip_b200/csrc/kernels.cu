@@ -518,36 +518,34 @@ __global__ void __launch_bounds__(256) peak_smem_kernel(double* out, int iters) 
 // ---------------------------------------------------------------------------
 namespace {
 using MccKernel = void (*)(BatchDev);
-// minb = 2: 64-register build, BAND-wide sums; minb = 1: 128 registers, bands of `wide` diagonals (5, 10 or 15)
-MccKernel mcc_kernel(int minb, int wide, int* w_out) {
+// minb = 2: 64-register build, BAND-wide sums; minb = 1: 128 registers, bands of 10 diagonals
+MccKernel mcc_kernel(int minb, int* w_out) {
   if (minb >= 2) { *w_out = BAND; return mcc_persistent<RP_MCC_MIN_CTAS, BAND>; }
-  if (wide >= 15) { *w_out = 15; return mcc_persistent<1, 15>; }
-  if (wide >= 10) { *w_out = 10; return mcc_persistent<1, 10>; }
-  *w_out = BAND;
-  return mcc_persistent<1, BAND>;
+  *w_out = 10;
+  return mcc_persistent<1, 10>;
 }
 }  // namespace
 
-int mcc_max_ctas_per_sm(int threads, int minb, int wide) {
+int mcc_max_ctas_per_sm(int minb) {
   int n = 0, w = BAND;
-  MccKernel k = mcc_kernel(minb, wide, &w);
-  size_t smem = shared_bytes(threads, w);
+  MccKernel k = mcc_kernel(minb, &w);
+  size_t smem = shared_bytes(RP_MCC_THREADS, w);
   if (cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess) { cudaGetLastError(); return 0; }
-  if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, k, threads, smem) != cudaSuccess) return 0;
+  if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, k, RP_MCC_THREADS, smem) != cudaSuccess) return 0;
   return minb >= 2 ? n : (n > 1 ? 1 : n);
 }
 
-cudaError_t launch_mcc(const BatchDev& b, int grid, int threads, int minb, int wide, cudaStream_t st) {
+cudaError_t launch_mcc(const BatchDev& b, int grid, int minb, cudaStream_t st) {
   int w = BAND;
-  MccKernel k = mcc_kernel(minb, wide, &w);
-  size_t smem = shared_bytes(threads, w);
+  MccKernel k = mcc_kernel(minb, &w);
+  size_t smem = shared_bytes(RP_MCC_THREADS, w);
   cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-  k<<<grid, threads, smem, st>>>(b);
+  k<<<grid, RP_MCC_THREADS, smem, st>>>(b);
   return cudaGetLastError();
 }
 
-cudaError_t launch_mcc_cluster(const BatchDev& b, int nclusters, int ctas, int threads, cudaStream_t st) {
-  size_t smem = shared_bytes(threads, 10);
+cudaError_t launch_mcc_cluster(const BatchDev& b, int nclusters, int ctas, cudaStream_t st) {
+  size_t smem = shared_bytes(RP_MCC_THREADS, 10);
   MccKernel k = ctas >= 16 ? mcc_cluster_kernel<10, 16> : mcc_cluster_kernel<10, 8>;
   const int G = ctas >= 16 ? 16 : 8;
   cudaError_t e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
@@ -556,7 +554,7 @@ cudaError_t launch_mcc_cluster(const BatchDev& b, int nclusters, int ctas, int t
     e = cudaFuncSetAttribute(k, cudaFuncAttributeNonPortableClusterSizeAllowed, 1);
     if (e != cudaSuccess) return e;
   }
-  k<<<nclusters * G, threads, smem, st>>>(b);
+  k<<<nclusters * G, RP_MCC_THREADS, smem, st>>>(b);
   return cudaGetLastError();
 }
 

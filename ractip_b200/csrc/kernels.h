@@ -17,9 +17,6 @@
 #endif
 namespace rp {
 
-// queue entries: problem index, + RP_JOB_UNPAIRED for the unpaired-window pass of a deferred problem as a job of its own
-constexpr int RP_JOB_UNPAIRED = 0x40000000;
-
 struct BatchDev {
   const DevModel* model;
   const uint8_t* seq;      // encoded sequences, one zero byte of padding around each
@@ -59,11 +56,12 @@ struct SparseDev {
   int min_w, max_w;                    // window-length indices min_w-1 .. max_w-1 are scanned (src/ractip.cpp:622)
 };
 
-// minb = 2: 64-register build, two CTAs per SM; 1: 128 registers, one CTA per SM, split sums in bands of `wide` diagonals
-int mcc_max_ctas_per_sm(int threads, int minb, int wide);
-cudaError_t launch_mcc(const BatchDev& b, int grid, int threads, int minb, int wide, cudaStream_t st);
+// general kernel, RP_MCC_THREADS threads.  minb = 2: 64-register build, two CTAs per SM; 1: 128 registers, one CTA
+// per SM, split sums in bands of 10 diagonals
+int mcc_max_ctas_per_sm(int minb);
+cudaError_t launch_mcc(const BatchDev& b, int grid, int minb, cudaStream_t st);
 // multi-CTA wavefront: `nclusters` clusters of `ctas` (8 or 16) CTAs, one problem (and one workspace slot) per cluster
-cudaError_t launch_mcc_cluster(const BatchDev& b, int nclusters, int ctas, int threads, cudaStream_t st);
+cudaError_t launch_mcc_cluster(const BatchDev& b, int nclusters, int ctas, cudaStream_t st);
 int band_max_ctas_per_sm(int threads, size_t smem);   // threads = 256 (2 CTAs/SM) or 512 (1 CTA/SM)
 cudaError_t launch_band(const BatchDev& b, int grid, int threads, size_t smem, cudaStream_t st);
 cudaError_t launch_duplex(const BatchDev& b, int grid, cudaStream_t st);

@@ -78,21 +78,23 @@ RP_HD int band_ldb(int n) { return ((n + 1 + 7) / 8) * 8; }
 RP_HD int band_ngp(int n) { return (n + 7) / 8 + 3; }
 // partial sums of the split-sum band phases / of the interior items (they alias).  The CUDA build runs the
 // shuffle form of the band phases (mcc_band_shfl.cuh), where a warp owns 32-(BAND-1) rows: 2*BAND partials for
-// 28 rows per warp.  The host emulation runs the direct form: 2*BAND partials per thread.
-RP_HD size_t band_part_doubles(int n, int T) {
+// 28 rows per warp.  The host emulation runs the direct form: 2*BAND partials per thread.  Host code that sizes a
+// launch of the CUDA build (plan.cpp) asks for the shuffle form: shfl = true.
 #ifdef __CUDACC__
-  const size_t a = (size_t)2 * BAND * (32 - (BAND - 1)) * (T / 32);
+constexpr bool BAND_SHFL = true;
 #else
-  const size_t a = (size_t)2 * BAND * T;
+constexpr bool BAND_SHFL = false;
 #endif
+RP_HD size_t band_part_doubles(int n, int T, bool shfl = BAND_SHFL) {
+  const size_t a = shfl ? (size_t)2 * BAND * (32 - (BAND - 1)) * (T / 32) : (size_t)2 * BAND * T;
   const size_t b = (size_t)(NSLICE + 1) * BR * band_ngp(n);
   return a > b ? a : b;
 }
-RP_HD size_t band_shared_doubles(int n, int T) {
-  return band_part_doubles(n, T) + 128 /*red*/ + (size_t)3 * BSLOTS * band_ldb(n) + (size_t)3 * BR * band_ngp(n) +
+RP_HD size_t band_shared_doubles(int n, int T, bool shfl = BAND_SHFL) {
+  return band_part_doubles(n, T, shfl) + 128 /*red*/ + (size_t)3 * BSLOTS * band_ldb(n) + (size_t)3 * BR * band_ngp(n) +
          GPACK + 64 + (size_t)(n + 2) + SM_DOUBLES + DESC_DOUBLES + (size_t)(n + 2 + 7) / 8 + 2;
 }
-RP_HD size_t band_shared_bytes(int n, int T) { return band_shared_doubles(n, T) * sizeof(double); }
+RP_HD size_t band_shared_bytes(int n, int T, bool shfl = BAND_SHFL) { return band_shared_doubles(n, T, shfl) * sizeof(double); }
 
 RP_HD void carve_band(Shared& sh, BandShared& bs, void* base, int n, int T) {
   sh.T = T;

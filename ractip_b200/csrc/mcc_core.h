@@ -65,6 +65,8 @@ struct Problem {
   int defer_up;       // 1: the unpaired-window pass runs later in its own kernel (unstru_kernel) on the tables left in ws_off
   long long ws_off;   // >= 0: private workspace (doubles from BatchDev::ws_up) that outlives the wavefront kernel; -1: the CTA's slot
 };
+// queue entries: problem index, + RP_JOB_UNPAIRED for the unpaired-window pass of a deferred problem as a job of its own
+constexpr int RP_JOB_UNPAIRED = 0x40000000;
 
 enum {
   T_Q = 0, T_QQ, T_QM, T_QM1, T_QM2, T_QB, T_QBI, T_QB1N, T_QBAU,
