@@ -23,10 +23,12 @@ namespace rp {
 
 namespace {
 
-template <int NB = 4, int W = BAND>
+// executor of the phase schedules (mcc_driver.h) on the G CTAs that share one problem: one CTA (G = 1) or the CTAs of
+// a thread-block cluster (G > 1, launched with __cluster_dims__(G, 1, 1))
+template <int G = 1, int NB = 4, int W = BAND>
 struct CtaExecT {
+  static constexpr int kCtas = G;
   static constexpr int kBatch = NB;   // load-batch depth of the split-sum band phases (mcc_band_shfl.cuh)
-  static constexpr int kWideBatch = 8;   // ... of the wide far passes: one sum at a time leaves registers for 8 steps' loads
   static constexpr int kWide = W;     // diagonals per split-sum band of the general kernel (solve_mcc_wide when > BAND)
   long long* prof;  // optional per-phase cycle counters (RP_PROFILE=1), else null
   __device__ __forceinline__ int nthreads() const { return blockDim.x; }
@@ -41,33 +43,13 @@ struct CtaExecT {
       atomicAdd(reinterpret_cast<unsigned long long*>(prof + 32 + id), 1ull);
     }
   }
+  // G > 1 only: this CTA's rank in the cluster, and the cluster barrier
+  __device__ __forceinline__ int rank_begin() const { return (int)cooperative_groups::this_cluster().block_rank(); }
+  __device__ __forceinline__ int rank_end() const { return rank_begin() + 1; }
+  __device__ __forceinline__ void sync() { cooperative_groups::this_cluster().sync(); }
 };
 
-using CtaExec = CtaExecT<4>;
-
-// one CTA of a thread-block cluster that works on ONE problem (solve_mcc_cluster)
-template <int W>
-struct ClusterExec {
-  static constexpr int kBatch = 4;
-  static constexpr int kWideBatch = 8;
-  static constexpr int kWide = W;
-  long long* prof;
-  __device__ __forceinline__ int rank() const { return (int)cooperative_groups::this_cluster().block_rank(); }
-  __device__ __forceinline__ int nranks() const { return (int)cooperative_groups::this_cluster().num_blocks(); }
-  __device__ __forceinline__ int nthreads() const { return blockDim.x; }
-  template <class F>
-  __device__ __forceinline__ void phase(int id, F f) {
-    long long t0 = 0;
-    if (RP_EXPROF(prof) && threadIdx.x == 0) t0 = clock64();
-    f(threadIdx.x);
-    __syncthreads();
-    if (RP_EXPROF(prof) && threadIdx.x == 0) {
-      atomicAdd(reinterpret_cast<unsigned long long*>(prof + id), (unsigned long long)(clock64() - t0));
-      atomicAdd(reinterpret_cast<unsigned long long*>(prof + 32 + id), 1ull);
-    }
-  }
-  __device__ __forceinline__ void csync() { cooperative_groups::this_cluster().sync(); }
-};
+using CtaExec = CtaExecT<>;
 
 }  // namespace
 
@@ -81,7 +63,7 @@ template <int MINB, int W>
 __global__ void __launch_bounds__(RP_MCC_THREADS, MINB) mcc_persistent(BatchDev b) {
   extern __shared__ double smem_raw[];
   __shared__ int s_next;
-  CtaExecT<(MINB >= 2 ? 2 : 4), W> ex;
+  CtaExecT<1, (MINB >= 2 ? 2 : 4), W> ex;
   ex.prof = b.prof;
   Shared sh;
   carve_shared(sh, smem_raw, blockDim.x, W);
@@ -102,7 +84,7 @@ __global__ void __launch_bounds__(RP_MCC_THREADS, MINB) mcc_persistent(BatchDev 
 }
 
 // mcc_cluster_kernel: the multi-CTA wavefront for long problems when there are few of them (a single long
-// pair rather than a shuffle batch).  A cluster of G CTAs works on one problem (solve_mcc_cluster); clusters
+// pair rather than a shuffle batch).  A cluster of G CTAs works on one problem (solve_mcc_wide); clusters
 // pull problems from the same cost-ordered queue, one workspace slot each.  G = 16 (beyond the portable
 // cluster size, opted in at launch) when there are at most sm_count/16 problems, else 8.
 template <int W, int G>
@@ -111,7 +93,7 @@ __global__ void __cluster_dims__(G, 1, 1) __launch_bounds__(RP_MCC_THREADS, 1) m
   extern __shared__ double smem_raw[];
   __shared__ int s_next;
   cg::cluster_group cl = cg::this_cluster();
-  ClusterExec<W> ex;
+  CtaExecT<G, 4, W> ex;
   ex.prof = b.prof;
   Shared sh;
   carve_shared(sh, smem_raw, blockDim.x, W);
@@ -127,7 +109,7 @@ __global__ void __cluster_dims__(G, 1, 1) __launch_bounds__(RP_MCC_THREADS, 1) m
     Ctx c;
     bind_ctx(c, b.model, b.seq + p.seq_off - 1, p, b.ws + (size_t)cid * b.slot_stride);
     c.dbg = b.dbg;
-    solve_mcc_cluster(ex, c, p, b.dense, b.logz, sh);
+    solve_mcc_wide(ex, c, p, b.dense, b.logz, sh);
   }
 }
 
@@ -202,23 +184,9 @@ __global__ void __launch_bounds__(RP_UP_THREADS, 1) unstru_kernel(BatchDev b) {
     bind_ctx(c, b.model, b.seq + p.seq_off - 1, p, b.ws_up + p.ws_off);
     c.dbg = b.dbg;
     c.prof = b.prof;
-    if (p.n + 2 <= RP_SMEM_SEQ) {
-      for (int x = threadIdx.x; x <= p.n + 1; x += T) s_seq[x] = c.S[x];
-      __syncthreads();
-      c.S = s_seq;
-    }
+    if (p.n + 2 <= RP_SMEM_SEQ) stage_sequence(ex, c, s_seq, [](int) {});
     inside_end(c);   // 1/Z from the finished inside table
-    // the phases of emit_unpaired (mcc_driver.h)
-    ex.phase(PH_UN_HAIRPIN, [&](int tid) {
-      unstru_hairpin(c, tid, T);
-      unstru_gap_specials(c, *b.model, tid, T);
-    });
-    ex.phase(PH_UN_GAPS0, [&](int tid) { unstru_gaps(c, s_gfull, 0, tid, T); });
-    ex.phase(PH_UN_GAPS1, [&](int tid) { unstru_gaps(c, s_gfull, 1, tid, T); });
-    ex.phase(PH_UN_DOMROWS, [&](int tid) { unstru_dom_rows(c, tid, T); });
-    ex.phase(PH_UN_DOMCOLS, [&](int tid) { unstru_dom_cols(c, tid, T); });
-    ex.phase(PH_UN_MLTAB, [&](int tid) { unstru_ml_tables(c, tid, T); });
-    if (p.out_up >= 0) ex.phase(PH_UN_WINDOWS, [&](int tid) { unstru_windows(c, b.dense + p.out_up, tid, T); });
+    emit_unpaired(ex, c, p, b.dense, *b.model, s_gfull);
   }
 }
 

@@ -9,13 +9,10 @@
 #include "mcc_core.h"
 #include "ractip_prob.h"
 
-#ifndef RP_MCC_THREADS
-#define RP_MCC_THREADS 512
-#endif
-#ifndef RP_MCC_MIN_CTAS
-#define RP_MCC_MIN_CTAS 2
-#endif
 namespace rp {
+
+constexpr int RP_MCC_THREADS = 512;   // threads per CTA of the general kernel
+constexpr int RP_MCC_MIN_CTAS = 2;    // CTAs per SM of its 64-register build
 
 struct BatchDev {
   const DevModel* model;

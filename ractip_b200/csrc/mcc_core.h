@@ -1040,6 +1040,10 @@ template <int W>
 RP_HD int wide_start_inside(int d) { return TURN + 1 + (d - TURN - 1) / W * W; }
 template <int W>
 RP_HD int wide_start_outside(int n, int d) { return n - 1 - (n - 1 - d) / W * W; }
+// rows one far-pass call takes with T threads: a warp of the shuffle variants owns 32-(W-1) rows
+// (W = BAND: mcc_band_shfl.cuh, W > BAND: mcc_wide_shfl.cuh)
+template <int W>
+RP_HD int wide_chunk(int T) { return (32 - (W - 1)) * (T / 32); }
 
 // host / reference form of the far pass (the CUDA build runs the shuffle variants of mcc_band_shfl.cuh)
 template <int W>

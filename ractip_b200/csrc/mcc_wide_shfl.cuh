@@ -38,9 +38,8 @@ struct WideSplit {
     CP = NW * HWW;
   }
 };
-// rows one far-pass call can take with T threads
-template <int W>
-RP_HD int wide_chunk(int T) { return (32 - (W - 1)) * (T / 32); }
+// load-batch depth of the far passes: one sum at a time leaves registers for 8 steps' loads
+constexpr int WIDE_NB = 8;
 // partial (sum w, diagonal e, slice sl, row cell) at part[((w*W+e)*S + sl)*CP + cell]
 
 template <int W, int NB>

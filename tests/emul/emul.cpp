@@ -11,8 +11,11 @@
 #include "seq_encode.h"
 
 namespace {
-template <int W>
+// The executor (contract at the top of mcc_driver.h) of G CTAs that share one problem, run as one serial flow with one
+// copy of shared memory: it runs the work of every rank, rank after rank, as the device deals it out.
+template <int W, int G = 1>
 struct SerialExecT {
+  static constexpr int kCtas = G;
   static constexpr int kWide = W;   // width of the wide split-sum bands (solve_mcc_wide)
   int T;
   int nthreads() const { return T; }
@@ -20,6 +23,9 @@ struct SerialExecT {
   void phase(int, F f) {
     for (int t = 0; t < T; t++) f(t);
   }
+  int rank_begin() const { return 0; }
+  int rank_end() const { return G; }
+  void sync() {}
 };
 using SerialExec = SerialExecT<rp::BAND>;
 
@@ -33,8 +39,9 @@ void layout(int n, int max_w, int n1, int n2, size_t& nbp, size_t& nup, size_t& 
 }  // namespace
 
 // one problem; band = 0: general kernel (solve_mcc), band = 1: shared-memory band kernel (solve_band),
-// band = 5, 8, 10, 15: general kernel with wide split-sum bands of that width (solve_mcc_wide)
-static int run_problem(int band, const rp_model* m, const char* seq, int n, int cp, int kind, int max_w, int n1, int n2,
+// band = 5, 8, 10, 15: general kernel with wide split-sum bands of that width (solve_mcc_wide);
+// G = 8, 16 (band = 10 only): solve_mcc_wide on a cluster of G CTAs
+static int run_problem(int band, int G, const rp_model* m, const char* seq, int n, int cp, int kind, int max_w, int n1, int n2,
                        float th_hy, int T, float* bp, float* up, float* hp, double* logz) {
   int rc = rp::build_dev_model(*m, &g_model);
   if (rc) return rc;
@@ -59,7 +66,13 @@ static int run_problem(int band, const rp_model* m, const char* seq, int n, int 
   rp::Ctx c;
   rp::bind_ctx(c, &g_model, S.data(), p, ws.data());
   SerialExec ex{T};
-  if (band == 5) {
+  if (G == 8) {
+    SerialExecT<10, 8> wx{T};
+    rp::solve_mcc_wide(wx, c, p, dense.data(), lz, sh);
+  } else if (G == 16) {
+    SerialExecT<10, 16> wx{T};
+    rp::solve_mcc_wide(wx, c, p, dense.data(), lz, sh);
+  } else if (band == 5) {
     SerialExecT<5> wx{T};
     rp::solve_mcc_wide(wx, c, p, dense.data(), lz, sh);
   } else if (band == 8) {
@@ -86,14 +99,19 @@ static int run_problem(int band, const rp_model* m, const char* seq, int n, int 
 
 extern "C" int emul_problem(const rp_model* m, const char* seq, int n, int cp, int kind, int max_w, int n1, int n2,
                             float th_hy, int T, float* bp, float* up, float* hp, double* logz) {
-  return run_problem(0, m, seq, n, cp, kind, max_w, n1, n2, th_hy, T, bp, up, hp, logz);
+  return run_problem(0, 1, m, seq, n, cp, kind, max_w, n1, n2, th_hy, T, bp, up, hp, logz);
 }
 extern "C" int emul_wide_problem(int W, const rp_model* m, const char* seq, int n, int cp, int kind, int max_w, int n1,
                                  int n2, float th_hy, int T, float* bp, float* up, float* hp, double* logz) {
   if (W != 5 && W != 8 && W != 10 && W != 15) return -1;
-  return run_problem(W, m, seq, n, cp, kind, max_w, n1, n2, th_hy, T, bp, up, hp, logz);
+  return run_problem(W, 1, m, seq, n, cp, kind, max_w, n1, n2, th_hy, T, bp, up, hp, logz);
 }
 extern "C" int emul_band_problem(const rp_model* m, const char* seq, int n, int cp, int kind, int max_w, int n1, int n2,
                                  float th_hy, int T, float* bp, float* up, float* hp, double* logz) {
-  return run_problem(1, m, seq, n, cp, kind, max_w, n1, n2, th_hy, T, bp, up, hp, logz);
+  return run_problem(1, 1, m, seq, n, cp, kind, max_w, n1, n2, th_hy, T, bp, up, hp, logz);
+}
+extern "C" int emul_cluster_problem(int G, const rp_model* m, const char* seq, int n, int cp, int kind, int max_w, int n1,
+                                    int n2, float th_hy, int T, float* bp, float* up, float* hp, double* logz) {
+  if (G != 8 && G != 16) return -1;
+  return run_problem(10, G, m, seq, n, cp, kind, max_w, n1, n2, th_hy, T, bp, up, hp, logz);
 }
