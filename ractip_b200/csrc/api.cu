@@ -497,9 +497,9 @@ int rp_batch_run(rp_batch* b) {
     long long h[64];
     CU(cudaMemcpyAsync(h, ctx->d_prof, sizeof h, cudaMemcpyDeviceToHost, st));
     CU(cudaStreamSynchronize(st));
-    static const char* names[32] = {"stage", "prologue", "prologue2", "inside_A", "inside_B", "generic_in", "generic_out", "outside_A", "outside_B", "write_bp", "un_hairpin", "un_gaps0", "un_gaps1", "un_domrows", "un_domcols", "un_mltab", "un_windows", "write_hp", "logz", "band_A", "band_B", "collect", "un_hairpin.cells(t0)", "un_hairpin.specials(t0)", "finish_in.loads(t0)", "finish_in.rest(t0)", "bandA_in.head(t0)", "bandA_in.main(t0)", "bandA_in.tail(t0)", "bandA_out.PR(t0)", "bandA_out.need(t0)", "bandA_out.ML(t0)"};
+    static const char* names[32] = {"stage", "prologue", "prologue2", "inside_A", "inside_B", "generic_in", "generic_out", "outside_A", "outside_B", "write_bp", "un_items", "un_domrows", "un_domcols", "un_windows", "write_hp", "logz", "band_A", "band_B", "collect", "", "", "", "", "", "finish_in.loads(t0)", "finish_in.rest(t0)", "bandA_in.head(t0)", "bandA_in.main(t0)", "bandA_in.tail(t0)", "bandA_out.PR(t0)", "bandA_out.need(t0)", "bandA_out.ML(t0)"};
     long long tot = 0;
-    for (int k = 0; k < 22; k++) tot += h[k];
+    for (int k = 0; k < 19; k++) tot += h[k];   // the phase counters (PH_COUNT, mcc_driver.h)
     for (int k = 0; k < 32; k++)
       if (h[32 + k]) std::fprintf(stderr, "[rp_profile] %-11s %6.2f%%  calls %9lld  cycles/call %9.0f\n", names[k], 100.0 * h[k] / tot, h[32 + k], (double)h[k] / h[32 + k]);
   }

@@ -86,14 +86,18 @@ enum {
 constexpr int RP_MAX_N = 12000;
 RP_HD size_t table_elems(int n) { return (size_t)n * (size_t)(n + 1) + 8; }
 RP_HD size_t vector_elems(int n) { return (size_t)n + 8; }
-RP_HD size_t slot_doubles(int n) { return T_COUNT * table_elems(n) + V_COUNT * vector_elems(n); }
+// scratch of the unpaired-window pass, after the vectors: the generic gap sums of both sides and the slices of the
+// table-driven shapes' gap sums (up_gap_idx / up_special_idx)
+constexpr int UP_SLICES_MAX = 4;   // gap_special_slices(n) <= 4
+RP_HD size_t up_scratch_elems(int n) { return (size_t)(2 * (MAXLOOP + 1) + 2 * 3 * UP_SLICES_MAX) * n + 8; }
+RP_HD size_t slot_doubles(int n) { return T_COUNT * table_elems(n) + V_COUNT * vector_elems(n) + up_scratch_elems(n); }
 
 // one problem per CTA (or cluster), elements contiguous; the work of a cell is sliced over threads
 struct Ctx {
   const DevModel* M;
   const uint8_t* S;   // S[1..n]; low 3 bits base code 0..4, bit 3 = "letter is not A/C/G/U"
   int n, cp, ld, kind, max_w;
-  double* ws;         // slot workspace: T_COUNT tables then V_COUNT vectors
+  double* ws;         // slot workspace: T_COUNT tables, V_COUNT vectors, then the unpaired-window scratch
   unsigned te, ve;    // elements per table / per vector (a slot is < 2^32 doubles: n <= RP_MAX_N, checked by the host)
   double invZ;        // set after the inside pass
   int dbg;            // tuning aid (RP_DEBUG_SKIP): 1 skip interior rows, 2 skip split sums, 4 skip gap sums
@@ -114,6 +118,7 @@ struct Ctx {
   // row-major copies they are neighbours.
   RP_HD double* rptr(int t, int i, int j) const { return ws + ((unsigned)t * te + (unsigned)(i - 1) * (unsigned)ld + (unsigned)j); }
   RP_HD double& v(int vv, int k) const { return ws[(unsigned)T_COUNT * te + (unsigned)vv * ve + (unsigned)k]; }
+  RP_HD double* up_scratch() const { return ws + ((unsigned)T_COUNT * te + (unsigned)V_COUNT * ve); }
   RP_HD int dstep() const { return ld; }   // one diagonal up, same position
   RP_HD int pstep() const { return 1; }    // same diagonal, next position
   RP_HD int sraw(int i) const { return S[i]; }
@@ -1511,21 +1516,22 @@ RP_HD void generic_items(const Ctx& c, const Shared& sh, int d, int i0, int C, i
 // ---------------------------------------------------------------------------
 // unpaired windows (single strand): up(i,d) = P(i..i+d unpaired), d < max_w
 // ---------------------------------------------------------------------------
-// U1: DG(p,o) = out(p,o)*hairpin(p,o)   (loop whose unpaired run is (p,o))
+// The pass runs in four phases: P1 (unstru_items: every sum that depends only on the finished wavefront tables),
+// the row scan (which also adds P1's pieces of DG up), the column scan, and the windows.
+//
+// U1: DG(p,o) = out(p,o)*hairpin(p,o)   (loop whose unpaired run is (p,o)); cell x = d*ld + i of the table
 template <class C>
-RP_HD void unstru_hairpin(C& c, int tid, int T) {
+RP_HD void unstru_hairpin_cell(C& c, unsigned x) {
   const int n = c.n;
-  const unsigned total = (unsigned)n * (unsigned)c.ld, ld = (unsigned)c.ld;   // n <= RP_MAX_N: 32-bit index arithmetic
-  for (unsigned x = tid; x < total; x += T) {
-    const int d = (int)(x / ld), i = (int)(x - (unsigned)d * ld);
-    if (i < 1 || i + d > n) continue;
-    double v = 0.;
-    if (d > TURN) {
-      const double o = TB(c, T_OUT, d, i);
-      if (o != 0.) v = o * hairpin(c, i, i + d, pair_type(base(c, i), base(c, i + d)));
-    }
-    TB(c, T_DG, d, i) = v;
+  const unsigned ld = (unsigned)c.ld;   // n <= RP_MAX_N: 32-bit index arithmetic
+  const int d = (int)(x / ld), i = (int)(x - (unsigned)d * ld);
+  if (i < 1 || i + d > n) return;
+  double v = 0.;
+  if (d > TURN) {
+    const double o = TB(c, T_OUT, d, i);
+    if (o != 0.) v = o * hairpin(c, i, i + d, pair_type(base(c, i), base(c, i + d)));
   }
+  TB(c, T_DG, d, i) = v;
 }
 // class of the loop shape (u1,u2), u1+u2 <= MAXLOOP: the rule of build_dev_model (dev_model.cpp), in registers
 RP_HD int loop_class(int u1, int u2) {
@@ -1535,193 +1541,178 @@ RP_HD int loop_class(int u1, int u2) {
   return (us == 2 && (ul == 2 || ul == 3)) ? CLS_SPECIAL : CLS_GENERIC;
 }
 
-// The table-driven shapes (9 small loops, dev_model.h) of the gap sums: item (side, gap size
-// ug <= 3, gap start a, slice) sums the loops of all special shapes with that gap size over
-// every `nsl`-th position of the free pair end and leaves the partial in a scratch row of T_RR
-// (free until unstru_ml_tables): row (side*3+ug-1)*nsl+slice, position a.  unstru_gaps adds the
-// slices up in fixed order.  Branch-free body: cells that cannot pair carry qb = out = 0.
-RP_HD int gap_special_slices(int n) { return n >= 48 ? 4 : 1; }
-template <class C, class MT>
-RP_HD void unstru_gap_specials(C& c, const MT& M, int tid, int T) {
-  const int n = c.n;
-  if (n < 7) return;   // rows 0..5 of the scratch must exist; shorter sequences have no such loops to speak of (handled below)
-  const int nsl = gap_special_slices(n);
-  const int items = (RP_DBG(c) & 4) ? 0 : 2 * 3 * nsl * n;
-  for (int x = tid; x < items; x += T) {
-    const int a = x % n + 1;
-    int y = x / n;
-    const int sl = y % nsl; y /= nsl;
-    const int ug = y % 3 + 1, side = y / 3;
-    const int b = a + ug + 1;
-    double acc = 0.;
-    if (b <= n) {
-      if (side == 0) {
-        const int p = a, k = b, u1 = ug, lmin = k + TURN + 1;
-        const int sp1 = base(c, k - 1), si1 = base(c, p + 1);
-        for (int u2 = 0; u2 <= 3; u2++) {
-          if (loop_class(u1, u2) != CLS_SPECIAL) continue;
-          const int lmax = n - 1 - u2, sidx = special_index(u1, u2);
-          // four positions per round trip: the eight table loads go out before the first weight is looked up
-          for (int l0 = lmin + sl; l0 <= lmax; l0 += 4 * nsl) {
-            double qb[4], ou[4];
-#pragma unroll
-            for (int u = 0; u < 4; u++) {
-              const int l = l0 + u * nsl;
-              const bool on = l <= lmax;
-              qb[u] = on ? TB(c, T_QB, l - k, k) : 0.;
-              ou[u] = on ? TB(c, T_OUT, l + 1 + u2 - p, p) : 0.;
-            }
-            double w[4];
-#pragma unroll
-            for (int u = 0; u < 4; u++) {   // branch-free: the four weight look-ups (L2) are in flight together
-              const int l = l0 + u * nsl <= lmax ? l0 + u * nsl : lmax, o = l + 1 + u2;
-              w[u] = special_loop(M, sidx, pair_type(base(c, p), base(c, o)), rtype(pair_type(base(c, k), base(c, l))),
-                                  si1, base(c, o - 1), sp1, base(c, l + 1));
-            }
-#pragma unroll
-            for (int u = 0; u < 4; u++) acc += ou[u] * qb[u] * w[u];
-          }
-        }
-      } else {
-        const int l = a, o = b, u2 = ug;
-        const int sq1 = base(c, l + 1), sj1 = base(c, o - 1);
-        for (int u1 = 0; u1 <= 3; u1++) {
-          if (loop_class(u1, u2) != CLS_SPECIAL) continue;
-          const int pmax = l - TURN - 2 - u1, sidx = special_index(u1, u2);
-          for (int p0 = 1 + sl; p0 <= pmax; p0 += 4 * nsl) {
-            double qb[4], ou[4];
-#pragma unroll
-            for (int u = 0; u < 4; u++) {
-              const int p = p0 + u * nsl;
-              const bool on = p <= pmax;
-              ou[u] = on ? TB(c, T_OUT, o - p, p) : 0.;
-              qb[u] = on ? TB(c, T_QB, l - (p + 1 + u1), p + 1 + u1) : 0.;
-            }
-            double w[4];
-#pragma unroll
-            for (int u = 0; u < 4; u++) {
-              const int p = p0 + u * nsl <= pmax ? p0 + u * nsl : pmax, k = p + 1 + u1;
-              w[u] = special_loop(M, sidx, pair_type(base(c, p), base(c, o)), rtype(pair_type(base(c, k), base(c, l))),
-                                  base(c, p + 1), sj1, base(c, k - 1), sq1);
-            }
-#pragma unroll
-            for (int u = 0; u < 4; u++) acc += ou[u] * qb[u] * w[u];
-          }
-        }
-      }
-    }
-    TB(c, T_RR, ((side * 3 + ug - 1) * nsl + sl), a) = acc;
-  }
+// Scratch of the pass (Ctx::up_scratch): the generic gap sum of side s, gap size ug, gap start a at
+// up_gap_idx (the sizes of one gap start side by side, as the row scan reads them), then the slices of the
+// table-driven shapes' gap sums at up_special_idx.
+RP_HD unsigned up_gap_idx(int n, int side, int ug, int a) {
+  return ((unsigned)side * (unsigned)n + (unsigned)(a - 1)) * (MAXLOOP + 1) + (unsigned)ug;
+}
+RP_HD unsigned up_special_idx(int n, int side, int ug, int nsl, int sl, int a) {
+  return 2u * (MAXLOOP + 1) * (unsigned)n + (unsigned)((side * 3 + ug - 1) * nsl + sl) * (unsigned)n + (unsigned)(a - 1);
 }
 
-// U2 (side=0): DG(p,k) += weight of all interior loops closed by some (p,o) with inner pair (k,l): 5' gap (p,k)
-// U3 (side=1): DG(l,o) += the same loops seen from their 3' gap (l,o)
-// One item per gap.  For the factorised classes the sum over the free pair end is a dot
-// product of two table rows that already carry the pair factors:
-//   side 0:  sum_l  outX(p, l+1+u2) * qbX(k, l)          (both advance one diagonal per l)
-//   side 1:  sum_p  outX(p, o)      * qbX(p+1+u1, l)     (both step one diagonal down, one cell right)
-// Runs of up to 8 shifts of one class share the streamed operand (multi_dot).
-// gfull: the weights g(u1,u2) incl. scale, row stride GROW_LD (DevModel::gfull, or a shared-memory copy)
-template <class C>
-RP_HD void unstru_gaps(C& c, const double* gfull, int side, int tid, int T) {
-  const int n = c.n, ds = c.dstep(), ps = c.pstep();
-  const int items = (RP_DBG(c) & 4) ? 0 : n * (MAXLOOP + 1);
-  const int tabO[3] = {T_OUTI, T_OUT1N, T_OUTAU};
-  const int tabQ[3] = {T_QBI, T_QB1N, T_QBAU};
-  for (int x = tid; x < items; x += T) {
-    const int ug = x / n;      // size of the gap this item owns
-    const int a = x % n + 1;   // gap is the open interval (a, a+ug+1)
-    const int b = a + ug + 1;
-    if (b > n || ug < 1) continue;  // an empty gap cannot contain a window
-    double acc = 0.;
+// The table-driven shapes (9 small loops, dev_model.h) of the gap sums: item x = (side, gap size
+// ug <= 3, gap start a, slice) sums the loops of all special shapes with that gap size over
+// every `nsl`-th position of the free pair end into its scratch slot.  The row scan adds the
+// slices up in fixed order.  Branch-free body: cells that cannot pair carry qb = out = 0.
+// Only for n >= 7: shorter sequences have no such loops to speak of.
+RP_HD int gap_special_slices(int n) { return n >= 48 ? 4 : 1; }
+template <class C, class MT>
+RP_HD void unstru_gap_special(C& c, const MT& M, int x) {
+  const int n = c.n;
+  const int nsl = gap_special_slices(n);
+  const int a = x % n + 1;
+  int y = x / n;
+  const int sl = y % nsl; y /= nsl;
+  const int ug = y % 3 + 1, side = y / 3;
+  const int b = a + ug + 1;
+  double acc = 0.;
+  if (b <= n) {
     if (side == 0) {
-      const int p = a, k = b, u1 = ug;
-      const int lmin = k + TURN + 1;
-      for (int u2 = 0; u1 + u2 <= MAXLOOP;) {
-        if (n - 1 - u2 < lmin) break;
-        const int cls = loop_class(u1, u2);
-        if (cls != CLS_SPECIAL) {
-          // run of up to 8 consecutive u2 of the same class
-          int nu = 1;
-          while (nu < 8 && u1 + u2 + nu <= MAXLOOP && loop_class(u1, u2 + nu) == cls && n - 1 - (u2 + nu) >= lmin) nu++;
-          double av[8] = {0., 0., 0., 0., 0., 0., 0., 0.};
-          const double* Q = c.ptr(tabQ[cls], lmin - k, k);           // qbX(k,l), one diagonal per l
-          const double* O = c.ptr(tabO[cls], lmin + 1 + u2 - p, p);  // outX(p,l+1+u2), one diagonal per u2
-          const int cmain = n - 1 - (u2 + nu - 1) - lmin + 1;        // l range valid for every u2 of the run
-          // the shorter shifts reach further (l up to n-1-(u2+t)): walk to the end of the longest one;
-          // window elements past the last diagonal count as 0
-          const int X = cmain + nu - 1;
-          if (nu == 1) av[0] = dot_range(Q, ds, O, ds, 0, X, 0, 1);   // a lone shift (the bulge / 1xn heads): plain dot product
-          else multi_dot_slide(Q, ds, O, ds, X, 0, X - 1, av);
-          for (int t = 0; t < nu; t++) acc += gfull[u1 * GROW_LD + u2 + t] * av[t];
-          u2 += nu;
-        } else {
-          u2++;  // table-driven shapes: summed by unstru_gap_specials into the scratch rows
+      const int p = a, k = b, u1 = ug, lmin = k + TURN + 1;
+      const int sp1 = base(c, k - 1), si1 = base(c, p + 1);
+      for (int u2 = 0; u2 <= 3; u2++) {
+        if (loop_class(u1, u2) != CLS_SPECIAL) continue;
+        const int lmax = n - 1 - u2, sidx = special_index(u1, u2);
+        // four positions per round trip: the eight table loads go out before the first weight is looked up
+        for (int l0 = lmin + sl; l0 <= lmax; l0 += 4 * nsl) {
+          double qb[4], ou[4];
+#pragma unroll
+          for (int u = 0; u < 4; u++) {
+            const int l = l0 + u * nsl;
+            const bool on = l <= lmax;
+            qb[u] = on ? TB(c, T_QB, l - k, k) : 0.;
+            ou[u] = on ? TB(c, T_OUT, l + 1 + u2 - p, p) : 0.;
+          }
+          double w[4];
+#pragma unroll
+          for (int u = 0; u < 4; u++) {   // branch-free: the four weight look-ups (L2) are in flight together
+            const int l = l0 + u * nsl <= lmax ? l0 + u * nsl : lmax, o = l + 1 + u2;
+            w[u] = special_loop(M, sidx, pair_type(base(c, p), base(c, o)), rtype(pair_type(base(c, k), base(c, l))),
+                                si1, base(c, o - 1), sp1, base(c, l + 1));
+          }
+#pragma unroll
+          for (int u = 0; u < 4; u++) acc += ou[u] * qb[u] * w[u];
         }
       }
     } else {
       const int l = a, o = b, u2 = ug;
-      for (int u1 = 0; u1 + u2 <= MAXLOOP;) {
-        if (l - TURN - 2 - u1 < 1) break;  // k = p+1+u1 <= l-TURN-1 needs p >= 1
-        const int cls = loop_class(u1, u2);
-        if (cls != CLS_SPECIAL) {
-          int nu = 1;
-          while (nu < 8 && u1 + nu + u2 <= MAXLOOP && loop_class(u1 + nu, u2) == cls && l - TURN - 2 - (u1 + nu) >= 1) nu++;
-          double av[8] = {0., 0., 0., 0., 0., 0., 0., 0.};
-          const double* O = c.ptr(tabO[cls], o - 1, 1);               // outX(p,o): one diagonal down, one cell right per p
-          const double* Q = c.ptr(tabQ[cls], l - 2 - u1, 2 + u1);     // qbX(p+1+u1,l); per u1 likewise
-          const int cmain = l - TURN - 2 - (u1 + nu - 1);             // p = 1..cmain valid for every u1 of the run
-          // walked from the largest p downwards: then the lanes of a warp (consecutive gaps) read
-          // consecutive addresses.  Reversed window: element z holds Q[X+6-z], shift t' = 7-t.
-          if (cmain > 0) {
-            const long st = ps - ds;
-            const int X = cmain + nu - 1;   // steps of the longest shift (t = 0)
-            if (nu == 1) {
-              av[0] = dot_range(O + (long)(X - 1) * st, (int)-st, Q + (long)(X - 1) * st, (int)-st, 0, X, 0, 1);
-            } else {
-              double rv[8] = {0., 0., 0., 0., 0., 0., 0., 0.};
-              multi_dot_slide(O + (long)(X - 1) * st, -st, Q + (long)(X + 6) * st, -st, X, 7, X + 6, rv);
+      const int sq1 = base(c, l + 1), sj1 = base(c, o - 1);
+      for (int u1 = 0; u1 <= 3; u1++) {
+        if (loop_class(u1, u2) != CLS_SPECIAL) continue;
+        const int pmax = l - TURN - 2 - u1, sidx = special_index(u1, u2);
+        for (int p0 = 1 + sl; p0 <= pmax; p0 += 4 * nsl) {
+          double qb[4], ou[4];
 #pragma unroll
-              for (int t = 0; t < 8; t++) av[t] = rv[7 - t];
-            }
+          for (int u = 0; u < 4; u++) {
+            const int p = p0 + u * nsl;
+            const bool on = p <= pmax;
+            ou[u] = on ? TB(c, T_OUT, o - p, p) : 0.;
+            qb[u] = on ? TB(c, T_QB, l - (p + 1 + u1), p + 1 + u1) : 0.;
           }
-          for (int t = 0; t < nu; t++) acc += gfull[(u1 + t) * GROW_LD + u2] * av[t];
-          u1 += nu;
-        } else {
-          u1++;
+          double w[4];
+#pragma unroll
+          for (int u = 0; u < 4; u++) {
+            const int p = p0 + u * nsl <= pmax ? p0 + u * nsl : pmax, k = p + 1 + u1;
+            w[u] = special_loop(M, sidx, pair_type(base(c, p), base(c, o)), rtype(pair_type(base(c, k), base(c, l))),
+                                base(c, p + 1), sj1, base(c, k - 1), sq1);
+          }
+#pragma unroll
+          for (int u = 0; u < 4; u++) acc += ou[u] * qb[u] * w[u];
         }
       }
     }
-    if (ug <= 3 && n >= 7) {
-      const int nsl = gap_special_slices(n);
-      for (int sl = 0; sl < nsl; sl++) acc += TB(c, T_RR, ((side * 3 + ug - 1) * nsl + sl), a);
-    }
-    TB(c, T_DG, b - a, a) += acc;
   }
+  c.up_scratch()[up_special_idx(n, side, ug, nsl, sl, a)] = acc;
 }
-// U4a: suffix sums over b for each a ; U4b: prefix sums over a for each b
+
+// U2 (side=0): the weight of all interior loops closed by some (p,o) with inner pair (k,l) whose 5' gap is (p,k)
+// U3 (side=1): the same loops seen from their 3' gap (l,o)
+// Item x: rank r, gap size ug = 1..MAXLOOP, side; gap start a = 1+r on side 0, a = n-1-r-ug on side 1, so that the
+// free pair end of both walks about n-r-ug positions.  A group of 32 items (x >> 5) is one side and gap size over 32
+// consecutive ranks: the lanes of a warp take neighbouring gaps, whose streams are neighbouring addresses, with the
+// same runs of classes.  The groups go by block of ranks, then gap size (32 slots, bit fields of x), then side:
+// ascending x is about longest first.  Items with ug > MAXLOOP or r+ug > n-2 have no gap.  For the factorised classes the sum over the free pair end is a dot product of two table rows that already
+// carry the pair factors:
+//   side 0:  sum_l  outX(p, l+1+u2) * qbX(k, l)          (both advance one diagonal per l)
+//   side 1:  sum_p  outX(p, o)      * qbX(p+1+u1, l)     (both step one diagonal down, one cell right)
+// Runs of up to 8 shifts of one class share the streamed operand (multi_dot).  The table-driven shapes are left to
+// unstru_gap_special.  The sum goes to the item's scratch slot.
+// gfull: the weights g(u1,u2) incl. scale, row stride GROW_LD (DevModel::gfull, or a shared-memory copy)
 template <class C>
-RP_HD void unstru_dom_rows(C& c, int tid, int T) {
-  const int n = c.n;
-  for (int a = 1 + tid; a <= n; a += T) {
-    double s = 0.;
-    for (int b = n; b > a; b--) {
-      s += TB(c, T_DG, b - a, a);
-      TB(c, T_DG, b - a, a) = s;
+RP_HD void unstru_gap_item(C& c, const double* gfull, int x) {
+  const int n = c.n, ds = c.dstep(), ps = c.pstep();
+  static_assert(MAXLOOP <= 32, "gap sizes per block of ranks");
+  const int side = (x >> 5) & 1, ug = ((x >> 6) & 31) + 1, r = (x >> 11 << 5) | (x & 31);
+  if (ug > MAXLOOP || r + ug > n - 2) return;
+  const int a = side ? n - 1 - r - ug : 1 + r;   // the gap is the open interval (a, a+ug+1)
+  const int b = a + ug + 1;
+  // the class tables of class cls: T_OUTI + cls, T_QBI + cls
+  static_assert(T_OUT1N == T_OUTI + CLS_1N && T_OUTAU == T_OUTI + CLS_BULGE && T_QB1N == T_QBI + CLS_1N &&
+                T_QBAU == T_QBI + CLS_BULGE && CLS_GENERIC == 0, "class table order");
+  double acc = 0.;
+  if (side == 0) {
+    const int p = a, k = b, u1 = ug;
+    const int lmin = k + TURN + 1;
+    for (int u2 = 0; u1 + u2 <= MAXLOOP;) {
+      if (n - 1 - u2 < lmin) break;
+      const int cls = loop_class(u1, u2);
+      if (cls != CLS_SPECIAL) {
+        // run of up to 8 consecutive u2 of the same class
+        int nu = 1;
+        while (nu < 8 && u1 + u2 + nu <= MAXLOOP && loop_class(u1, u2 + nu) == cls && n - 1 - (u2 + nu) >= lmin) nu++;
+        double av[8] = {0., 0., 0., 0., 0., 0., 0., 0.};
+        const double* Q = c.ptr(T_QBI + cls, lmin - k, k);           // qbX(k,l), one diagonal per l
+        const double* O = c.ptr(T_OUTI + cls, lmin + 1 + u2 - p, p);  // outX(p,l+1+u2), one diagonal per u2
+        const int cmain = n - 1 - (u2 + nu - 1) - lmin + 1;        // l range valid for every u2 of the run
+        // the shorter shifts reach further (l up to n-1-(u2+t)): walk to the end of the longest one;
+        // window elements past the last diagonal count as 0
+        const int X = cmain + nu - 1;
+        if (nu == 1) av[0] = dot_range(Q, ds, O, ds, 0, X, 0, 1);   // a lone shift (the bulge / 1xn heads): plain dot product
+        else multi_dot_slide(Q, ds, O, ds, X, 0, X - 1, av);
+        for (int t = 0; t < nu; t++) acc += gfull[u1 * GROW_LD + u2 + t] * av[t];
+        u2 += nu;
+      } else {
+        u2++;  // table-driven shapes: summed by unstru_gap_special
+      }
     }
+    c.up_scratch()[up_gap_idx(n, 0, u1, p)] = acc;   // (in terms of what the loop kept live: no spill at 80 registers)
+  } else {
+    const int l = a, o = b, u2 = ug;
+    for (int u1 = 0; u1 + u2 <= MAXLOOP;) {
+      if (l - TURN - 2 - u1 < 1) break;  // k = p+1+u1 <= l-TURN-1 needs p >= 1
+      const int cls = loop_class(u1, u2);
+      if (cls != CLS_SPECIAL) {
+        int nu = 1;
+        while (nu < 8 && u1 + nu + u2 <= MAXLOOP && loop_class(u1 + nu, u2) == cls && l - TURN - 2 - (u1 + nu) >= 1) nu++;
+        double av[8] = {0., 0., 0., 0., 0., 0., 0., 0.};
+        const double* O = c.ptr(T_OUTI + cls, o - 1, 1);               // outX(p,o): one diagonal down, one cell right per p
+        const double* Q = c.ptr(T_QBI + cls, l - 2 - u1, 2 + u1);     // qbX(p+1+u1,l); per u1 likewise
+        const int cmain = l - TURN - 2 - (u1 + nu - 1);             // p = 1..cmain valid for every u1 of the run
+        // walked from the largest p downwards: then the lanes of a warp (consecutive gaps) read
+        // consecutive addresses.  Reversed window: element z holds Q[X+6-z], shift t' = 7-t.
+        if (cmain > 0) {
+          const long st = ps - ds;
+          const int X = cmain + nu - 1;   // steps of the longest shift (t = 0)
+          if (nu == 1) {
+            av[0] = dot_range(O + (long)(X - 1) * st, (int)-st, Q + (long)(X - 1) * st, (int)-st, 0, X, 0, 1);
+          } else {
+            double rv[8] = {0., 0., 0., 0., 0., 0., 0., 0.};
+            multi_dot_slide(O + (long)(X - 1) * st, -st, Q + (long)(X + 6) * st, -st, X, 7, X + 6, rv);
+#pragma unroll
+            for (int t = 0; t < 8; t++) av[t] = rv[7 - t];
+          }
+        }
+        for (int t = 0; t < nu; t++) acc += gfull[(u1 + t) * GROW_LD + u2] * av[t];
+        u1 += nu;
+      } else {
+        u1++;
+      }
+    }
+    c.up_scratch()[up_gap_idx(n, 1, u2, l)] = acc;
   }
 }
-template <class C>
-RP_HD void unstru_dom_cols(C& c, int tid, int T) {
-  const int n = c.n;
-  for (int b = 2 + tid; b <= n; b += T) {
-    double s = 0.;
-    for (int a = 1; a < b; a++) {
-      s += TB(c, T_DG, b - a, a);
-      TB(c, T_DG, b - a, a) = s;
-    }
-  }
-}
+
 // U5/U6: the multiloop part of the unpaired-window probabilities.  The window [i..j] (dd = j-i) lies in
 // the loop closed by (p,o), p < i, j < o, next to the closing pair's unpaired run or between stems:
 //   m1 = sum_{p<i} mlb^(j-p)  sum_{o>=j+2} Mc(p,o) QM2(j+1,o-1)           window in the 5' run, >= 2 stems follow
@@ -1734,32 +1725,165 @@ RP_HD void unstru_dom_cols(C& c, int tid, int T) {
 //   m3 = mlb^(dd+1) sum_p qm(p+1,i-1)  PR(p,j),    PR(p,j)  = sum_o Mc(p,o) qm(j+1,o-1)
 // and PR is the outside pass's own right-hand multiloop sum, which the band phases leave in T_XX for
 // single-strand problems with windows.  Tables: K -> T_RR, PLf -> T_LL.
+// One scan per item, p = 1+i (row) / o = 2+i (column).  Both walk the diagonals downwards from the top one of the
+// item's group of 32, so that the lanes of a warp, which take one group, touch consecutive elements at every step;
+// the loads of 8 steps go out before their stores.
+constexpr int UP_NB = 8;
 template <class C>
-RP_HD void unstru_ml_tables(C& c, int tid, int T) {
-  const int n = c.n;
+RP_HD void unstru_ml_row(C& c, int i) {   // PLf(p,j), j = n .. p+1
+  const int n = c.n, p = 1 + i, top = n - 1 - (i & ~31);
   const double mlb1 = c.M->mlb1;
-  // both scans walk the diagonals downwards, every thread on the same diagonal at the same step, so
-  // that the threads of a warp touch consecutive elements
-  for (int p0 = 1; p0 < n; p0 += T) {          // row p: PLf(p,j), j = n .. p+1
-    const int p = p0 + tid;
-    double s = 0.;
-#pragma unroll 8
-    for (int d = n - p0; d >= 1; d--) {
-      if (d > n - p) continue;
-      const double mc = TB(c, T_MC, d, p);
+  double s = 0.;
+  for (int d0 = top; d0 >= 1; d0 -= UP_NB) {
+    double mc[UP_NB];
+#pragma unroll
+    for (int u = 0; u < UP_NB; u++) mc[u] = d0 - u >= 1 && d0 - u <= n - p ? TB(c, T_MC, d0 - u, p) : 0.;
+#pragma unroll
+    for (int u = 0; u < UP_NB; u++) {
+      const int d = d0 - u;
+      if (d < 1 || d > n - p) continue;
       TB(c, T_LL, d, p) = s;
-      s = s * mlb1 + mc;
+      s = s * mlb1 + mc[u];
     }
   }
-  for (int o0 = 2; o0 <= n; o0 += T) {         // column o: K(i,o), i = 1 .. o-1
-    const int o = o0 + tid, top = (o0 + T - 1 < n ? o0 + T - 1 : n) - 1;
-    double s = 0.;
-#pragma unroll 8
-    for (int d = top; d >= 1; d--) {
-      if (o > n || d > o - 1) continue;
-      const double mc = TB(c, T_MC, d, o - d);
+}
+template <class C>
+RP_HD void unstru_ml_col(C& c, int i) {   // K(i',o), i' = 1 .. o-1
+  const int n = c.n, o = 2 + i, last = 2 + (i | 31), top = (last < n ? last : n) - 1;
+  const double mlb1 = c.M->mlb1;
+  double s = 0.;
+  for (int d0 = top; d0 >= 1; d0 -= UP_NB) {
+    double mc[UP_NB];
+#pragma unroll
+    for (int u = 0; u < UP_NB; u++) mc[u] = d0 - u >= 1 && d0 - u <= o - 1 ? TB(c, T_MC, d0 - u, o - (d0 - u)) : 0.;
+#pragma unroll
+    for (int u = 0; u < UP_NB; u++) {
+      const int d = d0 - u;
+      if (d < 1 || d > o - 1) continue;
       TB(c, T_RR, d, o - d) = s;
-      s = mlb1 * (s + mc);
+      s = mlb1 * (s + mc[u]);
+    }
+  }
+}
+
+// Items [first, first+count) of the list P1 deals out: round k of GT consecutive items goes to the threads in order
+// for even k and in reverse for odd k, so that two rounds of items sorted by length even out; body(item - first)
+template <class F>
+RP_HD void deal_snake(int first, int count, int gt, int GT, F body) {
+  const int end = first + count;
+  for (int k = first / GT; k * GT < end; k++) {
+    const int x = k * GT + ((k & 1) ? GT - 1 - gt : gt);
+    if (x >= first && x < end) body(x - first);
+  }
+}
+
+// P1: the hairpin cells, the gap sums of both sides, the table-driven shapes' slices and the two multiloop scans
+// depend on the finished wavefront tables only, so they are the items of one phase, dealt longest first: the gap items
+// of the first half of the rank blocks, the scans (starting on a whole warp), the other gap items, the table-driven
+// slices, the hairpin cells.  The deal is fixed, so every run computes the same values.
+template <class C, class MT>
+RP_HD void unstru_items(C& c, const MT& M, const double* gfull, int gt, int GT) {
+  const int n = c.n;
+  const bool gaps = !(RP_DBG(c) & 4);
+  const int blocks = n > 2 ? (n - 2 + 31) / 32 : 0, blong = (blocks + 1) / 2;   // blocks of 32 gap ranks
+  const int nlong = gaps ? blong << 11 : 0, nshort = gaps ? (blocks - blong) << 11 : 0;   // 2 sides x 32 sizes x 32
+  const int nscan = (n - 1 + 31) & ~31;   // per scan kind, whole warps
+  const int nspec = gaps && n >= 7 ? 2 * 3 * gap_special_slices(n) * n : 0;
+  const int xshort = nlong + 2 * nscan, xspec = xshort + nshort, xhp = xspec + nspec;
+  // one loop per kind of item, each body inlined once (the gap items: the two ranges around the scans)
+  deal_snake(0, xspec, gt, GT, [&](int x) {
+    if (x < nlong || x >= xshort) unstru_gap_item(c, gfull, x < nlong ? x : x - 2 * nscan);
+  });
+  deal_snake(nlong, 2 * nscan, gt, GT, [&](int i) {
+    if (i < nscan) {
+      if (i < n - 1) unstru_ml_row(c, i);
+    } else if (i - nscan < n - 1) {
+      unstru_ml_col(c, i - nscan);
+    }
+  });
+  deal_snake(xspec, nspec, gt, GT, [&](int x) { unstru_gap_special(c, M, x); });
+  deal_snake(xhp, n * c.ld, gt, GT, [&](int x) { unstru_hairpin_cell(c, (unsigned)x); });
+}
+
+// U4a: DG(a,b) = hairpin + side-0 gap sum + side-1 gap sum (the sizes ug <= 3 with their table-driven slices added
+// to each side's generic sum first, in slice order), then suffix sums over b for each a; U4b: prefix sums over a for
+// each b.  One row / column per thread; the loads of UP_NB elements go out before their stores.
+template <class C>
+RP_HD void unstru_dom_rows(C& c, int tid, int T) {
+  const int n = c.n;
+  const bool gaps = !(RP_DBG(c) & 4), specials = gaps && n >= 7;
+  const int nsl = gap_special_slices(n);
+  const double* G = c.up_scratch();
+  for (int a = 1 + tid; a <= n; a += T) {
+    double s0[3], s1[3];   // side sums of the gap sizes 1..3
+#pragma unroll
+    for (int g = 0; g < 3; g++) {
+      s0[g] = s1[g] = 0.;
+      if (gaps && a + g + 2 <= n) {
+        s0[g] = G[up_gap_idx(n, 0, g + 1, a)];
+        s1[g] = G[up_gap_idx(n, 1, g + 1, a)];
+        if (specials)
+          for (int sl = 0; sl < nsl; sl++) {
+            s0[g] += G[up_special_idx(n, 0, g + 1, nsl, sl, a)];
+            s1[g] += G[up_special_idx(n, 1, g + 1, nsl, sl, a)];
+          }
+      }
+    }
+    double s = 0.;
+    const int bnear = a + MAXLOOP + 1 < n ? a + MAXLOOP + 1 : n;   // b <= bnear: gap sizes 0..MAXLOOP
+    for (int b0 = n; b0 > bnear; b0 -= UP_NB) {
+      double v[UP_NB];
+#pragma unroll
+      for (int u = 0; u < UP_NB; u++) v[u] = b0 - u > bnear ? TB(c, T_DG, b0 - u - a, a) : 0.;
+#pragma unroll
+      for (int u = 0; u < UP_NB; u++) {
+        if (b0 - u <= bnear) continue;
+        s += v[u];
+        TB(c, T_DG, b0 - u - a, a) = s;
+      }
+    }
+    constexpr int NBN = UP_NB / 2;   // three loads per element here
+    for (int b0 = bnear; b0 > a; b0 -= NBN) {
+      double v[NBN], g0[NBN], g1[NBN];
+#pragma unroll
+      for (int u = 0; u < NBN; u++) {
+        const int b = b0 - u, ug = b - a - 1;
+        const bool gen = gaps && ug > 3;
+        v[u] = b > a ? TB(c, T_DG, b - a, a) : 0.;
+        g0[u] = gen ? G[up_gap_idx(n, 0, ug, a)] : 0.;
+        g1[u] = gen ? G[up_gap_idx(n, 1, ug, a)] : 0.;
+      }
+#pragma unroll
+      for (int u = 0; u < NBN; u++) {
+        const int b = b0 - u, ug = b - a - 1;
+        if (b <= a) continue;
+        double x = v[u];
+        if (gaps && ug >= 1) {
+          const double x0 = ug > 3 ? g0[u] : ug == 1 ? s0[0] : ug == 2 ? s0[1] : s0[2];
+          const double x1 = ug > 3 ? g1[u] : ug == 1 ? s1[0] : ug == 2 ? s1[1] : s1[2];
+          x = (x + x0) + x1;
+        }
+        s += x;
+        TB(c, T_DG, b - a, a) = s;
+      }
+    }
+  }
+}
+template <class C>
+RP_HD void unstru_dom_cols(C& c, int tid, int T) {
+  const int n = c.n;
+  for (int b = 2 + tid; b <= n; b += T) {
+    double s = 0.;
+    for (int a0 = 1; a0 < b; a0 += UP_NB) {
+      double v[UP_NB];
+#pragma unroll
+      for (int u = 0; u < UP_NB; u++) v[u] = a0 + u < b ? TB(c, T_DG, b - a0 - u, a0 + u) : 0.;
+#pragma unroll
+      for (int u = 0; u < UP_NB; u++) {
+        if (a0 + u >= b) continue;
+        s += v[u];
+        TB(c, T_DG, b - a0 - u, a0 + u) = s;
+      }
     }
   }
 }

@@ -32,7 +32,7 @@ namespace rp {
 
 enum {
   PH_STAGE = 0, PH_PROLOGUE, PH_PROLOGUE2, PH_INSIDE_A, PH_INSIDE_B, PH_GENERIC_IN, PH_GENERIC_OUT, PH_OUTSIDE_A, PH_OUTSIDE_B,
-  PH_WRITE_BP, PH_UN_HAIRPIN, PH_UN_GAPS0, PH_UN_GAPS1, PH_UN_DOMROWS, PH_UN_DOMCOLS, PH_UN_MLTAB, PH_UN_WINDOWS,
+  PH_WRITE_BP, PH_UN_ITEMS, PH_UN_DOMROWS, PH_UN_DOMCOLS, PH_UN_WINDOWS,
   PH_WRITE_HP, PH_LOGZ, PH_BAND_A, PH_BAND_B, PH_CFAC, PH_COUNT
 };
 
@@ -159,30 +159,9 @@ RP_HD void split_sums_outside(Exec& ex, Ctx& c, const Shared& sh, int d) {
 // `gfull`: DevModel::gfull or a shared-memory copy of it
 template <class Exec, class MT>
 RP_HD void emit_unpaired(Exec& ex, Ctx& c, const Problem& p, float* dense, const MT& SM, const double* gfull) {
-  flat(ex, PH_UN_HAIRPIN, [&](int tid, int gt, int GT) {
-#ifdef __CUDA_ARCH__
-    long long* prof = RP_PROF(c);
-    const long long t0 = (prof && tid == 0) ? clock64() : 0;
-#endif
-    unstru_hairpin(c, gt, GT);
-#ifdef __CUDA_ARCH__
-    const long long t1 = (prof && tid == 0) ? clock64() : 0;
-#endif
-    unstru_gap_specials(c, SM, gt, GT);
-#ifdef __CUDA_ARCH__
-    if (prof && tid == 0) {   // RP_PROFILE probes of thread 0: the two halves of the phase
-      atomicAdd(reinterpret_cast<unsigned long long*>(prof + 22), (unsigned long long)(t1 - t0));
-      atomicAdd(reinterpret_cast<unsigned long long*>(prof + 32 + 22), 1ull);
-      atomicAdd(reinterpret_cast<unsigned long long*>(prof + 23), (unsigned long long)(clock64() - t1));
-      atomicAdd(reinterpret_cast<unsigned long long*>(prof + 32 + 23), 1ull);
-    }
-#endif
-  });
-  flat(ex, PH_UN_GAPS0, [&](int, int gt, int GT) { unstru_gaps(c, gfull, 0, gt, GT); });
-  flat(ex, PH_UN_GAPS1, [&](int, int gt, int GT) { unstru_gaps(c, gfull, 1, gt, GT); });
+  flat(ex, PH_UN_ITEMS, [&](int, int gt, int GT) { unstru_items(c, SM, gfull, gt, GT); });
   flat(ex, PH_UN_DOMROWS, [&](int, int gt, int GT) { unstru_dom_rows(c, gt, GT); });
   flat(ex, PH_UN_DOMCOLS, [&](int, int gt, int GT) { unstru_dom_cols(c, gt, GT); });
-  flat(ex, PH_UN_MLTAB, [&](int, int gt, int GT) { unstru_ml_tables(c, gt, GT); });
   if (p.out_up >= 0) flat(ex, PH_UN_WINDOWS, [&](int, int gt, int GT) { unstru_windows(c, dense + p.out_up, gt, GT); });
 }
 
