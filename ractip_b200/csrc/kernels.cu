@@ -28,6 +28,7 @@ namespace {
 template <int G = 1, int NB = 4, int W = BAND>
 struct CtaExecT {
   static constexpr int kCtas = G;
+  static constexpr bool kShfl = true;   // the split sums run the warp-shuffle forms
   static constexpr int kBatch = NB;   // load-batch depth of the split-sum band phases (mcc_band_shfl.cuh)
   static constexpr int kWide = W;     // diagonals per split-sum band of the general kernel (solve_mcc_wide when > BAND)
   long long* prof;  // optional per-phase cycle counters (RP_PROFILE=1), else null

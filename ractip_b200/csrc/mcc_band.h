@@ -78,8 +78,8 @@ RP_HD int band_ldb(int n) { return ((n + 1 + 7) / 8) * 8; }
 RP_HD int band_ngp(int n) { return (n + 7) / 8 + 3; }
 // partial sums of the split-sum band phases / of the interior items (they alias).  The CUDA build runs the
 // shuffle form of the band phases (mcc_band_shfl.cuh), where a warp owns 32-(BAND-1) rows: 2*BAND partials for
-// 28 rows per warp.  The host emulation runs the direct form: 2*BAND partials per thread.  Host code that sizes a
-// launch of the CUDA build (plan.cpp) asks for the shuffle form: shfl = true.
+// 28 rows per warp.  The direct form takes 2*BAND partials per thread.  Host code that sizes a launch of the CUDA
+// build (plan.cpp) asks for the shuffle form: shfl = true; solve_band carves the form its executor runs (kShfl).
 #ifdef __CUDACC__
 constexpr bool BAND_SHFL = true;
 #else
@@ -96,10 +96,10 @@ RP_HD size_t band_shared_doubles(int n, int T, bool shfl = BAND_SHFL) {
 }
 RP_HD size_t band_shared_bytes(int n, int T, bool shfl = BAND_SHFL) { return band_shared_doubles(n, T, shfl) * sizeof(double); }
 
-RP_HD void carve_band(Shared& sh, BandShared& bs, void* base, int n, int T) {
+RP_HD void carve_band(Shared& sh, BandShared& bs, void* base, int n, int T, bool shfl = BAND_SHFL) {
   sh.T = T;
   double* p = static_cast<double*>(base);
-  sh.part = p; bs.ipart = p; p += band_part_doubles(n, T);
+  sh.part = p; bs.ipart = p; p += band_part_doubles(n, T, shfl);
   sh.red = p; p += 128;
   bs.LDB = band_ldb(n); bs.LD8 = bs.LDB / 8; bs.NGP = band_ngp(n);
   bs.TI = p; p += (size_t)BSLOTS * bs.LDB;

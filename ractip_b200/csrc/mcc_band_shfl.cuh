@@ -1,4 +1,4 @@
-// mcc_band_shfl.cuh -- device-only variants of the split-sum band phases
+// mcc_band_shfl.cuh -- the device's variants of the split-sum band phases
 // (inside_band_A / outside_band_A of mcc_core.h) that fetch every element of the streamed
 // table ONCE per warp and pass it along the lanes with warp shuffles.
 //
@@ -12,8 +12,12 @@
 // the phase drops ~2.5x.
 // A warp owns 28 rows; its last 4 lanes shadow the next warp's first rows to feed the chain.
 // Loads of 4 consecutive steps are issued together (the phase is latency-bound otherwise).
-// Same sums in a different association order than the host-emulated path (a slice covers a
-// contiguous run of steps instead of every S-th one).
+// Same sums in a different association order than the direct forms (a slice covers a contiguous
+// run of steps instead of every S-th one).  For two strands the outside forms here and in
+// mcc_wide_shfl.cuh skip the PR / ML-left terms of cells that do not join the strands (pr_live,
+// ml_live, the nick test of cand) and leave other values than the direct forms in those PRB / MLB
+// cells: the outside pass finishes only inter-strand cells (cross_lo .. cross_hi) and never reads them.  The host emulation runs these forms too, with each warp's
+// lanes as fibers that meet at every shuffle (tests/emul/warp_emul.h).
 #ifndef RP_MCC_BAND_SHFL_CUH
 #define RP_MCC_BAND_SHFL_CUH
 
@@ -22,6 +26,14 @@
 namespace rp {
 
 __device__ __forceinline__ double shfl_down_f64(double v, int delta) { return __shfl_down_sync(0xffffffffu, v, delta); }
+// starts the line of `p` towards the L2 (no register, no scoreboard slot); nothing in the host emulation
+__device__ __forceinline__ void prefetch_l2(const void* p) {
+#ifdef __CUDA_ARCH__
+  asm volatile("prefetch.global.L2 [%0];" ::"l"(p));
+#else
+  (void)p;
+#endif
+}
 // fine-grained probes (RP_PROFILE): thread 0 accumulates the cycles between two marks into slot k
 #define RP_MARK(k)                                                                                       \
   do {                                                                                                   \
@@ -194,7 +206,7 @@ __device__ __forceinline__ void outside_band_A_shfl(const Ctx& c, const Shared& 
 #pragma unroll
         for (int e = 0; e < BAND; e++) {
           const int k = k0 + e, d = d0 - e;
-          if (k > 2 && d > TURN) asm volatile("prefetch.global.L2 [%0];" ::"l"(c.ptr(T_QB, d, k)));
+          if (k > 2 && d > TURN) prefetch_l2(c.ptr(T_QB, d, k));
         }
       }
     }

@@ -1,5 +1,6 @@
 // mcc_driver.h -- the phase schedules, written once against an "executor".  kernels.cu instantiates them with
-// CtaExecT (one CTA, or the G CTAs of a thread-block cluster that share one problem); tests/emul with a serial one.
+// CtaExecT (one CTA, or the G CTAs of a thread-block cluster that share one problem); tests/emul with a serial one
+// and with a warp-lockstep one (tests/emul/warp_emul.h: each warp's 32 threads as fibers that meet at every shuffle).
 //
 //   solve_mcc        one problem per CTA, tables in HBM (the 64-register build)
 //   solve_mcc_wide   one problem per CTA or per cluster, tables in HBM (long problems)
@@ -9,7 +10,10 @@
 //   nthreads()      threads per CTA
 //   phase(id, f)    f(tid) on every thread of this CTA, then a CTA barrier
 //   kWide           diagonals per split-sum band of solve_mcc_wide
-//   kBatch          load-batch depth of the BAND-wide shuffle far passes (device only, mcc_band_shfl.cuh)
+//   kShfl           (optional, false if absent) true: the split sums run the warp-shuffle forms (mcc_band_shfl.cuh,
+//                   mcc_wide_shfl.cuh), which need the 32 threads of a warp to meet at every shuffle, and solve_band's
+//                   shared memory is carved for them; false: the direct forms of mcc_core.h, thread by thread
+//   kBatch          (kShfl only) load-batch depth of the BAND-wide shuffle forms
 // and, when G = kCtas > 1 CTAs share one problem (a thread-block cluster), also
 //   rank_begin(), rank_end()   the ranks of the CTAs whose work this flow of control runs: its own on the device,
 //                              all G in the serial host emulation
@@ -23,7 +27,9 @@
 
 #include "mcc_band.h"
 #include "mcc_core.h"
-#ifdef __CUDACC__
+// (the host emulation defines RP_HOST_SHFL and host stand-ins for the warp intrinsics to run the shuffle forms)
+#if defined(__CUDACC__) || defined(RP_HOST_SHFL)
+#define RP_SHFL_FORMS 1
 #include "mcc_band_shfl.cuh"
 #include "mcc_wide_shfl.cuh"
 #endif
@@ -41,6 +47,12 @@ template <class Exec, class = void>
 struct CtasOf { static constexpr int value = 1; };
 template <class Exec>
 struct CtasOf<Exec, std::void_t<decltype(Exec::kCtas)>> { static constexpr int value = Exec::kCtas; };
+
+// whether executor Exec runs the warp-shuffle forms of the split sums (Exec::kShfl; an executor without it does not)
+template <class Exec, class = void>
+struct ShflOf { static constexpr bool value = false; };
+template <class Exec>
+struct ShflOf<Exec, std::void_t<decltype(Exec::kShfl)>> { static constexpr bool value = Exec::kShfl; };
 
 // chunk size of chunks(): `total` items spread over G CTAs, at most `cap` per chunk
 RP_HD int deal_chunk(int total, int G, int cap) {
@@ -103,28 +115,36 @@ RP_HD void emit_logz(Exec& ex, Ctx& c, const Problem& p, double* logz) {
 }
 
 // Split sums of the band of W diagonals d .. d+W-1 (inside) / d .. d-W+1 (outside): inside_band_* / outside_band_*
-// for W = BAND, the far pass wide_* for W > BAND; the shuffle forms on the device, the reference forms on the host.
+// for W = BAND, the far pass wide_* for W > BAND; the shuffle forms when Exec::kShfl, else the direct forms.
 // Rows are dealt in chunks of at most wide_chunk<W>(T), the rows one shuffle-form call takes.
 template <int W, class Exec>
 RP_HD void split_sums_inside(Exec& ex, Ctx& c, const Shared& sh, int d) {
   chunks(ex, 1, c.n - d + 1, wide_chunk<W>(sh.T), [&](int i0, int C) {
     ex.phase(PH_BAND_A, [&](int tid) {
-#ifdef __CUDA_ARCH__
-      if constexpr (W == BAND) inside_band_A_shfl<Exec::kBatch>(c, sh, d, i0, C, tid);
-      else wide_inside_A_shfl<W, WIDE_NB>(c, sh, d, i0, C, tid);
+      if constexpr (ShflOf<Exec>::value) {
+#ifdef RP_SHFL_FORMS
+        if constexpr (W == BAND) inside_band_A_shfl<Exec::kBatch>(c, sh, d, i0, C, tid);
+        else wide_inside_A_shfl<W, WIDE_NB>(c, sh, d, i0, C, tid);
 #else
-      if constexpr (W == BAND) inside_band_A(c, sh, d, i0, C, tid);
-      else wide_inside_A<W>(c, sh, d, i0, C, tid);
+        static_assert(!ShflOf<Exec>::value, "the shuffle forms are not compiled in");
 #endif
+      } else {
+        if constexpr (W == BAND) inside_band_A(c, sh, d, i0, C, tid);
+        else wide_inside_A<W>(c, sh, d, i0, C, tid);
+      }
     });
     ex.phase(PH_BAND_B, [&](int tid) {
-#ifdef __CUDA_ARCH__
-      if constexpr (W == BAND) inside_band_B_shfl(c, sh, d, i0, C, tid);
-      else wide_inside_B_shfl<W>(c, sh, d, i0, C, tid);
+      if constexpr (ShflOf<Exec>::value) {
+#ifdef RP_SHFL_FORMS
+        if constexpr (W == BAND) inside_band_B_shfl(c, sh, d, i0, C, tid);
+        else wide_inside_B_shfl<W>(c, sh, d, i0, C, tid);
 #else
-      if constexpr (W == BAND) inside_band_B(c, sh, d, i0, C, tid);
-      else wide_inside_B<W>(c, sh, d, i0, C, tid);
+        static_assert(!ShflOf<Exec>::value, "the shuffle forms are not compiled in");
 #endif
+      } else {
+        if constexpr (W == BAND) inside_band_B(c, sh, d, i0, C, tid);
+        else wide_inside_B<W>(c, sh, d, i0, C, tid);
+      }
     });
   });
 }
@@ -132,22 +152,30 @@ template <int W, class Exec>
 RP_HD void split_sums_outside(Exec& ex, Ctx& c, const Shared& sh, int d) {
   chunks(ex, 0, c.n - d + W - 1, wide_chunk<W>(sh.T), [&](int r0, int C) {
     ex.phase(PH_BAND_A, [&](int tid) {
-#ifdef __CUDA_ARCH__
-      if constexpr (W == BAND) outside_band_A_shfl<Exec::kBatch>(c, sh, d, r0, C, tid);
-      else wide_outside_A_shfl<W, WIDE_NB>(c, sh, d, r0, C, tid);
+      if constexpr (ShflOf<Exec>::value) {
+#ifdef RP_SHFL_FORMS
+        if constexpr (W == BAND) outside_band_A_shfl<Exec::kBatch>(c, sh, d, r0, C, tid);
+        else wide_outside_A_shfl<W, WIDE_NB>(c, sh, d, r0, C, tid);
 #else
-      if constexpr (W == BAND) outside_band_A(c, sh, d, r0, C, tid);
-      else wide_outside_A<W>(c, sh, d, r0, C, tid);
+        static_assert(!ShflOf<Exec>::value, "the shuffle forms are not compiled in");
 #endif
+      } else {
+        if constexpr (W == BAND) outside_band_A(c, sh, d, r0, C, tid);
+        else wide_outside_A<W>(c, sh, d, r0, C, tid);
+      }
     });
     ex.phase(PH_BAND_B, [&](int tid) {
-#ifdef __CUDA_ARCH__
-      if constexpr (W == BAND) outside_band_B_shfl(c, sh, d, r0, C, tid);
-      else wide_outside_B_shfl<W>(c, sh, d, r0, C, tid);
+      if constexpr (ShflOf<Exec>::value) {
+#ifdef RP_SHFL_FORMS
+        if constexpr (W == BAND) outside_band_B_shfl(c, sh, d, r0, C, tid);
+        else wide_outside_B_shfl<W>(c, sh, d, r0, C, tid);
 #else
-      if constexpr (W == BAND) outside_band_B(c, sh, d, r0, C, tid);
-      else wide_outside_B<W>(c, sh, d, r0, C, tid);
+        static_assert(!ShflOf<Exec>::value, "the shuffle forms are not compiled in");
 #endif
+      } else {
+        if constexpr (W == BAND) outside_band_B(c, sh, d, r0, C, tid);
+        else wide_outside_B<W>(c, sh, d, r0, C, tid);
+      }
     });
   });
 }
@@ -333,7 +361,7 @@ RP_HD void solve_band(Exec& ex, Ctx& c, const Problem& p, float* dense, double* 
   const int n = c.n;
   Shared sh;
   BandShared bs;
-  carve_band(sh, bs, smem, n, T);
+  carve_band(sh, bs, smem, n, T, ShflOf<Exec>::value);
   const bool wide = c.kind == KIND_LINEAR && c.max_w > 0;  // the unpaired-window pass reads the class tables' full history
   stage_sequence(ex, c, sh.S, [&](int tid) {
     load_band_weights(*c.M, bs, tid, T);
@@ -398,7 +426,7 @@ RP_HD void solve_band_unpaired(Exec& ex, Ctx& c, const Problem& p, float* dense,
   const int T = ex.nthreads(), n = c.n;
   Shared sh;
   BandShared bs;
-  carve_band(sh, bs, smem, n, T);
+  carve_band(sh, bs, smem, n, T, ShflOf<Exec>::value);
   stage_sequence(ex, c, sh.S, [&](int tid) { load_band_weights(*c.M, bs, tid, T); });
   inside_end(c);
   emit_unpaired(ex, c, p, dense, *bs.sm, stage_gap_weights(ex, c, bs));

@@ -1,4 +1,4 @@
-// mcc_wide_shfl.cuh -- device-only far passes of the WIDE split-sum bands (mcc_core.h, "Wide bands"),
+// mcc_wide_shfl.cuh -- the device's far passes of the WIDE split-sum bands (mcc_core.h, "Wide bands"),
 // general kernel, long problems.
 //
 // Same scheme as mcc_band_shfl.cuh -- a thread keeps one accumulator per diagonal of the band for its

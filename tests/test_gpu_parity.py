@@ -574,3 +574,36 @@ def test_single_sequence_request_and_context_lifetime(oracle, model, bundled):
     flat = b.fetch_dense()
     assert np.abs(b.split_dense(flat)[0].bp1.astype(np.float64) - obp).max() <= TOL
     b.close()
+
+
+# The lengths and nick positions the host emulation runs through the warp-shuffle forms of the split sums
+# (test_emul.py, test_lockstep_routes_match_oracle), on the device routes that run those forms, in one ragged batch.
+# Strand 1 of 22..24 / 27..29 nt puts the nick of the two-strand problem just before, on and just after the second
+# warp's first row (32-(W-1) rows a warp, W = 10 / 5); 60, 96 and 175 nt put a split-sum chunk on each edge class of
+# the warp split at 512 threads; strands of 1..8 nt are too short for a band.
+SPLIT_SUM_SWEEP = [(1, 2), (3, 4), (5, 6), (7, 8), (22, 115), (23, 175), (24, 40), (27, 60), (28, 96), (29, 24)]
+
+
+@pytest.mark.parametrize("route", [
+    {"RP_BAND": "0", "RP_CLUSTER": "0"},                         # mcc_persistent<2,5>: the 64-register build
+    {"RP_BAND": "0", "RP_CLUSTER": "0", "RP_MCC_LONG_N": "1"},   # mcc_persistent<1,10>: wide bands, every length
+    {"RP_BAND": "0", "RP_CLUSTER": "8"},                         # mcc_cluster_kernel<10,8>
+    {"RP_BAND": "0", "RP_CLUSTER": "16"},                        # mcc_cluster_kernel<10,16>
+], ids=["general64", "wide10", "cluster8", "cluster16"])
+def test_split_sum_shapes_on_every_general_route(model, oracle, monkeypatch, route):
+    """The shapes of the host emulation's warp-lockstep runs on each general-kernel route of the device, against the
+    oracle: the device confirms what the emulated warps model."""
+    from ractip_b200 import ProbabilityStage, default_opts
+    for k, v in route.items():
+        monkeypatch.setenv(k, v)   # read when a context is created
+    rng = np.random.default_rng(13000)
+    pairs = [(rand_seq(rng, n1), rand_seq(rng, n2)) for n1, n2 in SPLIT_SUM_SWEEP]
+    opts = default_opts()
+    st = ProbabilityStage(model)
+    try:
+        res = st.run_dense(pairs, opts)
+    finally:
+        st.close()
+    tag = " ".join("%s=%s" % kv for kv in route.items())
+    for (s1, s2), r in zip(pairs, res):
+        _compare(r, _oracle_pair(oracle, s1, s2, opts), s1, s2, opts, f"{tag} {len(s1)}x{len(s2)}")
