@@ -194,6 +194,9 @@ const char* rp_strerror(int code);
 /* Use an externally owned cudaStream_t (e.g. torch's current stream). NULL
  * restores the context's own stream. */
 int rp_set_stream(rp_ctx* ctx, void* cuda_stream);
+/* The stream the context enqueues on now (its own one unless rp_set_stream
+ * chose another), so that a caller can set it back after borrowing it. */
+int rp_get_stream(const rp_ctx* ctx, void** cuda_stream);
 
 /* Pinned host memory for output buffers (plain malloc'd buffers also work). */
 void* rp_host_alloc(size_t bytes);
@@ -240,6 +243,37 @@ int rp_batch_fetch_sparse(rp_batch* batch, rp_rec* recs, size_t n_recs,
  * context stream.  counts_dev receives n_pairs rp_sparse_counts. */
 int rp_batch_sparse_device(rp_batch* batch, void* recs_dev, size_t n_recs,
                            void* ups_dev, size_t n_floats, void* counts_dev);
+/* The dense outputs left in DEVICE memory the caller owns, in the layout of
+ * rp_dense_plan (the bytes rp_batch_fetch_dense delivers): one device-to-device
+ * copy, asynchronous on the context's current stream.  If the batch last ran
+ * on another stream, the current stream first waits for it (no host
+ * synchronisation).  RP_ERR_CAPACITY when out_floats < total_floats. */
+int rp_batch_dense_device(rp_batch* batch, void* out_dev, size_t out_floats);
+
+/* Padded square layout of a batch: the dense outputs of every pair expanded
+ * into five fp32 tensors, row-major, 1-based like the reference (index 0 and
+ * everything past a pair's own lengths are 0):
+ *   bp1 [B][N1+1][N1+1]   symmetric: P[i][j] = P[j][i] = bp[offset[i]+j], 1<=i<j<=n1
+ *   bp2 [B][N2+1][N2+1]
+ *   up1 [B][N1][W]        up[i][d] as in rp_dense_layout, rows past n1 are 0
+ *   up2 [B][N2][W]
+ *   hp  [B][N1+1][N2+1]   hp[i][j] as in rp_dense_layout (thresholded zeros kept)
+ * with N1 = max n1, N2 = max n2 over the batch and W = max(max_w, 0).  A pair
+ * with n2 == 0 has all-zero bp2, up2 and hp slices.  n_* are element counts;
+ * RP_ERR_ARG if one of them (or its size in bytes) overflows size_t.  Host
+ * arithmetic only. */
+typedef struct rp_square_layout {
+  int B, N1, N2, W;
+  size_t n_bp1, n_bp2, n_up1, n_up2, n_hp;
+} rp_square_layout;
+int rp_square_plan(const rp_pair* pairs, int n_pairs, const rp_opts* opts,
+                   rp_square_layout* layout);
+/* Expand the batch's dense outputs into the square tensors of rp_square_plan,
+ * in DEVICE memory the caller owns (each sized as rp_square_plan says; NULL
+ * skips that tensor).  Every element, padding included, is written: the
+ * buffers need no clearing.  Same stream rules as rp_batch_dense_device. */
+int rp_batch_square_device(rp_batch* batch, float* bp1, float* bp2, float* up1,
+                           float* up2, float* hp);
 /* log of the (unscaled) partition function per problem: 3 doubles per pair
  * (s1, s2, s1&s2); parity / debugging aid. */
 int rp_batch_fetch_logz(rp_batch* batch, double* logz, size_t n);

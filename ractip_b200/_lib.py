@@ -67,6 +67,11 @@ class RpDenseLayout(C.Structure):
                 ("bp1", "bp2", "up1", "up2", "hp", "n_bp1", "n_bp2", "n_up1", "n_up2", "n_hp")]
 
 
+class RpSquareLayout(C.Structure):
+    _fields_ = [("B", C.c_int), ("N1", C.c_int), ("N2", C.c_int), ("W", C.c_int)] + \
+        [(n, C.c_size_t) for n in ("n_bp1", "n_bp2", "n_up1", "n_up2", "n_hp")]
+
+
 class RpRec(C.Structure):
     _fields_ = [("i", C.c_int32), ("j", C.c_int32), ("p", C.c_float)]
 
@@ -98,9 +103,10 @@ class RpTiming(C.Structure):
 EXPORTS = [
     "rp_model_default", "rp_model_read_par", "rp_model_digest", "rp_opts_default",
     "rp_dense_plan", "rp_sparse_plan", "rp_create", "rp_destroy", "rp_last_error",
-    "rp_strerror", "rp_set_stream", "rp_host_alloc", "rp_host_free", "rp_run_dense",
+    "rp_strerror", "rp_set_stream", "rp_get_stream", "rp_host_alloc", "rp_host_free", "rp_run_dense",
     "rp_run_sparse", "rp_batch_create", "rp_batch_run", "rp_batch_sync",
-    "rp_batch_fetch_dense", "rp_batch_fetch_sparse", "rp_batch_sparse_device", "rp_batch_fetch_logz",
+    "rp_batch_fetch_dense", "rp_batch_fetch_sparse", "rp_batch_sparse_device", "rp_batch_dense_device",
+    "rp_square_plan", "rp_batch_square_device", "rp_batch_fetch_logz",
     "rp_batch_destroy", "rp_last_timing", "rp_measure_peaks", "rp_zscore_shuffles",
     "rp_alg_flops_mcc", "rp_version", "rp_kernel_plan",
     "rp_multi_create", "rp_multi_destroy", "rp_multi_devices", "rp_multi_last_error", "rp_multi_run_dense",
@@ -141,6 +147,7 @@ def load() -> C.CDLL:
         "rp_last_error": (C.c_char_p, [vp]),
         "rp_strerror": (C.c_char_p, [i]),
         "rp_set_stream": (i, [vp, vp]),
+        "rp_get_stream": (i, [vp, P(vp)]),
         "rp_host_alloc": (vp, [sz]),
         "rp_host_free": (None, [vp]),
         "rp_run_dense": (i, [vp, P(RpPair), i, P(RpOpts), vp, sz]),
@@ -151,6 +158,9 @@ def load() -> C.CDLL:
         "rp_batch_fetch_dense": (i, [vp, vp, sz]),
         "rp_batch_fetch_sparse": (i, [vp, vp, sz, vp, sz, vp]),
         "rp_batch_sparse_device": (i, [vp, vp, sz, vp, sz, vp]),
+        "rp_batch_dense_device": (i, [vp, vp, sz]),
+        "rp_square_plan": (i, [P(RpPair), i, P(RpOpts), P(RpSquareLayout)]),
+        "rp_batch_square_device": (i, [vp, vp, vp, vp, vp, vp]),
         "rp_batch_fetch_logz": (i, [vp, vp, sz]),
         "rp_batch_destroy": (i, [vp]),
         "rp_last_timing": (i, [vp, P(RpTiming)]),

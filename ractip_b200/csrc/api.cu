@@ -37,6 +37,7 @@ struct rp_ctx {
   cudaEvent_t ev_fork = nullptr, ev_join = nullptr;
   cudaStream_t copy_stream = nullptr;   // rp_batch_fetch_dense: outputs of the long band class leave while the short class still runs
   cudaEvent_t ev_main = nullptr, ev_copy = nullptr;
+  cudaEvent_t ev_handoff = nullptr;     // rp_batch_*_device: the reading stream waits for the stream the batch ran on
   cudaStream_t stream = nullptr;
   cudaEvent_t ev[6] = {};
   cudaEvent_t ev_dom[2] = {};   // around the launch that carries most of the algorithmic flops (rp_timing::ms_dominant)
@@ -272,6 +273,7 @@ int rp_create(rp_ctx** out, const rp_model* m, int device) {
   if ((e = cudaStreamCreateWithFlags(&ctx->copy_stream, cudaStreamNonBlocking)) != cudaSuccess) return bail(RP_ERR_CUDA, cudaGetErrorString(e));
   if ((e = cudaEventCreateWithFlags(&ctx->ev_main, cudaEventDisableTiming)) != cudaSuccess) return bail(RP_ERR_CUDA, cudaGetErrorString(e));
   if ((e = cudaEventCreateWithFlags(&ctx->ev_copy, cudaEventDisableTiming)) != cudaSuccess) return bail(RP_ERR_CUDA, cudaGetErrorString(e));
+  if ((e = cudaEventCreateWithFlags(&ctx->ev_handoff, cudaEventDisableTiming)) != cudaSuccess) return bail(RP_ERR_CUDA, cudaGetErrorString(e));
   for (auto& ev : ctx->ev)
     if ((e = cudaEventCreate(&ev)) != cudaSuccess) return bail(RP_ERR_CUDA, cudaGetErrorString(e));
   for (auto& ev : ctx->ev_dom)
@@ -312,6 +314,7 @@ int rp_destroy(rp_ctx* ctx) {
   if (ctx->copy_stream) { cudaStreamSynchronize(ctx->copy_stream); cudaStreamDestroy(ctx->copy_stream); }
   if (ctx->ev_main) cudaEventDestroy(ctx->ev_main);
   if (ctx->ev_copy) cudaEventDestroy(ctx->ev_copy);
+  if (ctx->ev_handoff) cudaEventDestroy(ctx->ev_handoff);
   if (ctx->ev_fork) cudaEventDestroy(ctx->ev_fork);
   if (ctx->ev_join) cudaEventDestroy(ctx->ev_join);
   if (ctx->own_stream) cudaStreamDestroy(ctx->own_stream);
@@ -322,6 +325,12 @@ int rp_destroy(rp_ctx* ctx) {
 int rp_set_stream(rp_ctx* ctx, void* cuda_stream) {
   if (!ctx) return RP_ERR_ARG;
   ctx->stream = cuda_stream ? static_cast<cudaStream_t>(cuda_stream) : ctx->own_stream;
+  return RP_OK;
+}
+
+int rp_get_stream(const rp_ctx* ctx, void** cuda_stream) {
+  if (!ctx || !cuda_stream) return RP_ERR_ARG;
+  *cuda_stream = ctx->stream;
   return RP_OK;
 }
 
@@ -584,7 +593,56 @@ int sparse_launch(rp_batch* b, rp_rec* d_recs, float* d_ups, rp_sparse_counts* d
   ctx->timing.kernel_launches += d_ups ? 2 : 1;
   return RP_OK;
 }
+
+// Work that reads the batch's outputs on the context's current stream: that stream waits (on the device) for the stream
+// the batch last ran on, and becomes the one rp_batch_destroy waits for before the buffers go back to the pool.
+int order_after_run(rp_batch* b) {
+  rp_ctx* ctx = b->ctx;
+  if (b->last_stream && b->last_stream != ctx->stream) {
+    CU(cudaEventRecord(ctx->ev_handoff, b->last_stream));
+    CU(cudaStreamWaitEvent(ctx->stream, ctx->ev_handoff, 0));
+  }
+  b->last_stream = ctx->stream;
+  return RP_OK;
+}
 }  // namespace
+
+extern "C" int rp_batch_dense_device(rp_batch* b, void* out_dev, size_t out_floats) {
+  if (!b || !out_dev) return RP_ERR_ARG;
+  rp_ctx* ctx = b->ctx;
+  const rp::BatchPlan& p = b->plan;
+  if (out_floats < p.total_floats) return fail(ctx, RP_ERR_CAPACITY, "rp_batch_dense_device: buffer too small");
+  CU(cudaSetDevice(ctx->device));
+  if (b->n_pairs == 0) return RP_OK;
+  int rc = order_after_run(b);
+  if (rc) return rc;
+  CU(cudaMemcpyAsync(out_dev, b->d_dense, p.total_floats * sizeof(float), cudaMemcpyDeviceToDevice, ctx->stream));
+  return RP_OK;
+}
+
+extern "C" int rp_batch_square_device(rp_batch* b, float* bp1, float* bp2, float* up1, float* up2, float* hp) {
+  if (!b) return RP_ERR_ARG;
+  rp_ctx* ctx = b->ctx;
+  const rp::BatchPlan& p = b->plan;
+  CU(cudaSetDevice(ctx->device));
+  if (b->n_pairs == 0 || !(bp1 || bp2 || up1 || up2 || hp)) return RP_OK;
+  rp::SquareDev s;
+  s.probs = b->d_probs; s.dense = b->d_dense;
+  s.out[rp::SQ_BP1] = bp1; s.out[rp::SQ_BP2] = bp2; s.out[rp::SQ_UP1] = up1; s.out[rp::SQ_UP2] = up2; s.out[rp::SQ_HP] = hp;
+  s.N1 = s.N2 = 0;
+  for (int k = 0; k < b->n_pairs; k++) {   // the dimensions rp_square_plan gives the batch's pairs
+    s.N1 = std::max(s.N1, p.probs[3 * k].n1);
+    s.N2 = std::max(s.N2, p.probs[3 * k].n2);
+  }
+  s.W = std::max(b->opts.max_w, 0);
+  s.tiles = (std::max(s.N1, s.N2) + 1 + 31) / 32;
+  if ((long long)b->n_pairs * s.tiles > 0x7fffffffLL)
+    return fail(ctx, RP_ERR_ARG, "rp_batch_square_device: batch too large for one launch");
+  int rc = order_after_run(b);
+  if (rc) return rc;
+  CU(rp::launch_square(s, b->n_pairs, ctx->stream));
+  return RP_OK;
+}
 
 extern "C" int rp_batch_sparse_device(rp_batch* b, void* recs_dev, size_t n_recs, void* ups_dev, size_t n_floats,
                                       void* counts_dev) {

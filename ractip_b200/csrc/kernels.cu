@@ -456,6 +456,79 @@ __global__ void gather_up_kernel(SparseDev s) {
 }
 
 // ---------------------------------------------------------------------------
+// square_kernel (rp_batch_square_device): the packed sections of a batch expanded into the padded square tensors of
+// rp_square_plan.  One CTA per (pair, tile of 32 output rows, section), each writing every element of its rows, padding
+// included: the caller's buffers need no clearing.  bp: the upper triangle of output row i is packed row i
+// (bp[offset[i]+i+1 .. offset[i]+L]), a coalesced row copy; the mirrored lower triangle of the row is a column of the
+// packed layout, so it goes through a 32 x 32 shared-memory transpose -- loads along packed rows, stores along output
+// rows.  up and hp are row-major already: row by row into the padded rows.
+// ---------------------------------------------------------------------------
+constexpr int RP_SQUARE_THREADS = 256;
+constexpr int RP_SQUARE_ROWS = 32;
+__global__ void __launch_bounds__(RP_SQUARE_THREADS) square_kernel(SquareDev s) {
+  __shared__ float tile[RP_SQUARE_ROWS][RP_SQUARE_ROWS + 1];   // +1: the transposed reads fall in 32 different banks
+  const int sec = blockIdx.y;
+  float* out_sec = s.out[0];   // selected, not indexed: a parameter array indexed at run time is copied to local memory
+#pragma unroll
+  for (int k = 1; k < SQ_SECTIONS; k++) out_sec = sec == k ? s.out[k] : out_sec;
+  if (!out_sec) return;
+  const int pair = blockIdx.x / s.tiles, r0 = (blockIdx.x - pair * s.tiles) * RP_SQUARE_ROWS;
+  const Problem* pp = s.probs + 3 * pair;   // s1, s2, s1&s2
+  const int n1 = pp[0].n1, n2 = pp[0].n2;
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, NW = RP_SQUARE_THREADS / 32;
+  if (sec == SQ_BP1 || sec == SQ_BP2) {
+    const int L = sec == SQ_BP1 ? n1 : n2, M = (sec == SQ_BP1 ? s.N1 : s.N2) + 1;
+    if (r0 >= M) return;
+    const float* bp = s.dense + pp[sec == SQ_BP1 ? 0 : 1].out_bp;
+    float* out = out_sec + (size_t)pair * M * M;
+    auto off = [L](int i) { return i * (2 * L + 1 - i) / 2; };   // offset[i], src/ractip.cpp:316-317
+    // columns 0 .. r0+31: the lower triangle by transposed tiles (packed row j = lower-triangle column j); the tile
+    // on the diagonal also takes its upper part straight from the packed rows
+    for (int c0 = 0; c0 <= r0; c0 += RP_SQUARE_ROWS) {
+      for (int jj = warp; jj < RP_SQUARE_ROWS; jj += NW) {
+        const int j = c0 + jj, i = r0 + lane;
+        tile[jj][lane] = (j >= 1 && j < i && i <= L) ? bp[off(j) + i] : 0.f;
+      }
+      __syncthreads();
+      for (int ii = warp; ii < RP_SQUARE_ROWS; ii += NW) {
+        const int i = r0 + ii, j = c0 + lane;
+        if (i < M && j < M) out[(size_t)i * M + j] = j > i ? (i >= 1 && j <= L ? bp[off(i) + j] : 0.f) : tile[lane][ii];
+      }
+      __syncthreads();
+    }
+    // columns r0+32 .. M-1: upper triangle only
+    for (int ii = warp; ii < RP_SQUARE_ROWS; ii += NW) {
+      const int i = r0 + ii;
+      if (i >= M) break;
+      float* o = out + (size_t)i * M;
+      for (int j = r0 + RP_SQUARE_ROWS + lane; j < M; j += 32) o[j] = (i >= 1 && j <= L) ? bp[off(i) + j] : 0.f;
+    }
+  } else if (sec == SQ_HP) {
+    const int rows = s.N1 + 1, cols = s.N2 + 1;
+    if (r0 >= rows) return;
+    const long long o = pp[2].out_hp;   // -1 for a lone sequence (n2 == 0): an all-zero slice
+    const int Lr = o >= 0 ? n1 + 1 : 0, Lc = n2 + 1;
+    const float* hp = s.dense + (o >= 0 ? o : 0);
+    float* out = out_sec + (size_t)pair * rows * cols;
+    const int r1 = min(r0 + RP_SQUARE_ROWS, rows);
+    for (int i = r0 + warp; i < r1; i += NW)
+      for (int j = lane; j < cols; j += 32)
+        out[(size_t)i * cols + j] = (i < Lr && j < Lc) ? hp[(size_t)i * Lc + j] : 0.f;
+  } else {
+    // up rows have the width W in both layouts: the tile's rows are one contiguous range, the pair's own rows first
+    const bool first = sec == SQ_UP1;
+    const int rows = first ? s.N1 : s.N2;
+    if (r0 >= rows) return;
+    const long long o = pp[first ? 0 : 1].out_up;   // -1 when W == 0
+    const size_t W = (size_t)s.W, e0 = (size_t)r0 * W, e1 = (size_t)min(r0 + RP_SQUARE_ROWS, rows) * W;
+    const size_t own = o >= 0 ? (size_t)(first ? n1 : n2) * W : 0;
+    const float* up = s.dense + (o >= 0 ? o : 0);
+    float* out = out_sec + (size_t)pair * rows * W;
+    for (size_t e = e0 + threadIdx.x; e < e1; e += RP_SQUARE_THREADS) out[e] = e < own ? up[e] : 0.f;
+  }
+}
+
+// ---------------------------------------------------------------------------
 // roofline denominators measured live: fp64 FMA pipe and shared-memory reads
 // ---------------------------------------------------------------------------
 __global__ void __launch_bounds__(256) peak_fp64_kernel(double* out, int iters) {
@@ -570,6 +643,11 @@ cudaError_t launch_sparse(const SparseDev& s, int n_pairs, bool with_ups, cudaSt
   cudaError_t e = cudaGetLastError();
   if (e != cudaSuccess || !with_ups) return e;
   gather_up_kernel<<<n_pairs, 256, 0, st>>>(s);
+  return cudaGetLastError();
+}
+
+cudaError_t launch_square(const SquareDev& s, int n_pairs, cudaStream_t st) {
+  square_kernel<<<dim3((unsigned)n_pairs * (unsigned)s.tiles, SQ_SECTIONS), RP_SQUARE_THREADS, 0, st>>>(s);
   return cudaGetLastError();
 }
 

@@ -53,6 +53,17 @@ struct SparseDev {
   int min_w, max_w;                    // window-length indices min_w-1 .. max_w-1 are scanned (src/ractip.cpp:622)
 };
 
+// rp_batch_square_device: the dense outputs of a batch (three problems per pair, in pair order: s1, s2, s1&s2, whose
+// out_* offsets locate the pair's sections) expanded into the padded square tensors of rp_square_plan
+enum { SQ_BP1 = 0, SQ_BP2, SQ_UP1, SQ_UP2, SQ_HP, SQ_SECTIONS };
+struct SquareDev {
+  const Problem* probs;
+  const float* dense;
+  float* out[SQ_SECTIONS];             // null: section skipped
+  int N1, N2, W;
+  int tiles;                           // 32-row tiles per pair: ceil((max(N1, N2) + 1) / 32)
+};
+
 // general kernel, RP_MCC_THREADS threads.  minb = 2: 64-register build, two CTAs per SM; 1: 128 registers, one CTA
 // per SM, split sums in bands of 10 diagonals
 int mcc_max_ctas_per_sm(int minb);
@@ -65,6 +76,7 @@ cudaError_t launch_duplex(const BatchDev& b, int grid, cudaStream_t st);
 int unstru_max_ctas_per_sm();
 cudaError_t launch_unstru(const BatchDev& b, int grid, cudaStream_t st);   // deferred unpaired-window passes: b.order/nprob = their queue
 cudaError_t launch_sparse(const SparseDev& s, int n_pairs, bool with_ups, cudaStream_t st);
+cudaError_t launch_square(const SquareDev& s, int n_pairs, cudaStream_t st);
 cudaError_t launch_peak_fp64(double* out, int grid, int iters, cudaStream_t st);
 cudaError_t launch_peak_smem(double* out, int grid, int iters, cudaStream_t st);
 

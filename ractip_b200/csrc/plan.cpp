@@ -58,6 +58,36 @@ int rp_dense_plan(const rp_pair* pairs, int n_pairs, const rp_opts* opts, rp_den
   return RP_OK;
 }
 
+int rp_square_plan(const rp_pair* pairs, int n_pairs, const rp_opts* opts, rp_square_layout* layout) {
+  int rc = rp::check_pairs(pairs, n_pairs, opts);
+  if (rc) return rc;
+  if (!layout) return RP_ERR_ARG;
+  rp_square_layout s = {};
+  s.B = n_pairs;
+  s.W = std::max(opts->max_w, 0);
+  for (int p = 0; p < n_pairs; p++) {
+    s.N1 = std::max(s.N1, pairs[p].n1);
+    s.N2 = std::max(s.N2, pairs[p].n2);
+  }
+  // B * rows * cols elements, and their size in bytes, must fit size_t
+  bool overflow = false;
+  auto count = [&](size_t rows, size_t cols) {
+    size_t n = 0;
+    overflow |= __builtin_mul_overflow((size_t)s.B, rows, &n) || __builtin_mul_overflow(n, cols, &n) ||
+                n > SIZE_MAX / sizeof(float);
+    return n;
+  };
+  const size_t m1 = (size_t)s.N1 + 1, m2 = (size_t)s.N2 + 1;
+  s.n_bp1 = count(m1, m1);
+  s.n_bp2 = count(m2, m2);
+  s.n_up1 = count(s.N1, s.W);
+  s.n_up2 = count(s.N2, s.W);
+  s.n_hp = count(m1, m2);
+  if (overflow) return RP_ERR_ARG;
+  *layout = s;
+  return RP_OK;
+}
+
 int rp_sparse_plan(const rp_pair* pairs, int n_pairs, const rp_opts* opts, rp_sparse_layout* layout, size_t* total_recs,
                    size_t* total_floats) {
   int rc = rp::check_pairs(pairs, n_pairs, opts);

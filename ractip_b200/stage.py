@@ -13,15 +13,16 @@ All arithmetic runs in the CUDA library; torch/numpy are only used for buffers.
 """
 from __future__ import annotations
 
+import contextlib
 import ctypes as C
 from dataclasses import dataclass
-from typing import List, Optional, Sequence, Tuple
+from typing import Dict, List, Optional, Sequence, Tuple
 
 import numpy as np
 
 from . import _lib
 from ._lib import (RpDenseLayout, RpModel, RpOpts, RpPair, RpRec, RpSparseCounts,
-                   RpSparseLayout, RpTiming)
+                   RpSparseLayout, RpSquareLayout, RpTiming)
 
 
 class RpError(RuntimeError):
@@ -89,6 +90,11 @@ class PairRecords:
 
 REC_DTYPE = np.dtype([("i", np.int32), ("j", np.int32), ("p", np.float32)])
 
+# the tensors of DeviceBatch.tensors(), in the argument order of rp_batch_square_device
+SQUARE_KEYS = ("bp1", "bp2", "up1", "up2", "hp")
+# cudaStreamLegacy: torch's default stream has handle 0, which rp_set_stream reads as "the context's own stream"
+_CUDA_STREAM_LEGACY = 1
+
 
 def _make_pairs(pairs: Sequence[Tuple[str, str]]):
     n = len(pairs)
@@ -151,6 +157,42 @@ class DeviceBatch:
         self.stage._check(self.lib.rp_batch_fetch_logz(self.handle, lz.ctypes.data, lz.size))
         return lz[:self.n]
 
+    def square_layout(self) -> RpSquareLayout:
+        """rp_square_plan of the batch: B, N1, N2, W and the element count of each square tensor."""
+        arr, keep = _make_pairs(self.pairs)
+        lay = RpSquareLayout()
+        self.stage._check(self.lib.rp_square_plan(arr, self.n, C.byref(self.opts), C.byref(lay)))
+        return lay
+
+    def dense_tensor(self):
+        """The dense outputs as one flat float32 CUDA tensor in the layout of rp_dense_plan (the values
+        fetch_dense() returns), copied on the device.  Enqueued on torch's current stream: torch ops that
+        follow on that stream see the result without a host synchronisation."""
+        with self.stage._torch_stream() as torch:
+            out = torch.empty(max(self.total_floats, 1), dtype=torch.float32, device=self.stage.torch_device())
+            self.stage._check(self.lib.rp_batch_dense_device(self.handle, C.c_void_p(out.data_ptr()), out.numel()))
+        return out[:self.total_floats]
+
+    def tensors(self) -> Dict[str, "torch.Tensor"]:
+        """The outputs as padded square float32 CUDA tensors (rp_batch_square_device), 1-based like the reference:
+        bp1 [B, N1+1, N1+1] and bp2 [B, N2+1, N2+1] symmetric, up1 [B, N1, W], up2 [B, N2, W], hp [B, N1+1, N2+1],
+        N1 / N2 the longest first / second sequence of the batch, W = max_w; index 0 and everything past a pair's
+        own lengths are 0.  n1 and n2 (int32 [B]) hold each pair's lengths for masking.  Enqueued on torch's
+        current stream, like dense_tensor()."""
+        lay = self.square_layout()
+        B, N1, N2, W = lay.B, lay.N1, lay.N2, lay.W
+        shapes = {"bp1": (B, N1 + 1, N1 + 1), "bp2": (B, N2 + 1, N2 + 1), "up1": (B, N1, W), "up2": (B, N2, W),
+                  "hp": (B, N1 + 1, N2 + 1)}
+        with self.stage._torch_stream() as torch:
+            dev = self.stage.torch_device()
+            out = {k: torch.empty(shapes[k], dtype=torch.float32, device=dev) for k in SQUARE_KEYS}
+            ptrs = [C.c_void_p(out[k].data_ptr() if out[k].numel() else None) for k in SQUARE_KEYS]
+            self.stage._check(self.lib.rp_batch_square_device(self.handle, *ptrs))
+            lens = torch.tensor([len(a) for a, _ in self.pairs] + [len(b) for _, b in self.pairs], dtype=torch.int32)
+            lens = lens.pin_memory().to(dev, non_blocking=True)
+        out["n1"], out["n2"] = lens[:self.n], lens[self.n:]
+        return out
+
     def split_dense(self, flat: np.ndarray) -> List[PairProbabilities]:
         out = []
         w = max(self.opts.max_w, 0)
@@ -210,6 +252,27 @@ class ProbabilityStage:
             msg = self.lib.rp_last_error(self.ctx).decode() or self.lib.rp_strerror(rc).decode()
             raise RpError(rc, msg)
 
+    def torch_device(self):
+        import torch
+        return torch.device("cuda", self.device)
+
+    @contextlib.contextmanager
+    def _torch_stream(self):
+        """Run the block's library calls on torch's current stream, then give the context its previous stream
+        back.  torch is imported here only: the rest of the stage works without it."""
+        import torch
+        if torch.cuda.current_device() != self.device:
+            raise RuntimeError(f"torch's current device is cuda:{torch.cuda.current_device()}, this stage runs on "
+                               f"cuda:{self.device}: select it with torch.cuda.device({self.device})")
+        prev = C.c_void_p()
+        self._check(self.lib.rp_get_stream(self.ctx, C.byref(prev)))
+        stream = torch.cuda.current_stream(self.device).cuda_stream or _CUDA_STREAM_LEGACY
+        self._check(self.lib.rp_set_stream(self.ctx, C.c_void_p(stream)))
+        try:
+            yield torch
+        finally:
+            self.lib.rp_set_stream(self.ctx, prev)
+
     def close(self):
         if getattr(self, "ctx", None):
             self.lib.rp_destroy(self.ctx)
@@ -260,6 +323,16 @@ class ProbabilityStage:
                 up2=flat[L.up2:L.up2 + L.n_up2].reshape(n2, w),
                 hp=flat[L.hp:L.hp + L.n_hp].reshape(n1 + 1, n2 + 1)))
         return out
+
+    def run_tensors(self, pairs: Sequence[Tuple[str, str]], opts: Optional[RpOpts] = None) -> Dict[str, "torch.Tensor"]:
+        """batch + run + DeviceBatch.tensors(): the square CUDA tensors of `pairs`.  Closing the batch waits for
+        the expansion (the batch's buffers go back to the context's pool)."""
+        b = self.batch(pairs, opts)
+        try:
+            b.run()
+            return b.tensors()
+        finally:
+            b.close()
 
     def run_sparse(self, pairs: Sequence[Tuple[str, str]], opts: Optional[RpOpts] = None) -> List[PairRecords]:
         opts = opts if opts is not None else default_opts()
