@@ -233,6 +233,36 @@ int rp_multi_run_sparse(rp_multi* multi, const rp_pair* pairs, int n_pairs,
 typedef struct rp_batch rp_batch;
 int rp_batch_create(rp_ctx* ctx, const rp_pair* pairs, int n_pairs,
                     const rp_opts* opts, rp_batch** batch);
+
+/* Structure constraints of one pair (RactIP -c, the FASTA record's structure
+ * line): c1 over s1 (n1 chars), c2 over s2 (n2 chars), NUL-terminated; NULL
+ * means unconstrained.  Alphabet of RactIP's joint structures:
+ *   .      no constraint
+ *   x      the base pairs with nothing
+ *   ( )    intramolecular pair, bracket-matched within the same string
+ *   [ ]    intermolecular pair, '[' in c1 only, ']' in c2 only: the k-th '['
+ *          from the 3' end of s1 pairs with the k-th ']' from the 5' end of s2
+ * A constraint only removes pairs (no base is forced to pair, no energy
+ * changes).  s1's fold sees the () of c1 and keeps x and [ unpaired; s2's fold
+ * the () of c2, x and ] unpaired; the s1&s2 co-fold the [] pairs, x ( )
+ * unpaired; the --duplex branch is unconstrained.  A pair (i,j) of a problem is
+ * allowed when neither base is unpaired there, a bracketed base pairs only with
+ * its partner, and (i,j) crosses no bracket pair.  A bracket pair that cannot
+ * form leaves both bases unpaired. */
+typedef struct rp_constraint {
+  const char* c1;
+  const char* c2;
+} rp_constraint;
+/* rp_batch_create with one rp_constraint per pair (cons == NULL, or an entry
+ * with both strings NULL: unconstrained).  The problems a constraint restricts
+ * run on the general kernel.  RP_ERR_ARG, with rp_last_error naming the pair,
+ * the string and the position, for a string whose length differs from its
+ * sequence's, a character outside .x()[], unbalanced (), ] in c1 or [ in c2,
+ * or different numbers of [ in c1 and ] in c2.  Everything that takes an
+ * rp_batch works on the result unchanged. */
+int rp_batch_create_constrained(rp_ctx* ctx, const rp_pair* pairs,
+                                const rp_constraint* cons, int n_pairs,
+                                const rp_opts* opts, rp_batch** batch);
 int rp_batch_run(rp_batch* batch);                 /* async on the ctx stream */
 int rp_batch_sync(rp_batch* batch);
 int rp_batch_fetch_dense(rp_batch* batch, float* out, size_t out_floats);

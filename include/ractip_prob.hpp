@@ -76,6 +76,26 @@ class ProbabilityStage {
     out = std::move(res[0]);
   }
 
+  // The same under structure constraints c1 over s1, c2 over s2 (RactIP -c: the FASTA records' structure lines in
+  // the alphabet .x()[] of rp_constraint; an empty string leaves its sequence unconstrained).  One context only.
+  void solve_probabilities(const std::string& s1, const std::string& s2, const std::string& c1, const std::string& c2,
+                           PairProbabilities& out) {
+    if (!ctx_) throw std::runtime_error("ractip_prob: constrained problems run on a single-device stage");
+    rp_pair pair = {s1.data(), static_cast<int>(s1.size()), s2.data(), static_cast<int>(s2.size())};
+    rp_constraint con = {c1.empty() ? nullptr : c1.c_str(), c2.empty() ? nullptr : c2.c_str()};
+    rp_dense_layout lay;
+    size_t total = 0;
+    check(rp_dense_plan(&pair, 1, &opts_, &lay, &total), ctx_);
+    std::vector<float> flat(total ? total : 1);
+    rp_batch* b = nullptr;
+    check(rp_batch_create_constrained(ctx_, &pair, &con, 1, &opts_, &b), ctx_);
+    int rc = rp_batch_run(b);
+    if (!rc) rc = rp_batch_fetch_dense(b, flat.data(), flat.size());
+    rp_batch_destroy(b);
+    check(rc, ctx_);
+    unpack(pair, lay, flat.data(), out);
+  }
+
   // the same for a whole batch (the shuffles of src/ractip.cpp:1638-1657) in one call
   void solve_batch(const std::vector<std::pair<std::string, std::string> >& seqs, std::vector<PairProbabilities>& out) {
     const int n = static_cast<int>(seqs.size());
@@ -97,16 +117,7 @@ class ProbabilityStage {
       check(rp_run_dense(ctx_, pairs.data(), n, &opts_, flat.data(), flat.size()), ctx_);
     }
     out.assign(n, PairProbabilities());
-    const int w = opts_.max_w > 0 ? opts_.max_w : 0;
-    for (int k = 0; k < n; k++) {
-      const rp_dense_layout& L = lay[k];
-      PairProbabilities& r = out[k];
-      fill_bp(flat.data() + L.bp1, pairs[k].n1, r.bp1, r.offset1);
-      fill_bp(flat.data() + L.bp2, pairs[k].n2, r.bp2, r.offset2);
-      fill_rows(flat.data() + L.up1, pairs[k].n1, w, r.up1);
-      fill_rows(flat.data() + L.up2, pairs[k].n2, w, r.up2);
-      fill_rows(flat.data() + L.hp, pairs[k].n1 + 1, pairs[k].n2 + 1, r.hp);
-    }
+    for (int k = 0; k < n; k++) unpack(pairs[k], lay[k], flat.data(), out[k]);
   }
 
   // RactIP::rnafold(fa, bp, offset, up, max_w), src/ractip.cpp:308-382: a pair with an empty second
@@ -132,6 +143,15 @@ class ProbabilityStage {
  private:
   static void check(int rc, rp_ctx* ctx) {
     if (rc) throw std::runtime_error(std::string("ractip_prob: ") + rp_strerror(rc) + " -- " + rp_last_error(ctx));
+  }
+  // one pair's sections of a dense output buffer
+  void unpack(const rp_pair& p, const rp_dense_layout& L, const float* flat, PairProbabilities& r) const {
+    const int w = opts_.max_w > 0 ? opts_.max_w : 0;
+    fill_bp(flat + L.bp1, p.n1, r.bp1, r.offset1);
+    fill_bp(flat + L.bp2, p.n2, r.bp2, r.offset2);
+    fill_rows(flat + L.up1, p.n1, w, r.up1);
+    fill_rows(flat + L.up2, p.n2, w, r.up2);
+    fill_rows(flat + L.hp, p.n1 + 1, p.n2 + 1, r.hp);
   }
   static void fill_bp(const float* src, int L, VF& bp, VI& offset) {
     bp.assign(src, src + static_cast<size_t>(L + 1) * (L + 2) / 2);

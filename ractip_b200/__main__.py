@@ -2,9 +2,11 @@
 import argparse
 import sys
 
-from .frontend import format_result, input_pairs, predict
+from .frontend import constraint_line, format_result, input_pairs, predict
 from .ip import default_ip_opts
-from .stage import ProbabilityStage, default_opts
+from .stage import ProbabilityStage, RpError, default_opts
+
+RP_ERR_ARG = 1
 
 
 def main(argv=None) -> int:
@@ -25,6 +27,8 @@ def main(argv=None) -> int:
     ap.add_argument("--seed", type=int, default=1)
     ap.add_argument("--allow-isolated", action="store_true")
     ap.add_argument("-e", "--show-energy", action="store_true")
+    ap.add_argument("-c", "--use-constraint", action="store_true",
+                    help="constrain the probabilities by the records' structure lines (.x()[]; ? and space as .)")
     ap.add_argument("-P", "--param-file", default=None)
     ap.add_argument("--no-pk", action="store_true")
     ap.add_argument("--duplex", action="store_true")
@@ -36,6 +40,9 @@ def main(argv=None) -> int:
         ap.error("at most two FASTA files")
     try:
         pairs = input_pairs(args.fasta[0], args.fasta[1] if len(args.fasta) > 1 else None, args.all_pairs)
+        if args.use_constraint:
+            for a, b in pairs:
+                constraint_line(a), constraint_line(b)
     except ValueError as e:   # the reference prints the message and exits 1 (src/ractip.cpp:1684-1697)
         print(e)
         return 1
@@ -48,8 +55,14 @@ def main(argv=None) -> int:
                           stacking=int(not args.allow_isolated))
     stage = ProbabilityStage(device=args.device, use_bl=not args.no_bl, param_file=args.param_file)
     try:
-        for r in predict(stage, pairs, opts, ipo, args.show_energy, args.zscore, args.num_shuffling, args.seed):
+        for r in predict(stage, pairs, opts, ipo, args.show_energy, args.zscore, args.num_shuffling, args.seed,
+                         use_constraint=args.use_constraint):
             print(format_result(r, args.show_energy))
+    except RpError as e:
+        if not (args.use_constraint and e.code == RP_ERR_ARG):
+            raise
+        print(e)   # a malformed structure line is an input error like the others
+        return 1
     finally:
         stage.close()
     return 0

@@ -57,6 +57,10 @@ class RpPair(C.Structure):
     _fields_ = [("s1", C.c_char_p), ("n1", C.c_int), ("s2", C.c_char_p), ("n2", C.c_int)]
 
 
+class RpConstraint(C.Structure):
+    _fields_ = [("c1", C.c_char_p), ("c2", C.c_char_p)]
+
+
 class RpOpts(C.Structure):
     _fields_ = [("max_w", C.c_int), ("min_w", C.c_int), ("th_ss", C.c_float), ("th_hy", C.c_float),
                 ("th_ac", C.c_float), ("use_pf_duplex", C.c_int)]
@@ -104,7 +108,7 @@ EXPORTS = [
     "rp_model_default", "rp_model_read_par", "rp_model_digest", "rp_opts_default",
     "rp_dense_plan", "rp_sparse_plan", "rp_create", "rp_destroy", "rp_last_error",
     "rp_strerror", "rp_set_stream", "rp_get_stream", "rp_host_alloc", "rp_host_free", "rp_run_dense",
-    "rp_run_sparse", "rp_batch_create", "rp_batch_run", "rp_batch_sync",
+    "rp_run_sparse", "rp_batch_create", "rp_batch_create_constrained", "rp_batch_run", "rp_batch_sync",
     "rp_batch_fetch_dense", "rp_batch_fetch_sparse", "rp_batch_sparse_device", "rp_batch_dense_device",
     "rp_square_plan", "rp_batch_square_device", "rp_batch_fetch_logz",
     "rp_batch_destroy", "rp_last_timing", "rp_measure_peaks", "rp_zscore_shuffles",
@@ -153,6 +157,7 @@ def load() -> C.CDLL:
         "rp_run_dense": (i, [vp, P(RpPair), i, P(RpOpts), vp, sz]),
         "rp_run_sparse": (i, [vp, P(RpPair), i, P(RpOpts), vp, sz, vp, sz, vp]),
         "rp_batch_create": (i, [vp, P(RpPair), i, P(RpOpts), P(vp)]),
+        "rp_batch_create_constrained": (i, [vp, P(RpPair), P(RpConstraint), i, P(RpOpts), P(vp)]),
         "rp_batch_run": (i, [vp]),
         "rp_batch_sync": (i, [vp]),
         "rp_batch_fetch_dense": (i, [vp, vp, sz]),

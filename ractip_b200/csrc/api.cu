@@ -71,6 +71,7 @@ struct rp_batch {
   rp::BatchPlan plan;
   // device
   uint8_t* d_seq = nullptr;
+  uint16_t* d_key = nullptr;  // structure-constraint keys (BatchPlan::key), null when no problem is constrained
   Problem* d_probs = nullptr;
   int* d_order = nullptr;
   int* d_counter = nullptr;
@@ -353,7 +354,7 @@ int rp_batch_destroy(rp_batch* b) {
   }
   if (b->ctx) {
     rp_ctx* ctx = b->ctx;
-    for (void* p : {(void*)b->d_seq, (void*)b->d_probs, (void*)b->d_order, (void*)b->d_counter, (void*)b->d_dense,
+    for (void* p : {(void*)b->d_seq, (void*)b->d_key, (void*)b->d_probs, (void*)b->d_order, (void*)b->d_counter, (void*)b->d_dense,
                     (void*)b->d_logz, (void*)b->d_done, (void*)b->d_spairs, (void*)b->d_recs, (void*)b->d_ups, (void*)b->d_counts})
       pool_release(ctx, p);
     ctx->live_batches--;
@@ -366,7 +367,11 @@ int rp_batch_destroy(rp_batch* b) {
   return RP_OK;
 }
 
-int rp_batch_create(rp_ctx* ctx, const rp_pair* pairs, int n_pairs, const rp_opts* opts, rp_batch** out) {
+}  // extern "C"
+
+namespace {
+int batch_create(rp_ctx* ctx, const rp_pair* pairs, const rp_constraint* cons, int n_pairs, const rp_opts* opts,
+                 rp_batch** out) {
   if (!ctx || !out) return fail(ctx, RP_ERR_ARG, "rp_batch_create: null argument");
   *out = nullptr;
   int rc = rp::check_pairs(pairs, n_pairs, opts);
@@ -374,6 +379,8 @@ int rp_batch_create(rp_ctx* ctx, const rp_pair* pairs, int n_pairs, const rp_opt
   for (int p = 0; p < n_pairs; p++)
     if ((long long)pairs[p].n1 + pairs[p].n2 > rp::RP_MAX_N)
       return fail(ctx, RP_ERR_TOO_LONG, "rp_batch_create: n1+n2 exceeds the 32-bit workspace indexing limit (12000 nt)");
+  std::string msg;
+  if ((rc = rp::check_constraints(pairs, cons, n_pairs, &msg)) != RP_OK) return fail(ctx, rc, "rp_batch_create_constrained: " + msg);
   CU(cudaSetDevice(ctx->device));
   rp_batch* b = new rp_batch;
   b->ctx = ctx;
@@ -382,7 +389,7 @@ int rp_batch_create(rp_ctx* ctx, const rp_pair* pairs, int n_pairs, const rp_opt
   b->opts = *opts;
   b->slayout.resize(n_pairs);
   rp_sparse_plan(pairs, n_pairs, opts, b->slayout.data(), &b->total_recs, &b->total_upf);
-  if (rp::plan_batch(pairs, n_pairs, opts, device_facts(ctx), ctx->route, &b->plan) != RP_OK) {
+  if (rp::plan_batch(pairs, n_pairs, opts, device_facts(ctx), ctx->route, &b->plan, cons) != RP_OK) {
     rp_batch_destroy(b);
     return fail(ctx, RP_ERR_CUDA, "rp_batch_create: band kernel does not fit on this device");
   }
@@ -403,6 +410,11 @@ int rp_batch_create(rp_ctx* ctx, const rp_pair* pairs, int n_pairs, const rp_opt
   if ((e = pool_alloc(ctx, &b->d_logz, std::max<size_t>(1, (size_t)n_pairs * 3) * sizeof(double))) != cudaSuccess) return bail(e, "cudaMalloc logz");
   cudaStream_t st = ctx->stream;
   if ((e = cudaMemcpyAsync(b->d_seq, p.seq.data(), p.seq.size(), cudaMemcpyHostToDevice, st)) != cudaSuccess) return bail(e, "H2D seq");
+  if (!p.key.empty()) {   // only batches with a constrained problem carry keys
+    const size_t kb = p.key.size() * sizeof(uint16_t);
+    if ((e = pool_alloc(ctx, &b->d_key, kb)) != cudaSuccess) return bail(e, "cudaMalloc key");
+    if ((e = cudaMemcpyAsync(b->d_key, p.key.data(), kb, cudaMemcpyHostToDevice, st)) != cudaSuccess) return bail(e, "H2D key");
+  }
   if (np) {
     if ((e = cudaMemcpyAsync(b->d_probs, p.probs.data(), np * sizeof(Problem), cudaMemcpyHostToDevice, st)) != cudaSuccess) return bail(e, "H2D probs");
     if (!p.order.empty() && (e = cudaMemcpyAsync(b->d_order, p.order.data(), p.order.size() * sizeof(int), cudaMemcpyHostToDevice, st)) != cudaSuccess) return bail(e, "H2D order");
@@ -411,8 +423,21 @@ int rp_batch_create(rp_ctx* ctx, const rp_pair* pairs, int n_pairs, const rp_opt
   if ((e = cudaMemsetAsync(b->d_logz, 0, std::max<size_t>(1, (size_t)n_pairs * 3) * sizeof(double), st)) != cudaSuccess) return bail(e, "memset logz");
   if ((e = cudaStreamSynchronize(st)) != cudaSuccess) return bail(e, "sync");  // the host copies are complete
   std::vector<uint8_t>().swap(p.seq);   // the sequences live on the device from here
+  std::vector<uint16_t>().swap(p.key);
   *out = b;
   return RP_OK;
+}
+}  // namespace
+
+extern "C" {
+
+int rp_batch_create(rp_ctx* ctx, const rp_pair* pairs, int n_pairs, const rp_opts* opts, rp_batch** out) {
+  return batch_create(ctx, pairs, nullptr, n_pairs, opts, out);
+}
+
+int rp_batch_create_constrained(rp_ctx* ctx, const rp_pair* pairs, const rp_constraint* cons, int n_pairs,
+                                const rp_opts* opts, rp_batch** out) {
+  return batch_create(ctx, pairs, cons, n_pairs, opts, out);
 }
 
 int rp_batch_run(rp_batch* b) {
@@ -428,7 +453,7 @@ int rp_batch_run(rp_batch* b) {
   if (rc) return rc;
   const int n_bandall = p.n_band[0] + p.n_band[1];
   rp::BatchDev d;
-  d.model = ctx->d_model; d.seq = b->d_seq; d.probs = b->d_probs; d.order = b->d_order + n_bandall; d.nprob = p.n_general;
+  d.model = ctx->d_model; d.seq = b->d_seq; d.key = b->d_key; d.probs = b->d_probs; d.order = b->d_order + n_bandall; d.nprob = p.n_general;
   d.counter = b->d_counter; d.ws = ctx->ws; d.slot_stride = p.slot_doubles; d.nslots = std::max(p.grid, 1);
   d.dense = b->d_dense; d.logz = b->d_logz;
   d.ws_up = ctx->ws + p.ws_up; d.done = b->d_done;

@@ -60,7 +60,9 @@ using CtaExec = CtaExecT<>;
 // as many problem histories compete for the L2).
 // <1, W> with W > BAND sums the split sums in wide bands (solve_mcc_wide): W-fold reuse of every element
 // streamed from HBM.
-template <int MINB, int W>
+// KEYS: the batch has structure-constrained problems (BatchDev::key).  The instances without compile the constraint
+// out (Ctx::key stays null), so that unconstrained batches run exactly the code they ran before constraints existed.
+template <int MINB, int W, bool KEYS>
 __global__ void __launch_bounds__(RP_MCC_THREADS, MINB) mcc_persistent(BatchDev b) {
   extern __shared__ double smem_raw[];
   __shared__ int s_next;
@@ -78,6 +80,7 @@ __global__ void __launch_bounds__(RP_MCC_THREADS, MINB) mcc_persistent(BatchDev 
     if (p.kind == KIND_DUPLEX) continue;  // handled by duplex_kernel
     Ctx c;
     bind_ctx(c, b.model, b.seq + p.seq_off - 1, p, b.ws + (size_t)blockIdx.x * b.slot_stride);
+    if (KEYS && p.constrained) c.key = b.key + p.seq_off - 1;
     c.dbg = b.dbg;
     if (W > BAND) solve_mcc_wide(ex, c, p, b.dense, b.logz, sh);
     else solve_mcc(ex, c, p, b.dense, b.logz, sh);
@@ -88,7 +91,7 @@ __global__ void __launch_bounds__(RP_MCC_THREADS, MINB) mcc_persistent(BatchDev 
 // pair rather than a shuffle batch).  A cluster of G CTAs works on one problem (solve_mcc_wide); clusters
 // pull problems from the same cost-ordered queue, one workspace slot each.  G = 16 (beyond the portable
 // cluster size, opted in at launch) when there are at most sm_count/16 problems, else 8.
-template <int W, int G>
+template <int W, int G, bool KEYS>
 __global__ void __cluster_dims__(G, 1, 1) __launch_bounds__(RP_MCC_THREADS, 1) mcc_cluster_kernel(BatchDev b) {
   namespace cg = cooperative_groups;
   extern __shared__ double smem_raw[];
@@ -109,6 +112,7 @@ __global__ void __cluster_dims__(G, 1, 1) __launch_bounds__(RP_MCC_THREADS, 1) m
     if (p.kind == KIND_DUPLEX) continue;
     Ctx c;
     bind_ctx(c, b.model, b.seq + p.seq_off - 1, p, b.ws + (size_t)cid * b.slot_stride);
+    if (KEYS && p.constrained) c.key = b.key + p.seq_off - 1;
     c.dbg = b.dbg;
     solve_mcc_wide(ex, c, p, b.dense, b.logz, sh);
   }
@@ -561,16 +565,16 @@ __global__ void __launch_bounds__(256) peak_smem_kernel(double* out, int iters) 
 namespace {
 using MccKernel = void (*)(BatchDev);
 // minb = 2: 64-register build, BAND-wide sums; minb = 1: 128 registers, bands of 10 diagonals
-MccKernel mcc_kernel(int minb, int* w_out) {
-  if (minb >= 2) { *w_out = BAND; return mcc_persistent<RP_MCC_MIN_CTAS, BAND>; }
+MccKernel mcc_kernel(int minb, bool keys, int* w_out) {
+  if (minb >= 2) { *w_out = BAND; return keys ? mcc_persistent<RP_MCC_MIN_CTAS, BAND, true> : mcc_persistent<RP_MCC_MIN_CTAS, BAND, false>; }
   *w_out = 10;
-  return mcc_persistent<1, 10>;
+  return keys ? mcc_persistent<1, 10, true> : mcc_persistent<1, 10, false>;
 }
 }  // namespace
 
 int mcc_max_ctas_per_sm(int minb) {
   int n = 0, w = BAND;
-  MccKernel k = mcc_kernel(minb, &w);
+  MccKernel k = mcc_kernel(minb, false, &w);
   size_t smem = shared_bytes(RP_MCC_THREADS, w);
   if (cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess) { cudaGetLastError(); return 0; }
   if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, k, RP_MCC_THREADS, smem) != cudaSuccess) return 0;
@@ -579,7 +583,7 @@ int mcc_max_ctas_per_sm(int minb) {
 
 cudaError_t launch_mcc(const BatchDev& b, int grid, int minb, cudaStream_t st) {
   int w = BAND;
-  MccKernel k = mcc_kernel(minb, &w);
+  MccKernel k = mcc_kernel(minb, b.key != nullptr, &w);
   size_t smem = shared_bytes(RP_MCC_THREADS, w);
   cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
   k<<<grid, RP_MCC_THREADS, smem, st>>>(b);
@@ -588,7 +592,8 @@ cudaError_t launch_mcc(const BatchDev& b, int grid, int minb, cudaStream_t st) {
 
 cudaError_t launch_mcc_cluster(const BatchDev& b, int nclusters, int ctas, cudaStream_t st) {
   size_t smem = shared_bytes(RP_MCC_THREADS, 10);
-  MccKernel k = ctas >= 16 ? mcc_cluster_kernel<10, 16> : mcc_cluster_kernel<10, 8>;
+  MccKernel k = ctas >= 16 ? (b.key ? mcc_cluster_kernel<10, 16, true> : mcc_cluster_kernel<10, 16, false>)
+                           : (b.key ? mcc_cluster_kernel<10, 8, true> : mcc_cluster_kernel<10, 8, false>);
   const int G = ctas >= 16 ? 16 : 8;
   cudaError_t e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
   if (e != cudaSuccess) return e;

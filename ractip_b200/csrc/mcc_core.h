@@ -58,6 +58,7 @@ struct Problem {
   int which;          // 0: s1, 1: s2, 2: s1&s2
   int max_w;
   int n1, n2;
+  int constrained;    // 1: a structure constraint removes some pairs (BatchDev::key); general kernel only
   long long out_bp;   // float offsets into the dense output, -1 if absent
   long long out_up;
   long long out_hp;
@@ -102,6 +103,7 @@ struct Ctx {
   double invZ;        // set after the inside pass
   int dbg;            // tuning aid (RP_DEBUG_SKIP): 1 skip interior rows, 2 skip split sums, 4 skip gap sums
   long long* prof;    // RP_PROFILE counters (slots 40..: fine-grained probes of thread 0) or null
+  const uint16_t* key;   // key[1..n] of a constrained problem (pair (i,j) allowed iff key[i] == key[j]), else null
   // Tables whose rows are only read while they are recent are RINGS of a few rows (row d at d & mask):
   // PR/PL/PMLB are read one diagonal after they are written, the band results QS/PRB/MLB within a
   // band.  A full table would leave every written line behind in L2, where it pushes out the history
@@ -130,6 +132,7 @@ RP_HD void bind_ctx(Ctx& c, const DevModel* M, const uint8_t* S, const Problem& 
   c.invZ = 0;
   c.dbg = 0;
   c.prof = nullptr;
+  c.key = nullptr;
 }
 #define TB(c, t, d, i) ((c).tb(t, d, i))
 // store of a value that is not read again soon (qb, out, class tables, outputs): evict-first, so that
@@ -213,6 +216,14 @@ RP_HD int pair_type(int a, int b) {
   return (a && b) ? t : 0;
 }
 RP_HD int rtype(int t) { return t == 0 ? 0 : (t == 7 ? 7 : ((t - 1) ^ 1) + 1); }
+// Pair type of cell (i,j) in the general kernel: 0 also when the problem's structure constraint removes the pair.
+// Every decision of the general kernel on whether a cell or an enclosing pair can pair goes through here; type 0
+// leaves qb, the outside value and the class tables of the cell at 0, so nothing of a removed pair reaches other
+// cells or the unpaired-window pass.  (The band kernel runs unconstrained problems only and calls pair_type.)
+RP_HD int cell_type(const Ctx& c, int i, int j) {
+  const int t = pair_type(c.sraw(i) & 7, c.sraw(j) & 7);
+  return (c.key && c.key[i] != c.key[j]) ? 0 : t;
+}
 
 // ViennaRNA SAME_STRAND(a,b) for a<b
 template <class C>
@@ -515,7 +526,7 @@ RP_HD void prologue_lists(Ctx& c, int tid, int T) {
     int cnt = 0;
     for (int i = 1; i <= n - d; i++) {
       P[i] = (uint16_t)cnt;
-      if (d > TURN && pair_type(base(c, i), base(c, i + d))) L[cnt++] = (uint16_t)i;
+      if (d > TURN && cell_type(c, i, i + d)) L[cnt++] = (uint16_t)i;
     }
     P[n - d + 1 <= n ? n - d + 1 : n] = (uint16_t)cnt;  // d = 0: i = n+1 does not exist and is never asked for
     if (d == 0) P[n] = 0;
@@ -603,7 +614,7 @@ RP_HD double inside_interior(const C& c, const Shared& sh, int d, int i, int typ
     const int dd = u1 + u2 + 2;
     if (dd > ddmax || u1 + 1 > maxpo || u2 > maxu2) continue;
     const int k = i + 1 + u1, l = j - 1 - u2;
-    const int t2 = pair_type(base(c, k), base(c, l));
+    const int t2 = cell_type(c, k, l);
     if (!t2) continue;
     accI += TB(c, T_QB, d - dd, k) * special_loop(M, s, type, rtype(t2), si1, sj1, base(c, k - 1), base(c, l + 1));
   }
@@ -768,7 +779,7 @@ RP_HD void inside_A(const Ctx& c, const Shared& sh, int d, int i0, int C, int ti
   const int r = tid % is.cntp, sl = tid / is.cntp;
   if (sl < is.SI && r < is.cnt) {
     const int i = listp(c)[(size_t)d * c.ld + is.lo + r];
-    sh.part[tid] = inside_interior(c, sh, d, i, pair_type(base(c, i), base(c, i + d)), sl, is.SI);
+    sh.part[tid] = inside_interior(c, sh, d, i, cell_type(c, i, i + d), sl, is.SI);
   }
 }
 // per diagonal, phase B: one thread per cell
@@ -782,7 +793,7 @@ RP_HD void inside_B(Ctx& c, const Shared& sh, int d, int i0, int C, int tid) {
   // the terms of the q-split that the band pass could not see yet: a < e, qq on diagonals >= d0
   const int e = d - band_start_inside(d);
   for (int a = 0; a < e && a <= d - TURN - 2; a++) sQ += TB(c, T_Q, a, i) * TB(c, T_QQ, d - 1 - a, i + 1 + a);
-  const int type = pair_type(base(c, i), base(c, i + d));
+  const int type = cell_type(c, i, i + d);
   if (type && d - (TURN + 1) >= 2) {
     const ISplit is = make_isplit(c, d, i0, C, T);
     const int r = (int)posp(c)[(size_t)d * c.ld + i] - is.lo;
@@ -811,7 +822,7 @@ RP_HD double outside_interior(const C& c, const Shared& sh, int d, int k, int sl
     if (l < c.cp && c.cp - 2 - l < maxu2) maxu2 = c.cp - 2 - l;  // j must stay on l's strand
   }
   if (maxpo < 1 || maxu2 < 0 || TB(c, T_QB, d, k) == 0.) return 0.;
-  const int type = pair_type(base(c, k), base(c, l));
+  const int type = cell_type(c, k, l);
   const int t2 = rtype(type), sp1 = base(c, k - 1), sq1 = base(c, l + 1);
   int u1max = ddmax - 2 < MAXLOOP ? ddmax - 2 : MAXLOOP;
   if (maxpo - 1 < u1max) u1max = maxpo - 1;
@@ -826,7 +837,7 @@ RP_HD double outside_interior(const C& c, const Shared& sh, int d, int k, int sl
     const int dd = u1 + u2 + 2;
     if (dd > ddmax || u1 + 1 > maxpo || u2 > maxu2) continue;
     const int i = k - 1 - u1, j = l + 1 + u2;
-    const int t1 = pair_type(base(c, i), base(c, j));
+    const int t1 = cell_type(c, i, j);
     if (!t1) continue;
     const double o = TB(c, T_OUT, d + dd, i);
     if (o == 0.) continue;
@@ -944,7 +955,7 @@ RP_HD void outside_band_A(const Ctx& c, const Shared& sh, int d0, int r0, int C,
         unsigned need = 0;
         for (int e = 0; e < BAND; e++) {
           const int k = k0 + e, d = d0 - e;
-          if (k > 2 && d > TURN && pair_type(base(c, k), base(c, l)) && TB(c, T_QB, d, k) != 0.) need |= 1u << e;
+          if (k > 2 && d > TURN && cell_type(c, k, l) && TB(c, T_QB, d, k) != 0.) need |= 1u << e;
         }
         if (need) {
           const int imax = k0 + (BAND - 1) - TURN - 3, imain = k0 - TURN - 3;
@@ -1014,7 +1025,7 @@ RP_HD void outside_B(Ctx& c, const Shared& sh, int d, int i0, int C, int tid) {
   const int k = i0 + tid;
   double sI = 0.;
   const double sP = TB(c, T_PRB, d, k), sL = TB(c, T_MLB, d, k);
-  const int type = pair_type(base(c, k), base(c, k + d));
+  const int type = cell_type(c, k, k + d);
   if (type && c.n - 1 - d >= 2 && TB(c, T_QB, d, k) != 0.) {
     const ISplit is = make_isplit(c, d, i0, C, T);
     const int r = (int)posp(c)[(size_t)d * c.ld + k] - is.lo;
@@ -1153,7 +1164,7 @@ RP_HD void wide_outside_A(const Ctx& c, const Shared& sh, int d0, int r0, int C,
         unsigned need = 0;
         for (int e = 0; e < W; e++) {
           const int k = k0 + e, d = d0 - e;
-          if (k > 2 && d > TURN && pair_type(base(c, k), base(c, l)) && TB(c, T_QB, d, k) != 0.) need |= 1u << e;
+          if (k > 2 && d > TURN && cell_type(c, k, l) && TB(c, T_QB, d, k) != 0.) need |= 1u << e;
         }
         if (need) {
           const int ifar = k0 - 2;
@@ -1277,7 +1288,7 @@ RP_HD double inside_ends_item(const Ctx& c, const Shared& sh, int d, int i, int 
   const DevModel& M = *c.M;
   const int ddmax = d - (TURN + 1) < MAXLOOP + 2 ? d - (TURN + 1) : MAXLOOP + 2;
   if (ddmax < 2) return 0.;
-  const int j = i + d, type = pair_type(base(c, i), base(c, j));
+  const int j = i + d, type = cell_type(c, i, j);
   const int maxpo = (c.cp > 0 && i < c.cp) ? c.cp - 1 - i : 1000;
   const int maxu2 = (c.cp > 0 && j >= c.cp) ? j - 1 - c.cp : 1000;
   const int si1 = base(c, i + 1), sj1 = base(c, j - 1);
@@ -1297,7 +1308,7 @@ RP_HD double inside_ends_item(const Ctx& c, const Shared& sh, int d, int i, int 
     const int dd = u1 + u2 + 2;
     const bool ok = dd <= ddmax && u1 + 1 <= maxpo && u2 <= maxu2;
     const int k = i + 1 + u1, l = j - 1 - u2;
-    t2v[s] = ok ? pair_type(base(c, k), base(c, l)) : 0;
+    t2v[s] = ok ? cell_type(c, k, l) : 0;
     qv[s] = t2v[s] ? TB(c, T_QB, d - dd, k) : 0.;
   }
   double acc = 0.;
@@ -1322,7 +1333,7 @@ RP_HD double outside_ends_item(const Ctx& c, const Shared& sh, int d, int k, int
     if (l < c.cp && c.cp - 2 - l < maxu2) maxu2 = c.cp - 2 - l;
   }
   if (maxpo < 1 || maxu2 < 0 || TB(c, T_QB, d, k) == 0.) return 0.;
-  const int type = pair_type(base(c, k), base(c, l));
+  const int type = cell_type(c, k, l);
   const int t2 = rtype(type), sp1 = base(c, k - 1), sq1 = base(c, l + 1);
   if (kind < 4) {
     int u1max = ddmax - 2 < MAXLOOP ? ddmax - 2 : MAXLOOP;
@@ -1339,7 +1350,7 @@ RP_HD double outside_ends_item(const Ctx& c, const Shared& sh, int d, int k, int
     const int dd = u1 + u2 + 2;
     const bool ok = dd <= ddmax && u1 + 1 <= maxpo && u2 <= maxu2;
     const int i = k - 1 - u1, j = l + 1 + u2;
-    t1v[s] = ok ? pair_type(base(c, i), base(c, j)) : 0;
+    t1v[s] = ok ? cell_type(c, i, j) : 0;
     ov[s] = t1v[s] ? TB(c, T_OUT, d + dd, i) : 0.;
   }
   double acc = 0.;
@@ -1374,7 +1385,7 @@ RP_HD void wide_inside_finish(Ctx& c, const Shared& sh, int d, int i0, int C, in
   double sI = 0.;
   double sM = TB(c, T_QM2, d, i), sQ = TB(c, T_QS, d, i);
   inside_near<W>(c, d, i, sM, sQ);
-  const int type = pair_type(base(c, i), base(c, i + d));
+  const int type = cell_type(c, i, i + d);
   if (type && d - (TURN + 1) >= 2) {
     const ISplit is = make_isplit(c, d, i0, C, T);
     const int r = (int)posp(c)[(size_t)d * c.ld + i] - is.lo;
@@ -1402,7 +1413,7 @@ RP_HD void wide_outside_finish(Ctx& c, const Shared& sh, int d, int i0, int C, i
   const int k = i0 + tid, l = k + d;
   double sI = 0.;
   double sP = TB(c, T_PRB, d, k), sL = TB(c, T_MLB, d, k);
-  const int type = pair_type(base(c, k), base(c, l));
+  const int type = cell_type(c, k, l);
   const bool pairs = type && TB(c, T_QB, d, k) != 0.;
   outside_near<W>(c, d, k, pairs && k > 2 && l < c.n, sP, sL);
   if (pairs && c.n - 1 - d >= 2) {

@@ -201,7 +201,7 @@ __device__ __forceinline__ void wide_outside_A_shfl(const Ctx& c, const Shared& 
 #pragma unroll
       for (int e = 0; e < W; e++) {
         const int k = k0 + e, d = d0 - e;
-        cand[e] = k > 2 && d > TURN && pair_type(base(c, k), base(c, l)) != 0 && (c.cp <= 0 || (k < c.cp && l >= c.cp));
+        cand[e] = k > 2 && d > TURN && cell_type(c, k, l) != 0 && (c.cp <= 0 || (k < c.cp && l >= c.cp));
         qbv[e] = cand[e] ? TB(c, T_QB, d, k) : 0.;
       }
 #pragma unroll

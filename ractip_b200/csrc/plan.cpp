@@ -2,7 +2,9 @@
 #include "plan.h"
 
 #include <algorithm>
+#include <cctype>
 #include <cmath>
+#include <cstdio>
 #include <cstring>
 
 #include "mcc_band.h"
@@ -18,6 +20,111 @@ int check_pairs(const rp_pair* pairs, int n_pairs, const rp_opts* opts) {
     if (!pairs[p].s1 || pairs[p].n1 < 1 || pairs[p].n2 < 0 || (pairs[p].n2 > 0 && !pairs[p].s2)) return RP_ERR_ARG;   // n2 == 0: s1 alone
   return RP_OK;
 }
+
+// Structure constraints: c1 over s1, c2 over s2, in the alphabet of RactIP's joint structures --
+//   .  no constraint      x  the base pairs with nothing
+//   ( )  an intramolecular pair, bracket-matched within its string
+//   [ (c1 only), ] (c2 only)  an intermolecular pair: the k-th '[' from the 3' end of s1 pairs with the k-th ']' from
+//        the 5' end of s2 (nested, as RactIP's joint structures are)
+// A constraint only removes pairs.  Each of a pair's problems sees the brackets of its own kind and keeps unpaired
+// the bases the other kind pairs (a base paired on the other strand has no partner in its own strand's problem; a
+// base paired within its strand forms no intermolecular pair):
+//   s1:     bracket pairs () of c1,   unpaired x [
+//   s2:     bracket pairs () of c2,   unpaired x ]
+//   s1&s2:  bracket pairs [] across,  unpaired x ( )
+// Pair (i,j) of a problem is allowed when neither base is unpaired, either base is bracketed only if they are each
+// other's partner, and (i,j) crosses no bracket pair.
+int check_constraints(const rp_pair* pairs, const rp_constraint* cons, int n_pairs, std::string* msg) {
+  if (!cons) return RP_OK;
+  char buf[200];
+  auto bad = [&](int p, int s, int pos, const char* what) {
+    std::snprintf(buf, sizeof buf, "pair %d, c%d, position %d: %s", p, s + 1, pos, what);
+    if (msg) *msg = buf;
+    return RP_ERR_ARG;
+  };
+  for (int p = 0; p < n_pairs; p++) {
+    const char* cs[2] = {cons[p].c1, cons[p].c2};
+    const int ns[2] = {pairs[p].n1, pairs[p].n2};
+    std::vector<int> inter[2];   // positions of '[' in c1 / ']' in c2
+    for (int s = 0; s < 2; s++) {
+      const char* c = cs[s];
+      if (!c) continue;
+      const size_t len = strnlen(c, (size_t)ns[s] + 1);
+      if (len != (size_t)ns[s]) {
+        char what[96];
+        std::snprintf(what, sizeof what, "the string is %s than s%d (%d nt)", len < (size_t)ns[s] ? "shorter" : "longer",
+                      s + 1, ns[s]);
+        return bad(p, s, (int)std::min(len, (size_t)ns[s]) + 1, what);
+      }
+      std::vector<int> open;
+      for (int i = 0; i < ns[s]; i++) {
+        switch (c[i]) {
+          case '.': case 'x': break;
+          case '(': open.push_back(i); break;
+          case ')':
+            if (open.empty()) return bad(p, s, i + 1, "')' closes no '('");
+            open.pop_back();
+            break;
+          case '[':
+            if (s == 1) return bad(p, s, i + 1, "'[' (an intermolecular pair's s1 end) may appear in c1 only");
+            inter[s].push_back(i);
+            break;
+          case ']':
+            if (s == 0) return bad(p, s, i + 1, "']' (an intermolecular pair's s2 end) may appear in c2 only");
+            inter[s].push_back(i);
+            break;
+          default: {
+            char what[64];
+            std::snprintf(what, sizeof what, "character '%c' (code %d) is not one of .x()[]", std::isprint((unsigned char)c[i]) ? c[i] : '?',
+                          (unsigned char)c[i]);
+            return bad(p, s, i + 1, what);
+          }
+        }
+      }
+      if (!open.empty()) return bad(p, s, open.back() + 1, "'(' is never closed");
+    }
+    const size_t k1 = inter[0].size(), k2 = inter[1].size();
+    if (k1 > k2) return bad(p, 0, inter[0][k1 - 1 - k2] + 1, "'[' has no partner ']' in c2");
+    if (k2 > k1) return bad(p, 1, inter[1][k1] + 1, "']' has no partner '[' in c1");
+  }
+  return RP_OK;
+}
+
+namespace {
+// Keys of one problem of length m from its bracket pairs: partner[i] = j for the ends of a bracket pair (i,j), 0 for a
+// base left free, -1 for a base kept unpaired (1-based).  Bracket pair number t (from 1, in the order they open) gets
+// 2t+1 at both ends, a free base 2t for the innermost bracket pair around it (0 for none), an unpaired base
+// 0x8000 + i, which no other base carries: then pair (i,j) is allowed iff key[i] == key[j].  n <= RP_MAX_N keeps
+// every key below 2^16.  Returns whether any key differs from 0 (whether the constraint removes any pair).
+bool fill_keys(const std::vector<int>& partner, int m, uint16_t* key) {
+  std::vector<int> open;   // numbers of the bracket pairs around the current base
+  int count = 0;
+  bool any = false;
+  for (int i = 1; i <= m; i++) {
+    const int q = partner[i];
+    int k;
+    if (q < 0) k = 0x8000 + i;
+    else if (q > i) { open.push_back(++count); k = 2 * count + 1; }
+    else if (q > 0) { k = key[q]; open.pop_back(); }
+    else k = open.empty() ? 0 : 2 * open.back();
+    key[i] = (uint16_t)k;
+    any |= k != 0;
+  }
+  return any;
+}
+
+// partners of the ( ) pairs of constraint string c (n bases), the bases of `unpaired` kept unpaired
+void intra_partners(const char* c, int n, const char* unpaired, std::vector<int>& partner) {
+  partner.assign(n + 1, 0);
+  if (!c) return;
+  std::vector<int> open;
+  for (int i = 1; i <= n; i++) {
+    if (c[i - 1] == '(') open.push_back(i);
+    else if (c[i - 1] == ')') { partner[i] = open.back(); partner[open.back()] = i; open.pop_back(); }
+    else if (std::strchr(unpaired, c[i - 1])) partner[i] = -1;
+  }
+}
+}  // namespace
 
 }  // namespace rp
 
@@ -160,7 +267,7 @@ static double alg_flops_mcc_uncached(int n) {
 namespace rp {
 
 int plan_batch(const rp_pair* pairs, int n_pairs, const rp_opts* opts, const DeviceFacts& dev, const RouteSettings& rs,
-               BatchPlan* out) {
+               BatchPlan* out, const rp_constraint* cons) {
   BatchPlan& b = *out;
   b = BatchPlan{};
   size_t mem = 0;   // DeviceFacts::memory, asked once
@@ -176,6 +283,9 @@ int plan_batch(const rp_pair* pairs, int n_pairs, const rp_opts* opts, const Dev
   for (int p = 0; p < n_pairs; p++) bytes += 2 * ((size_t)pairs[p].n1 + pairs[p].n2) + 4;
   std::vector<uint8_t>& seq = b.seq;
   seq.reserve(bytes + 16);
+  std::vector<uint16_t>& key = b.key;   // (filled only for batches with constraints, then dropped if none restricts)
+  bool any_constrained = false;
+  std::vector<int> partner;
   const int w = opts->max_w > 0 ? opts->max_w : 0;
   size_t ws_need = 0;
   for (int p = 0; p < n_pairs; p++) {
@@ -192,6 +302,30 @@ int plan_batch(const rp_pair* pairs, int n_pairs, const rp_opts* opts, const Dev
     for (int i = 0; i < pr.n1; i++) seq.push_back(encode_base(pr.s1[i]));
     for (int i = 0; i < pr.n2; i++) seq.push_back(encode_base(pr.s2[i]));
     seq.push_back(0);
+    int con[3] = {0, 0, 0};   // s1, s2, s1&s2 restricted by the constraint
+    if (cons && (cons[p].c1 || cons[p].c2)) {
+      const char *c1 = cons[p].c1, *c2 = cons[p].c2;
+      key.resize(seq.size(), 0);
+      intra_partners(c1, pr.n1, "x[", partner);
+      con[0] = fill_keys(partner, pr.n1, &key[off1 - 1]);
+      intra_partners(c2, pr.n2, "x]", partner);
+      con[1] = fill_keys(partner, pr.n2, &key[off2 - 1]);
+      // s1&s2: the k-th '[' from the 3' end of c1 with the k-th ']' from the 5' end of c2
+      const int n12 = pr.n1 + pr.n2;
+      partner.assign(n12 + 1, 0);
+      std::vector<int> ends;
+      for (int i = pr.n1; i >= 1; i--)
+        if (c1 && c1[i - 1] == '[') ends.push_back(i);
+      size_t k = 0;
+      for (int j = 1; j <= pr.n2; j++)
+        if (c2 && c2[j - 1] == ']') { partner[ends[k]] = pr.n1 + j; partner[pr.n1 + j] = ends[k]; k++; }
+      for (int i = 1; i <= n12; i++) {
+        const char ch = i <= pr.n1 ? (c1 ? c1[i - 1] : '.') : (c2 ? c2[i - pr.n1 - 1] : '.');
+        if (ch == 'x' || ch == '(' || ch == ')') partner[i] = -1;
+      }
+      con[2] = pr.n2 > 0 && !opts->use_pf_duplex && fill_keys(partner, n12, &key[off12 - 1]);   // --duplex: unconstrained
+      any_constrained |= con[0] || con[1] || con[2];
+    }
     Problem q;
     std::memset(&q, 0, sizeof q);
     q.pair = p; q.max_w = w; q.n1 = pr.n1; q.n2 = pr.n2; q.th_hy = opts->th_hy;
@@ -199,10 +333,10 @@ int plan_batch(const rp_pair* pairs, int n_pairs, const rp_opts* opts, const Dev
     q.ws_off = -1;
     // rnafold(fa1, ...), rnafold(fa2, ...)  src/ractip.cpp:546-547
     Problem a = q;
-    a.kind = KIND_LINEAR; a.which = 0; a.seq_off = off1; a.n = pr.n1; a.cp = 0;
+    a.kind = KIND_LINEAR; a.which = 0; a.seq_off = off1; a.n = pr.n1; a.cp = 0; a.constrained = con[0];
     a.out_bp = (long long)L.bp1; a.out_up = w > 0 ? (long long)L.up1 : -1;
     b.probs.push_back(a);
-    a.which = 1; a.seq_off = off2; a.n = pr.n2;
+    a.which = 1; a.seq_off = off2; a.n = pr.n2; a.constrained = con[1];
     a.out_bp = (long long)L.bp2; a.out_up = w > 0 ? (long long)L.up2 : -1;
     b.probs.push_back(a);
     if (pr.n2 == 0) {   // a lone sequence (RactIP::rnafold on its own, src/ractip.cpp:1599-1601): no second fold, no hybridization
@@ -221,17 +355,19 @@ int plan_batch(const rp_pair* pairs, int n_pairs, const rp_opts* opts, const Dev
       b.n_duplex++;
       ws_need = std::max(ws_need, 2 * (size_t)(pr.n1 + 2) * (size_t)(pr.n2 + 2));
     } else {
-      c.kind = KIND_COFOLD; c.n = pr.n1 + pr.n2; c.cp = pr.n1 + 1;
+      c.kind = KIND_COFOLD; c.n = pr.n1 + pr.n2; c.cp = pr.n1 + 1; c.constrained = con[2];
       b.alg_flops += rp_alg_flops_mcc(c.n);
     }
     b.probs.push_back(c);
     b.alg_flops += rp_alg_flops_mcc(pr.n1) + rp_alg_flops_mcc(pr.n2);
   }
+  if (any_constrained) key.resize(seq.size(), 0);
+  else std::vector<uint16_t>().swap(key);
 
   // Band class of a problem: 0 = L (512 threads, ring needs more than half an SM), 1 = S (256 threads, 2 CTAs/SM),
-  // -1 = the general kernel.
+  // -1 = the general kernel, which alone applies structure constraints.
   auto cls = [&](const Problem& q) {
-    if (!rs.band || q.kind == KIND_DUPLEX) return -1;
+    if (!rs.band || q.kind == KIND_DUPLEX || q.constrained) return -1;
     const int k = rp_kernel_plan(q.n, dev.smem_optin, nullptr);
     return k >= RP_KERNEL_GENERAL ? -1 : k;
   };

@@ -8,6 +8,7 @@
 #include <stdint.h>
 
 #include <functional>
+#include <string>
 #include <utility>
 #include <vector>
 
@@ -45,6 +46,9 @@ struct DeviceFacts {
 
 struct BatchPlan {
   std::vector<uint8_t> seq;              // encoded sequences, per pair  0 s1 0 s2 0 s1s2 0
+  // structure-constraint keys of the constrained problems, laid out like seq (pair (i,j) of a problem is allowed iff
+  // its two bases carry the same key); empty when no problem of the batch is constrained
+  std::vector<uint16_t> key;
   std::vector<Problem> probs;            // three per pair: s1, s2, s1&s2
   std::vector<rp_dense_layout> layout;
   size_t total_floats = 0;
@@ -88,10 +92,14 @@ struct BatchPlan {
 
 size_t bp_len(int L);
 int check_pairs(const rp_pair* pairs, int n_pairs, const rp_opts* opts);
+// The structure constraints of pairs that pass check_pairs (cons may be null: none).  RP_OK, or RP_ERR_ARG with a
+// message in *msg that names the pair, the string and the (1-based) position.
+int check_constraints(const rp_pair* pairs, const rp_constraint* cons, int n_pairs, std::string* msg);
 
-// The pairs must pass check_pairs.  Returns RP_OK, or RP_ERR_CUDA when a band launch shape fits no SM.
+// The pairs must pass check_pairs and the constraints check_constraints (cons == null: none).  A problem that a
+// constraint restricts runs on the general kernel.  Returns RP_OK, or RP_ERR_CUDA when a band launch shape fits no SM.
 int plan_batch(const rp_pair* pairs, int n_pairs, const rp_opts* opts, const DeviceFacts& dev, const RouteSettings& rs,
-               BatchPlan* plan);
+               BatchPlan* plan, const rp_constraint* cons = nullptr);
 
 }  // namespace rp
 #endif

@@ -21,7 +21,7 @@ from typing import Dict, List, Optional, Sequence, Tuple
 import numpy as np
 
 from . import _lib
-from ._lib import (RpDenseLayout, RpModel, RpOpts, RpPair, RpRec, RpSparseCounts,
+from ._lib import (RpConstraint, RpDenseLayout, RpModel, RpOpts, RpPair, RpRec, RpSparseCounts,
                    RpSparseLayout, RpSquareLayout, RpTiming)
 
 
@@ -107,10 +107,25 @@ def _make_pairs(pairs: Sequence[Tuple[str, str]]):
     return arr, keep
 
 
-class DeviceBatch:
-    """A batch whose inputs are resident in HBM (rp_batch_*)."""
+def _make_constraints(constraints: Sequence[Optional[Tuple[Optional[str], Optional[str]]]], n: int):
+    if len(constraints) != n:
+        raise ValueError(f"constraints: {len(constraints)} entries for {n} pairs")
+    arr = (RpConstraint * max(n, 1))()
+    keep = []
+    for k, con in enumerate(constraints):
+        c1, c2 = con if con is not None else (None, None)
+        b1, b2 = (c.encode() if c is not None else None for c in (c1, c2))
+        keep.append((b1, b2))
+        arr[k].c1, arr[k].c2 = b1, b2
+    return arr, keep
 
-    def __init__(self, stage: "ProbabilityStage", pairs: Sequence[Tuple[str, str]], opts: RpOpts):
+
+class DeviceBatch:
+    """A batch whose inputs are resident in HBM (rp_batch_*).  constraints: None, or one (c1, c2) per pair -- the
+    structure constraints of rp_batch_create_constrained, either string (or the whole entry) None for none."""
+
+    def __init__(self, stage: "ProbabilityStage", pairs: Sequence[Tuple[str, str]], opts: RpOpts,
+                 constraints: Optional[Sequence[Optional[Tuple[Optional[str], Optional[str]]]]] = None):
         self.stage, self.lib, self.opts = stage, stage.lib, opts
         self.pairs = list(pairs)
         self.n = len(self.pairs)
@@ -124,7 +139,12 @@ class DeviceBatch:
         stage._check(self.lib.rp_sparse_plan(arr, self.n, C.byref(opts), self.slayout, C.byref(tr), C.byref(tf)))
         self.total_recs, self.total_upf = tr.value, tf.value
         self.handle = C.c_void_p()
-        stage._check(self.lib.rp_batch_create(stage.ctx, arr, self.n, C.byref(opts), C.byref(self.handle)))
+        if constraints is None:
+            stage._check(self.lib.rp_batch_create(stage.ctx, arr, self.n, C.byref(opts), C.byref(self.handle)))
+        else:
+            cons, ckeep = _make_constraints(constraints, self.n)
+            stage._check(self.lib.rp_batch_create_constrained(stage.ctx, arr, cons, self.n, C.byref(opts),
+                                                              C.byref(self.handle)))
 
     def run(self):
         self.stage._check(self.lib.rp_batch_run(self.handle))
@@ -285,14 +305,24 @@ class ProbabilityStage:
             pass
 
     # ------------------------------------------------------------- batches
-    def batch(self, pairs: Sequence[Tuple[str, str]], opts: Optional[RpOpts] = None) -> DeviceBatch:
-        return DeviceBatch(self, pairs, opts if opts is not None else default_opts())
+    def batch(self, pairs: Sequence[Tuple[str, str]], opts: Optional[RpOpts] = None,
+              constraints=None) -> DeviceBatch:
+        """constraints: None, or one (c1, c2) structure-constraint pair per pair (DeviceBatch)."""
+        return DeviceBatch(self, pairs, opts if opts is not None else default_opts(), constraints)
 
     def run_dense(self, pairs: Sequence[Tuple[str, str]], opts: Optional[RpOpts] = None,
-                  pinned: bool = False) -> List[PairProbabilities]:
+                  pinned: bool = False, constraints=None) -> List[PairProbabilities]:
         """rp_run_dense: host buffers in, host buffers out.  pinned=True hands the library a page-locked
-        buffer (rp_host_alloc) as the target of its device-to-host copy."""
+        buffer (rp_host_alloc) as the target of its device-to-host copy.  With constraints (one (c1, c2) per
+        pair, see DeviceBatch) the pairs run as a constrained device batch."""
         opts = opts if opts is not None else default_opts()
+        if constraints is not None:
+            b = self.batch(pairs, opts, constraints)
+            try:
+                b.run()
+                return b.split_dense(b.fetch_dense())
+            finally:
+                b.close()
         arr, keep = _make_pairs(pairs)
         n = len(pairs)
         layout = (RpDenseLayout * max(n, 1))()
@@ -334,9 +364,10 @@ class ProbabilityStage:
         finally:
             b.close()
 
-    def run_sparse(self, pairs: Sequence[Tuple[str, str]], opts: Optional[RpOpts] = None) -> List[PairRecords]:
+    def run_sparse(self, pairs: Sequence[Tuple[str, str]], opts: Optional[RpOpts] = None,
+                   constraints=None) -> List[PairRecords]:
         opts = opts if opts is not None else default_opts()
-        b = self.batch(pairs, opts)
+        b = self.batch(pairs, opts, constraints)
         try:
             b.run()
             return b.split_sparse(*b.fetch_sparse())
