@@ -263,6 +263,44 @@ typedef struct rp_constraint {
 int rp_batch_create_constrained(rp_ctx* ctx, const rp_pair* pairs,
                                 const rp_constraint* cons, int n_pairs,
                                 const rp_opts* opts, rp_batch** batch);
+
+/* Stacking pseudo-energies of one pair (chemical probing data, e.g. SHAPE
+ * reactivities through rp_shape_deigan): e1[0..n1-1] over s1, e2[0..n2-1]
+ * over s2, in kcal/mol; NULL means none.  ViennaRNA's vrna_sc_set_stack
+ * semantics, to which RNAfold --shape (Deigan method) reduces:
+ *   - each value is rounded to an integer number of 0.01 kcal/mol, half away
+ *     from zero: E_i;
+ *   - every stack, an interior loop closed by (i,j) around (i+1,j-1), has its
+ *     Boltzmann weight multiplied by f(i) f(i+1) f(j-1) f(j), where
+ *     f(x) = exp(-E_x * 10 / kT) at the model's kT (37 C);
+ *   - nothing else changes: no other loop (bulges of one base included), no
+ *     pf_scale, no energy of rp_energy_of_structure (-e, z-scores).
+ * s1's fold takes e1, s2's fold e2.  The s1&s2 co-fold applies them to the
+ * stacks within one strand, with that strand's values; a stack that joins the
+ * strands gets no pseudo-energy (data measured on each RNA alone describe its
+ * own structure).  The --duplex branch takes none. */
+typedef struct rp_stack_energy {
+  const double* e1;
+  const double* e2;
+} rp_stack_energy;
+/* rp_batch_create with structure constraints (cons, as
+ * rp_batch_create_constrained; NULL: none) and stacking pseudo-energies (se,
+ * one rp_stack_energy per pair; NULL, or an entry with both NULL: none).  A
+ * problem whose rounded values are all 0 has no data: it is planned and
+ * computed exactly as without them.  Problems with data run on the general
+ * kernel.  RP_ERR_ARG, with rp_last_error naming the pair, the vector and
+ * the position, for a value that is not finite; constraint errors as
+ * rp_batch_create_constrained.  Everything that takes an rp_batch works on
+ * the result unchanged. */
+int rp_batch_create_soft(rp_ctx* ctx, const rp_pair* pairs,
+                         const rp_constraint* cons, const rp_stack_energy* se,
+                         int n_pairs, const rp_opts* opts, rp_batch** batch);
+/* Deigan et al. (2009) pseudo-energies from probing reactivities, host only:
+ * e[i] = slope * ln(r[i] + 1) + intercept for r[i] >= 0, 0 for r[i] < 0 or
+ * NaN (missing data).  RNAfold --shapeMethod=D uses slope 1.8 and intercept
+ * -0.6 kcal/mol.  RP_ERR_ARG for n < 0 or a NULL array with n > 0. */
+int rp_shape_deigan(const double* r, int n, double slope, double intercept,
+                    double* e);
 int rp_batch_run(rp_batch* batch);                 /* async on the ctx stream */
 int rp_batch_sync(rp_batch* batch);
 int rp_batch_fetch_dense(rp_batch* batch, float* out, size_t out_floats);

@@ -80,20 +80,17 @@ class ProbabilityStage {
   // the alphabet .x()[] of rp_constraint; an empty string leaves its sequence unconstrained).  One context only.
   void solve_probabilities(const std::string& s1, const std::string& s2, const std::string& c1, const std::string& c2,
                            PairProbabilities& out) {
-    if (!ctx_) throw std::runtime_error("ractip_prob: constrained problems run on a single-device stage");
-    rp_pair pair = {s1.data(), static_cast<int>(s1.size()), s2.data(), static_cast<int>(s2.size())};
-    rp_constraint con = {c1.empty() ? nullptr : c1.c_str(), c2.empty() ? nullptr : c2.c_str()};
-    rp_dense_layout lay;
-    size_t total = 0;
-    check(rp_dense_plan(&pair, 1, &opts_, &lay, &total), ctx_);
-    std::vector<float> flat(total ? total : 1);
-    rp_batch* b = nullptr;
-    check(rp_batch_create_constrained(ctx_, &pair, &con, 1, &opts_, &b), ctx_);
-    int rc = rp_batch_run(b);
-    if (!rc) rc = rp_batch_fetch_dense(b, flat.data(), flat.size());
-    rp_batch_destroy(b);
-    check(rc, ctx_);
-    unpack(pair, lay, flat.data(), out);
+    solve_one(s1, s2, c1, c2, nullptr, out);
+  }
+
+  // The same with stacking pseudo-energies e1 over s1, e2 over s2 in kcal/mol as well (rp_stack_energy; SHAPE data
+  // through rp_shape_deigan; an empty vector means none, as an empty constraint string does).  One context only.
+  void solve_probabilities(const std::string& s1, const std::string& s2, const std::string& c1, const std::string& c2,
+                           const std::vector<double>& e1, const std::vector<double>& e2, PairProbabilities& out) {
+    if ((!e1.empty() && e1.size() != s1.size()) || (!e2.empty() && e2.size() != s2.size()))
+      throw std::runtime_error("ractip_prob: a pseudo-energy vector's length differs from its sequence's");
+    rp_stack_energy se = {e1.empty() ? nullptr : e1.data(), e2.empty() ? nullptr : e2.data()};
+    solve_one(s1, s2, c1, c2, &se, out);
   }
 
   // the same for a whole batch (the shuffles of src/ractip.cpp:1638-1657) in one call
@@ -141,6 +138,25 @@ class ProbabilityStage {
   }
 
  private:
+  // one pair on the context under constraints and, when se is set, stacking pseudo-energies
+  void solve_one(const std::string& s1, const std::string& s2, const std::string& c1, const std::string& c2,
+                 const rp_stack_energy* se, PairProbabilities& out) {
+    if (!ctx_) throw std::runtime_error("ractip_prob: constrained problems run on a single-device stage");
+    rp_pair pair = {s1.data(), static_cast<int>(s1.size()), s2.data(), static_cast<int>(s2.size())};
+    rp_constraint con = {c1.empty() ? nullptr : c1.c_str(), c2.empty() ? nullptr : c2.c_str()};
+    rp_dense_layout lay;
+    size_t total = 0;
+    check(rp_dense_plan(&pair, 1, &opts_, &lay, &total), ctx_);
+    std::vector<float> flat(total ? total : 1);
+    rp_batch* b = nullptr;
+    check(se ? rp_batch_create_soft(ctx_, &pair, &con, se, 1, &opts_, &b)
+             : rp_batch_create_constrained(ctx_, &pair, &con, 1, &opts_, &b), ctx_);
+    int rc = rp_batch_run(b);
+    if (!rc) rc = rp_batch_fetch_dense(b, flat.data(), flat.size());
+    rp_batch_destroy(b);
+    check(rc, ctx_);
+    unpack(pair, lay, flat.data(), out);
+  }
   static void check(int rc, rp_ctx* ctx) {
     if (rc) throw std::runtime_error(std::string("ractip_prob: ") + rp_strerror(rc) + " -- " + rp_last_error(ctx));
   }

@@ -2,7 +2,7 @@
 import argparse
 import sys
 
-from .frontend import constraint_line, format_result, input_pairs, predict
+from .frontend import constraint_line, format_result, input_pairs, predict, read_shape
 from .ip import default_ip_opts
 from .stage import ProbabilityStage, RpError, default_opts
 
@@ -29,6 +29,11 @@ def main(argv=None) -> int:
     ap.add_argument("-e", "--show-energy", action="store_true")
     ap.add_argument("-c", "--use-constraint", action="store_true",
                     help="constrain the probabilities by the records' structure lines (.x()[]; ? and space as .)")
+    ap.add_argument("--shape", action="append", default=[], metavar="NAME=FILE",
+                    help="probing reactivities (lines 'position [nucleotide] value') of the record NAME, turned into "
+                         "stacking pseudo-energies (Deigan); repeatable")
+    ap.add_argument("--shape-slope", type=float, default=1.8, help="m of E = m ln(r+1) + b, kcal/mol (default 1.8)")
+    ap.add_argument("--shape-intercept", type=float, default=-0.6, help="b of E = m ln(r+1) + b, kcal/mol (default -0.6)")
     ap.add_argument("-P", "--param-file", default=None)
     ap.add_argument("--no-pk", action="store_true")
     ap.add_argument("--duplex", action="store_true")
@@ -43,6 +48,18 @@ def main(argv=None) -> int:
         if args.use_constraint:
             for a, b in pairs:
                 constraint_line(a), constraint_line(b)
+        records = {r.name: r for ab in pairs for r in ab}
+        shape = {}
+        for arg in args.shape:
+            name, eq, path = arg.partition("=")
+            if not eq or not name or not path:
+                raise ValueError(f"--shape {arg}: expected NAME=FILE")
+            if name not in records:
+                raise ValueError(f"--shape {arg}: no record named {name!r}")
+            try:
+                shape[name] = read_shape(path, records[name].seq)
+            except OSError as e:
+                raise ValueError(f"--shape {arg}: {e.strerror}") from None
     except ValueError as e:   # the reference prints the message and exits 1 (src/ractip.cpp:1684-1697)
         print(e)
         return 1
@@ -56,7 +73,8 @@ def main(argv=None) -> int:
     stage = ProbabilityStage(device=args.device, use_bl=not args.no_bl, param_file=args.param_file)
     try:
         for r in predict(stage, pairs, opts, ipo, args.show_energy, args.zscore, args.num_shuffling, args.seed,
-                         use_constraint=args.use_constraint):
+                         use_constraint=args.use_constraint, shape=shape, shape_slope=args.shape_slope,
+                         shape_intercept=args.shape_intercept):
             print(format_result(r, args.show_energy))
     except RpError as e:
         if not (args.use_constraint and e.code == RP_ERR_ARG):

@@ -71,7 +71,10 @@ struct rp_batch {
   rp::BatchPlan plan;
   // device
   uint8_t* d_seq = nullptr;
-  uint16_t* d_key = nullptr;  // structure-constraint keys (BatchPlan::key), null when no problem is constrained
+  // per-base data (BatchDev::perbase): BatchPlan::key, then BatchPlan::stack from stack_off doubles on; null when no
+  // problem is constrained or carries pseudo-energies
+  double* d_perbase = nullptr;
+  unsigned stack_off = 0;
   Problem* d_probs = nullptr;
   int* d_order = nullptr;
   int* d_counter = nullptr;
@@ -354,7 +357,7 @@ int rp_batch_destroy(rp_batch* b) {
   }
   if (b->ctx) {
     rp_ctx* ctx = b->ctx;
-    for (void* p : {(void*)b->d_seq, (void*)b->d_key, (void*)b->d_probs, (void*)b->d_order, (void*)b->d_counter, (void*)b->d_dense,
+    for (void* p : {(void*)b->d_seq, (void*)b->d_perbase, (void*)b->d_probs, (void*)b->d_order, (void*)b->d_counter, (void*)b->d_dense,
                     (void*)b->d_logz, (void*)b->d_done, (void*)b->d_spairs, (void*)b->d_recs, (void*)b->d_ups, (void*)b->d_counts})
       pool_release(ctx, p);
     ctx->live_batches--;
@@ -370,8 +373,8 @@ int rp_batch_destroy(rp_batch* b) {
 }  // extern "C"
 
 namespace {
-int batch_create(rp_ctx* ctx, const rp_pair* pairs, const rp_constraint* cons, int n_pairs, const rp_opts* opts,
-                 rp_batch** out) {
+int batch_create(const char* who, rp_ctx* ctx, const rp_pair* pairs, const rp_constraint* cons,
+                 const rp_stack_energy* se, int n_pairs, const rp_opts* opts, rp_batch** out) {
   if (!ctx || !out) return fail(ctx, RP_ERR_ARG, "rp_batch_create: null argument");
   *out = nullptr;
   int rc = rp::check_pairs(pairs, n_pairs, opts);
@@ -380,7 +383,8 @@ int batch_create(rp_ctx* ctx, const rp_pair* pairs, const rp_constraint* cons, i
     if ((long long)pairs[p].n1 + pairs[p].n2 > rp::RP_MAX_N)
       return fail(ctx, RP_ERR_TOO_LONG, "rp_batch_create: n1+n2 exceeds the 32-bit workspace indexing limit (12000 nt)");
   std::string msg;
-  if ((rc = rp::check_constraints(pairs, cons, n_pairs, &msg)) != RP_OK) return fail(ctx, rc, "rp_batch_create_constrained: " + msg);
+  if ((rc = rp::check_constraints(pairs, cons, n_pairs, &msg)) != RP_OK) return fail(ctx, rc, std::string(who) + ": " + msg);
+  if ((rc = rp::check_stack_energies(pairs, se, n_pairs, &msg)) != RP_OK) return fail(ctx, rc, std::string(who) + ": " + msg);
   CU(cudaSetDevice(ctx->device));
   rp_batch* b = new rp_batch;
   b->ctx = ctx;
@@ -389,7 +393,7 @@ int batch_create(rp_ctx* ctx, const rp_pair* pairs, const rp_constraint* cons, i
   b->opts = *opts;
   b->slayout.resize(n_pairs);
   rp_sparse_plan(pairs, n_pairs, opts, b->slayout.data(), &b->total_recs, &b->total_upf);
-  if (rp::plan_batch(pairs, n_pairs, opts, device_facts(ctx), ctx->route, &b->plan, cons) != RP_OK) {
+  if (rp::plan_batch(pairs, n_pairs, opts, device_facts(ctx), ctx->route, &b->plan, cons, se) != RP_OK) {
     rp_batch_destroy(b);
     return fail(ctx, RP_ERR_CUDA, "rp_batch_create: band kernel does not fit on this device");
   }
@@ -410,10 +414,14 @@ int batch_create(rp_ctx* ctx, const rp_pair* pairs, const rp_constraint* cons, i
   if ((e = pool_alloc(ctx, &b->d_logz, std::max<size_t>(1, (size_t)n_pairs * 3) * sizeof(double))) != cudaSuccess) return bail(e, "cudaMalloc logz");
   cudaStream_t st = ctx->stream;
   if ((e = cudaMemcpyAsync(b->d_seq, p.seq.data(), p.seq.size(), cudaMemcpyHostToDevice, st)) != cudaSuccess) return bail(e, "H2D seq");
-  if (!p.key.empty()) {   // only batches with a constrained problem carry keys
-    const size_t kb = p.key.size() * sizeof(uint16_t);
-    if ((e = pool_alloc(ctx, &b->d_key, kb)) != cudaSuccess) return bail(e, "cudaMalloc key");
-    if ((e = cudaMemcpyAsync(b->d_key, p.key.data(), kb, cudaMemcpyHostToDevice, st)) != cudaSuccess) return bail(e, "H2D key");
+  // per-base data only for batches with a constrained problem (keys) or one whose pseudo-energies are not all 0
+  if (!p.key.empty() || !p.stack.empty()) {
+    const size_t kb = p.key.size() * sizeof(uint16_t), fb = p.stack.size() * sizeof(double);
+    b->stack_off = (unsigned)((kb + sizeof(double) - 1) / sizeof(double));
+    if ((e = pool_alloc(ctx, &b->d_perbase, b->stack_off * sizeof(double) + fb)) != cudaSuccess) return bail(e, "cudaMalloc per-base data");
+    if (kb && (e = cudaMemcpyAsync(b->d_perbase, p.key.data(), kb, cudaMemcpyHostToDevice, st)) != cudaSuccess) return bail(e, "H2D key");
+    if (fb && (e = cudaMemcpyAsync(b->d_perbase + b->stack_off, p.stack.data(), fb, cudaMemcpyHostToDevice, st)) != cudaSuccess)
+      return bail(e, "H2D stack");
   }
   if (np) {
     if ((e = cudaMemcpyAsync(b->d_probs, p.probs.data(), np * sizeof(Problem), cudaMemcpyHostToDevice, st)) != cudaSuccess) return bail(e, "H2D probs");
@@ -424,6 +432,7 @@ int batch_create(rp_ctx* ctx, const rp_pair* pairs, const rp_constraint* cons, i
   if ((e = cudaStreamSynchronize(st)) != cudaSuccess) return bail(e, "sync");  // the host copies are complete
   std::vector<uint8_t>().swap(p.seq);   // the sequences live on the device from here
   std::vector<uint16_t>().swap(p.key);
+  std::vector<double>().swap(p.stack);
   *out = b;
   return RP_OK;
 }
@@ -432,12 +441,17 @@ int batch_create(rp_ctx* ctx, const rp_pair* pairs, const rp_constraint* cons, i
 extern "C" {
 
 int rp_batch_create(rp_ctx* ctx, const rp_pair* pairs, int n_pairs, const rp_opts* opts, rp_batch** out) {
-  return batch_create(ctx, pairs, nullptr, n_pairs, opts, out);
+  return batch_create("rp_batch_create", ctx, pairs, nullptr, nullptr, n_pairs, opts, out);
 }
 
 int rp_batch_create_constrained(rp_ctx* ctx, const rp_pair* pairs, const rp_constraint* cons, int n_pairs,
                                 const rp_opts* opts, rp_batch** out) {
-  return batch_create(ctx, pairs, cons, n_pairs, opts, out);
+  return batch_create("rp_batch_create_constrained", ctx, pairs, cons, nullptr, n_pairs, opts, out);
+}
+
+int rp_batch_create_soft(rp_ctx* ctx, const rp_pair* pairs, const rp_constraint* cons, const rp_stack_energy* se,
+                         int n_pairs, const rp_opts* opts, rp_batch** out) {
+  return batch_create("rp_batch_create_soft", ctx, pairs, cons, se, n_pairs, opts, out);
 }
 
 int rp_batch_run(rp_batch* b) {
@@ -453,7 +467,7 @@ int rp_batch_run(rp_batch* b) {
   if (rc) return rc;
   const int n_bandall = p.n_band[0] + p.n_band[1];
   rp::BatchDev d;
-  d.model = ctx->d_model; d.seq = b->d_seq; d.key = b->d_key; d.probs = b->d_probs; d.order = b->d_order + n_bandall; d.nprob = p.n_general;
+  d.model = ctx->d_model; d.seq = b->d_seq; d.perbase = b->d_perbase; d.stack_off = b->stack_off; d.probs = b->d_probs; d.order = b->d_order + n_bandall; d.nprob = p.n_general;
   d.counter = b->d_counter; d.ws = ctx->ws; d.slot_stride = p.slot_doubles; d.nslots = std::max(p.grid, 1);
   d.dense = b->d_dense; d.logz = b->d_logz;
   d.ws_up = ctx->ws + p.ws_up; d.done = b->d_done;

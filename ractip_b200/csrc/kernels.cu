@@ -54,15 +54,22 @@ using CtaExec = CtaExecT<>;
 
 }  // namespace
 
+template <bool PB>
+__device__ __forceinline__ void bind_per_base(Ctx& c, const BatchDev& b, const Problem& p) {
+  if (PB && (p.constrained & CON_KEYS)) c.key = static_cast<const uint16_t*>(b.perbase) + p.seq_off - 1;
+  if (PB && (p.constrained & CON_STACK)) c.stk = static_cast<const double*>(b.perbase) + b.stack_off + p.seq_off - 1;
+}
+
 // Instantiated for two register budgets: <2> two CTAs per SM at 64 registers (many short problems
 // in flight) and <1> one CTA per SM at 128 registers (long problems: the split-sum band phases keep
 // their accumulators, operand windows and four steps' loads in registers without spilling, and half
 // as many problem histories compete for the L2).
 // <1, W> with W > BAND sums the split sums in wide bands (solve_mcc_wide): W-fold reuse of every element
 // streamed from HBM.
-// KEYS: the batch has structure-constrained problems (BatchDev::key).  The instances without compile the constraint
-// out (Ctx::key stays null), so that unconstrained batches run exactly the code they ran before constraints existed.
-template <int MINB, int W, bool KEYS>
+// PB: the batch has per-base data (BatchDev::perbase), structure-constraint keys or stacking pseudo-energies; each
+// problem binds what it carries.  The instances without compile both out (Ctx::key and Ctx::stk stay null), so that
+// unconstrained batches run exactly the code they ran before constraints existed.
+template <int MINB, int W, bool PB>
 __global__ void __launch_bounds__(RP_MCC_THREADS, MINB) mcc_persistent(BatchDev b) {
   extern __shared__ double smem_raw[];
   __shared__ int s_next;
@@ -80,7 +87,7 @@ __global__ void __launch_bounds__(RP_MCC_THREADS, MINB) mcc_persistent(BatchDev 
     if (p.kind == KIND_DUPLEX) continue;  // handled by duplex_kernel
     Ctx c;
     bind_ctx(c, b.model, b.seq + p.seq_off - 1, p, b.ws + (size_t)blockIdx.x * b.slot_stride);
-    if (KEYS && p.constrained) c.key = b.key + p.seq_off - 1;
+    bind_per_base<PB>(c, b, p);
     c.dbg = b.dbg;
     if (W > BAND) solve_mcc_wide(ex, c, p, b.dense, b.logz, sh);
     else solve_mcc(ex, c, p, b.dense, b.logz, sh);
@@ -91,7 +98,7 @@ __global__ void __launch_bounds__(RP_MCC_THREADS, MINB) mcc_persistent(BatchDev 
 // pair rather than a shuffle batch).  A cluster of G CTAs works on one problem (solve_mcc_wide); clusters
 // pull problems from the same cost-ordered queue, one workspace slot each.  G = 16 (beyond the portable
 // cluster size, opted in at launch) when there are at most sm_count/16 problems, else 8.
-template <int W, int G, bool KEYS>
+template <int W, int G, bool PB>
 __global__ void __cluster_dims__(G, 1, 1) __launch_bounds__(RP_MCC_THREADS, 1) mcc_cluster_kernel(BatchDev b) {
   namespace cg = cooperative_groups;
   extern __shared__ double smem_raw[];
@@ -112,7 +119,7 @@ __global__ void __cluster_dims__(G, 1, 1) __launch_bounds__(RP_MCC_THREADS, 1) m
     if (p.kind == KIND_DUPLEX) continue;
     Ctx c;
     bind_ctx(c, b.model, b.seq + p.seq_off - 1, p, b.ws + (size_t)cid * b.slot_stride);
-    if (KEYS && p.constrained) c.key = b.key + p.seq_off - 1;
+    bind_per_base<PB>(c, b, p);
     c.dbg = b.dbg;
     solve_mcc_wide(ex, c, p, b.dense, b.logz, sh);
   }
@@ -565,10 +572,10 @@ __global__ void __launch_bounds__(256) peak_smem_kernel(double* out, int iters) 
 namespace {
 using MccKernel = void (*)(BatchDev);
 // minb = 2: 64-register build, BAND-wide sums; minb = 1: 128 registers, bands of 10 diagonals
-MccKernel mcc_kernel(int minb, bool keys, int* w_out) {
-  if (minb >= 2) { *w_out = BAND; return keys ? mcc_persistent<RP_MCC_MIN_CTAS, BAND, true> : mcc_persistent<RP_MCC_MIN_CTAS, BAND, false>; }
+MccKernel mcc_kernel(int minb, bool pb, int* w_out) {
+  if (minb >= 2) { *w_out = BAND; return pb ? mcc_persistent<RP_MCC_MIN_CTAS, BAND, true> : mcc_persistent<RP_MCC_MIN_CTAS, BAND, false>; }
   *w_out = 10;
-  return keys ? mcc_persistent<1, 10, true> : mcc_persistent<1, 10, false>;
+  return pb ? mcc_persistent<1, 10, true> : mcc_persistent<1, 10, false>;
 }
 }  // namespace
 
@@ -583,7 +590,7 @@ int mcc_max_ctas_per_sm(int minb) {
 
 cudaError_t launch_mcc(const BatchDev& b, int grid, int minb, cudaStream_t st) {
   int w = BAND;
-  MccKernel k = mcc_kernel(minb, b.key != nullptr, &w);
+  MccKernel k = mcc_kernel(minb, b.perbase != nullptr, &w);
   size_t smem = shared_bytes(RP_MCC_THREADS, w);
   cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
   k<<<grid, RP_MCC_THREADS, smem, st>>>(b);
@@ -592,8 +599,9 @@ cudaError_t launch_mcc(const BatchDev& b, int grid, int minb, cudaStream_t st) {
 
 cudaError_t launch_mcc_cluster(const BatchDev& b, int nclusters, int ctas, cudaStream_t st) {
   size_t smem = shared_bytes(RP_MCC_THREADS, 10);
-  MccKernel k = ctas >= 16 ? (b.key ? mcc_cluster_kernel<10, 16, true> : mcc_cluster_kernel<10, 16, false>)
-                           : (b.key ? mcc_cluster_kernel<10, 8, true> : mcc_cluster_kernel<10, 8, false>);
+  const bool pb = b.perbase != nullptr;
+  MccKernel k = ctas >= 16 ? (pb ? mcc_cluster_kernel<10, 16, true> : mcc_cluster_kernel<10, 16, false>)
+                           : (pb ? mcc_cluster_kernel<10, 8, true> : mcc_cluster_kernel<10, 8, false>);
   const int G = ctas >= 16 ? 16 : 8;
   cudaError_t e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
   if (e != cudaSuccess) return e;

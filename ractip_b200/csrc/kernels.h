@@ -30,7 +30,11 @@ struct BatchDev {
   double* logz;            // 3 per pair, may be null
   long long* prof;         // 64 counters (cycles, calls per phase id) or null
   int dbg;                 // RP_DEBUG_SKIP bits (tuning aid; results are wrong when set)
-  const uint16_t* key;     // structure-constraint keys laid out like seq (Problem::constrained), or null
+  unsigned stack_off;      // doubles from perbase to the stacking factors
+  // Per-base data of the batch, or null: structure-constraint keys (uint16) laid out like seq at the start
+  // (Problem::constrained & CON_KEYS), stacking pseudo-energy factors (double) laid out like seq at stack_off
+  // (CON_STACK).  One pointer, so that the parameter block of every kernel keeps the layout it had before factors.
+  const void* perbase;
 };
 
 struct SparsePair {
@@ -66,8 +70,8 @@ struct SquareDev {
 };
 
 // general kernel, RP_MCC_THREADS threads.  minb = 2: 64-register build, two CTAs per SM; 1: 128 registers, one CTA
-// per SM, split sums in bands of 10 diagonals.  Both launches run the instances that apply structure constraints when
-// b.key is set, else the ones that compile them out.
+// per SM, split sums in bands of 10 diagonals.  Both launches run the instances that apply per-base data (structure
+// constraints, stacking pseudo-energies) when b.perbase is set, else the ones that compile it out.
 int mcc_max_ctas_per_sm(int minb);
 cudaError_t launch_mcc(const BatchDev& b, int grid, int minb, cudaStream_t st);
 // multi-CTA wavefront: `nclusters` clusters of `ctas` (8 or 16) CTAs, one problem (and one workspace slot) per cluster

@@ -58,7 +58,8 @@ struct Problem {
   int which;          // 0: s1, 1: s2, 2: s1&s2
   int max_w;
   int n1, n2;
-  int constrained;    // 1: a structure constraint removes some pairs (BatchDev::key); general kernel only
+  int constrained;    // general kernel only, bits (BatchDev::perbase): CON_KEYS a structure constraint removes some
+                      // pairs, CON_STACK stacking pseudo-energies weight its stacks
   long long out_bp;   // float offsets into the dense output, -1 if absent
   long long out_up;
   long long out_hp;
@@ -66,6 +67,7 @@ struct Problem {
   int defer_up;       // 1: the unpaired-window pass runs later in its own kernel (unstru_kernel) on the tables left in ws_off
   long long ws_off;   // >= 0: private workspace (doubles from BatchDev::ws_up) that outlives the wavefront kernel; -1: the CTA's slot
 };
+enum { CON_KEYS = 1, CON_STACK = 2 };
 // queue entries: problem index, + RP_JOB_UNPAIRED for the unpaired-window pass of a deferred problem as a job of its own
 constexpr int RP_JOB_UNPAIRED = 0x40000000;
 
@@ -104,6 +106,7 @@ struct Ctx {
   int dbg;            // tuning aid (RP_DEBUG_SKIP): 1 skip interior rows, 2 skip split sums, 4 skip gap sums
   long long* prof;    // RP_PROFILE counters (slots 40..: fine-grained probes of thread 0) or null
   const uint16_t* key;   // key[1..n] of a constrained problem (pair (i,j) allowed iff key[i] == key[j]), else null
+  const double* stk;     // stk[1..n]: per-base factors exp(-E/kT) of stacking pseudo-energies (CON_STACK), else null
   // Tables whose rows are only read while they are recent are RINGS of a few rows (row d at d & mask):
   // PR/PL/PMLB are read one diagonal after they are written, the band results QS/PRB/MLB within a
   // band.  A full table would leave every written line behind in L2, where it pushes out the history
@@ -133,6 +136,7 @@ RP_HD void bind_ctx(Ctx& c, const DevModel* M, const uint8_t* S, const Problem& 
   c.dbg = 0;
   c.prof = nullptr;
   c.key = nullptr;
+  c.stk = nullptr;
 }
 #define TB(c, t, d, i) ((c).tb(t, d, i))
 // store of a value that is not read again soon (qb, out, class tables, outputs): evict-first, so that
@@ -228,6 +232,16 @@ RP_HD int cell_type(const Ctx& c, int i, int j) {
 // ViennaRNA SAME_STRAND(a,b) for a<b
 template <class C>
 RP_HD bool ss(const C& c, int a, int b) { return c.cp <= 0 || a >= c.cp || b < c.cp; }
+
+// Weight w of table-driven shape s closed by (i,j) with the stacking pseudo-energies of the problem (soft constraint,
+// CON_STACK): a stack (s = 0) gets the factor stk[i] stk[i+1] stk[j-1] stk[j], unless it joins the strands (probing
+// data of each RNA alone say nothing about its pairs with the partner).  Every other shape, and every problem without
+// factors, keeps w as it is; the instances without per-base data know c.stk is null and compile this away.
+template <class C>
+RP_HD double stack_sc(const C& c, int s, int i, int j, double w) {
+  if (s != 0 || !c.stk || !ss(c, i, j)) return w;
+  return w * (c.stk[i] * c.stk[i + 1] * c.stk[j - 1] * c.stk[j]);
+}
 
 // Outside pass of a two-strand problem: RactIP keeps only the probabilities of pairs that JOIN the strands
 // (i < cp <= j; reference src/ractip.cpp:451-453), and the outside value of such a pair depends on enclosing
@@ -616,7 +630,7 @@ RP_HD double inside_interior(const C& c, const Shared& sh, int d, int i, int typ
     const int k = i + 1 + u1, l = j - 1 - u2;
     const int t2 = cell_type(c, k, l);
     if (!t2) continue;
-    accI += TB(c, T_QB, d - dd, k) * special_loop(M, s, type, rtype(t2), si1, sj1, base(c, k - 1), base(c, l + 1));
+    accI += TB(c, T_QB, d - dd, k) * stack_sc(c, s, i, j, special_loop(M, s, type, rtype(t2), si1, sj1, base(c, k - 1), base(c, l + 1)));
   }
   return accI;
 }
@@ -841,7 +855,7 @@ RP_HD double outside_interior(const C& c, const Shared& sh, int d, int k, int sl
     if (!t1) continue;
     const double o = TB(c, T_OUT, d + dd, i);
     if (o == 0.) continue;
-    accI += o * special_loop(M, s, t1, t2, base(c, i + 1), base(c, j - 1), sp1, sq1);
+    accI += o * stack_sc(c, s, i, j, special_loop(M, s, t1, t2, base(c, i + 1), base(c, j - 1), sp1, sq1));
   }
   return accI;
 }
@@ -1318,7 +1332,7 @@ RP_HD double inside_ends_item(const Ctx& c, const Shared& sh, int d, int i, int 
     int u1, u2;
     special_uv(s, u1, u2);
     const int k = i + 1 + u1, l = j - 1 - u2;
-    acc += qv[s] * special_loop(M, s, type, rtype(t2v[s]), si1, sj1, base(c, k - 1), base(c, l + 1));
+    acc += qv[s] * stack_sc(c, s, i, j, special_loop(M, s, type, rtype(t2v[s]), si1, sj1, base(c, k - 1), base(c, l + 1)));
   }
   return acc;
 }
@@ -1360,7 +1374,7 @@ RP_HD double outside_ends_item(const Ctx& c, const Shared& sh, int d, int k, int
     int u1, u2;
     special_uv(s, u1, u2);
     const int i = k - 1 - u1, j = l + 1 + u2;
-    acc += ov[s] * special_loop(M, s, t1v[s], t2, base(c, i + 1), base(c, j - 1), sp1, sq1);
+    acc += ov[s] * stack_sc(c, s, i, j, special_loop(M, s, t1v[s], t2, base(c, i + 1), base(c, j - 1), sp1, sq1));
   }
   return acc;
 }
@@ -1566,6 +1580,8 @@ RP_HD unsigned up_special_idx(int n, int side, int ug, int nsl, int sl, int a) {
 // ug <= 3, gap start a, slice) sums the loops of all special shapes with that gap size over
 // every `nsl`-th position of the free pair end into its scratch slot.  The row scan adds the
 // slices up in fixed order.  Branch-free body: cells that cannot pair carry qb = out = 0.
+// A gap here holds at least one base (ug >= 1), so no shape is a stack and no stacking pseudo-energy (Ctx::stk)
+// enters these sums: a stack leaves no base unpaired.
 // Only for n >= 7: shorter sequences have no such loops to speak of.
 RP_HD int gap_special_slices(int n) { return n >= 48 ? 4 : 1; }
 template <class C, class MT>

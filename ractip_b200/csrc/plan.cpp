@@ -90,7 +90,43 @@ int check_constraints(const rp_pair* pairs, const rp_constraint* cons, int n_pai
   return RP_OK;
 }
 
+// Stacking pseudo-energies: e1 over s1, e2 over s2, in kcal/mol (either may be null).
+int check_stack_energies(const rp_pair* pairs, const rp_stack_energy* se, int n_pairs, std::string* msg) {
+  if (!se) return RP_OK;
+  for (int p = 0; p < n_pairs; p++) {
+    const double* es[2] = {se[p].e1, se[p].e2};
+    const int ns[2] = {pairs[p].n1, pairs[p].n2};
+    for (int s = 0; s < 2; s++) {
+      if (!es[s]) continue;
+      for (int i = 0; i < ns[s]; i++)
+        if (!std::isfinite(es[s][i])) {
+          char buf[160];
+          std::snprintf(buf, sizeof buf, "pair %d, e%d, position %d: %g kcal/mol is not finite", p, s + 1, i + 1, es[s][i]);
+          if (msg) *msg = buf;
+          return RP_ERR_ARG;
+        }
+    }
+  }
+  return RP_OK;
+}
+
 namespace {
+// Stacking factors of one strand of length m from its pseudo-energies e[0..m-1] (kcal/mol): each value rounded to an
+// integer number of 0.01 kcal/mol, half away from zero (as ViennaRNA stores soft-constraint energies), then
+// f[i] = exp(-E_i * 10 / kT) at 37 C, the Boltzmann factor of every other integer energy of the model (dev_model.cpp).
+// Returns whether any rounded value differs from 0 (whether the data changes anything).
+bool fill_stack(const double* e, int m, double* f) {
+  if (!e) return false;
+  const double kT = (37.0 + RP_K0) * RP_GASCONST;
+  bool any = false;
+  for (int i = 1; i <= m; i++) {
+    const double E = std::round(e[i - 1] * 100.0);
+    f[i] = std::exp(-E * 10.0 / kT);
+    any |= E != 0.;
+  }
+  return any;
+}
+
 // Keys of one problem of length m from its bracket pairs: partner[i] = j for the ends of a bracket pair (i,j), 0 for a
 // base left free, -1 for a base kept unpaired (1-based).  Bracket pair number t (from 1, in the order they open) gets
 // 2t+1 at both ends, a free base 2t for the innermost bracket pair around it (0 for none), an unpaired base
@@ -195,6 +231,12 @@ int rp_square_plan(const rp_pair* pairs, int n_pairs, const rp_opts* opts, rp_sq
   return RP_OK;
 }
 
+int rp_shape_deigan(const double* r, int n, double slope, double intercept, double* e) {
+  if (n < 0 || (n > 0 && (!r || !e))) return RP_ERR_ARG;
+  for (int i = 0; i < n; i++) e[i] = r[i] >= 0. ? slope * std::log(r[i] + 1.) + intercept : 0.;   // r < 0, NaN: missing
+  return RP_OK;
+}
+
 int rp_sparse_plan(const rp_pair* pairs, int n_pairs, const rp_opts* opts, rp_sparse_layout* layout, size_t* total_recs,
                    size_t* total_floats) {
   int rc = rp::check_pairs(pairs, n_pairs, opts);
@@ -267,7 +309,7 @@ static double alg_flops_mcc_uncached(int n) {
 namespace rp {
 
 int plan_batch(const rp_pair* pairs, int n_pairs, const rp_opts* opts, const DeviceFacts& dev, const RouteSettings& rs,
-               BatchPlan* out, const rp_constraint* cons) {
+               BatchPlan* out, const rp_constraint* cons, const rp_stack_energy* se) {
   BatchPlan& b = *out;
   b = BatchPlan{};
   size_t mem = 0;   // DeviceFacts::memory, asked once
@@ -286,6 +328,8 @@ int plan_batch(const rp_pair* pairs, int n_pairs, const rp_opts* opts, const Dev
   std::vector<uint16_t>& key = b.key;   // (filled only for batches with constraints, then dropped if none restricts)
   bool any_constrained = false;
   std::vector<int> partner;
+  std::vector<double>& stack = b.stack;   // (the same for the stacking factors)
+  bool any_stack = false;
   const int w = opts->max_w > 0 ? opts->max_w : 0;
   size_t ws_need = 0;
   for (int p = 0; p < n_pairs; p++) {
@@ -326,6 +370,17 @@ int plan_batch(const rp_pair* pairs, int n_pairs, const rp_opts* opts, const Dev
       con[2] = pr.n2 > 0 && !opts->use_pf_duplex && fill_keys(partner, n12, &key[off12 - 1]);   // --duplex: unconstrained
       any_constrained |= con[0] || con[1] || con[2];
     }
+    // stacking pseudo-energies: s1's fold takes e1, s2's e2, the co-fold both (stack_sc, mcc_core.h, leaves out the
+    // stacks that join the strands); --duplex takes none
+    int stk[2] = {0, 0};
+    if (se && (se[p].e1 || se[p].e2)) {
+      stack.resize(seq.size(), 1.0);
+      stk[0] = fill_stack(se[p].e1, pr.n1, &stack[off1 - 1]) ? CON_STACK : 0;
+      stk[1] = fill_stack(se[p].e2, pr.n2, &stack[off2 - 1]) ? CON_STACK : 0;
+      std::copy(&stack[off1], &stack[off1] + pr.n1, &stack[off12]);
+      std::copy(&stack[off2], &stack[off2] + pr.n2, &stack[off12] + pr.n1);
+      any_stack |= stk[0] || stk[1];
+    }
     Problem q;
     std::memset(&q, 0, sizeof q);
     q.pair = p; q.max_w = w; q.n1 = pr.n1; q.n2 = pr.n2; q.th_hy = opts->th_hy;
@@ -333,10 +388,10 @@ int plan_batch(const rp_pair* pairs, int n_pairs, const rp_opts* opts, const Dev
     q.ws_off = -1;
     // rnafold(fa1, ...), rnafold(fa2, ...)  src/ractip.cpp:546-547
     Problem a = q;
-    a.kind = KIND_LINEAR; a.which = 0; a.seq_off = off1; a.n = pr.n1; a.cp = 0; a.constrained = con[0];
+    a.kind = KIND_LINEAR; a.which = 0; a.seq_off = off1; a.n = pr.n1; a.cp = 0; a.constrained = con[0] | stk[0];
     a.out_bp = (long long)L.bp1; a.out_up = w > 0 ? (long long)L.up1 : -1;
     b.probs.push_back(a);
-    a.which = 1; a.seq_off = off2; a.n = pr.n2; a.constrained = con[1];
+    a.which = 1; a.seq_off = off2; a.n = pr.n2; a.constrained = con[1] | stk[1];
     a.out_bp = (long long)L.bp2; a.out_up = w > 0 ? (long long)L.up2 : -1;
     b.probs.push_back(a);
     if (pr.n2 == 0) {   // a lone sequence (RactIP::rnafold on its own, src/ractip.cpp:1599-1601): no second fold, no hybridization
@@ -355,7 +410,7 @@ int plan_batch(const rp_pair* pairs, int n_pairs, const rp_opts* opts, const Dev
       b.n_duplex++;
       ws_need = std::max(ws_need, 2 * (size_t)(pr.n1 + 2) * (size_t)(pr.n2 + 2));
     } else {
-      c.kind = KIND_COFOLD; c.n = pr.n1 + pr.n2; c.cp = pr.n1 + 1; c.constrained = con[2];
+      c.kind = KIND_COFOLD; c.n = pr.n1 + pr.n2; c.cp = pr.n1 + 1; c.constrained = con[2] | stk[0] | stk[1];
       b.alg_flops += rp_alg_flops_mcc(c.n);
     }
     b.probs.push_back(c);
@@ -363,9 +418,11 @@ int plan_batch(const rp_pair* pairs, int n_pairs, const rp_opts* opts, const Dev
   }
   if (any_constrained) key.resize(seq.size(), 0);
   else std::vector<uint16_t>().swap(key);
+  if (any_stack) stack.resize(seq.size(), 1.0);
+  else std::vector<double>().swap(stack);
 
   // Band class of a problem: 0 = L (512 threads, ring needs more than half an SM), 1 = S (256 threads, 2 CTAs/SM),
-  // -1 = the general kernel, which alone applies structure constraints.
+  // -1 = the general kernel, which alone applies structure constraints and stacking pseudo-energies.
   auto cls = [&](const Problem& q) {
     if (!rs.band || q.kind == KIND_DUPLEX || q.constrained) return -1;
     const int k = rp_kernel_plan(q.n, dev.smem_optin, nullptr);

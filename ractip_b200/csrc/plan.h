@@ -49,6 +49,9 @@ struct BatchPlan {
   // structure-constraint keys of the constrained problems, laid out like seq (pair (i,j) of a problem is allowed iff
   // its two bases carry the same key); empty when no problem of the batch is constrained
   std::vector<uint16_t> key;
+  // stacking pseudo-energy factors exp(-E/kT) of the problems that carry such data (CON_STACK), laid out like seq, 1
+  // elsewhere; empty when no problem of the batch does
+  std::vector<double> stack;
   std::vector<Problem> probs;            // three per pair: s1, s2, s1&s2
   std::vector<rp_dense_layout> layout;
   size_t total_floats = 0;
@@ -95,11 +98,16 @@ int check_pairs(const rp_pair* pairs, int n_pairs, const rp_opts* opts);
 // The structure constraints of pairs that pass check_pairs (cons may be null: none).  RP_OK, or RP_ERR_ARG with a
 // message in *msg that names the pair, the string and the (1-based) position.
 int check_constraints(const rp_pair* pairs, const rp_constraint* cons, int n_pairs, std::string* msg);
+// The stacking pseudo-energies of pairs that pass check_pairs (se may be null: none).  RP_OK, or RP_ERR_ARG with a
+// message in *msg that names the pair, the vector and the (1-based) position of a value that is not finite.
+int check_stack_energies(const rp_pair* pairs, const rp_stack_energy* se, int n_pairs, std::string* msg);
 
-// The pairs must pass check_pairs and the constraints check_constraints (cons == null: none).  A problem that a
-// constraint restricts runs on the general kernel.  Returns RP_OK, or RP_ERR_CUDA when a band launch shape fits no SM.
+// The pairs must pass check_pairs, the constraints check_constraints (cons == null: none) and the stacking
+// pseudo-energies check_stack_energies (se == null: none).  A problem that a constraint restricts, or whose rounded
+// pseudo-energies are not all 0, runs on the general kernel.  Returns RP_OK, or RP_ERR_CUDA when a band launch shape
+// fits no SM.
 int plan_batch(const rp_pair* pairs, int n_pairs, const rp_opts* opts, const DeviceFacts& dev, const RouteSettings& rs,
-               BatchPlan* plan, const rp_constraint* cons = nullptr);
+               BatchPlan* plan, const rp_constraint* cons = nullptr, const rp_stack_energy* se = nullptr);
 
 }  // namespace rp
 #endif

@@ -13,13 +13,16 @@ z-score run).  The IP itself stays on the host, as in the reference.
 from __future__ import annotations
 
 import ctypes as C
+import math
 from dataclasses import dataclass
-from typing import List, Optional, Sequence, Tuple
+from typing import Dict, List, Optional, Sequence, Tuple
+
+import numpy as np
 
 from . import _lib
 from ._lib import RpIpOpts, RpModel, RpOpts
 from .ip import JointPrediction, default_ip_opts, solve_joint, solve_ss, zscore_statistic
-from .stage import ProbabilityStage, RpError, default_opts, zscore_shuffles
+from .stage import ProbabilityStage, RpError, default_opts, shape_deigan, zscore_shuffles
 
 
 @dataclass
@@ -93,6 +96,45 @@ def constraint_line(rec: FastaRecord) -> Optional[str]:
     return rec.str.replace("?", ".").replace(" ", ".")
 
 
+def read_shape(path: str, seq: str) -> np.ndarray:
+    """Probing reactivities of `seq` from a file in the usual format (RNAfold --shape): one `position [nucleotide]
+    value` per line, position 1-based; blank lines and lines starting with '#' are skipped.  Returns len(seq) values,
+    NaN (missing) at the positions the file does not list; a negative value also counts as missing (shape_deigan).
+    A ValueError for a position outside 1..len(seq) or listed twice, a nucleotide that differs from the sequence's
+    base (T and U alike, any case), or a value that is not a finite number."""
+    r = np.full(len(seq), np.nan)
+    seen = set()
+    with open(path) as f:
+        for k, line in enumerate(f, 1):
+            t = line.split()
+            if not t or t[0].startswith("#"):
+                continue
+            where = f"{path}, line {k}"
+            if len(t) not in (2, 3):
+                raise ValueError(f"{where}: expected 'position [nucleotide] value', got {line.strip()!r}")
+            try:
+                pos = int(t[0])
+            except ValueError:
+                raise ValueError(f"{where}: position {t[0]!r} is not an integer") from None
+            if not 1 <= pos <= len(seq):
+                raise ValueError(f"{where}: position {pos} is outside 1..{len(seq)}")
+            if pos in seen:
+                raise ValueError(f"{where}: position {pos} is listed twice")
+            seen.add(pos)
+            if len(t) == 3:
+                nt, base = t[1].upper().replace("T", "U"), seq[pos - 1].upper().replace("T", "U")
+                if nt != base:
+                    raise ValueError(f"{where}: nucleotide {t[1]!r} at position {pos}, the sequence has {seq[pos - 1]!r}")
+            try:
+                v = float(t[-1])
+            except ValueError:
+                raise ValueError(f"{where}: value {t[-1]!r} is not a number") from None
+            if not math.isfinite(v):
+                raise ValueError(f"{where}: value {t[-1]!r} is not finite")
+            r[pos - 1] = v
+    return r
+
+
 @dataclass
 class PairResult:
     a: FastaRecord
@@ -123,19 +165,29 @@ def format_result(r: PairResult, show_energy: bool = False) -> str:
 
 def predict(stage: ProbabilityStage, pairs: Sequence[Tuple[FastaRecord, FastaRecord]], opts: Optional[RpOpts] = None,
             ip_opts: Optional[RpIpOpts] = None, show_energy: bool = False, zscore: int = 0, num_shuffling: int = 1000,
-            seed: int = 1, use_constraint: bool = False) -> List[PairResult]:
+            seed: int = 1, use_constraint: bool = False, shape: Optional[Dict[str, Sequence[float]]] = None,
+            shape_slope: float = 1.8, shape_intercept: float = -0.6) -> List[PairResult]:
     """Joint structures of all `pairs`: one GPU batch for every pair's matrices, then the integer programmes on the
     host.  zscore in (1, 2, 12): per pair one more GPU batch with all its dinucleotide shuffles (the loop of
     src/ractip.cpp:1636-1657 with the probability work hoisted out of it).  use_constraint (-c): the records'
     structure lines constrain the pairs' probability matrices (constraint_line); shuffles have no structure line and
-    stay unconstrained."""
+    stay unconstrained.  shape: probing reactivities by record name (read_shape), turned into stacking
+    pseudo-energies by shape_deigan(shape_slope, shape_intercept) for every record of that name; they bias the
+    probability matrices only, not the energies of -e, and the shuffles carry none."""
     opts = opts if opts is not None else default_opts()
     ip_opts = ip_opts if ip_opts is not None else default_ip_opts()
     model: RpModel = stage.model
     energies = show_energy or zscore in (1, 2, 12)
     seqs = [(a.seq, b.seq) for a, b in pairs]
     cons = [(constraint_line(a), constraint_line(b)) for a, b in pairs] if use_constraint else None
-    probs = stage.run_dense(seqs, opts, constraints=cons)
+    kw = {}
+    if shape:
+        unknown = set(shape) - {r.name for ab in pairs for r in ab}
+        if unknown:
+            raise ValueError(f"reactivities for {', '.join(sorted(unknown))}: no such record")
+        de = lambda r: shape_deigan(shape[r.name], shape_slope, shape_intercept) if r.name in shape else None
+        kw["stack_energies"] = [(de(a), de(b)) for a, b in pairs]
+    probs = stage.run_dense(seqs, opts, constraints=cons, **kw)
     out = []
     for (a, b), p in zip(pairs, probs):
         res = PairResult(a, b, solve_joint(model, a.seq, b.seq, p, ip_opts, energies=energies))

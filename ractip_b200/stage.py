@@ -22,7 +22,7 @@ import numpy as np
 
 from . import _lib
 from ._lib import (RpConstraint, RpDenseLayout, RpModel, RpOpts, RpPair, RpRec, RpSparseCounts,
-                   RpSparseLayout, RpSquareLayout, RpTiming)
+                   RpSparseLayout, RpSquareLayout, RpStackEnergy, RpTiming)
 
 
 class RpError(RuntimeError):
@@ -120,12 +120,45 @@ def _make_constraints(constraints: Sequence[Optional[Tuple[Optional[str], Option
     return arr, keep
 
 
+def _make_stack_energies(stack_energies, pairs: Sequence[Tuple[str, str]]):
+    n = len(pairs)
+    if len(stack_energies) != n:
+        raise ValueError(f"stack_energies: {len(stack_energies)} entries for {n} pairs")
+    arr = (RpStackEnergy * max(n, 1))()
+    keep = []
+    for k, (ent, seqs) in enumerate(zip(stack_energies, pairs)):
+        for s, (e, seq) in enumerate(zip(ent if ent is not None else (None, None), seqs)):
+            if e is None:
+                continue
+            a = np.ascontiguousarray(e, dtype=np.float64)
+            if a.shape != (len(seq),):
+                raise ValueError(f"stack_energies: pair {k}, e{s + 1} has shape {a.shape} for {len(seq)} nt")
+            keep.append(a)
+            setattr(arr[k], f"e{s + 1}", a.ctypes.data)
+    return arr, keep
+
+
+def shape_deigan(reactivities, slope: float = 1.8, intercept: float = -0.6) -> np.ndarray:
+    """Stacking pseudo-energies (kcal/mol) from probing reactivities by Deigan et al.'s rule (rp_shape_deigan):
+    slope * ln(r + 1) + intercept for r >= 0, 0 for a missing value (r < 0 or NaN).  The defaults are RNAfold's
+    --shapeMethod=D."""
+    r = np.ascontiguousarray(reactivities, dtype=np.float64).reshape(-1)
+    e = np.empty_like(r)
+    rc = _lib.load().rp_shape_deigan(r.ctypes.data, r.size, slope, intercept, e.ctypes.data)
+    if rc:
+        raise RpError(rc, "rp_shape_deigan")
+    return e
+
+
 class DeviceBatch:
     """A batch whose inputs are resident in HBM (rp_batch_*).  constraints: None, or one (c1, c2) per pair -- the
-    structure constraints of rp_batch_create_constrained, either string (or the whole entry) None for none."""
+    structure constraints of rp_batch_create_constrained, either string (or the whole entry) None for none.
+    stack_energies: None, or one (e1, e2) per pair -- stacking pseudo-energies in kcal/mol over s1 and s2
+    (rp_batch_create_soft, e.g. from shape_deigan), either array (or the whole entry) None for none."""
 
     def __init__(self, stage: "ProbabilityStage", pairs: Sequence[Tuple[str, str]], opts: RpOpts,
-                 constraints: Optional[Sequence[Optional[Tuple[Optional[str], Optional[str]]]]] = None):
+                 constraints: Optional[Sequence[Optional[Tuple[Optional[str], Optional[str]]]]] = None,
+                 stack_energies=None):
         self.stage, self.lib, self.opts = stage, stage.lib, opts
         self.pairs = list(pairs)
         self.n = len(self.pairs)
@@ -139,7 +172,12 @@ class DeviceBatch:
         stage._check(self.lib.rp_sparse_plan(arr, self.n, C.byref(opts), self.slayout, C.byref(tr), C.byref(tf)))
         self.total_recs, self.total_upf = tr.value, tf.value
         self.handle = C.c_void_p()
-        if constraints is None:
+        if stack_energies is not None:
+            cons, ckeep = _make_constraints(constraints, self.n) if constraints is not None else (None, None)
+            se, ekeep = _make_stack_energies(stack_energies, self.pairs)
+            stage._check(self.lib.rp_batch_create_soft(stage.ctx, arr, cons, se, self.n, C.byref(opts),
+                                                       C.byref(self.handle)))
+        elif constraints is None:
             stage._check(self.lib.rp_batch_create(stage.ctx, arr, self.n, C.byref(opts), C.byref(self.handle)))
         else:
             cons, ckeep = _make_constraints(constraints, self.n)
@@ -306,18 +344,19 @@ class ProbabilityStage:
 
     # ------------------------------------------------------------- batches
     def batch(self, pairs: Sequence[Tuple[str, str]], opts: Optional[RpOpts] = None,
-              constraints=None) -> DeviceBatch:
-        """constraints: None, or one (c1, c2) structure-constraint pair per pair (DeviceBatch)."""
-        return DeviceBatch(self, pairs, opts if opts is not None else default_opts(), constraints)
+              constraints=None, stack_energies=None) -> DeviceBatch:
+        """constraints: None, or one (c1, c2) structure-constraint pair per pair; stack_energies: None, or one (e1, e2)
+        pair of stacking pseudo-energy arrays per pair (DeviceBatch)."""
+        return DeviceBatch(self, pairs, opts if opts is not None else default_opts(), constraints, stack_energies)
 
     def run_dense(self, pairs: Sequence[Tuple[str, str]], opts: Optional[RpOpts] = None,
-                  pinned: bool = False, constraints=None) -> List[PairProbabilities]:
+                  pinned: bool = False, constraints=None, stack_energies=None) -> List[PairProbabilities]:
         """rp_run_dense: host buffers in, host buffers out.  pinned=True hands the library a page-locked
-        buffer (rp_host_alloc) as the target of its device-to-host copy.  With constraints (one (c1, c2) per
-        pair, see DeviceBatch) the pairs run as a constrained device batch."""
+        buffer (rp_host_alloc) as the target of its device-to-host copy.  With constraints or stack_energies
+        (one entry per pair, see DeviceBatch) the pairs run as a device batch that carries them."""
         opts = opts if opts is not None else default_opts()
-        if constraints is not None:
-            b = self.batch(pairs, opts, constraints)
+        if constraints is not None or stack_energies is not None:
+            b = self.batch(pairs, opts, constraints, stack_energies)
             try:
                 b.run()
                 return b.split_dense(b.fetch_dense())
@@ -365,9 +404,9 @@ class ProbabilityStage:
             b.close()
 
     def run_sparse(self, pairs: Sequence[Tuple[str, str]], opts: Optional[RpOpts] = None,
-                   constraints=None) -> List[PairRecords]:
+                   constraints=None, stack_energies=None) -> List[PairRecords]:
         opts = opts if opts is not None else default_opts()
-        b = self.batch(pairs, opts, constraints)
+        b = self.batch(pairs, opts, constraints, stack_energies)
         try:
             b.run()
             return b.split_sparse(*b.fetch_sparse())
