@@ -301,6 +301,49 @@ int rp_batch_create_soft(rp_ctx* ctx, const rp_pair* pairs,
  * -0.6 kcal/mol.  RP_ERR_ARG for n < 0 or a NULL array with n > 0. */
 int rp_shape_deigan(const double* r, int n, double slope, double intercept,
                     double* e);
+/* Stochastic sampling of secondary structures (RNAfold -p --stochBT,
+ * RNAsubopt -p): `num` structures per requested problem, each drawn with
+ * probability exp(-E/kT) / Z from exactly the ensemble whose log Z
+ * rp_batch_fetch_logz reports (dangles = 2, MAXLOOP, special hairpins, -P
+ * tables; the batch's constraints and stacking pseudo-energies apply; the
+ * co-fold without DuplexInit).  `problems` is a mask of RP_SAMPLE_*; --duplex
+ * has no co-fold ensemble to sample (RP_ERR_UNSUPPORTED), a pair with n2 == 0
+ * only s1.  Random numbers: Philox4x64-10, key (seed, 3 pair + problem),
+ * counter (sample, decision / 4, 0, 0): a pair's samples do not depend on the
+ * other pairs of the batch, and one seed gives the same samples. */
+enum { RP_SAMPLE_S1 = 1, RP_SAMPLE_S2 = 2, RP_SAMPLE_COFOLD = 4 };
+typedef struct rp_sample_opts {
+  int num;          /* samples per requested problem, >= 0 */
+  uint64_t seed;
+  int problems;     /* RP_SAMPLE_* mask */
+} rp_sample_opts;
+/* Where a pair's samples live in the batch's sample buffer, in int16
+ * elements: num pair tables of n1 at s1, of n2 at s2, of n1+n2 at co (the
+ * concatenation s1 s2: base b of s2 is n1 + b); a problem that is not
+ * sampled has length 0.  Pair table t: t[k-1] = partner of base k (1-based),
+ * 0 if k is unpaired. */
+typedef struct rp_sample_layout {
+  size_t s1, s2, co;          /* offsets */
+  size_t len_s1, len_s2, len_co;
+} rp_sample_layout;
+/* Host arithmetic: per_pair[p] and *total (int16 elements).  RP_ERR_ARG for a
+ * bad argument or when a size overflows size_t. */
+int rp_sample_plan(const rp_pair* pairs, int n_pairs, const rp_sample_opts* so,
+                   rp_sample_layout* per_pair, size_t* total);
+/* rp_batch_create_soft plus samples, drawn by every rp_batch_run between the
+ * inside and the outside pass of the sampled problems, which run on the
+ * general kernel (so == NULL or num == 0: exactly rp_batch_create_soft).
+ * RP_ERR_ARG for num < 0 or an unknown bit in problems, RP_ERR_UNSUPPORTED for
+ * RP_SAMPLE_COFOLD with use_pf_duplex; rp_last_error names the pair. */
+int rp_batch_create_sampled(rp_ctx* ctx, const rp_pair* pairs,
+                            const rp_constraint* cons, const rp_stack_energy* se,
+                            int n_pairs, const rp_opts* opts,
+                            const rp_sample_opts* so, rp_batch** batch);
+/* The samples of the last run, in the layout of rp_sample_plan: to the host
+ * (synchronous), or device to device into memory the caller owns (the stream
+ * rules of rp_batch_dense_device).  RP_ERR_CAPACITY when n < total. */
+int rp_batch_fetch_samples(rp_batch* batch, int16_t* out, size_t n);
+int rp_batch_samples_device(rp_batch* batch, void* out_dev, size_t n);
 int rp_batch_run(rp_batch* batch);                 /* async on the ctx stream */
 int rp_batch_sync(rp_batch* batch);
 int rp_batch_fetch_dense(rp_batch* batch, float* out, size_t out_floats);

@@ -14,6 +14,7 @@
 #ifndef RACTIP_PROB_HPP
 #define RACTIP_PROB_HPP
 
+#include <cstdint>
 #include <stdexcept>
 #include <string>
 #include <utility>
@@ -80,7 +81,7 @@ class ProbabilityStage {
   // the alphabet .x()[] of rp_constraint; an empty string leaves its sequence unconstrained).  One context only.
   void solve_probabilities(const std::string& s1, const std::string& s2, const std::string& c1, const std::string& c2,
                            PairProbabilities& out) {
-    solve_one(s1, s2, c1, c2, nullptr, out);
+    solve_one(s1, s2, c1, c2, nullptr, nullptr, out);
   }
 
   // The same with stacking pseudo-energies e1 over s1, e2 over s2 in kcal/mol as well (rp_stack_energy; SHAPE data
@@ -90,7 +91,26 @@ class ProbabilityStage {
     if ((!e1.empty() && e1.size() != s1.size()) || (!e2.empty() && e2.size() != s2.size()))
       throw std::runtime_error("ractip_prob: a pseudo-energy vector's length differs from its sequence's");
     rp_stack_energy se = {e1.empty() ? nullptr : e1.data(), e2.empty() ? nullptr : e2.data()};
-    solve_one(s1, s2, c1, c2, &se, out);
+    solve_one(s1, s2, c1, c2, &se, nullptr, out);
+  }
+
+  // The same, and num structures sampled from one of the pair's ensembles with seed (rp_batch_create_sampled):
+  // problem is RP_SAMPLE_S1, RP_SAMPLE_S2 or RP_SAMPLE_COFOLD; samples[s] is a pair table, samples[s][k-1] the
+  // 1-based partner of base k, 0 if unpaired (co-fold: over s1 s2, base b of s2 at n1 + b).  One context only.
+  void solve_probabilities(const std::string& s1, const std::string& s2, const std::string& c1, const std::string& c2,
+                           const std::vector<double>& e1, const std::vector<double>& e2, int problem, int num,
+                           std::uint64_t seed, PairProbabilities& out, std::vector<std::vector<int16_t> >& samples) {
+    if ((!e1.empty() && e1.size() != s1.size()) || (!e2.empty() && e2.size() != s2.size()))
+      throw std::runtime_error("ractip_prob: a pseudo-energy vector's length differs from its sequence's");
+    if (problem != RP_SAMPLE_S1 && problem != RP_SAMPLE_S2 && problem != RP_SAMPLE_COFOLD)
+      throw std::runtime_error("ractip_prob: sample one problem: RP_SAMPLE_S1, RP_SAMPLE_S2 or RP_SAMPLE_COFOLD");
+    rp_stack_energy se = {e1.empty() ? nullptr : e1.data(), e2.empty() ? nullptr : e2.data()};
+    rp_sample_opts so = {num, seed, problem};
+    std::vector<int16_t> flat;
+    solve_one(s1, s2, c1, c2, &se, &so, out, &flat);
+    const size_t n = problem == RP_SAMPLE_S1 ? s1.size() : problem == RP_SAMPLE_S2 ? s2.size() : s1.size() + s2.size();
+    samples.assign(n && flat.size() >= n * static_cast<size_t>(num) ? num : 0, std::vector<int16_t>(n));
+    for (size_t k = 0; k < samples.size(); k++) samples[k].assign(flat.begin() + k * n, flat.begin() + (k + 1) * n);
   }
 
   // the same for a whole batch (the shuffles of src/ractip.cpp:1638-1657) in one call
@@ -138,9 +158,11 @@ class ProbabilityStage {
   }
 
  private:
-  // one pair on the context under constraints and, when se is set, stacking pseudo-energies
+  // one pair on the context under constraints and, when se is set, stacking pseudo-energies; when so is set, its
+  // samples (the layout of rp_sample_plan for the one pair) to *samples
   void solve_one(const std::string& s1, const std::string& s2, const std::string& c1, const std::string& c2,
-                 const rp_stack_energy* se, PairProbabilities& out) {
+                 const rp_stack_energy* se, const rp_sample_opts* so, PairProbabilities& out,
+                 std::vector<int16_t>* samples = nullptr) {
     if (!ctx_) throw std::runtime_error("ractip_prob: constrained problems run on a single-device stage");
     rp_pair pair = {s1.data(), static_cast<int>(s1.size()), s2.data(), static_cast<int>(s2.size())};
     rp_constraint con = {c1.empty() ? nullptr : c1.c_str(), c2.empty() ? nullptr : c2.c_str()};
@@ -148,11 +170,19 @@ class ProbabilityStage {
     size_t total = 0;
     check(rp_dense_plan(&pair, 1, &opts_, &lay, &total), ctx_);
     std::vector<float> flat(total ? total : 1);
+    size_t n_samples = 0;
+    if (so) {
+      rp_sample_layout sl;
+      check(rp_sample_plan(&pair, 1, so, &sl, &n_samples), ctx_);
+      samples->assign(n_samples ? n_samples : 1, 0);
+    }
     rp_batch* b = nullptr;
-    check(se ? rp_batch_create_soft(ctx_, &pair, &con, se, 1, &opts_, &b)
-             : rp_batch_create_constrained(ctx_, &pair, &con, 1, &opts_, &b), ctx_);
+    check(so   ? rp_batch_create_sampled(ctx_, &pair, &con, se, 1, &opts_, so, &b)
+          : se ? rp_batch_create_soft(ctx_, &pair, &con, se, 1, &opts_, &b)
+               : rp_batch_create_constrained(ctx_, &pair, &con, 1, &opts_, &b), ctx_);
     int rc = rp_batch_run(b);
     if (!rc) rc = rp_batch_fetch_dense(b, flat.data(), flat.size());
+    if (!rc && so) rc = rp_batch_fetch_samples(b, samples->data(), samples->size());
     rp_batch_destroy(b);
     check(rc, ctx_);
     unpack(pair, lay, flat.data(), out);

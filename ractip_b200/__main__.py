@@ -40,10 +40,17 @@ def main(argv=None) -> int:
     ap.add_argument("--no-bl", action="store_true")
     ap.add_argument("--all-pairs", action="store_true", help="every record of the first file against every record of the second")
     ap.add_argument("--device", type=int, default=0)
+    ap.add_argument("--sample", type=int, default=0, metavar="N",
+                    help="after each pair, N structures sampled from its s1&s2 co-fold ensemble, one r1&r2 per line")
+    ap.add_argument("--sample-seed", type=int, default=1, metavar="S", help="seed of --sample (default 1)")
     args = ap.parse_args(argv)
     if len(args.fasta) > 2:
         ap.error("at most two FASTA files")
     try:
+        if args.sample < 0:
+            raise ValueError(f"--sample {args.sample}: the number of samples cannot be negative")
+        if args.sample and args.duplex:
+            raise ValueError("--sample: --duplex has no co-fold ensemble to sample")
         pairs = input_pairs(args.fasta[0], args.fasta[1] if len(args.fasta) > 1 else None, args.all_pairs)
         if args.use_constraint:
             for a, b in pairs:
@@ -74,7 +81,7 @@ def main(argv=None) -> int:
     try:
         for r in predict(stage, pairs, opts, ipo, args.show_energy, args.zscore, args.num_shuffling, args.seed,
                          use_constraint=args.use_constraint, shape=shape, shape_slope=args.shape_slope,
-                         shape_intercept=args.shape_intercept):
+                         shape_intercept=args.shape_intercept, samples=args.sample, sample_seed=args.sample_seed):
             print(format_result(r, args.show_energy))
     except RpError as e:
         if not (args.use_constraint and e.code == RP_ERR_ARG):

@@ -12,6 +12,7 @@
 #include <algorithm>
 #include <cstdio>
 #include <cstdlib>
+#include <cstring>
 #include <string>
 #include <utility>
 #include <vector>
@@ -71,8 +72,8 @@ struct rp_batch {
   rp::BatchPlan plan;
   // device
   uint8_t* d_seq = nullptr;
-  // per-base data (BatchDev::perbase): BatchPlan::key, then BatchPlan::stack from stack_off doubles on; null when no
-  // problem is constrained or carries pseudo-energies
+  // per-base data (BatchDev::perbase): PerBaseHead, BatchPlan::key, then BatchPlan::stack from stack_off doubles on, then
+  // the sample offsets; null when no problem is constrained, carries pseudo-energies or is sampled
   double* d_perbase = nullptr;
   unsigned stack_off = 0;
   Problem* d_probs = nullptr;
@@ -81,6 +82,7 @@ struct rp_batch {
   float* d_dense = nullptr;
   double* d_logz = nullptr;
   int* d_done = nullptr;      // completion flags of the deferred problems (indexed by problem)
+  int16_t* d_samples = nullptr;   // stochastic samples (BatchPlan::sample_total int16), null when nothing is sampled
   cudaStream_t last_stream = nullptr;   // stream the batch last ran on (rp_set_stream may have moved the context on)
   // sparse
   std::vector<rp_sparse_layout> slayout;
@@ -358,7 +360,8 @@ int rp_batch_destroy(rp_batch* b) {
   if (b->ctx) {
     rp_ctx* ctx = b->ctx;
     for (void* p : {(void*)b->d_seq, (void*)b->d_perbase, (void*)b->d_probs, (void*)b->d_order, (void*)b->d_counter, (void*)b->d_dense,
-                    (void*)b->d_logz, (void*)b->d_done, (void*)b->d_spairs, (void*)b->d_recs, (void*)b->d_ups, (void*)b->d_counts})
+                    (void*)b->d_logz, (void*)b->d_done, (void*)b->d_spairs, (void*)b->d_recs, (void*)b->d_ups, (void*)b->d_counts,
+                    (void*)b->d_samples})
       pool_release(ctx, p);
     ctx->live_batches--;
     if (ctx->closing && ctx->live_batches == 0) {
@@ -374,7 +377,8 @@ int rp_batch_destroy(rp_batch* b) {
 
 namespace {
 int batch_create(const char* who, rp_ctx* ctx, const rp_pair* pairs, const rp_constraint* cons,
-                 const rp_stack_energy* se, int n_pairs, const rp_opts* opts, rp_batch** out) {
+                 const rp_stack_energy* se, int n_pairs, const rp_opts* opts, rp_batch** out,
+                 const rp_sample_opts* so = nullptr) {
   if (!ctx || !out) return fail(ctx, RP_ERR_ARG, "rp_batch_create: null argument");
   *out = nullptr;
   int rc = rp::check_pairs(pairs, n_pairs, opts);
@@ -385,6 +389,7 @@ int batch_create(const char* who, rp_ctx* ctx, const rp_pair* pairs, const rp_co
   std::string msg;
   if ((rc = rp::check_constraints(pairs, cons, n_pairs, &msg)) != RP_OK) return fail(ctx, rc, std::string(who) + ": " + msg);
   if ((rc = rp::check_stack_energies(pairs, se, n_pairs, &msg)) != RP_OK) return fail(ctx, rc, std::string(who) + ": " + msg);
+  if ((rc = rp::check_samples(pairs, n_pairs, opts, so, &msg)) != RP_OK) return fail(ctx, rc, std::string(who) + ": " + msg);
   CU(cudaSetDevice(ctx->device));
   rp_batch* b = new rp_batch;
   b->ctx = ctx;
@@ -393,7 +398,7 @@ int batch_create(const char* who, rp_ctx* ctx, const rp_pair* pairs, const rp_co
   b->opts = *opts;
   b->slayout.resize(n_pairs);
   rp_sparse_plan(pairs, n_pairs, opts, b->slayout.data(), &b->total_recs, &b->total_upf);
-  if (rp::plan_batch(pairs, n_pairs, opts, device_facts(ctx), ctx->route, &b->plan, cons, se) != RP_OK) {
+  if (rp::plan_batch(pairs, n_pairs, opts, device_facts(ctx), ctx->route, &b->plan, cons, se, so) != RP_OK) {
     rp_batch_destroy(b);
     return fail(ctx, RP_ERR_CUDA, "rp_batch_create: band kernel does not fit on this device");
   }
@@ -414,14 +419,33 @@ int batch_create(const char* who, rp_ctx* ctx, const rp_pair* pairs, const rp_co
   if ((e = pool_alloc(ctx, &b->d_logz, std::max<size_t>(1, (size_t)n_pairs * 3) * sizeof(double))) != cudaSuccess) return bail(e, "cudaMalloc logz");
   cudaStream_t st = ctx->stream;
   if ((e = cudaMemcpyAsync(b->d_seq, p.seq.data(), p.seq.size(), cudaMemcpyHostToDevice, st)) != cudaSuccess) return bail(e, "H2D seq");
-  // per-base data only for batches with a constrained problem (keys) or one whose pseudo-energies are not all 0
-  if (!p.key.empty() || !p.stack.empty()) {
-    const size_t kb = p.key.size() * sizeof(uint16_t), fb = p.stack.size() * sizeof(double);
-    b->stack_off = (unsigned)((kb + sizeof(double) - 1) / sizeof(double));
-    if ((e = pool_alloc(ctx, &b->d_perbase, b->stack_off * sizeof(double) + fb)) != cudaSuccess) return bail(e, "cudaMalloc per-base data");
-    if (kb && (e = cudaMemcpyAsync(b->d_perbase, p.key.data(), kb, cudaMemcpyHostToDevice, st)) != cudaSuccess) return bail(e, "H2D key");
-    if (fb && (e = cudaMemcpyAsync(b->d_perbase + b->stack_off, p.stack.data(), fb, cudaMemcpyHostToDevice, st)) != cudaSuccess)
-      return bail(e, "H2D stack");
+  // per-base data only for batches with a constrained problem (keys), one whose pseudo-energies are not all 0, or a
+  // sampled one (the instances that sample are the per-base ones).  One block: PerBaseHead, keys, factors, sample offsets.
+  if (!p.key.empty() || !p.stack.empty() || p.sample_total) {
+    const size_t kd = (p.key.size() * sizeof(uint16_t) + sizeof(double) - 1) / sizeof(double);
+    b->stack_off = (unsigned)(rp::PB_HEAD + kd);
+    std::vector<double> blk(b->stack_off + p.stack.size() + 3 * (size_t)n_pairs, 0.);
+    rp::PerBaseHead h = {};
+    if (p.sample_total) {
+      if ((e = pool_alloc(ctx, &b->d_samples, p.sample_total * sizeof(int16_t))) != cudaSuccess) return bail(e, "cudaMalloc samples");
+      if ((e = cudaMemsetAsync(b->d_samples, 0, p.sample_total * sizeof(int16_t), st)) != cudaSuccess) return bail(e, "memset samples");
+      h.samples = b->d_samples;
+      h.seed = p.sample_seed;
+      h.num = p.sample_num;
+      h.off_doubles = (long long)(b->stack_off + p.stack.size());
+      long long* off = reinterpret_cast<long long*>(blk.data() + h.off_doubles);
+      for (int k = 0; k < n_pairs; k++) {
+        const rp_sample_layout& L = p.sample_layout[k];
+        off[3 * k] = (long long)L.s1; off[3 * k + 1] = (long long)L.s2; off[3 * k + 2] = (long long)L.co;
+      }
+    }
+    std::memcpy(blk.data(), &h, sizeof h);
+    if (!p.key.empty()) std::memcpy(blk.data() + rp::PB_HEAD, p.key.data(), p.key.size() * sizeof(uint16_t));
+    std::copy(p.stack.begin(), p.stack.end(), blk.begin() + b->stack_off);
+    if ((e = pool_alloc(ctx, &b->d_perbase, blk.size() * sizeof(double))) != cudaSuccess) return bail(e, "cudaMalloc per-base data");
+    if ((e = cudaMemcpyAsync(b->d_perbase, blk.data(), blk.size() * sizeof(double), cudaMemcpyHostToDevice, st)) != cudaSuccess)
+      return bail(e, "H2D per-base data");
+    if ((e = cudaStreamSynchronize(st)) != cudaSuccess) return bail(e, "sync");   // blk is released at the end of the block
   }
   if (np) {
     if ((e = cudaMemcpyAsync(b->d_probs, p.probs.data(), np * sizeof(Problem), cudaMemcpyHostToDevice, st)) != cudaSuccess) return bail(e, "H2D probs");
@@ -452,6 +476,11 @@ int rp_batch_create_constrained(rp_ctx* ctx, const rp_pair* pairs, const rp_cons
 int rp_batch_create_soft(rp_ctx* ctx, const rp_pair* pairs, const rp_constraint* cons, const rp_stack_energy* se,
                          int n_pairs, const rp_opts* opts, rp_batch** out) {
   return batch_create("rp_batch_create_soft", ctx, pairs, cons, se, n_pairs, opts, out);
+}
+
+int rp_batch_create_sampled(rp_ctx* ctx, const rp_pair* pairs, const rp_constraint* cons, const rp_stack_energy* se,
+                            int n_pairs, const rp_opts* opts, const rp_sample_opts* so, rp_batch** out) {
+  return batch_create("rp_batch_create_sampled", ctx, pairs, cons, se, n_pairs, opts, out, so);
 }
 
 int rp_batch_run(rp_batch* b) {
@@ -545,9 +574,9 @@ int rp_batch_run(rp_batch* b) {
     long long h[64];
     CU(cudaMemcpyAsync(h, ctx->d_prof, sizeof h, cudaMemcpyDeviceToHost, st));
     CU(cudaStreamSynchronize(st));
-    static const char* names[32] = {"stage", "prologue", "prologue2", "inside_A", "inside_B", "generic_in", "generic_out", "outside_A", "outside_B", "write_bp", "un_items", "un_domrows", "un_domcols", "un_windows", "write_hp", "logz", "band_A", "band_B", "collect", "", "", "", "", "", "finish_in.loads(t0)", "finish_in.rest(t0)", "bandA_in.head(t0)", "bandA_in.main(t0)", "bandA_in.tail(t0)", "bandA_out.PR(t0)", "bandA_out.need(t0)", "bandA_out.ML(t0)"};
+    static const char* names[32] = {"stage", "prologue", "prologue2", "inside_A", "inside_B", "generic_in", "generic_out", "outside_A", "outside_B", "write_bp", "un_items", "un_domrows", "un_domcols", "un_windows", "write_hp", "logz", "band_A", "band_B", "collect", "sample", "", "", "", "", "finish_in.loads(t0)", "finish_in.rest(t0)", "bandA_in.head(t0)", "bandA_in.main(t0)", "bandA_in.tail(t0)", "bandA_out.PR(t0)", "bandA_out.need(t0)", "bandA_out.ML(t0)"};
     long long tot = 0;
-    for (int k = 0; k < 19; k++) tot += h[k];   // the phase counters (PH_COUNT, mcc_driver.h)
+    for (int k = 0; k < 20; k++) tot += h[k];   // the phase counters (PH_COUNT, mcc_driver.h)
     for (int k = 0; k < 32; k++)
       if (h[32 + k]) std::fprintf(stderr, "[rp_profile] %-11s %6.2f%%  calls %9lld  cycles/call %9.0f\n", names[k], 100.0 * h[k] / tot, h[32 + k], (double)h[k] / h[32 + k]);
   }
@@ -656,6 +685,33 @@ extern "C" int rp_batch_dense_device(rp_batch* b, void* out_dev, size_t out_floa
   int rc = order_after_run(b);
   if (rc) return rc;
   CU(cudaMemcpyAsync(out_dev, b->d_dense, p.total_floats * sizeof(float), cudaMemcpyDeviceToDevice, ctx->stream));
+  return RP_OK;
+}
+
+extern "C" int rp_batch_samples_device(rp_batch* b, void* out_dev, size_t n) {
+  if (!b || !out_dev) return RP_ERR_ARG;
+  rp_ctx* ctx = b->ctx;
+  const rp::BatchPlan& p = b->plan;
+  if (n < p.sample_total) return fail(ctx, RP_ERR_CAPACITY, "rp_batch_samples_device: buffer too small");
+  CU(cudaSetDevice(ctx->device));
+  if (!p.sample_total) return RP_OK;
+  int rc = order_after_run(b);
+  if (rc) return rc;
+  CU(cudaMemcpyAsync(out_dev, b->d_samples, p.sample_total * sizeof(int16_t), cudaMemcpyDeviceToDevice, ctx->stream));
+  return RP_OK;
+}
+
+extern "C" int rp_batch_fetch_samples(rp_batch* b, int16_t* out, size_t n) {
+  if (!b || !out) return RP_ERR_ARG;
+  rp_ctx* ctx = b->ctx;
+  const rp::BatchPlan& p = b->plan;
+  if (n < p.sample_total) return fail(ctx, RP_ERR_CAPACITY, "rp_batch_fetch_samples: buffer too small");
+  CU(cudaSetDevice(ctx->device));
+  if (!p.sample_total) return RP_OK;
+  int rc = order_after_run(b);
+  if (rc) return rc;
+  CU(cudaMemcpyAsync(out, b->d_samples, p.sample_total * sizeof(int16_t), cudaMemcpyDeviceToHost, ctx->stream));
+  CU(cudaStreamSynchronize(ctx->stream));
   return RP_OK;
 }
 

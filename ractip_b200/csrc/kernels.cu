@@ -56,8 +56,15 @@ using CtaExec = CtaExecT<>;
 
 template <bool PB>
 __device__ __forceinline__ void bind_per_base(Ctx& c, const BatchDev& b, const Problem& p) {
-  if (PB && (p.constrained & CON_KEYS)) c.key = static_cast<const uint16_t*>(b.perbase) + p.seq_off - 1;
-  if (PB && (p.constrained & CON_STACK)) c.stk = static_cast<const double*>(b.perbase) + b.stack_off + p.seq_off - 1;
+  const double* pb = static_cast<const double*>(b.perbase);
+  if (PB && (p.constrained & CON_KEYS)) c.key = reinterpret_cast<const uint16_t*>(pb + PB_HEAD) + p.seq_off - 1;
+  if (PB && (p.constrained & CON_STACK)) c.stk = pb + b.stack_off + p.seq_off - 1;
+  if (PB && (p.constrained & CON_SAMPLE)) {
+    const PerBaseHead& h = *reinterpret_cast<const PerBaseHead*>(pb);
+    c.smp = h.samples + reinterpret_cast<const long long*>(pb + h.off_doubles)[(size_t)p.pair * 3 + p.which];
+    c.smp_seed = h.seed;
+    c.smp_num = (int)h.num;
+  }
 }
 
 // Instantiated for two register budgets: <2> two CTAs per SM at 64 registers (many short problems
@@ -66,8 +73,8 @@ __device__ __forceinline__ void bind_per_base(Ctx& c, const BatchDev& b, const P
 // as many problem histories compete for the L2).
 // <1, W> with W > BAND sums the split sums in wide bands (solve_mcc_wide): W-fold reuse of every element
 // streamed from HBM.
-// PB: the batch has per-base data (BatchDev::perbase), structure-constraint keys or stacking pseudo-energies; each
-// problem binds what it carries.  The instances without compile both out (Ctx::key and Ctx::stk stay null), so that
+// PB: the batch has per-base data (BatchDev::perbase): structure-constraint keys, stacking pseudo-energies or samples
+// (PerBaseHead); each problem binds what it carries.  The instances without compile all out (Ctx::key, Ctx::stk and Ctx::smp stay null), so that
 // unconstrained batches run exactly the code they ran before constraints existed.
 template <int MINB, int W, bool PB>
 __global__ void __launch_bounds__(RP_MCC_THREADS, MINB) mcc_persistent(BatchDev b) {

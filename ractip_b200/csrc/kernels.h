@@ -31,11 +31,23 @@ struct BatchDev {
   long long* prof;         // 64 counters (cycles, calls per phase id) or null
   int dbg;                 // RP_DEBUG_SKIP bits (tuning aid; results are wrong when set)
   unsigned stack_off;      // doubles from perbase to the stacking factors
-  // Per-base data of the batch, or null: structure-constraint keys (uint16) laid out like seq at the start
-  // (Problem::constrained & CON_KEYS), stacking pseudo-energy factors (double) laid out like seq at stack_off
-  // (CON_STACK).  One pointer, so that the parameter block of every kernel keeps the layout it had before factors.
+  // Per-base data of the batch, or null: a PerBaseHead (below), structure-constraint keys (uint16) laid out like seq
+  // after it (Problem::constrained & CON_KEYS), stacking pseudo-energy factors (double) laid out like seq at stack_off
+  // (CON_STACK), the sample offsets.  One pointer, so that the parameter block of every kernel keeps the layout it had
+  // before factors and samples.
   const void* perbase;
 };
+
+// Head of the per-base block (BatchDev::perbase): the batch's stochastic samples (Problem::constrained & CON_SAMPLE):
+// `num` pair tables per sampled problem, problem `which` of pair p at samples + off[3p + which] (rp_sample_plan), where
+// off = (const long long*)perbase + off_doubles.  The structure-constraint keys follow the head, at PB_HEAD doubles.
+struct PerBaseHead {
+  int16_t* samples;   // null: nothing sampled
+  unsigned long long seed;
+  long long off_doubles;
+  long long num;
+};
+constexpr int PB_HEAD = sizeof(PerBaseHead) / sizeof(double);
 
 struct SparsePair {
   int n1, n2;

@@ -59,7 +59,7 @@ struct Problem {
   int max_w;
   int n1, n2;
   int constrained;    // general kernel only, bits (BatchDev::perbase): CON_KEYS a structure constraint removes some
-                      // pairs, CON_STACK stacking pseudo-energies weight its stacks
+                      // pairs, CON_STACK stacking pseudo-energies weight its stacks, CON_SAMPLE structures are sampled
   long long out_bp;   // float offsets into the dense output, -1 if absent
   long long out_up;
   long long out_hp;
@@ -67,7 +67,7 @@ struct Problem {
   int defer_up;       // 1: the unpaired-window pass runs later in its own kernel (unstru_kernel) on the tables left in ws_off
   long long ws_off;   // >= 0: private workspace (doubles from BatchDev::ws_up) that outlives the wavefront kernel; -1: the CTA's slot
 };
-enum { CON_KEYS = 1, CON_STACK = 2 };
+enum { CON_KEYS = 1, CON_STACK = 2, CON_SAMPLE = 4 };
 // queue entries: problem index, + RP_JOB_UNPAIRED for the unpaired-window pass of a deferred problem as a job of its own
 constexpr int RP_JOB_UNPAIRED = 0x40000000;
 
@@ -107,6 +107,11 @@ struct Ctx {
   long long* prof;    // RP_PROFILE counters (slots 40..: fine-grained probes of thread 0) or null
   const uint16_t* key;   // key[1..n] of a constrained problem (pair (i,j) allowed iff key[i] == key[j]), else null
   const double* stk;     // stk[1..n]: per-base factors exp(-E/kT) of stacking pseudo-energies (CON_STACK), else null
+  // stochastic sampling (CON_SAMPLE, mcc_sample.h): smp_num pair tables of n int16 at smp, drawn with seed smp_seed;
+  // smp null: none (the instances without per-base data know it and compile the sampling phase away)
+  int16_t* smp;
+  unsigned long long smp_seed;
+  int smp_num;
   // Tables whose rows are only read while they are recent are RINGS of a few rows (row d at d & mask):
   // PR/PL/PMLB are read one diagonal after they are written, the band results QS/PRB/MLB within a
   // band.  A full table would leave every written line behind in L2, where it pushes out the history
@@ -137,6 +142,9 @@ RP_HD void bind_ctx(Ctx& c, const DevModel* M, const uint8_t* S, const Problem& 
   c.prof = nullptr;
   c.key = nullptr;
   c.stk = nullptr;
+  c.smp = nullptr;
+  c.smp_seed = 0;
+  c.smp_num = 0;
 }
 #define TB(c, t, d, i) ((c).tb(t, d, i))
 // store of a value that is not read again soon (qb, out, class tables, outputs): evict-first, so that

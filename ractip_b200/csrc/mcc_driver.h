@@ -27,6 +27,7 @@
 
 #include "mcc_band.h"
 #include "mcc_core.h"
+#include "mcc_sample.h"
 // (the host emulation defines RP_HOST_SHFL and host stand-ins for the warp intrinsics to run the shuffle forms)
 #if defined(__CUDACC__) || defined(RP_HOST_SHFL)
 #define RP_SHFL_FORMS 1
@@ -39,7 +40,7 @@ namespace rp {
 enum {
   PH_STAGE = 0, PH_PROLOGUE, PH_PROLOGUE2, PH_INSIDE_A, PH_INSIDE_B, PH_GENERIC_IN, PH_GENERIC_OUT, PH_OUTSIDE_A, PH_OUTSIDE_B,
   PH_WRITE_BP, PH_UN_ITEMS, PH_UN_DOMROWS, PH_UN_DOMCOLS, PH_UN_WINDOWS,
-  PH_WRITE_HP, PH_LOGZ, PH_BAND_A, PH_BAND_B, PH_CFAC, PH_COUNT
+  PH_WRITE_HP, PH_LOGZ, PH_BAND_A, PH_BAND_B, PH_CFAC, PH_SAMPLE, PH_COUNT
 };
 
 // number of CTAs that share one problem under executor Exec
@@ -111,6 +112,26 @@ RP_HD void emit_logz(Exec& ex, Ctx& c, const Problem& p, double* logz) {
   }
   ex.phase(PH_LOGZ, [&](int tid) {
     if (tid == 0) logz[(size_t)p.pair * 3 + p.which] = log(TB(c, T_Q, c.n - 1, 1)) + c.n * log(c.M->pf_scale);
+  });
+}
+
+// Stochastic samples of a problem whose inside pass is finished (Ctx::smp, mcc_sample.h): the pair tables are cleared,
+// then each warp of the problem (at most te / (n+2) of them, the room in T_RR for their pending segments) takes samples
+// w, w + nw, ...: the shuffle form on all 32 lanes when Exec::kShfl, else the direct form on lane 0.
+template <class Exec>
+RP_HD void emit_samples(Exec& ex, Ctx& c, const Problem& p) {
+  const int n = c.n, num = c.smp_num;
+  int16_t* out = c.smp;
+  flat(ex, PH_SAMPLE, [&](int, int gt, int GT) {
+    for (size_t x = gt; x < (size_t)num * n; x += GT) out[x] = 0;
+  });
+  const int cap = (int)(c.te / (unsigned)(n + 2));
+  flat(ex, PH_SAMPLE, [&](int, int gt, int GT) {
+    constexpr bool shfl = ShflOf<Exec>::value;
+    const int nw = GT / 32 < cap ? GT / 32 : cap, w = gt / 32, lane = gt & 31;
+    if (w >= nw || (!shfl && lane)) return;
+    uint64_t* stk = reinterpret_cast<uint64_t*>(c.ptr(T_RR, 0, 0)) + (size_t)w * (n + 2);
+    for (int s = w; s < num; s += nw) sample_one<shfl>(c, c.smp_seed, p.pair, p.which, s, out + (size_t)s * n, stk, lane);
   });
 }
 
@@ -239,6 +260,7 @@ RP_HD void solve_mcc(Exec& ex, Ctx& c, const Problem& p, float* dense, double* l
   }
   inside_end(c);
   emit_logz(ex, c, p, logz);
+  if (c.smp) emit_samples(ex, c, p);
 
   // ---- outside: longest spans first
   // (two strands: only the inter-strand cells of a diagonal, no nick sums -- cross_lo / cross_hi in mcc_core.h)
@@ -317,6 +339,7 @@ RP_HD void solve_mcc_wide(Exec& ex, Ctx& c, const Problem& p, float* dense, doub
   }
   inside_end(c);
   emit_logz(ex, c, p, logz);
+  if (c.smp) emit_samples(ex, c, p);
 
   for (int d = n - 1; d >= TURN + 1; d--) {
     if (d == wide_start_outside<W>(n, d)) split_sums_outside<W>(ex, c, sh, d);

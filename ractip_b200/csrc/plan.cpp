@@ -110,6 +110,38 @@ int check_stack_energies(const rp_pair* pairs, const rp_stack_energy* se, int n_
   return RP_OK;
 }
 
+int check_samples(const rp_pair* pairs, int n_pairs, const rp_opts* opts, const rp_sample_opts* so, std::string* msg) {
+  if (!so) return RP_OK;
+  char buf[160];
+  if (so->num < 0) {
+    std::snprintf(buf, sizeof buf, "sample count %d is negative", so->num);
+    if (msg) *msg = buf;
+    return RP_ERR_ARG;
+  }
+  if (so->problems & ~(RP_SAMPLE_S1 | RP_SAMPLE_S2 | RP_SAMPLE_COFOLD)) {
+    std::snprintf(buf, sizeof buf, "unknown bits 0x%x in the sampled problems", so->problems & ~7);
+    if (msg) *msg = buf;
+    return RP_ERR_ARG;
+  }
+  if (so->num > 0) {   // the sample buffer's size, and its size in bytes, must fit size_t (rp_sample_plan)
+    std::vector<rp_sample_layout> lay(n_pairs > 0 ? n_pairs : 1);
+    size_t total = 0;
+    if (rp_sample_plan(pairs, n_pairs, so, lay.data(), &total) != RP_OK) {
+      std::snprintf(buf, sizeof buf, "%d samples of the requested problems overflow the sample buffer's size", so->num);
+      if (msg) *msg = buf;
+      return RP_ERR_ARG;
+    }
+  }
+  if (so->num > 0 && (so->problems & RP_SAMPLE_COFOLD) && opts->use_pf_duplex)
+    for (int p = 0; p < n_pairs; p++)
+      if (pairs[p].n2 > 0) {
+        std::snprintf(buf, sizeof buf, "pair %d: --duplex has no co-fold ensemble to sample", p);
+        if (msg) *msg = buf;
+        return RP_ERR_UNSUPPORTED;
+      }
+  return RP_OK;
+}
+
 namespace {
 // Stacking factors of one strand of length m from its pseudo-energies e[0..m-1] (kcal/mol): each value rounded to an
 // integer number of 0.01 kcal/mol, half away from zero (as ViennaRNA stores soft-constraint energies), then
@@ -231,6 +263,30 @@ int rp_square_plan(const rp_pair* pairs, int n_pairs, const rp_opts* opts, rp_sq
   return RP_OK;
 }
 
+int rp_sample_plan(const rp_pair* pairs, int n_pairs, const rp_sample_opts* so, rp_sample_layout* per_pair, size_t* total) {
+  if (!pairs || n_pairs < 0 || !so || so->num < 0 || !total || (n_pairs > 0 && !per_pair)) return RP_ERR_ARG;
+  size_t off = 0;
+  bool overflow = false;
+  // num pair tables of n int16 each, or none; the running offset and its size in bytes must fit size_t
+  auto take = [&](bool on, size_t n, size_t* at, size_t* len) {
+    size_t m = 0;
+    if (on) overflow |= __builtin_mul_overflow((size_t)so->num, n, &m);
+    *at = off;
+    *len = m;
+    overflow |= __builtin_add_overflow(off, m, &off) || off > SIZE_MAX / sizeof(int16_t);
+  };
+  for (int p = 0; p < n_pairs; p++) {
+    const size_t n1 = (size_t)std::max(pairs[p].n1, 0), n2 = (size_t)std::max(pairs[p].n2, 0);
+    rp_sample_layout& L = per_pair[p];
+    take((so->problems & RP_SAMPLE_S1) != 0, n1, &L.s1, &L.len_s1);
+    take((so->problems & RP_SAMPLE_S2) != 0, n2, &L.s2, &L.len_s2);
+    take((so->problems & RP_SAMPLE_COFOLD) != 0 && n2 > 0, n1 + n2, &L.co, &L.len_co);
+  }
+  if (overflow) return RP_ERR_ARG;
+  *total = off;
+  return RP_OK;
+}
+
 int rp_shape_deigan(const double* r, int n, double slope, double intercept, double* e) {
   if (n < 0 || (n > 0 && (!r || !e))) return RP_ERR_ARG;
   for (int i = 0; i < n; i++) e[i] = r[i] >= 0. ? slope * std::log(r[i] + 1.) + intercept : 0.;   // r < 0, NaN: missing
@@ -309,9 +365,16 @@ static double alg_flops_mcc_uncached(int n) {
 namespace rp {
 
 int plan_batch(const rp_pair* pairs, int n_pairs, const rp_opts* opts, const DeviceFacts& dev, const RouteSettings& rs,
-               BatchPlan* out, const rp_constraint* cons, const rp_stack_energy* se) {
+               BatchPlan* out, const rp_constraint* cons, const rp_stack_energy* se, const rp_sample_opts* so) {
   BatchPlan& b = *out;
   b = BatchPlan{};
+  // sampled problems (CON_SAMPLE): those with room in the sample buffer
+  if (so && so->num > 0) {
+    b.sample_layout.resize(n_pairs);
+    rp_sample_plan(pairs, n_pairs, so, b.sample_layout.data(), &b.sample_total);   // cannot fail: check_samples
+    b.sample_num = so->num;
+    b.sample_seed = so->seed;
+  }
   size_t mem = 0;   // DeviceFacts::memory, asked once
   auto memory = [&]() {
     if (!mem) mem = std::max<size_t>(1, dev.memory());
@@ -388,10 +451,13 @@ int plan_batch(const rp_pair* pairs, int n_pairs, const rp_opts* opts, const Dev
     q.ws_off = -1;
     // rnafold(fa1, ...), rnafold(fa2, ...)  src/ractip.cpp:546-547
     Problem a = q;
+    const rp_sample_layout* sl = b.sample_total ? &b.sample_layout[p] : nullptr;
     a.kind = KIND_LINEAR; a.which = 0; a.seq_off = off1; a.n = pr.n1; a.cp = 0; a.constrained = con[0] | stk[0];
+    if (sl && sl->len_s1) a.constrained |= CON_SAMPLE;
     a.out_bp = (long long)L.bp1; a.out_up = w > 0 ? (long long)L.up1 : -1;
     b.probs.push_back(a);
     a.which = 1; a.seq_off = off2; a.n = pr.n2; a.constrained = con[1] | stk[1];
+    if (sl && sl->len_s2) a.constrained |= CON_SAMPLE;
     a.out_bp = (long long)L.bp2; a.out_up = w > 0 ? (long long)L.up2 : -1;
     b.probs.push_back(a);
     if (pr.n2 == 0) {   // a lone sequence (RactIP::rnafold on its own, src/ractip.cpp:1599-1601): no second fold, no hybridization
@@ -411,6 +477,7 @@ int plan_batch(const rp_pair* pairs, int n_pairs, const rp_opts* opts, const Dev
       ws_need = std::max(ws_need, 2 * (size_t)(pr.n1 + 2) * (size_t)(pr.n2 + 2));
     } else {
       c.kind = KIND_COFOLD; c.n = pr.n1 + pr.n2; c.cp = pr.n1 + 1; c.constrained = con[2] | stk[0] | stk[1];
+      if (sl && sl->len_co) c.constrained |= CON_SAMPLE;
       b.alg_flops += rp_alg_flops_mcc(c.n);
     }
     b.probs.push_back(c);
@@ -422,7 +489,7 @@ int plan_batch(const rp_pair* pairs, int n_pairs, const rp_opts* opts, const Dev
   else std::vector<double>().swap(stack);
 
   // Band class of a problem: 0 = L (512 threads, ring needs more than half an SM), 1 = S (256 threads, 2 CTAs/SM),
-  // -1 = the general kernel, which alone applies structure constraints and stacking pseudo-energies.
+  // -1 = the general kernel, which alone applies structure constraints and stacking pseudo-energies and samples.
   auto cls = [&](const Problem& q) {
     if (!rs.band || q.kind == KIND_DUPLEX || q.constrained) return -1;
     const int k = rp_kernel_plan(q.n, dev.smem_optin, nullptr);

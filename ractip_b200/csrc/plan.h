@@ -53,6 +53,11 @@ struct BatchPlan {
   // elsewhere; empty when no problem of the batch does
   std::vector<double> stack;
   std::vector<Problem> probs;            // three per pair: s1, s2, s1&s2
+  // stochastic samples (rp_sample_plan), empty / 0 when no problem is sampled
+  std::vector<rp_sample_layout> sample_layout;
+  size_t sample_total = 0;               // int16 elements
+  int sample_num = 0;
+  uint64_t sample_seed = 0;
   std::vector<rp_dense_layout> layout;
   size_t total_floats = 0;
   bool has_single = false;               // some pair has n2 == 0: its unused output sections are zero-filled once
@@ -102,12 +107,17 @@ int check_constraints(const rp_pair* pairs, const rp_constraint* cons, int n_pai
 // message in *msg that names the pair, the vector and the (1-based) position of a value that is not finite.
 int check_stack_energies(const rp_pair* pairs, const rp_stack_energy* se, int n_pairs, std::string* msg);
 
-// The pairs must pass check_pairs, the constraints check_constraints (cons == null: none) and the stacking
-// pseudo-energies check_stack_energies (se == null: none).  A problem that a constraint restricts, or whose rounded
-// pseudo-energies are not all 0, runs on the general kernel.  Returns RP_OK, or RP_ERR_CUDA when a band launch shape
-// fits no SM.
+// The sampling options of pairs that pass check_pairs (so may be null: none).  RP_OK; RP_ERR_ARG for a negative count
+// or an unknown problem bit; RP_ERR_UNSUPPORTED, naming the pair, for a co-fold sample under --duplex.
+int check_samples(const rp_pair* pairs, int n_pairs, const rp_opts* opts, const rp_sample_opts* so, std::string* msg);
+
+// The pairs must pass check_pairs, the constraints check_constraints (cons == null: none), the stacking
+// pseudo-energies check_stack_energies (se == null: none) and the sampling options check_samples (so == null or
+// so->num == 0: none).  A problem that a constraint restricts, whose rounded pseudo-energies are not all 0, or that is
+// sampled runs on the general kernel.  Returns RP_OK, or RP_ERR_CUDA when a band launch shape fits no SM.
 int plan_batch(const rp_pair* pairs, int n_pairs, const rp_opts* opts, const DeviceFacts& dev, const RouteSettings& rs,
-               BatchPlan* plan, const rp_constraint* cons = nullptr, const rp_stack_energy* se = nullptr);
+               BatchPlan* plan, const rp_constraint* cons = nullptr, const rp_stack_energy* se = nullptr,
+               const rp_sample_opts* so = nullptr);
 
 }  // namespace rp
 #endif

@@ -22,7 +22,7 @@ import numpy as np
 from . import _lib
 from ._lib import RpIpOpts, RpModel, RpOpts
 from .ip import JointPrediction, default_ip_opts, solve_joint, solve_ss, zscore_statistic
-from .stage import ProbabilityStage, RpError, default_opts, shape_deigan, zscore_shuffles
+from .stage import ProbabilityStage, RpError, default_opts, joint_structure, shape_deigan, zscore_shuffles
 
 
 @dataclass
@@ -143,6 +143,7 @@ class PairResult:
     e1s: Optional[float] = None   # solve_ss energies (for -e and the z-score)
     e2s: Optional[float] = None
     zscore: Optional[Tuple[float, float]] = None
+    samples: Optional[List[Tuple[str, str]]] = None   # co-fold samples (r1, r2) in RactIP's notation (predict(samples=))
 
 
 def _f(x: float) -> str:
@@ -160,20 +161,24 @@ def format_result(r: PairResult, show_energy: bool = False) -> str:
                    f"S1+S2= {_f(r.e1s + r.e2s)} = {_f(r.e1s)}{sg(r.e2s)})")
     if r.zscore is not None:
         out.append(f"z-score: {_f(r.zscore[0])}, {_f(r.zscore[1])}")
+    out.extend(f"{r1}&{r2}" for r1, r2 in r.samples or [])
     return "\n".join(out)
 
 
 def predict(stage: ProbabilityStage, pairs: Sequence[Tuple[FastaRecord, FastaRecord]], opts: Optional[RpOpts] = None,
             ip_opts: Optional[RpIpOpts] = None, show_energy: bool = False, zscore: int = 0, num_shuffling: int = 1000,
             seed: int = 1, use_constraint: bool = False, shape: Optional[Dict[str, Sequence[float]]] = None,
-            shape_slope: float = 1.8, shape_intercept: float = -0.6) -> List[PairResult]:
+            shape_slope: float = 1.8, shape_intercept: float = -0.6, samples: int = 0,
+            sample_seed: int = 1) -> List[PairResult]:
     """Joint structures of all `pairs`: one GPU batch for every pair's matrices, then the integer programmes on the
     host.  zscore in (1, 2, 12): per pair one more GPU batch with all its dinucleotide shuffles (the loop of
     src/ractip.cpp:1636-1657 with the probability work hoisted out of it).  use_constraint (-c): the records'
     structure lines constrain the pairs' probability matrices (constraint_line); shuffles have no structure line and
     stay unconstrained.  shape: probing reactivities by record name (read_shape), turned into stacking
     pseudo-energies by shape_deigan(shape_slope, shape_intercept) for every record of that name; they bias the
-    probability matrices only, not the energies of -e, and the shuffles carry none."""
+    probability matrices only, not the energies of -e, and the shuffles carry none.  samples > 0: that many structures
+    of each pair's s1&s2 co-fold ensemble (constraints and pseudo-energies included), drawn with sample_seed in the
+    same GPU batch, on PairResult.samples; the shuffles are never sampled."""
     opts = opts if opts is not None else default_opts()
     ip_opts = ip_opts if ip_opts is not None else default_ip_opts()
     model: RpModel = stage.model
@@ -187,10 +192,24 @@ def predict(stage: ProbabilityStage, pairs: Sequence[Tuple[FastaRecord, FastaRec
             raise ValueError(f"reactivities for {', '.join(sorted(unknown))}: no such record")
         de = lambda r: shape_deigan(shape[r.name], shape_slope, shape_intercept) if r.name in shape else None
         kw["stack_energies"] = [(de(a), de(b)) for a, b in pairs]
-    probs = stage.run_dense(seqs, opts, constraints=cons, **kw)
+    drawn = None
+    if samples:
+        bt = stage.batch(seqs, opts, cons, kw.get("stack_energies"), samples=samples, sample_seed=sample_seed,
+                         sample_problems=("co",))
+        try:
+            bt.run()
+            probs = bt.split_dense(bt.fetch_dense())
+            drawn = [[joint_structure(t, len(a.seq)) for t in d["co"]] if "co" in d else []
+                     for d, (a, _) in zip(bt.fetch_samples(), pairs)]
+        finally:
+            bt.close()
+    else:
+        probs = stage.run_dense(seqs, opts, constraints=cons, **kw)
     out = []
-    for (a, b), p in zip(pairs, probs):
+    for k, ((a, b), p) in enumerate(zip(pairs, probs)):
         res = PairResult(a, b, solve_joint(model, a.seq, b.seq, p, ip_opts, energies=energies))
+        if drawn is not None:
+            res.samples = drawn[k]
         if energies:
             _, _, res.e1s = solve_ss(model, a.seq, p.bp1, ip_opts, energy=True)
             _, _, res.e2s = solve_ss(model, b.seq, p.bp2, ip_opts, energy=True)

@@ -21,8 +21,8 @@ from typing import Dict, List, Optional, Sequence, Tuple
 import numpy as np
 
 from . import _lib
-from ._lib import (RpConstraint, RpDenseLayout, RpModel, RpOpts, RpPair, RpRec, RpSparseCounts,
-                   RpSparseLayout, RpSquareLayout, RpStackEnergy, RpTiming)
+from ._lib import (RpConstraint, RpDenseLayout, RpModel, RpOpts, RpPair, RpRec, RpSampleLayout, RpSampleOpts,
+                   RpSparseCounts, RpSparseLayout, RpSquareLayout, RpStackEnergy, RpTiming)
 
 
 class RpError(RuntimeError):
@@ -150,15 +150,55 @@ def shape_deigan(reactivities, slope: float = 1.8, intercept: float = -0.6) -> n
     return e
 
 
+# problem names of sample_problems= and the keys of fetch_samples() / sample_tensors(), with their RP_SAMPLE_* bits
+SAMPLE_BITS = {"s1": 1, "s2": 2, "co": 4}
+
+
+def sample_opts(num: int, seed: int = 1, problems: Sequence[str] = ("s1", "s2", "co")) -> RpSampleOpts:
+    """rp_sample_opts: `num` samples of each of `problems` ("s1", "s2", "co"), drawn with `seed`."""
+    bits = 0
+    for name in problems:
+        if name not in SAMPLE_BITS:
+            raise ValueError(f"sample_problems: unknown problem {name!r} (s1, s2 or co)")
+        bits |= SAMPLE_BITS[name]
+    return RpSampleOpts(int(num), int(seed) & (2 ** 64 - 1), bits)
+
+
+def dot_bracket(table) -> str:
+    """Dot-bracket string of a pair table (t[k-1] = 1-based partner of base k, 0 unpaired)."""
+    t = np.asarray(table)
+    return "".join("." if p == 0 else ("(" if p > k + 1 else ")") for k, p in enumerate(t.tolist()))
+
+
+def joint_structure(co_table, n1: int) -> Tuple[str, str]:
+    """A co-fold sample (pair table over s1 s2, s2's base b at n1 + b) in RactIP's notation for a joint structure:
+    () intramolecular, [ in s1 and ] in s2 for a pair that joins the strands (the k-th [ from the 3' end of s1 with the
+    k-th ] from the 5' end of s2).  The result is a valid -c constraint line for the pair."""
+    t = np.asarray(co_table).tolist()
+    out = []
+    for k, p in enumerate(t, start=1):
+        if p == 0:
+            out.append(".")
+        elif (k <= n1) != (p <= n1):
+            out.append("[" if k <= n1 else "]")
+        else:
+            out.append("(" if p > k else ")")
+    s = "".join(out)
+    return s[:n1], s[n1:]
+
+
 class DeviceBatch:
     """A batch whose inputs are resident in HBM (rp_batch_*).  constraints: None, or one (c1, c2) per pair -- the
     structure constraints of rp_batch_create_constrained, either string (or the whole entry) None for none.
     stack_energies: None, or one (e1, e2) per pair -- stacking pseudo-energies in kcal/mol over s1 and s2
-    (rp_batch_create_soft, e.g. from shape_deigan), either array (or the whole entry) None for none."""
+    (rp_batch_create_soft, e.g. from shape_deigan), either array (or the whole entry) None for none.
+    samples > 0: every run also draws that many structures of each of sample_problems ("s1", "s2", "co") with
+    sample_seed (rp_batch_create_sampled); fetch_samples() and sample_tensors() return them."""
 
     def __init__(self, stage: "ProbabilityStage", pairs: Sequence[Tuple[str, str]], opts: RpOpts,
                  constraints: Optional[Sequence[Optional[Tuple[Optional[str], Optional[str]]]]] = None,
-                 stack_energies=None):
+                 stack_energies=None, samples: int = 0, sample_seed: int = 1,
+                 sample_problems: Sequence[str] = ("s1", "s2", "co")):
         self.stage, self.lib, self.opts = stage, stage.lib, opts
         self.pairs = list(pairs)
         self.n = len(self.pairs)
@@ -172,7 +212,20 @@ class DeviceBatch:
         stage._check(self.lib.rp_sparse_plan(arr, self.n, C.byref(opts), self.slayout, C.byref(tr), C.byref(tf)))
         self.total_recs, self.total_upf = tr.value, tf.value
         self.handle = C.c_void_p()
-        if stack_energies is not None:
+        self.samples = int(samples)
+        self.sample_layout = (RpSampleLayout * max(self.n, 1))()
+        self.total_samples = 0
+        if self.samples != 0:
+            so = sample_opts(self.samples, sample_seed, sample_problems)
+            cons, ckeep = _make_constraints(constraints, self.n) if constraints is not None else (None, None)
+            se, ekeep = (_make_stack_energies(stack_energies, self.pairs) if stack_energies is not None
+                         else (None, None))
+            stage._check(self.lib.rp_batch_create_sampled(stage.ctx, arr, cons, se, self.n, C.byref(opts),
+                                                          C.byref(so), C.byref(self.handle)))
+            ts = C.c_size_t()
+            stage._check(self.lib.rp_sample_plan(arr, self.n, C.byref(so), self.sample_layout, C.byref(ts)))
+            self.total_samples = ts.value
+        elif stack_energies is not None:
             cons, ckeep = _make_constraints(constraints, self.n) if constraints is not None else (None, None)
             se, ekeep = _make_stack_energies(stack_energies, self.pairs)
             stage._check(self.lib.rp_batch_create_soft(stage.ctx, arr, cons, se, self.n, C.byref(opts),
@@ -214,6 +267,44 @@ class DeviceBatch:
         lz = np.zeros((max(self.n, 1), 3))
         self.stage._check(self.lib.rp_batch_fetch_logz(self.handle, lz.ctypes.data, lz.size))
         return lz[:self.n]
+
+    def fetch_samples(self) -> List[Dict[str, np.ndarray]]:
+        """The samples of the last run: per pair, {problem: int16 [num, n]} for each sampled problem ("s1", "s2",
+        "co"; n = n1, n2, n1+n2), each row a pair table (t[k-1] = 1-based partner of base k, 0 unpaired)."""
+        flat = np.zeros(max(self.total_samples, 1), dtype=np.int16)
+        self.stage._check(self.lib.rp_batch_fetch_samples(self.handle, flat.ctypes.data, flat.size))
+        out = []
+        for k, (s1, s2) in enumerate(self.pairs):
+            L = self.sample_layout[k]
+            d = {}
+            for name, off, ln, n in (("s1", L.s1, L.len_s1, len(s1)), ("s2", L.s2, L.len_s2, len(s2)),
+                                     ("co", L.co, L.len_co, len(s1) + len(s2))):
+                if ln:
+                    d[name] = flat[off:off + ln].reshape(self.samples, n)
+            out.append(d)
+        return out
+
+    def sample_tensors(self) -> Dict[str, "torch.Tensor"]:
+        """The samples as padded int16 CUDA tensors s1 [B, num, N1], s2 [B, num, N2], co [B, num, N1+N2] (N1 / N2 the
+        longest first / second sequence of the batch), zero past each pair's own length and for problems that were
+        not sampled.  Copied on the device and enqueued on torch's current stream, like dense_tensor()."""
+        B, num = self.n, self.samples
+        N1 = max([len(a) for a, _ in self.pairs], default=0)
+        N2 = max([len(b) for _, b in self.pairs], default=0)
+        with self.stage._torch_stream() as torch:
+            dev = self.stage.torch_device()
+            flat = torch.empty(max(self.total_samples, 1), dtype=torch.int16, device=dev)
+            self.stage._check(self.lib.rp_batch_samples_device(self.handle, C.c_void_p(flat.data_ptr()), flat.numel()))
+            out = {"s1": torch.zeros((B, num, N1), dtype=torch.int16, device=dev),
+                   "s2": torch.zeros((B, num, N2), dtype=torch.int16, device=dev),
+                   "co": torch.zeros((B, num, N1 + N2), dtype=torch.int16, device=dev)}
+            for k, (s1, s2) in enumerate(self.pairs):
+                L = self.sample_layout[k]
+                for name, off, ln, n in (("s1", L.s1, L.len_s1, len(s1)), ("s2", L.s2, L.len_s2, len(s2)),
+                                         ("co", L.co, L.len_co, len(s1) + len(s2))):
+                    if ln:
+                        out[name][k, :, :n] = flat[off:off + ln].view(num, n)
+        return out
 
     def square_layout(self) -> RpSquareLayout:
         """rp_square_plan of the batch: B, N1, N2, W and the element count of each square tensor."""
@@ -344,10 +435,13 @@ class ProbabilityStage:
 
     # ------------------------------------------------------------- batches
     def batch(self, pairs: Sequence[Tuple[str, str]], opts: Optional[RpOpts] = None,
-              constraints=None, stack_energies=None) -> DeviceBatch:
+              constraints=None, stack_energies=None, samples: int = 0, sample_seed: int = 1,
+              sample_problems: Sequence[str] = ("s1", "s2", "co")) -> DeviceBatch:
         """constraints: None, or one (c1, c2) structure-constraint pair per pair; stack_energies: None, or one (e1, e2)
-        pair of stacking pseudo-energy arrays per pair (DeviceBatch)."""
-        return DeviceBatch(self, pairs, opts if opts is not None else default_opts(), constraints, stack_energies)
+        pair of stacking pseudo-energy arrays per pair; samples, sample_seed, sample_problems: stochastic samples
+        (DeviceBatch)."""
+        return DeviceBatch(self, pairs, opts if opts is not None else default_opts(), constraints, stack_energies,
+                           samples, sample_seed, sample_problems)
 
     def run_dense(self, pairs: Sequence[Tuple[str, str]], opts: Optional[RpOpts] = None,
                   pinned: bool = False, constraints=None, stack_energies=None) -> List[PairProbabilities]:
