@@ -339,6 +339,41 @@ int rp_batch_create_sampled(rp_ctx* ctx, const rp_pair* pairs,
                             const rp_constraint* cons, const rp_stack_energy* se,
                             int n_pairs, const rp_opts* opts,
                             const rp_sample_opts* so, rp_batch** batch);
+
+/* Unpaired pseudo-energies of one pair (probing data that reward or penalise a
+ * base for staying unpaired, e.g. DMS or SHAPE perturbation vectors): u1[0..n1-1]
+ * over s1, u2[0..n2-1] over s2, in kcal/mol; NULL means none.  ViennaRNA's
+ * vrna_sc_set_up semantics (RNAfold --shapeMethod=W):
+ *   - each value is rounded to an integer number of 0.01 kcal/mol, half away
+ *     from zero: E_x;
+ *   - every base x a structure leaves unpaired, in hairpins, interior loops,
+ *     bulges, multiloops and the exterior loop alike, multiplies the
+ *     structure's Boltzmann weight by f(x) = exp(-E_x * 10 / kT) (37 C);
+ *   - nothing else changes: no pf_scale, no energy of rp_energy_of_structure.
+ * s1's fold takes u1, s2's fold u2.  The s1&s2 co-fold takes both; a base paired
+ * with the partner counts as unpaired there (data measured on each RNA alone
+ * describe only its own structure).  The --duplex branch takes none.  log Z
+ * (rp_batch_fetch_logz) is that of the ensemble with the factors.
+ * Range: pf_scale is not adapted to the data, so a problem whose
+ * B = sum_x |E_x| * 10 / kT over the bases it applies exceeds ln 10^150 is
+ * RP_ERR_UNSUPPORTED (about 425 nt at 0.5 kcal/mol per base). */
+typedef struct rp_unpaired_energy {
+  const double* u1;
+  const double* u2;
+} rp_unpaired_energy;
+/* rp_batch_create_sampled with unpaired pseudo-energies as well (ue, one
+ * rp_unpaired_energy per pair; NULL, or an entry with both NULL: none; ue ==
+ * NULL is exactly rp_batch_create_sampled).  A problem whose rounded values are
+ * all 0 has no such data and is planned and computed exactly as without it;
+ * problems with data run on the general kernel.  RP_ERR_ARG, with rp_last_error
+ * naming the pair, the vector and the position, for a value that is not
+ * finite; RP_ERR_UNSUPPORTED, naming the pair, the problem and B, for a problem
+ * beyond the range above. */
+int rp_batch_create_probed(rp_ctx* ctx, const rp_pair* pairs,
+                           const rp_constraint* cons, const rp_stack_energy* se,
+                           const rp_unpaired_energy* ue, int n_pairs,
+                           const rp_opts* opts, const rp_sample_opts* so,
+                           rp_batch** batch);
 /* The samples of the last run, in the layout of rp_sample_plan: to the host
  * (synchronous), or device to device into memory the caller owns (the stream
  * rules of rp_batch_dense_device).  RP_ERR_CAPACITY when n < total. */

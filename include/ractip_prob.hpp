@@ -113,6 +113,19 @@ class ProbabilityStage {
     for (size_t k = 0; k < samples.size(); k++) samples[k].assign(flat.begin() + k * n, flat.begin() + (k + 1) * n);
   }
 
+  // The same as the stacking overload with unpaired pseudo-energies u1 over s1, u2 over s2 in kcal/mol as well
+  // (rp_unpaired_energy, RNAfold --shapeMethod=W; an empty vector means none).  One context only.
+  void solve_probabilities(const std::string& s1, const std::string& s2, const std::string& c1, const std::string& c2,
+                           const std::vector<double>& e1, const std::vector<double>& e2, const std::vector<double>& u1,
+                           const std::vector<double>& u2, PairProbabilities& out) {
+    if ((!e1.empty() && e1.size() != s1.size()) || (!e2.empty() && e2.size() != s2.size()) ||
+        (!u1.empty() && u1.size() != s1.size()) || (!u2.empty() && u2.size() != s2.size()))
+      throw std::runtime_error("ractip_prob: a pseudo-energy vector's length differs from its sequence's");
+    rp_stack_energy se = {e1.empty() ? nullptr : e1.data(), e2.empty() ? nullptr : e2.data()};
+    rp_unpaired_energy ue = {u1.empty() ? nullptr : u1.data(), u2.empty() ? nullptr : u2.data()};
+    solve_one(s1, s2, c1, c2, &se, nullptr, out, nullptr, &ue);
+  }
+
   // the same for a whole batch (the shuffles of src/ractip.cpp:1638-1657) in one call
   void solve_batch(const std::vector<std::pair<std::string, std::string> >& seqs, std::vector<PairProbabilities>& out) {
     const int n = static_cast<int>(seqs.size());
@@ -158,11 +171,11 @@ class ProbabilityStage {
   }
 
  private:
-  // one pair on the context under constraints and, when se is set, stacking pseudo-energies; when so is set, its
-  // samples (the layout of rp_sample_plan for the one pair) to *samples
+  // one pair on the context under constraints and, when se is set, stacking pseudo-energies, when ue is set, unpaired
+  // pseudo-energies; when so is set, its samples (the layout of rp_sample_plan for the one pair) to *samples
   void solve_one(const std::string& s1, const std::string& s2, const std::string& c1, const std::string& c2,
                  const rp_stack_energy* se, const rp_sample_opts* so, PairProbabilities& out,
-                 std::vector<int16_t>* samples = nullptr) {
+                 std::vector<int16_t>* samples = nullptr, const rp_unpaired_energy* ue = nullptr) {
     if (!ctx_) throw std::runtime_error("ractip_prob: constrained problems run on a single-device stage");
     rp_pair pair = {s1.data(), static_cast<int>(s1.size()), s2.data(), static_cast<int>(s2.size())};
     rp_constraint con = {c1.empty() ? nullptr : c1.c_str(), c2.empty() ? nullptr : c2.c_str()};
@@ -177,7 +190,8 @@ class ProbabilityStage {
       samples->assign(n_samples ? n_samples : 1, 0);
     }
     rp_batch* b = nullptr;
-    check(so   ? rp_batch_create_sampled(ctx_, &pair, &con, se, 1, &opts_, so, &b)
+    check(ue   ? rp_batch_create_probed(ctx_, &pair, &con, se, ue, 1, &opts_, so, &b)
+          : so ? rp_batch_create_sampled(ctx_, &pair, &con, se, 1, &opts_, so, &b)
           : se ? rp_batch_create_soft(ctx_, &pair, &con, se, 1, &opts_, &b)
                : rp_batch_create_constrained(ctx_, &pair, &con, 1, &opts_, &b), ctx_);
     int rc = rp_batch_run(b);

@@ -7,6 +7,7 @@ from .ip import default_ip_opts
 from .stage import ProbabilityStage, RpError, default_opts
 
 RP_ERR_ARG = 1
+RP_ERR_UNSUPPORTED = 10
 
 
 def main(argv=None) -> int:
@@ -34,6 +35,9 @@ def main(argv=None) -> int:
                          "stacking pseudo-energies (Deigan); repeatable")
     ap.add_argument("--shape-slope", type=float, default=1.8, help="m of E = m ln(r+1) + b, kcal/mol (default 1.8)")
     ap.add_argument("--shape-intercept", type=float, default=-0.6, help="b of E = m ln(r+1) + b, kcal/mol (default -0.6)")
+    ap.add_argument("--shape-method", default="D", metavar="D|W",
+                    help="D: --shape values are reactivities, stacking pseudo-energies by Deigan (default); W: they are "
+                         "unpaired pseudo-energies in kcal/mol, missing positions 0 (RNAfold --shapeMethod=W)")
     ap.add_argument("-P", "--param-file", default=None)
     ap.add_argument("--no-pk", action="store_true")
     ap.add_argument("--duplex", action="store_true")
@@ -47,6 +51,8 @@ def main(argv=None) -> int:
     if len(args.fasta) > 2:
         ap.error("at most two FASTA files")
     try:
+        if args.shape_method not in ("D", "W"):
+            raise ValueError(f"--shape-method {args.shape_method}: expected D or W")
         if args.sample < 0:
             raise ValueError(f"--sample {args.sample}: the number of samples cannot be negative")
         if args.sample and args.duplex:
@@ -81,12 +87,15 @@ def main(argv=None) -> int:
     try:
         for r in predict(stage, pairs, opts, ipo, args.show_energy, args.zscore, args.num_shuffling, args.seed,
                          use_constraint=args.use_constraint, shape=shape, shape_slope=args.shape_slope,
-                         shape_intercept=args.shape_intercept, samples=args.sample, sample_seed=args.sample_seed):
+                         shape_intercept=args.shape_intercept, samples=args.sample, sample_seed=args.sample_seed,
+                         shape_method=args.shape_method):
             print(format_result(r, args.show_energy))
     except RpError as e:
-        if not (args.use_constraint and e.code == RP_ERR_ARG):
+        probed = bool(shape) and args.shape_method == "W"
+        if not ((args.use_constraint and e.code == RP_ERR_ARG) or (probed and e.code == RP_ERR_UNSUPPORTED)):
             raise
-        print(e)   # a malformed structure line is an input error like the others
+        # a malformed structure line, or unpaired pseudo-energies beyond the range, is an input error like the others
+        print(e)
         return 1
     finally:
         stage.close()

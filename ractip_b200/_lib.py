@@ -73,6 +73,10 @@ class RpSampleLayout(C.Structure):
     _fields_ = [(n, C.c_size_t) for n in ("s1", "s2", "co", "len_s1", "len_s2", "len_co")]
 
 
+class RpUnpairedEnergy(C.Structure):
+    _fields_ = [("u1", C.c_void_p), ("u2", C.c_void_p)]
+
+
 class RpOpts(C.Structure):
     _fields_ = [("max_w", C.c_int), ("min_w", C.c_int), ("th_ss", C.c_float), ("th_hy", C.c_float),
                 ("th_ac", C.c_float), ("use_pf_duplex", C.c_int)]
@@ -124,7 +128,7 @@ EXPORTS = [
     "rp_batch_run", "rp_batch_sync",
     "rp_batch_fetch_dense", "rp_batch_fetch_sparse", "rp_batch_sparse_device", "rp_batch_dense_device",
     "rp_square_plan", "rp_batch_square_device", "rp_batch_fetch_logz",
-    "rp_sample_plan", "rp_batch_create_sampled", "rp_batch_fetch_samples", "rp_batch_samples_device",
+    "rp_sample_plan", "rp_batch_create_sampled", "rp_batch_create_probed", "rp_batch_fetch_samples", "rp_batch_samples_device",
     "rp_batch_destroy", "rp_last_timing", "rp_measure_peaks", "rp_zscore_shuffles",
     "rp_alg_flops_mcc", "rp_version", "rp_kernel_plan",
     "rp_multi_create", "rp_multi_destroy", "rp_multi_devices", "rp_multi_last_error", "rp_multi_run_dense",
@@ -186,6 +190,8 @@ def load() -> C.CDLL:
         "rp_sample_plan": (i, [P(RpPair), i, P(RpSampleOpts), P(RpSampleLayout), P(sz)]),
         "rp_batch_create_sampled": (i, [vp, P(RpPair), P(RpConstraint), P(RpStackEnergy), i, P(RpOpts),
                                         P(RpSampleOpts), P(vp)]),
+        "rp_batch_create_probed": (i, [vp, P(RpPair), P(RpConstraint), P(RpStackEnergy), P(RpUnpairedEnergy), i,
+                                       P(RpOpts), P(RpSampleOpts), P(vp)]),
         "rp_batch_fetch_samples": (i, [vp, vp, sz]),
         "rp_batch_samples_device": (i, [vp, vp, sz]),
         "rp_batch_destroy": (i, [vp]),

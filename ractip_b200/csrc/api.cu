@@ -378,7 +378,7 @@ int rp_batch_destroy(rp_batch* b) {
 namespace {
 int batch_create(const char* who, rp_ctx* ctx, const rp_pair* pairs, const rp_constraint* cons,
                  const rp_stack_energy* se, int n_pairs, const rp_opts* opts, rp_batch** out,
-                 const rp_sample_opts* so = nullptr) {
+                 const rp_sample_opts* so = nullptr, const rp_unpaired_energy* ue = nullptr) {
   if (!ctx || !out) return fail(ctx, RP_ERR_ARG, "rp_batch_create: null argument");
   *out = nullptr;
   int rc = rp::check_pairs(pairs, n_pairs, opts);
@@ -390,6 +390,7 @@ int batch_create(const char* who, rp_ctx* ctx, const rp_pair* pairs, const rp_co
   if ((rc = rp::check_constraints(pairs, cons, n_pairs, &msg)) != RP_OK) return fail(ctx, rc, std::string(who) + ": " + msg);
   if ((rc = rp::check_stack_energies(pairs, se, n_pairs, &msg)) != RP_OK) return fail(ctx, rc, std::string(who) + ": " + msg);
   if ((rc = rp::check_samples(pairs, n_pairs, opts, so, &msg)) != RP_OK) return fail(ctx, rc, std::string(who) + ": " + msg);
+  if ((rc = rp::check_unpaired_energies(pairs, ue, n_pairs, opts, &msg)) != RP_OK) return fail(ctx, rc, std::string(who) + ": " + msg);
   CU(cudaSetDevice(ctx->device));
   rp_batch* b = new rp_batch;
   b->ctx = ctx;
@@ -398,7 +399,7 @@ int batch_create(const char* who, rp_ctx* ctx, const rp_pair* pairs, const rp_co
   b->opts = *opts;
   b->slayout.resize(n_pairs);
   rp_sparse_plan(pairs, n_pairs, opts, b->slayout.data(), &b->total_recs, &b->total_upf);
-  if (rp::plan_batch(pairs, n_pairs, opts, device_facts(ctx), ctx->route, &b->plan, cons, se, so) != RP_OK) {
+  if (rp::plan_batch(pairs, n_pairs, opts, device_facts(ctx), ctx->route, &b->plan, cons, se, so, ue) != RP_OK) {
     rp_batch_destroy(b);
     return fail(ctx, RP_ERR_CUDA, "rp_batch_create: band kernel does not fit on this device");
   }
@@ -420,12 +421,18 @@ int batch_create(const char* who, rp_ctx* ctx, const rp_pair* pairs, const rp_co
   cudaStream_t st = ctx->stream;
   if ((e = cudaMemcpyAsync(b->d_seq, p.seq.data(), p.seq.size(), cudaMemcpyHostToDevice, st)) != cudaSuccess) return bail(e, "H2D seq");
   // per-base data only for batches with a constrained problem (keys), one whose pseudo-energies are not all 0, or a
-  // sampled one (the instances that sample are the per-base ones).  One block: PerBaseHead, keys, factors, sample offsets.
-  if (!p.key.empty() || !p.stack.empty() || p.sample_total) {
+  // sampled one (the instances that sample are the per-base ones).  One block: PerBaseHead, keys, factors, sample offsets,
+  // the unpaired pseudo-energies' pair factors and log-Z terms.
+  if (!p.key.empty() || !p.stack.empty() || p.sample_total || !p.unpaired.empty()) {
     const size_t kd = (p.key.size() * sizeof(uint16_t) + sizeof(double) - 1) / sizeof(double);
     b->stack_off = (unsigned)(rp::PB_HEAD + kd);
-    std::vector<double> blk(b->stack_off + p.stack.size() + 3 * (size_t)n_pairs, 0.);
+    const size_t unp_off = b->stack_off + p.stack.size() + 3 * (size_t)n_pairs;
+    std::vector<double> blk(unp_off + p.unpaired.size() + p.unpaired_lz.size(), 0.);
     rp::PerBaseHead h = {};
+    h.unp_off = (long long)unp_off;
+    h.unp_lz_off = (long long)(unp_off + p.unpaired.size());
+    std::copy(p.unpaired.begin(), p.unpaired.end(), blk.begin() + unp_off);
+    std::copy(p.unpaired_lz.begin(), p.unpaired_lz.end(), blk.begin() + h.unp_lz_off);
     if (p.sample_total) {
       if ((e = pool_alloc(ctx, &b->d_samples, p.sample_total * sizeof(int16_t))) != cudaSuccess) return bail(e, "cudaMalloc samples");
       if ((e = cudaMemsetAsync(b->d_samples, 0, p.sample_total * sizeof(int16_t), st)) != cudaSuccess) return bail(e, "memset samples");
@@ -457,6 +464,7 @@ int batch_create(const char* who, rp_ctx* ctx, const rp_pair* pairs, const rp_co
   std::vector<uint8_t>().swap(p.seq);   // the sequences live on the device from here
   std::vector<uint16_t>().swap(p.key);
   std::vector<double>().swap(p.stack);
+  std::vector<double>().swap(p.unpaired);
   *out = b;
   return RP_OK;
 }
@@ -481,6 +489,12 @@ int rp_batch_create_soft(rp_ctx* ctx, const rp_pair* pairs, const rp_constraint*
 int rp_batch_create_sampled(rp_ctx* ctx, const rp_pair* pairs, const rp_constraint* cons, const rp_stack_energy* se,
                             int n_pairs, const rp_opts* opts, const rp_sample_opts* so, rp_batch** out) {
   return batch_create("rp_batch_create_sampled", ctx, pairs, cons, se, n_pairs, opts, out, so);
+}
+
+int rp_batch_create_probed(rp_ctx* ctx, const rp_pair* pairs, const rp_constraint* cons, const rp_stack_energy* se,
+                           const rp_unpaired_energy* ue, int n_pairs, const rp_opts* opts, const rp_sample_opts* so,
+                           rp_batch** out) {
+  return batch_create("rp_batch_create_probed", ctx, pairs, cons, se, n_pairs, opts, out, so, ue);
 }
 
 int rp_batch_run(rp_batch* b) {

@@ -65,6 +65,11 @@ __device__ __forceinline__ void bind_per_base(Ctx& c, const BatchDev& b, const P
     c.smp_seed = h.seed;
     c.smp_num = (int)h.num;
   }
+  if (PB && (p.constrained & CON_UNPAIRED)) {
+    const PerBaseHead& h = *reinterpret_cast<const PerBaseHead*>(pb);
+    c.upf = pb + h.unp_off + p.seq_off - 1;
+    c.upf_lz = pb[h.unp_lz_off + (size_t)p.pair * 3 + p.which];
+  }
 }
 
 // Instantiated for two register budgets: <2> two CTAs per SM at 64 registers (many short problems
@@ -73,8 +78,9 @@ __device__ __forceinline__ void bind_per_base(Ctx& c, const BatchDev& b, const P
 // as many problem histories compete for the L2).
 // <1, W> with W > BAND sums the split sums in wide bands (solve_mcc_wide): W-fold reuse of every element
 // streamed from HBM.
-// PB: the batch has per-base data (BatchDev::perbase): structure-constraint keys, stacking pseudo-energies or samples
-// (PerBaseHead); each problem binds what it carries.  The instances without compile all out (Ctx::key, Ctx::stk and Ctx::smp stay null), so that
+// PB: the batch has per-base data (BatchDev::perbase): structure-constraint keys, stacking or unpaired pseudo-energies
+// or samples (PerBaseHead); each problem binds what it carries.  The instances without compile all out (Ctx::key,
+// Ctx::stk, Ctx::upf and Ctx::smp stay null), so that
 // unconstrained batches run exactly the code they ran before constraints existed.
 template <int MINB, int W, bool PB>
 __global__ void __launch_bounds__(RP_MCC_THREADS, MINB) mcc_persistent(BatchDev b) {

@@ -33,7 +33,7 @@ struct BatchDev {
   unsigned stack_off;      // doubles from perbase to the stacking factors
   // Per-base data of the batch, or null: a PerBaseHead (below), structure-constraint keys (uint16) laid out like seq
   // after it (Problem::constrained & CON_KEYS), stacking pseudo-energy factors (double) laid out like seq at stack_off
-  // (CON_STACK), the sample offsets.  One pointer, so that the parameter block of every kernel keeps the layout it had
+  // (CON_STACK), the sample offsets, the unpaired pseudo-energies' pair factors (CON_UNPAIRED).  One pointer, so that the parameter block of every kernel keeps the layout it had
   // before factors and samples.
   const void* perbase;
 };
@@ -41,11 +41,15 @@ struct BatchDev {
 // Head of the per-base block (BatchDev::perbase): the batch's stochastic samples (Problem::constrained & CON_SAMPLE):
 // `num` pair tables per sampled problem, problem `which` of pair p at samples + off[3p + which] (rp_sample_plan), where
 // off = (const long long*)perbase + off_doubles.  The structure-constraint keys follow the head, at PB_HEAD doubles.
+// Unpaired pseudo-energies (Problem::constrained & CON_UNPAIRED): the pair factors upf (double) laid out like seq at
+// unp_off, and at unp_lz_off one log-Z term per problem, problem `which` of pair p at [3p + which].
 struct PerBaseHead {
   int16_t* samples;   // null: nothing sampled
   unsigned long long seed;
   long long off_doubles;
   long long num;
+  long long unp_off;
+  long long unp_lz_off;
 };
 constexpr int PB_HEAD = sizeof(PerBaseHead) / sizeof(double);
 
@@ -83,7 +87,7 @@ struct SquareDev {
 
 // general kernel, RP_MCC_THREADS threads.  minb = 2: 64-register build, two CTAs per SM; 1: 128 registers, one CTA
 // per SM, split sums in bands of 10 diagonals.  Both launches run the instances that apply per-base data (structure
-// constraints, stacking pseudo-energies) when b.perbase is set, else the ones that compile it out.
+// constraints, stacking and unpaired pseudo-energies, samples) when b.perbase is set, else the ones that compile it out.
 int mcc_max_ctas_per_sm(int minb);
 cudaError_t launch_mcc(const BatchDev& b, int grid, int minb, cudaStream_t st);
 // multi-CTA wavefront: `nclusters` clusters of `ctas` (8 or 16) CTAs, one problem (and one workspace slot) per cluster

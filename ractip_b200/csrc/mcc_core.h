@@ -59,7 +59,8 @@ struct Problem {
   int max_w;
   int n1, n2;
   int constrained;    // general kernel only, bits (BatchDev::perbase): CON_KEYS a structure constraint removes some
-                      // pairs, CON_STACK stacking pseudo-energies weight its stacks, CON_SAMPLE structures are sampled
+                      // pairs, CON_STACK stacking pseudo-energies weight its stacks, CON_SAMPLE structures are sampled,
+                      // CON_UNPAIRED unpaired pseudo-energies weight its unpaired bases (as pair factors, see pair_sc)
   long long out_bp;   // float offsets into the dense output, -1 if absent
   long long out_up;
   long long out_hp;
@@ -67,7 +68,7 @@ struct Problem {
   int defer_up;       // 1: the unpaired-window pass runs later in its own kernel (unstru_kernel) on the tables left in ws_off
   long long ws_off;   // >= 0: private workspace (doubles from BatchDev::ws_up) that outlives the wavefront kernel; -1: the CTA's slot
 };
-enum { CON_KEYS = 1, CON_STACK = 2, CON_SAMPLE = 4 };
+enum { CON_KEYS = 1, CON_STACK = 2, CON_SAMPLE = 4, CON_UNPAIRED = 8 };
 // queue entries: problem index, + RP_JOB_UNPAIRED for the unpaired-window pass of a deferred problem as a job of its own
 constexpr int RP_JOB_UNPAIRED = 0x40000000;
 
@@ -107,6 +108,10 @@ struct Ctx {
   long long* prof;    // RP_PROFILE counters (slots 40..: fine-grained probes of thread 0) or null
   const uint16_t* key;   // key[1..n] of a constrained problem (pair (i,j) allowed iff key[i] == key[j]), else null
   const double* stk;     // stk[1..n]: per-base factors exp(-E/kT) of stacking pseudo-energies (CON_STACK), else null
+  // unpaired pseudo-energies (CON_UNPAIRED): upf[1..n] = exp(+E/kT), the inverse of each base's unpaired factor, and
+  // upf_lz = sum_x -E_x/kT, what they add to log Z; upf null: none
+  const double* upf;
+  double upf_lz;
   // stochastic sampling (CON_SAMPLE, mcc_sample.h): smp_num pair tables of n int16 at smp, drawn with seed smp_seed;
   // smp null: none (the instances without per-base data know it and compile the sampling phase away)
   int16_t* smp;
@@ -142,6 +147,8 @@ RP_HD void bind_ctx(Ctx& c, const DevModel* M, const uint8_t* S, const Problem& 
   c.prof = nullptr;
   c.key = nullptr;
   c.stk = nullptr;
+  c.upf = nullptr;
+  c.upf_lz = 0.;
   c.smp = nullptr;
   c.smp_seed = 0;
   c.smp_num = 0;
@@ -249,6 +256,21 @@ template <class C>
 RP_HD double stack_sc(const C& c, int s, int i, int j, double w) {
   if (s != 0 || !c.stk || !ss(c, i, j)) return w;
   return w * (c.stk[i] * c.stk[i + 1] * c.stk[j - 1] * c.stk[j]);
+}
+
+// Unpaired pseudo-energies (soft constraint, CON_UNPAIRED) as pair factors.  A base x left unpaired multiplies a
+// structure's weight by f(x) = exp(-E_x/kT).  Since w0(S) prod_{x unpaired} f(x) = prod_x f(x) * w0(S)
+// prod_{(i,j) in S} 1/(f(i) f(j)), the ensemble is the constant prod_x f(x) (emit_logz adds its log) times one in which
+// only pairs change: (i,j) gets upf[i] upf[j], upf = 1/f.  Every probability, and every sampled distribution, is that
+// of the second ensemble.  In the co-fold a base paired with the partner counts as unpaired (probing data of each RNA
+// alone describe only its own structure), so a pair that joins the strands gets 1.
+// Invariant: qb(i,j), and the weight of every loop closed by (i,j) wherever the outside pass or the unpaired-window
+// pass uses it (the class tables OUTI/OUT1N/OUTAU, Mc, the table-driven shapes, the hairpin and gap windows), carry
+// pair_sc(i,j) exactly once; out(i,j) carries none, so that P(i,j) = qb(i,j) out(i,j).  The instances without
+// per-base data know c.upf is null: the factor is the constant 1 and compiles away.
+template <class C>
+RP_HD double pair_sc(const C& c, int i, int j) {
+  return (c.upf && ss(c, i, j)) ? c.upf[i] * c.upf[j] : 1.;
 }
 
 // Outside pass of a two-strand problem: RactIP keeps only the probabilities of pairs that JOIN the strands
@@ -680,6 +702,7 @@ RP_HD void inside_finish(C& c, int d, int i, int type, double sI, double sM, dou
       t *= ext_stem(M, rtype(type), ss(c, j - 1, j) ? base(c, j - 1) : -1, ss(c, i, i + 1) ? base(c, i + 1) : -1);
       qb += t;
     }
+    qb *= pair_sc(c, i, j);
   }
   TB(c, T_QB, d, i) = qb;
   TB(c, T_QM2, d, i) = sM;
@@ -861,7 +884,7 @@ RP_HD double outside_interior(const C& c, const Shared& sh, int d, int k, int sl
     const int i = k - 1 - u1, j = l + 1 + u2;
     const int t1 = cell_type(c, i, j);
     if (!t1) continue;
-    const double o = TB(c, T_OUT, d + dd, i);
+    const double o = TB(c, T_OUT, d + dd, i) * pair_sc(c, i, j);
     if (o == 0.) continue;
     accI += o * stack_sc(c, s, i, j, special_loop(M, s, t1, t2, base(c, i + 1), base(c, j - 1), sp1, sq1));
   }
@@ -917,11 +940,12 @@ RP_HD void outside_finish(C& c, int d, int k, int type, double sI, double sP, do
   TB(c, T_OUT, d, k) = out;
   double fI = 0., f1 = 0., fA = 0., mc = 0.;
   if (out != 0.) {
+    const double og = out * pair_sc(c, k, l);   // the loops (k,l) closes carry its pair factor
     const int si1 = base(c, k + 1), sj1 = base(c, l - 1);
-    fI = out * M.mmI[type][si1][sj1];
-    f1 = out * M.mm1n[type][si1][sj1];
-    fA = type > 2 ? out * M.expTermAU : out;
-    if (ss(c, k, k + 1) && ss(c, l - 1, l)) mc = out * M.expMLclosing * ml_stem(M, rtype(type), sj1, si1);
+    fI = og * M.mmI[type][si1][sj1];
+    f1 = og * M.mm1n[type][si1][sj1];
+    fA = type > 2 ? og * M.expTermAU : og;
+    if (ss(c, k, k + 1) && ss(c, l - 1, l)) mc = og * M.expMLclosing * ml_stem(M, rtype(type), sj1, si1);
   }
   TB(c, T_OUTI, d, k) = fI;
   TB(c, T_OUT1N, d, k) = f1;
@@ -1373,7 +1397,7 @@ RP_HD double outside_ends_item(const Ctx& c, const Shared& sh, int d, int k, int
     const bool ok = dd <= ddmax && u1 + 1 <= maxpo && u2 <= maxu2;
     const int i = k - 1 - u1, j = l + 1 + u2;
     t1v[s] = ok ? cell_type(c, i, j) : 0;
-    ov[s] = t1v[s] ? TB(c, T_OUT, d + dd, i) : 0.;
+    ov[s] = t1v[s] ? TB(c, T_OUT, d + dd, i) * pair_sc(c, i, j) : 0.;
   }
   double acc = 0.;
 #pragma unroll
@@ -1561,7 +1585,7 @@ RP_HD void unstru_hairpin_cell(C& c, unsigned x) {
   if (i < 1 || i + d > n) return;
   double v = 0.;
   if (d > TURN) {
-    const double o = TB(c, T_OUT, d, i);
+    const double o = TB(c, T_OUT, d, i) * pair_sc(c, i, i + d);
     if (o != 0.) v = o * hairpin(c, i, i + d, pair_type(base(c, i), base(c, i + d)));
   }
   TB(c, T_DG, d, i) = v;
@@ -1617,7 +1641,7 @@ RP_HD void unstru_gap_special(C& c, const MT& M, int x) {
             const int l = l0 + u * nsl;
             const bool on = l <= lmax;
             qb[u] = on ? TB(c, T_QB, l - k, k) : 0.;
-            ou[u] = on ? TB(c, T_OUT, l + 1 + u2 - p, p) : 0.;
+            ou[u] = on ? TB(c, T_OUT, l + 1 + u2 - p, p) * pair_sc(c, p, l + 1 + u2) : 0.;
           }
           double w[4];
 #pragma unroll
@@ -1642,7 +1666,7 @@ RP_HD void unstru_gap_special(C& c, const MT& M, int x) {
           for (int u = 0; u < 4; u++) {
             const int p = p0 + u * nsl;
             const bool on = p <= pmax;
-            ou[u] = on ? TB(c, T_OUT, o - p, p) : 0.;
+            ou[u] = on ? TB(c, T_OUT, o - p, p) * pair_sc(c, p, o) : 0.;
             qb[u] = on ? TB(c, T_QB, l - (p + 1 + u1), p + 1 + u1) : 0.;
           }
           double w[4];
@@ -1956,7 +1980,8 @@ RP_HD void unstru_windows(C& c, float* up, int tid, int T) {
             m3 += A1[(long)t * st] * BR[(long)t * st];
           }
         }
-        // Mc carries no scale factor for the closing pair's two bases: apply it here
+        // Mc carries no scale factor for the closing pair's two bases: apply it here (its pair factor, pair_sc, it
+        // carries from outside_finish)
         v += (m1 * VEC(c, V_MLB, dd) + (m2 + m3) * VEC(c, V_MLB, dd + 1)) * VEC(c, V_SCALE, 2);
       }
     }

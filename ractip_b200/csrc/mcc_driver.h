@@ -103,7 +103,8 @@ RP_HD void stage_sequence(Exec& ex, Ctx& c, uint8_t* S, F with) {
   c.S = S;
 }
 
-// log Z of the finished inside pass: 3 doubles per pair (s1, s2, s1&s2)
+// log Z of the finished inside pass: 3 doubles per pair (s1, s2, s1&s2).  With unpaired pseudo-energies the tables
+// hold the pair-factor ensemble (pair_sc, mcc_core.h), whose log Z differs by Ctx::upf_lz.
 template <class Exec>
 RP_HD void emit_logz(Exec& ex, Ctx& c, const Problem& p, double* logz) {
   if (!logz) return;
@@ -111,7 +112,11 @@ RP_HD void emit_logz(Exec& ex, Ctx& c, const Problem& p, double* logz) {
     if (ex.rank_begin() != 0) return;   // the CTA of rank 0 writes it
   }
   ex.phase(PH_LOGZ, [&](int tid) {
-    if (tid == 0) logz[(size_t)p.pair * 3 + p.which] = log(TB(c, T_Q, c.n - 1, 1)) + c.n * log(c.M->pf_scale);
+    if (tid == 0) {
+      double lz = log(TB(c, T_Q, c.n - 1, 1)) + c.n * log(c.M->pf_scale);
+      if (c.upf) lz += c.upf_lz;
+      logz[(size_t)p.pair * 3 + p.which] = lz;
+    }
   });
 }
 

@@ -1,6 +1,6 @@
 // mcc_sample.h -- stochastic sampling of secondary structures (RNAfold -p --stochBT) from the inside tables the general
 // kernel leaves in a problem's workspace slot: structures drawn with probability exp(-E/kT) / Z of exactly the ensemble
-// whose log Z the kernel reports (constraint keys and stacking factors included).  A phase of its own between the
+// whose log Z the kernel reports (constraint keys, stacking factors and unpaired pseudo-energies included).  A phase of its own between the
 // inside and the outside pass (mcc_driver.h, emit_samples).
 //
 // Traceback.  A sample is a stack of pending SEGMENTS, each one term of the inside recursion:
@@ -56,6 +56,8 @@ RP_HD int sample_count(int kind, int i, int j) {
 //   SG_QB  x = 0: hairpin;  x = 1 + u1 (MAXLOOP+1) + u2: interior loop with inner pair (i+1+u1, j-1-u2), by its class
 //          (dev_model.h: bulge, 1xn and generic from the class tables QBAU / QB1N / QBI times g, the nine small shapes
 //          table-driven, with the stacking factor);  x = last-1: multiloop;  x = last: the exterior loop over the nick
+//          (without the pair factor of (i,j), pair_sc: it is common to every candidate, and the decision compares the
+//          candidates with their own sum, so it does not change which one is taken)
 //   SG_QM  x = 2(k-p): p..k-1 unpaired, mlb^(k-p) qm1(k,r);  x = 2(k-p)+1: qm(p,k-1) qm1(k,r)
 //   SG_QM1 x = l - (k+TURN+1): qb(k,l) mlstem mlb^(r-l)
 //   SG_QM2 x = k - (p+TURN+2): qm(p,k-1) qm1(k,r), not at the nick

@@ -110,6 +110,46 @@ int check_stack_energies(const rp_pair* pairs, const rp_stack_energy* se, int n_
   return RP_OK;
 }
 
+// Unpaired pseudo-energies: u1 over s1, u2 over s2, in kcal/mol (either may be null).  After rounding, a problem's
+// weights move by at most a factor e^B either way against the same problem without data, B = sum_x |E_x| 10 / kT over
+// the bases it applies; pf_scale is global, so B must leave the tables room in fp64 (UNPAIRED_MAX_B).
+int check_unpaired_energies(const rp_pair* pairs, const rp_unpaired_energy* ue, int n_pairs, const rp_opts* opts,
+                            std::string* msg) {
+  if (!ue) return RP_OK;
+  const double kT = (37.0 + RP_K0) * RP_GASCONST;
+  char buf[200];
+  for (int p = 0; p < n_pairs; p++) {
+    const double* us[2] = {ue[p].u1, ue[p].u2};
+    const int ns[2] = {pairs[p].n1, pairs[p].n2};
+    double B[2] = {0., 0.};
+    for (int s = 0; s < 2; s++) {
+      if (!us[s]) continue;
+      for (int i = 0; i < ns[s]; i++) {
+        if (!std::isfinite(us[s][i])) {
+          std::snprintf(buf, sizeof buf, "pair %d, u%d, position %d: %g kcal/mol is not finite", p, s + 1, i + 1, us[s][i]);
+          if (msg) *msg = buf;
+          return RP_ERR_ARG;
+        }
+        B[s] += std::fabs(std::round(us[s][i] * 100.0)) * 10.0 / kT;
+      }
+    }
+    // s1's fold takes u1, s2's u2, the co-fold both (not under --duplex)
+    const bool cofold = pairs[p].n2 > 0 && !opts->use_pf_duplex;
+    const double Bs[3] = {B[0], B[1], cofold ? B[0] + B[1] : 0.};
+    const char* names[3] = {"s1", "s2", "s1&s2"};
+    for (int w = 0; w < 3; w++)
+      if (Bs[w] > UNPAIRED_MAX_B) {
+        std::snprintf(buf, sizeof buf,
+                      "pair %d, problem %s: the unpaired pseudo-energies give B = sum |E| / kT = %.2f, beyond ln 10^150 "
+                      "= %.2f, the range a batch's global pf_scale leaves",
+                      p, names[w], Bs[w], UNPAIRED_MAX_B);
+        if (msg) *msg = buf;
+        return RP_ERR_UNSUPPORTED;
+      }
+  }
+  return RP_OK;
+}
+
 int check_samples(const rp_pair* pairs, int n_pairs, const rp_opts* opts, const rp_sample_opts* so, std::string* msg) {
   if (!so) return RP_OK;
   char buf[160];
@@ -154,6 +194,23 @@ bool fill_stack(const double* e, int m, double* f) {
   for (int i = 1; i <= m; i++) {
     const double E = std::round(e[i - 1] * 100.0);
     f[i] = std::exp(-E * 10.0 / kT);
+    any |= E != 0.;
+  }
+  return any;
+}
+
+// Pair factors of one strand of length m from its unpaired pseudo-energies u[0..m-1] (kcal/mol), rounded as fill_stack
+// rounds: g[i] = exp(+E_i * 10 / kT), the inverse of the unpaired factor f (pair_sc, mcc_core.h), and *lnf = sum_i
+// ln f(i) = -sum_i E_i * 10 / kT, what the data add to log Z.  Returns whether any rounded value differs from 0.
+bool fill_unpaired(const double* u, int m, double* g, double* lnf) {
+  *lnf = 0.;
+  if (!u) return false;
+  const double kT = (37.0 + RP_K0) * RP_GASCONST;
+  bool any = false;
+  for (int i = 1; i <= m; i++) {
+    const double E = std::round(u[i - 1] * 100.0);
+    g[i] = std::exp(E * 10.0 / kT);
+    *lnf -= E * 10.0 / kT;
     any |= E != 0.;
   }
   return any;
@@ -365,7 +422,8 @@ static double alg_flops_mcc_uncached(int n) {
 namespace rp {
 
 int plan_batch(const rp_pair* pairs, int n_pairs, const rp_opts* opts, const DeviceFacts& dev, const RouteSettings& rs,
-               BatchPlan* out, const rp_constraint* cons, const rp_stack_energy* se, const rp_sample_opts* so) {
+               BatchPlan* out, const rp_constraint* cons, const rp_stack_energy* se, const rp_sample_opts* so,
+               const rp_unpaired_energy* ue) {
   BatchPlan& b = *out;
   b = BatchPlan{};
   // sampled problems (CON_SAMPLE): those with room in the sample buffer
@@ -393,6 +451,8 @@ int plan_batch(const rp_pair* pairs, int n_pairs, const rp_opts* opts, const Dev
   std::vector<int> partner;
   std::vector<double>& stack = b.stack;   // (the same for the stacking factors)
   bool any_stack = false;
+  std::vector<double>& unp = b.unpaired;   // (and for the unpaired pseudo-energies' pair factors)
+  bool any_unp = false;
   const int w = opts->max_w > 0 ? opts->max_w : 0;
   size_t ws_need = 0;
   for (int p = 0; p < n_pairs; p++) {
@@ -444,6 +504,22 @@ int plan_batch(const rp_pair* pairs, int n_pairs, const rp_opts* opts, const Dev
       std::copy(&stack[off2], &stack[off2] + pr.n2, &stack[off12] + pr.n1);
       any_stack |= stk[0] || stk[1];
     }
+    // unpaired pseudo-energies: s1's fold takes u1, s2's u2, the co-fold both (pair_sc, mcc_core.h, gives the pairs
+    // that join the strands no factor); --duplex takes none
+    int unf[2] = {0, 0};
+    double lnf[2] = {0., 0.};
+    if (ue && (ue[p].u1 || ue[p].u2)) {
+      unp.resize(seq.size(), 1.0);
+      b.unpaired_lz.resize(3 * (size_t)n_pairs, 0.);
+      unf[0] = fill_unpaired(ue[p].u1, pr.n1, &unp[off1 - 1], &lnf[0]) ? CON_UNPAIRED : 0;
+      unf[1] = fill_unpaired(ue[p].u2, pr.n2, &unp[off2 - 1], &lnf[1]) ? CON_UNPAIRED : 0;
+      std::copy(&unp[off1], &unp[off1] + pr.n1, &unp[off12]);
+      std::copy(&unp[off2], &unp[off2] + pr.n2, &unp[off12] + pr.n1);
+      b.unpaired_lz[3 * (size_t)p] = lnf[0];
+      b.unpaired_lz[3 * (size_t)p + 1] = lnf[1];
+      b.unpaired_lz[3 * (size_t)p + 2] = lnf[0] + lnf[1];
+      any_unp |= unf[0] || unf[1];
+    }
     Problem q;
     std::memset(&q, 0, sizeof q);
     q.pair = p; q.max_w = w; q.n1 = pr.n1; q.n2 = pr.n2; q.th_hy = opts->th_hy;
@@ -452,11 +528,11 @@ int plan_batch(const rp_pair* pairs, int n_pairs, const rp_opts* opts, const Dev
     // rnafold(fa1, ...), rnafold(fa2, ...)  src/ractip.cpp:546-547
     Problem a = q;
     const rp_sample_layout* sl = b.sample_total ? &b.sample_layout[p] : nullptr;
-    a.kind = KIND_LINEAR; a.which = 0; a.seq_off = off1; a.n = pr.n1; a.cp = 0; a.constrained = con[0] | stk[0];
+    a.kind = KIND_LINEAR; a.which = 0; a.seq_off = off1; a.n = pr.n1; a.cp = 0; a.constrained = con[0] | stk[0] | unf[0];
     if (sl && sl->len_s1) a.constrained |= CON_SAMPLE;
     a.out_bp = (long long)L.bp1; a.out_up = w > 0 ? (long long)L.up1 : -1;
     b.probs.push_back(a);
-    a.which = 1; a.seq_off = off2; a.n = pr.n2; a.constrained = con[1] | stk[1];
+    a.which = 1; a.seq_off = off2; a.n = pr.n2; a.constrained = con[1] | stk[1] | unf[1];
     if (sl && sl->len_s2) a.constrained |= CON_SAMPLE;
     a.out_bp = (long long)L.bp2; a.out_up = w > 0 ? (long long)L.up2 : -1;
     b.probs.push_back(a);
@@ -476,7 +552,7 @@ int plan_batch(const rp_pair* pairs, int n_pairs, const rp_opts* opts, const Dev
       b.n_duplex++;
       ws_need = std::max(ws_need, 2 * (size_t)(pr.n1 + 2) * (size_t)(pr.n2 + 2));
     } else {
-      c.kind = KIND_COFOLD; c.n = pr.n1 + pr.n2; c.cp = pr.n1 + 1; c.constrained = con[2] | stk[0] | stk[1];
+      c.kind = KIND_COFOLD; c.n = pr.n1 + pr.n2; c.cp = pr.n1 + 1; c.constrained = con[2] | stk[0] | stk[1] | unf[0] | unf[1];
       if (sl && sl->len_co) c.constrained |= CON_SAMPLE;
       b.alg_flops += rp_alg_flops_mcc(c.n);
     }
@@ -487,9 +563,15 @@ int plan_batch(const rp_pair* pairs, int n_pairs, const rp_opts* opts, const Dev
   else std::vector<uint16_t>().swap(key);
   if (any_stack) stack.resize(seq.size(), 1.0);
   else std::vector<double>().swap(stack);
+  if (any_unp) {
+    unp.resize(seq.size(), 1.0);
+  } else {
+    std::vector<double>().swap(unp);
+    std::vector<double>().swap(b.unpaired_lz);
+  }
 
   // Band class of a problem: 0 = L (512 threads, ring needs more than half an SM), 1 = S (256 threads, 2 CTAs/SM),
-  // -1 = the general kernel, which alone applies structure constraints and stacking pseudo-energies and samples.
+  // -1 = the general kernel, which alone applies structure constraints, stacking and unpaired pseudo-energies and samples.
   auto cls = [&](const Problem& q) {
     if (!rs.band || q.kind == KIND_DUPLEX || q.constrained) return -1;
     const int k = rp_kernel_plan(q.n, dev.smem_optin, nullptr);

@@ -52,6 +52,11 @@ struct BatchPlan {
   // stacking pseudo-energy factors exp(-E/kT) of the problems that carry such data (CON_STACK), laid out like seq, 1
   // elsewhere; empty when no problem of the batch does
   std::vector<double> stack;
+  // pair factors exp(+E/kT) of the unpaired pseudo-energies of the problems that carry them (CON_UNPAIRED), laid out
+  // like seq, 1 elsewhere, and per problem (3 per pair: s1, s2, s1&s2) the term sum_x -E_x/kT they add to log Z;
+  // both empty when no problem of the batch carries such data
+  std::vector<double> unpaired;
+  std::vector<double> unpaired_lz;
   std::vector<Problem> probs;            // three per pair: s1, s2, s1&s2
   // stochastic samples (rp_sample_plan), empty / 0 when no problem is sampled
   std::vector<rp_sample_layout> sample_layout;
@@ -106,18 +111,24 @@ int check_constraints(const rp_pair* pairs, const rp_constraint* cons, int n_pai
 // The stacking pseudo-energies of pairs that pass check_pairs (se may be null: none).  RP_OK, or RP_ERR_ARG with a
 // message in *msg that names the pair, the vector and the (1-based) position of a value that is not finite.
 int check_stack_energies(const rp_pair* pairs, const rp_stack_energy* se, int n_pairs, std::string* msg);
+// The unpaired pseudo-energies of pairs that pass check_pairs (ue may be null: none).  RP_OK; RP_ERR_ARG with a message
+// that names the pair, the vector and the (1-based) position of a value that is not finite; RP_ERR_UNSUPPORTED, naming
+// the pair, the problem and B, for a problem whose rounded data give B = sum_x |E_x| 10 / kT > UNPAIRED_MAX_B.
+constexpr double UNPAIRED_MAX_B = 345.38776394910684;   // ln 10^150
+int check_unpaired_energies(const rp_pair* pairs, const rp_unpaired_energy* ue, int n_pairs, const rp_opts* opts,
+                            std::string* msg);
 
 // The sampling options of pairs that pass check_pairs (so may be null: none).  RP_OK; RP_ERR_ARG for a negative count
 // or an unknown problem bit; RP_ERR_UNSUPPORTED, naming the pair, for a co-fold sample under --duplex.
 int check_samples(const rp_pair* pairs, int n_pairs, const rp_opts* opts, const rp_sample_opts* so, std::string* msg);
 
 // The pairs must pass check_pairs, the constraints check_constraints (cons == null: none), the stacking
-// pseudo-energies check_stack_energies (se == null: none) and the sampling options check_samples (so == null or
-// so->num == 0: none).  A problem that a constraint restricts, whose rounded pseudo-energies are not all 0, or that is
-// sampled runs on the general kernel.  Returns RP_OK, or RP_ERR_CUDA when a band launch shape fits no SM.
+// pseudo-energies check_stack_energies (se == null: none), the sampling options check_samples (so == null or
+// so->num == 0: none) and the unpaired pseudo-energies check_unpaired_energies (ue == null: none).  A problem that a
+// constraint restricts, whose rounded pseudo-energies are not all 0, or that is sampled runs on the general kernel.  Returns RP_OK, or RP_ERR_CUDA when a band launch shape fits no SM.
 int plan_batch(const rp_pair* pairs, int n_pairs, const rp_opts* opts, const DeviceFacts& dev, const RouteSettings& rs,
                BatchPlan* plan, const rp_constraint* cons = nullptr, const rp_stack_energy* se = nullptr,
-               const rp_sample_opts* so = nullptr);
+               const rp_sample_opts* so = nullptr, const rp_unpaired_energy* ue = nullptr);
 
 }  // namespace rp
 #endif

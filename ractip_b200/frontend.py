@@ -169,14 +169,16 @@ def predict(stage: ProbabilityStage, pairs: Sequence[Tuple[FastaRecord, FastaRec
             ip_opts: Optional[RpIpOpts] = None, show_energy: bool = False, zscore: int = 0, num_shuffling: int = 1000,
             seed: int = 1, use_constraint: bool = False, shape: Optional[Dict[str, Sequence[float]]] = None,
             shape_slope: float = 1.8, shape_intercept: float = -0.6, samples: int = 0,
-            sample_seed: int = 1) -> List[PairResult]:
+            sample_seed: int = 1, shape_method: str = "D") -> List[PairResult]:
     """Joint structures of all `pairs`: one GPU batch for every pair's matrices, then the integer programmes on the
     host.  zscore in (1, 2, 12): per pair one more GPU batch with all its dinucleotide shuffles (the loop of
     src/ractip.cpp:1636-1657 with the probability work hoisted out of it).  use_constraint (-c): the records'
     structure lines constrain the pairs' probability matrices (constraint_line); shuffles have no structure line and
     stay unconstrained.  shape: probing reactivities by record name (read_shape), turned into stacking
     pseudo-energies by shape_deigan(shape_slope, shape_intercept) for every record of that name; they bias the
-    probability matrices only, not the energies of -e, and the shuffles carry none.  samples > 0: that many structures
+    probability matrices only, not the energies of -e, and the shuffles carry none.  shape_method "W" reads the values
+    as unpaired pseudo-energies in kcal/mol instead (RNAfold --shapeMethod=W; a missing position counts as 0, negative
+    values are valid, slope and intercept do not apply).  samples > 0: that many structures
     of each pair's s1&s2 co-fold ensemble (constraints and pseudo-energies included), drawn with sample_seed in the
     same GPU batch, on PairResult.samples; the shuffles are never sampled."""
     opts = opts if opts is not None else default_opts()
@@ -186,16 +188,22 @@ def predict(stage: ProbabilityStage, pairs: Sequence[Tuple[FastaRecord, FastaRec
     seqs = [(a.seq, b.seq) for a, b in pairs]
     cons = [(constraint_line(a), constraint_line(b)) for a, b in pairs] if use_constraint else None
     kw = {}
+    if shape_method not in ("D", "W"):
+        raise ValueError(f"shape method {shape_method!r}: expected D or W")
     if shape:
         unknown = set(shape) - {r.name for ab in pairs for r in ab}
         if unknown:
             raise ValueError(f"reactivities for {', '.join(sorted(unknown))}: no such record")
-        de = lambda r: shape_deigan(shape[r.name], shape_slope, shape_intercept) if r.name in shape else None
-        kw["stack_energies"] = [(de(a), de(b)) for a, b in pairs]
+        if shape_method == "W":
+            de = lambda r: np.nan_to_num(np.asarray(shape[r.name], dtype=np.float64), nan=0.0) if r.name in shape else None
+            kw["unpaired_energies"] = [(de(a), de(b)) for a, b in pairs]
+        else:
+            de = lambda r: shape_deigan(shape[r.name], shape_slope, shape_intercept) if r.name in shape else None
+            kw["stack_energies"] = [(de(a), de(b)) for a, b in pairs]
     drawn = None
     if samples:
         bt = stage.batch(seqs, opts, cons, kw.get("stack_energies"), samples=samples, sample_seed=sample_seed,
-                         sample_problems=("co",))
+                         sample_problems=("co",), unpaired_energies=kw.get("unpaired_energies"))
         try:
             bt.run()
             probs = bt.split_dense(bt.fetch_dense())

@@ -22,7 +22,8 @@ import numpy as np
 
 from . import _lib
 from ._lib import (RpConstraint, RpDenseLayout, RpModel, RpOpts, RpPair, RpRec, RpSampleLayout, RpSampleOpts,
-                   RpSparseCounts, RpSparseLayout, RpSquareLayout, RpStackEnergy, RpTiming)
+                   RpSparseCounts, RpSparseLayout, RpSquareLayout, RpStackEnergy, RpTiming,
+                   RpUnpairedEnergy)
 
 
 class RpError(RuntimeError):
@@ -120,22 +121,28 @@ def _make_constraints(constraints: Sequence[Optional[Tuple[Optional[str], Option
     return arr, keep
 
 
-def _make_stack_energies(stack_energies, pairs: Sequence[Tuple[str, str]]):
+def _make_energies(energies, pairs: Sequence[Tuple[str, str]], struct=RpStackEnergy, what="stack_energies",
+                   field="e"):
+    """one `struct` (rp_stack_energy or rp_unpaired_energy) per pair from (v1, v2) per-base arrays, either None"""
     n = len(pairs)
-    if len(stack_energies) != n:
-        raise ValueError(f"stack_energies: {len(stack_energies)} entries for {n} pairs")
-    arr = (RpStackEnergy * max(n, 1))()
+    if len(energies) != n:
+        raise ValueError(f"{what}: {len(energies)} entries for {n} pairs")
+    arr = (struct * max(n, 1))()
     keep = []
-    for k, (ent, seqs) in enumerate(zip(stack_energies, pairs)):
+    for k, (ent, seqs) in enumerate(zip(energies, pairs)):
         for s, (e, seq) in enumerate(zip(ent if ent is not None else (None, None), seqs)):
             if e is None:
                 continue
             a = np.ascontiguousarray(e, dtype=np.float64)
             if a.shape != (len(seq),):
-                raise ValueError(f"stack_energies: pair {k}, e{s + 1} has shape {a.shape} for {len(seq)} nt")
+                raise ValueError(f"{what}: pair {k}, {field}{s + 1} has shape {a.shape} for {len(seq)} nt")
             keep.append(a)
-            setattr(arr[k], f"e{s + 1}", a.ctypes.data)
+            setattr(arr[k], f"{field}{s + 1}", a.ctypes.data)
     return arr, keep
+
+
+def _make_stack_energies(stack_energies, pairs: Sequence[Tuple[str, str]]):
+    return _make_energies(stack_energies, pairs)
 
 
 def shape_deigan(reactivities, slope: float = 1.8, intercept: float = -0.6) -> np.ndarray:
@@ -193,12 +200,14 @@ class DeviceBatch:
     stack_energies: None, or one (e1, e2) per pair -- stacking pseudo-energies in kcal/mol over s1 and s2
     (rp_batch_create_soft, e.g. from shape_deigan), either array (or the whole entry) None for none.
     samples > 0: every run also draws that many structures of each of sample_problems ("s1", "s2", "co") with
-    sample_seed (rp_batch_create_sampled); fetch_samples() and sample_tensors() return them."""
+    sample_seed (rp_batch_create_sampled); fetch_samples() and sample_tensors() return them.
+    unpaired_energies: None, or one (u1, u2) per pair -- unpaired pseudo-energies in kcal/mol over s1 and s2
+    (rp_batch_create_probed, RNAfold --shapeMethod=W), either array (or the whole entry) None for none."""
 
     def __init__(self, stage: "ProbabilityStage", pairs: Sequence[Tuple[str, str]], opts: RpOpts,
                  constraints: Optional[Sequence[Optional[Tuple[Optional[str], Optional[str]]]]] = None,
                  stack_energies=None, samples: int = 0, sample_seed: int = 1,
-                 sample_problems: Sequence[str] = ("s1", "s2", "co")):
+                 sample_problems: Sequence[str] = ("s1", "s2", "co"), unpaired_energies=None):
         self.stage, self.lib, self.opts = stage, stage.lib, opts
         self.pairs = list(pairs)
         self.n = len(self.pairs)
@@ -215,13 +224,18 @@ class DeviceBatch:
         self.samples = int(samples)
         self.sample_layout = (RpSampleLayout * max(self.n, 1))()
         self.total_samples = 0
-        if self.samples != 0:
+        if self.samples != 0 or unpaired_energies is not None:
             so = sample_opts(self.samples, sample_seed, sample_problems)
             cons, ckeep = _make_constraints(constraints, self.n) if constraints is not None else (None, None)
             se, ekeep = (_make_stack_energies(stack_energies, self.pairs) if stack_energies is not None
                          else (None, None))
-            stage._check(self.lib.rp_batch_create_sampled(stage.ctx, arr, cons, se, self.n, C.byref(opts),
-                                                          C.byref(so), C.byref(self.handle)))
+            if unpaired_energies is None:
+                stage._check(self.lib.rp_batch_create_sampled(stage.ctx, arr, cons, se, self.n, C.byref(opts),
+                                                              C.byref(so), C.byref(self.handle)))
+            else:
+                ue, ukeep = _make_energies(unpaired_energies, self.pairs, RpUnpairedEnergy, "unpaired_energies", "u")
+                stage._check(self.lib.rp_batch_create_probed(stage.ctx, arr, cons, se, ue, self.n, C.byref(opts),
+                                                             C.byref(so), C.byref(self.handle)))
             ts = C.c_size_t()
             stage._check(self.lib.rp_sample_plan(arr, self.n, C.byref(so), self.sample_layout, C.byref(ts)))
             self.total_samples = ts.value
@@ -436,21 +450,22 @@ class ProbabilityStage:
     # ------------------------------------------------------------- batches
     def batch(self, pairs: Sequence[Tuple[str, str]], opts: Optional[RpOpts] = None,
               constraints=None, stack_energies=None, samples: int = 0, sample_seed: int = 1,
-              sample_problems: Sequence[str] = ("s1", "s2", "co")) -> DeviceBatch:
+              sample_problems: Sequence[str] = ("s1", "s2", "co"), unpaired_energies=None) -> DeviceBatch:
         """constraints: None, or one (c1, c2) structure-constraint pair per pair; stack_energies: None, or one (e1, e2)
-        pair of stacking pseudo-energy arrays per pair; samples, sample_seed, sample_problems: stochastic samples
-        (DeviceBatch)."""
+        pair of stacking pseudo-energy arrays per pair; samples, sample_seed, sample_problems: stochastic samples;
+        unpaired_energies: None, or one (u1, u2) pair of unpaired pseudo-energy arrays per pair (DeviceBatch)."""
         return DeviceBatch(self, pairs, opts if opts is not None else default_opts(), constraints, stack_energies,
-                           samples, sample_seed, sample_problems)
+                           samples, sample_seed, sample_problems, unpaired_energies)
 
     def run_dense(self, pairs: Sequence[Tuple[str, str]], opts: Optional[RpOpts] = None,
-                  pinned: bool = False, constraints=None, stack_energies=None) -> List[PairProbabilities]:
+                  pinned: bool = False, constraints=None, stack_energies=None,
+                  unpaired_energies=None) -> List[PairProbabilities]:
         """rp_run_dense: host buffers in, host buffers out.  pinned=True hands the library a page-locked
-        buffer (rp_host_alloc) as the target of its device-to-host copy.  With constraints or stack_energies
-        (one entry per pair, see DeviceBatch) the pairs run as a device batch that carries them."""
+        buffer (rp_host_alloc) as the target of its device-to-host copy.  With constraints, stack_energies or
+        unpaired_energies (one entry per pair, see DeviceBatch) the pairs run as a device batch that carries them."""
         opts = opts if opts is not None else default_opts()
-        if constraints is not None or stack_energies is not None:
-            b = self.batch(pairs, opts, constraints, stack_energies)
+        if constraints is not None or stack_energies is not None or unpaired_energies is not None:
+            b = self.batch(pairs, opts, constraints, stack_energies, unpaired_energies=unpaired_energies)
             try:
                 b.run()
                 return b.split_dense(b.fetch_dense())
@@ -498,9 +513,9 @@ class ProbabilityStage:
             b.close()
 
     def run_sparse(self, pairs: Sequence[Tuple[str, str]], opts: Optional[RpOpts] = None,
-                   constraints=None, stack_energies=None) -> List[PairRecords]:
+                   constraints=None, stack_energies=None, unpaired_energies=None) -> List[PairRecords]:
         opts = opts if opts is not None else default_opts()
-        b = self.batch(pairs, opts, constraints, stack_energies)
+        b = self.batch(pairs, opts, constraints, stack_energies, unpaired_energies=unpaired_energies)
         try:
             b.run()
             return b.split_sparse(*b.fetch_sparse())
