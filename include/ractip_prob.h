@@ -379,6 +379,45 @@ int rp_batch_create_probed(rp_ctx* ctx, const rp_pair* pairs,
  * rules of rp_batch_dense_device).  RP_ERR_CAPACITY when n < total. */
 int rp_batch_fetch_samples(rp_batch* batch, int16_t* out, size_t n);
 int rp_batch_samples_device(rp_batch* batch, void* out_dev, size_t n);
+/* Minimum free energy (MFE) structures (RNAfold / RNAcofold's first line):
+ * for each requested problem of each pair, the minimum over every structure S
+ * of exactly the ensemble the partition function sums over (canonical pairs
+ * with j-i > TURN across the nick too, interior loops up to MAXLOOP, the
+ * pair's constraint keys as rp_batch_create_constrained builds them; s1 takes
+ * e1/u1, s2 e2/u2, the co-fold both) of
+ *   E(S) = rp_energy_of_structure(seq, S, cut_point)     (0.01 kcal/mol)
+ *        + sum over stacks (i,j),(i+1,j-1) of S within one strand of
+ *          Es(i) + Es(i+1) + Es(j-1) + Es(j)
+ *        + sum over bases x unpaired in S of Eu(x)
+ * with Es, Eu rounded as rp_batch_create_soft / rp_batch_create_probed round
+ * them; in the co-fold a stack that joins the strands gets no Es, and a base
+ * paired with the partner counts as unpaired.  The co-fold (cut_point =
+ * n1+1) adds DuplexInit once when a pair joins the strands, as
+ * rp_energy_of_duplex and -e count it, so that
+ *   MFE(s1&s2) = min(MFE of the unjoined structures, i.e. s1's and s2's folds
+ *                under the co-fold's constraint,
+ *                min over joined structures + DuplexInit);
+ * the partition function (log Z, probabilities, samples) leaves DuplexInit
+ * out.  The result is exact integer arithmetic.  One structure that reaches
+ * the minimum is returned; ties are broken by a fixed candidate order.
+ *
+ * `problems` is a mask of RP_SAMPLE_* (unknown bits: RP_ERR_ARG); a pair with
+ * n2 == 0 has s1 only.  structures: the layout of rp_sample_plan with num = 1
+ * and the same mask (RP_ERR_CAPACITY when n_structures is smaller); energies:
+ * 3 int32 per pair (s1, s2, s1&s2) in 0.01 kcal/mol, RP_INF for a problem not
+ * computed.  cons, se, ue (each may be NULL) are checked as
+ * rp_batch_create_probed checks them, with the same messages, except that the
+ * pf_scale range of unpaired pseudo-energies does not apply.  Instead a
+ * problem whose sum over its bases of |Es| + |Eu| (0.01 kcal/mol, after
+ * rounding) exceeds RP_INF / 4 (25000 kcal/mol) is RP_ERR_UNSUPPORTED,
+ * naming the pair and the problem: every energy then stays far from the
+ * int32 range next to the kernel's INF sentinel.  rp_opts plays no part
+ * (--duplex changes how hp is computed, not the co-fold's MFE).  Synchronous,
+ * host buffers, on the context's stream. */
+int rp_run_mfe(rp_ctx* ctx, const rp_pair* pairs, const rp_constraint* cons,
+               const rp_stack_energy* se, const rp_unpaired_energy* ue,
+               int n_pairs, int problems, int16_t* structures,
+               size_t n_structures, int32_t* energies);
 int rp_batch_run(rp_batch* batch);                 /* async on the ctx stream */
 int rp_batch_sync(rp_batch* batch);
 int rp_batch_fetch_dense(rp_batch* batch, float* out, size_t out_floats);

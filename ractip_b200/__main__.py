@@ -47,6 +47,9 @@ def main(argv=None) -> int:
     ap.add_argument("--sample", type=int, default=0, metavar="N",
                     help="after each pair, N structures sampled from its s1&s2 co-fold ensemble, one r1&r2 per line")
     ap.add_argument("--sample-seed", type=int, default=1, metavar="S", help="seed of --sample (default 1)")
+    ap.add_argument("--mfe", action="store_true",
+                    help="after each pair (and its samples), the minimum free energy structures of s1, s2 and the s1&s2 "
+                         "co-fold, honouring -c and --shape")
     args = ap.parse_args(argv)
     if len(args.fasta) > 2:
         ap.error("at most two FASTA files")
@@ -88,7 +91,7 @@ def main(argv=None) -> int:
         for r in predict(stage, pairs, opts, ipo, args.show_energy, args.zscore, args.num_shuffling, args.seed,
                          use_constraint=args.use_constraint, shape=shape, shape_slope=args.shape_slope,
                          shape_intercept=args.shape_intercept, samples=args.sample, sample_seed=args.sample_seed,
-                         shape_method=args.shape_method):
+                         shape_method=args.shape_method, mfe=args.mfe):
             print(format_result(r, args.show_energy))
     except RpError as e:
         probed = bool(shape) and args.shape_method == "W"

@@ -129,7 +129,7 @@ EXPORTS = [
     "rp_batch_fetch_dense", "rp_batch_fetch_sparse", "rp_batch_sparse_device", "rp_batch_dense_device",
     "rp_square_plan", "rp_batch_square_device", "rp_batch_fetch_logz",
     "rp_sample_plan", "rp_batch_create_sampled", "rp_batch_create_probed", "rp_batch_fetch_samples", "rp_batch_samples_device",
-    "rp_batch_destroy", "rp_last_timing", "rp_measure_peaks", "rp_zscore_shuffles",
+    "rp_run_mfe", "rp_batch_destroy", "rp_last_timing", "rp_measure_peaks", "rp_zscore_shuffles",
     "rp_alg_flops_mcc", "rp_version", "rp_kernel_plan",
     "rp_multi_create", "rp_multi_destroy", "rp_multi_devices", "rp_multi_last_error", "rp_multi_run_dense",
     "rp_multi_run_sparse",
@@ -193,6 +193,7 @@ def load() -> C.CDLL:
         "rp_batch_create_probed": (i, [vp, P(RpPair), P(RpConstraint), P(RpStackEnergy), P(RpUnpairedEnergy), i,
                                        P(RpOpts), P(RpSampleOpts), P(vp)]),
         "rp_batch_fetch_samples": (i, [vp, vp, sz]),
+        "rp_run_mfe": (i, [vp, P(RpPair), P(RpConstraint), P(RpStackEnergy), P(RpUnpairedEnergy), i, i, vp, sz, vp]),
         "rp_batch_samples_device": (i, [vp, vp, sz]),
         "rp_batch_destroy": (i, [vp]),
         "rp_last_timing": (i, [vp, P(RpTiming)]),

@@ -30,6 +30,7 @@ struct rp_ctx {
   int ctas_per_sm = 0;       // general kernel, 64-register build (two CTAs per SM)
   int ctas_per_sm1 = 0;      // general kernel, 128-register build (one CTA per SM: long problems)
   int up_ctas_per_sm = 0;    // unstru_kernel occupancy
+  int mfe_ctas_per_sm = 0;   // mfe_kernel occupancy
   size_t smem_optin = 0;     // max dynamic shared memory per CTA
   rp::RouteSettings route;   // read from the environment at rp_create
   rp::DevModel* d_model = nullptr;
@@ -202,6 +203,7 @@ rp::DeviceFacts device_facts(rp_ctx* ctx) {
   f.ctas_per_sm = ctx->ctas_per_sm;
   f.ctas_per_sm1 = ctx->ctas_per_sm1;
   f.up_ctas_per_sm = ctx->up_ctas_per_sm;
+  f.mfe_ctas_per_sm = ctx->mfe_ctas_per_sm;
   f.ws_bytes = ctx->ws_bytes;
   f.band_occupancy = rp::band_max_ctas_per_sm;
   f.memory = [ctx]() -> size_t {   // cached buffers are freed on demand
@@ -291,6 +293,7 @@ int rp_create(rp_ctx** out, const rp_model* m, int device) {
   ctx->ctas_per_sm = rp::mcc_max_ctas_per_sm(2);
   ctx->ctas_per_sm1 = rp::mcc_max_ctas_per_sm(1);
   ctx->up_ctas_per_sm = rp::unstru_max_ctas_per_sm();
+  ctx->mfe_ctas_per_sm = rp::mfe_max_ctas_per_sm();
   if (ctx->ctas_per_sm < 1)
     return bail(RP_ERR_CUDA, "rp_create: kernel image not loadable on this device (built for sm_100a)");
   *out = ctx;
@@ -835,6 +838,88 @@ int rp_last_timing(const rp_ctx* cctx, rp_timing* t) {
 }
 
 // ------------------------------------------------------- one-shot host calls
+int rp_run_mfe(rp_ctx* ctx, const rp_pair* pairs, const rp_constraint* cons, const rp_stack_energy* se,
+               const rp_unpaired_energy* ue, int n_pairs, int problems, int16_t* structures, size_t n_structures,
+               int32_t* energies) {
+  if (!ctx || (n_pairs > 0 && !energies)) return fail(ctx, RP_ERR_ARG, "rp_run_mfe: null argument");
+  std::string msg;
+  const std::string who = "rp_run_mfe: ";
+  int rc = rp::check_mfe(pairs, n_pairs, cons, se, ue, problems, &msg);
+  if (rc != RP_OK) return fail(ctx, rc, who + msg);
+  rp::MfePlan m;
+  if ((rc = rp::plan_mfe(pairs, n_pairs, cons, se, ue, problems, device_facts(ctx), &m, &msg)) != RP_OK)
+    return fail(ctx, rc, who + (msg.empty() ? std::string("sizes overflow the structure buffer") : msg));
+  if (n_structures < m.total || (m.total && !structures))
+    return fail(ctx, RP_ERR_CAPACITY, "rp_run_mfe: the structure buffer holds fewer int16 than rp_sample_plan (num = 1) asks");
+  for (int k = 0; k < 3 * n_pairs; k++) energies[k] = RP_INF;
+  if (m.jobs.empty()) return RP_OK;
+  CU(cudaSetDevice(ctx->device));
+  cudaStream_t st = ctx->stream;
+  if ((rc = ensure_workspace(ctx, (size_t)m.grid * m.slot_ints * sizeof(int32_t))) != RP_OK) return rc;
+  if (ctx->ws_stream && ctx->ws_stream != st) CU(cudaStreamSynchronize(ctx->ws_stream));   // its last user is done
+  ctx->ws_stream = st;
+  // device buffers from the pool, released at the end of the call
+  std::vector<void*> bufs;
+  auto release = [&]() { for (void* p : bufs) pool_release(ctx, p); };
+  auto up = [&](const void* src, size_t bytes, void** dst) -> cudaError_t {
+    *dst = nullptr;
+    if (!bytes) return cudaSuccess;
+    cudaError_t e = pool_alloc(ctx, dst, bytes);
+    if (e != cudaSuccess) return e;
+    bufs.push_back(*dst);
+    return src ? cudaMemcpyAsync(*dst, src, bytes, cudaMemcpyHostToDevice, st) : cudaSuccess;
+  };
+  rp::MfeDev d = {};
+  std::vector<int32_t> e_init((size_t)3 * n_pairs, RP_INF);
+  const int zero = 0;
+  void *d_seq, *d_key, *d_es, *d_eu, *d_jobs, *d_counter, *d_struct, *d_energy;
+  cudaError_t e = cudaSuccess;
+  if (e == cudaSuccess) e = up(m.seq.data(), m.seq.size(), &d_seq);
+  if (e == cudaSuccess) e = up(m.key.data(), m.key.size() * sizeof(uint16_t), &d_key);
+  if (e == cudaSuccess) e = up(m.es.data(), m.es.size() * sizeof(int32_t), &d_es);
+  if (e == cudaSuccess) e = up(m.eu.data(), m.eu.size() * sizeof(int32_t), &d_eu);
+  if (e == cudaSuccess) e = up(m.jobs.data(), m.jobs.size() * sizeof(rp::MfeJob), &d_jobs);
+  if (e == cudaSuccess) e = up(&zero, sizeof(int), &d_counter);
+  if (e == cudaSuccess) e = up(nullptr, std::max<size_t>(m.total, 1) * sizeof(int16_t), &d_struct);
+  if (e == cudaSuccess) e = up(e_init.data(), e_init.size() * sizeof(int32_t), &d_energy);
+  if (e == cudaSuccess) {
+    d.model = ctx->d_model;
+    d.seq = static_cast<const uint8_t*>(d_seq);
+    d.key = static_cast<const uint16_t*>(d_key);
+    d.es = static_cast<const int32_t*>(d_es);
+    d.eu = static_cast<const int32_t*>(d_eu);
+    d.jobs = static_cast<const rp::MfeJob*>(d_jobs);
+    d.njobs = (int)m.jobs.size();
+    d.counter = static_cast<int*>(d_counter);
+    d.ws = reinterpret_cast<int32_t*>(ctx->ws);
+    d.slot_ints = m.slot_ints;
+    d.structures = static_cast<int16_t*>(d_struct);
+    d.energies = static_cast<int32_t*>(d_energy);
+    ctx->timing = rp_timing{};
+    cudaEventRecord(ctx->ev[0], st);
+    e = rp::launch_mfe(d, m.grid, st);
+    cudaEventRecord(ctx->ev[1], st);
+  }
+  if (e == cudaSuccess && m.total) e = cudaMemcpyAsync(structures, d_struct, m.total * sizeof(int16_t), cudaMemcpyDeviceToHost, st);
+  if (e == cudaSuccess) e = cudaMemcpyAsync(energies, d_energy, e_init.size() * sizeof(int32_t), cudaMemcpyDeviceToHost, st);
+  if (e == cudaSuccess) e = cudaStreamSynchronize(st);
+  if (e != cudaSuccess) {
+    cudaStreamSynchronize(st);
+    release();
+    return fail(ctx, RP_ERR_CUDA, std::string("rp_run_mfe: ") + cudaGetErrorString(e));
+  }
+  float ms = 0.f;
+  cudaEventElapsedTime(&ms, ctx->ev[0], ctx->ev[1]);
+  ctx->timing.ms_total = ms;
+  ctx->timing.kernel_launches = 1;
+  ctx->timing.dominant_kind = -1;
+  ctx->timing_pending = false;
+  ctx->dom_timed = false;
+  ctx->timed_copies = false;
+  release();
+  return RP_OK;
+}
+
 int rp_run_dense(rp_ctx* ctx, const rp_pair* pairs, int n_pairs, const rp_opts* opts, float* out, size_t out_floats) {
   if (!ctx || !out) return fail(ctx, RP_ERR_ARG, "rp_run_dense: null argument");
   rp_batch* b = nullptr;

@@ -148,6 +148,20 @@ int build_dev_model(const rp_model& m, DevModel* out) {
   D.i_ninio = m.ninio37;
   D.i_MAX_NINIO = m.MAX_NINIO;
   D.i_DuplexInit = m.DuplexInit37;
+  for (int u = 0; u <= 30; u++) D.i_hairpin[u] = m.hairpin37[u];
+  for (int t = 0; t < 8; t++)
+    for (int a = 0; a < 5; a++)
+      for (int b = 0; b < 5; b++) {
+        D.i_mmH[t][a][b] = m.mismatchH37[t][a][b];
+        D.i_mmM[t][a][b] = std::min(0, m.mismatchM37[t][a][b]);
+      }
+  D.i_MLbase = m.ML_BASE37;
+  D.i_MLclosing = m.ML_closing37;
+  D.i_MLintern = m.ML_intern37;
+  for (int i = 0; i < 200; i++) D.i_tetra[i] = m.Tetraloop37[i];
+  for (int i = 0; i < 40; i++) D.i_tri[i] = m.Triloop37[i];
+  for (int i = 0; i < 200; i++) D.i_hex[i] = m.Hexaloop37[i];
+  for (int u = 31; u <= HP_LONG_MAX; u++) D.i_hairpin_long[u] = m.hairpin37[30] + (int)(m.lxc37 * std::log(u / 30.));
 
   D.special_hp = m.special_hp;
   D.n_tetra = parse_special(m.Tetraloops, 6, 200, D.tetra_code);

@@ -29,6 +29,7 @@ constexpr int MAXLOOP = RP_MAXLOOP;
 // (class SPECIAL) and are evaluated directly.
 enum { CLS_GENERIC = 0, CLS_1N = 1, CLS_BULGE = 2, CLS_SPECIAL = 3, CLS_NONE = 255 };
 constexpr int GROW_LD = 32;
+constexpr int HP_LONG_MAX = 12000;   // longest hairpin loop of DevModel::i_hairpin_long (= RP_MAX_N, mcc_core.h)
 
 // Table-driven small loops (the nine shapes that do not factorise: stack, 1-bulge, 1x1, 1x2, 2x1, 2x2, 2x3,
 // 3x2): ONE flat table of finished weights, scale included, so that a look-up is an index computation and
@@ -80,6 +81,14 @@ struct DevModel {
   int i_stack[8][8], i_bulge[31], i_internal[31], i_mmI[8][5][5], i_mm1n[8][5][5], i_mm23[8][5][5];
   int i_int11[8][8][5][5], i_int21[8][8][5][5][5], i_int22[8][8][5][5][5][5];
   int i_TermAU, i_ninio, i_MAX_NINIO, i_DuplexInit;
+  // Integer view for the MFE kernel (mfe_core.h), appended so that every field above keeps its offset.  Exactly the
+  // values rp_energy_of_structure (eval.cpp) uses: mismatchM clipped to <= 0 like the dangles, the rest as is.
+  // i_hairpin_long[u] = hairpin37[30] + (int)(lxc37 * ln(u / 30)) for 30 < u <= HP_LONG_MAX, computed on the host with
+  // eval.cpp's expression, so that the truncation to int does not hinge on the device's log().
+  int i_hairpin[31], i_mmH[8][5][5], i_mmM[8][5][5];
+  int i_MLbase, i_MLclosing, i_MLintern;
+  int i_tetra[200], i_tri[40], i_hex[200];
+  int i_hairpin_long[HP_LONG_MAX + 1];
 };
 
 // Host: integer model -> DevModel.  Returns RP_OK or an error code.

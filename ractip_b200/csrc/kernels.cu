@@ -215,6 +215,32 @@ __global__ void __launch_bounds__(RP_UP_THREADS, 1) unstru_kernel(BatchDev b) {
   }
 }
 
+// mfe_kernel (rp_run_mfe): the minimum free energy and one structure that reaches it (mfe_core.h), one problem per CTA
+// from a queue ordered by decreasing length, in an int32 workspace slot per CTA.
+__global__ void __launch_bounds__(RP_MFE_THREADS, 1) mfe_kernel(MfeDev b) {
+  __shared__ int s_next;
+  __shared__ int s_red[RP_MFE_THREADS];
+  __shared__ int s_e;
+  CtaExec ex;
+  ex.prof = nullptr;
+  for (;;) {
+    if (threadIdx.x == 0) s_next = atomicAdd(b.counter, 1);
+    __syncthreads();
+    const int q = s_next;
+    __syncthreads();
+    if (q >= b.njobs) break;
+    const MfeJob j = b.jobs[q];
+    MfeCtx c;
+    bind_mfe(c, b.model, b.seq + j.seq_off - 1, j.n, j.cp, b.ws + (size_t)blockIdx.x * b.slot_ints);
+    if (j.flags & CON_KEYS) c.key = b.key + j.seq_off - 1;
+    if (j.flags & CON_STACK) c.es = b.es + j.seq_off - 1;
+    if (j.flags & CON_UNPAIRED) c.eu = b.eu + j.seq_off - 1;
+    solve_mfe(ex, c, s_red, b.structures + j.out, &s_e);
+    if (threadIdx.x == 0) b.energies[j.energy_at] = s_e >= MFE_BIG ? RP_INF : s_e + j.eu_const;
+    __syncthreads();
+  }
+}
+
 // ---------------------------------------------------------------------------
 // pf_duplex (--duplex): log-space forward/backward over pure duplexes.
 // Restates reference src/pf_duplex.c:128-164 (fw), :166-206 (bk), :97-103 (pr)
@@ -656,6 +682,16 @@ int unstru_max_ctas_per_sm() {
 }
 cudaError_t launch_unstru(const BatchDev& b, int grid, cudaStream_t st) {
   unstru_kernel<<<grid, RP_UP_THREADS, 0, st>>>(b);
+  return cudaGetLastError();
+}
+
+int mfe_max_ctas_per_sm() {
+  int n = 0;
+  if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, mfe_kernel, RP_MFE_THREADS, 0) != cudaSuccess) { cudaGetLastError(); return 0; }
+  return n;
+}
+cudaError_t launch_mfe(const MfeDev& m, int grid, cudaStream_t st) {
+  mfe_kernel<<<grid, RP_MFE_THREADS, 0, st>>>(m);
   return cudaGetLastError();
 }
 

@@ -7,6 +7,7 @@
 
 #include "mcc_band.h"
 #include "mcc_core.h"
+#include "mfe_core.h"
 #include "ractip_prob.h"
 
 namespace rp {
@@ -92,6 +93,25 @@ int mcc_max_ctas_per_sm(int minb);
 cudaError_t launch_mcc(const BatchDev& b, int grid, int minb, cudaStream_t st);
 // multi-CTA wavefront: `nclusters` clusters of `ctas` (8 or 16) CTAs, one problem (and one workspace slot) per cluster
 cudaError_t launch_mcc_cluster(const BatchDev& b, int nclusters, int ctas, cudaStream_t st);
+// mfe_kernel (rp_run_mfe): one CTA per problem of the queue `jobs` (longest first), RP_MFE_THREADS threads, int32
+// workspace slots of slot_ints; per-base arrays laid out like seq, null when no problem carries them
+constexpr int RP_MFE_THREADS = 512;
+struct MfeDev {
+  const DevModel* model;
+  const uint8_t* seq;
+  const uint16_t* key;
+  const int32_t* es;
+  const int32_t* eu;
+  const MfeJob* jobs;
+  int njobs;
+  int* counter;
+  int32_t* ws;
+  size_t slot_ints;
+  int16_t* structures;
+  int32_t* energies;   // 3 per pair; RP_INF stays where no problem writes
+};
+int mfe_max_ctas_per_sm();
+cudaError_t launch_mfe(const MfeDev& m, int grid, cudaStream_t st);
 int band_max_ctas_per_sm(int threads, size_t smem);   // threads = 256 (2 CTAs/SM) or 512 (1 CTA/SM)
 cudaError_t launch_band(const BatchDev& b, int grid, int threads, size_t smem, cudaStream_t st);
 cudaError_t launch_duplex(const BatchDev& b, int grid, cudaStream_t st);

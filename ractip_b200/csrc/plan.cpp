@@ -110,6 +110,19 @@ int check_stack_energies(const rp_pair* pairs, const rp_stack_energy* se, int n_
   return RP_OK;
 }
 
+namespace {
+// A pseudo-energy in kcal/mol as an integer number of 0.01 kcal/mol, half away from zero (as ViennaRNA stores
+// soft-constraint energies): the one rounding of every pseudo-energy the stage takes.
+double cal_units(double kcal) { return std::round(kcal * 100.0); }
+
+int unpaired_not_finite(int p, int s, int i, double v, std::string* msg) {
+  char buf[160];
+  std::snprintf(buf, sizeof buf, "pair %d, u%d, position %d: %g kcal/mol is not finite", p, s + 1, i + 1, v);
+  if (msg) *msg = buf;
+  return RP_ERR_ARG;
+}
+}  // namespace
+
 // Unpaired pseudo-energies: u1 over s1, u2 over s2, in kcal/mol (either may be null).  After rounding, a problem's
 // weights move by at most a factor e^B either way against the same problem without data, B = sum_x |E_x| 10 / kT over
 // the bases it applies; pf_scale is global, so B must leave the tables room in fp64 (UNPAIRED_MAX_B).
@@ -125,12 +138,8 @@ int check_unpaired_energies(const rp_pair* pairs, const rp_unpaired_energy* ue, 
     for (int s = 0; s < 2; s++) {
       if (!us[s]) continue;
       for (int i = 0; i < ns[s]; i++) {
-        if (!std::isfinite(us[s][i])) {
-          std::snprintf(buf, sizeof buf, "pair %d, u%d, position %d: %g kcal/mol is not finite", p, s + 1, i + 1, us[s][i]);
-          if (msg) *msg = buf;
-          return RP_ERR_ARG;
-        }
-        B[s] += std::fabs(std::round(us[s][i] * 100.0)) * 10.0 / kT;
+        if (!std::isfinite(us[s][i])) return unpaired_not_finite(p, s, i, us[s][i], msg);
+        B[s] += std::fabs(cal_units(us[s][i])) * 10.0 / kT;
       }
     }
     // s1's fold takes u1, s2's u2, the co-fold both (not under --duplex)
@@ -146,6 +155,18 @@ int check_unpaired_energies(const rp_pair* pairs, const rp_unpaired_energy* ue, 
         if (msg) *msg = buf;
         return RP_ERR_UNSUPPORTED;
       }
+  }
+  return RP_OK;
+}
+
+int check_unpaired_finite(const rp_pair* pairs, const rp_unpaired_energy* ue, int n_pairs, std::string* msg) {
+  if (!ue) return RP_OK;
+  for (int p = 0; p < n_pairs; p++) {
+    const double* us[2] = {ue[p].u1, ue[p].u2};
+    const int ns[2] = {pairs[p].n1, pairs[p].n2};
+    for (int s = 0; s < 2; s++)
+      for (int i = 0; us[s] && i < ns[s]; i++)
+        if (!std::isfinite(us[s][i])) return unpaired_not_finite(p, s, i, us[s][i], msg);
   }
   return RP_OK;
 }
@@ -192,7 +213,7 @@ bool fill_stack(const double* e, int m, double* f) {
   const double kT = (37.0 + RP_K0) * RP_GASCONST;
   bool any = false;
   for (int i = 1; i <= m; i++) {
-    const double E = std::round(e[i - 1] * 100.0);
+    const double E = cal_units(e[i - 1]);
     f[i] = std::exp(-E * 10.0 / kT);
     any |= E != 0.;
   }
@@ -208,7 +229,7 @@ bool fill_unpaired(const double* u, int m, double* g, double* lnf) {
   const double kT = (37.0 + RP_K0) * RP_GASCONST;
   bool any = false;
   for (int i = 1; i <= m; i++) {
-    const double E = std::round(u[i - 1] * 100.0);
+    const double E = cal_units(u[i - 1]);
     g[i] = std::exp(E * 10.0 / kT);
     *lnf -= E * 10.0 / kT;
     any |= E != 0.;
@@ -248,6 +269,32 @@ void intra_partners(const char* c, int n, const char* unpaired, std::vector<int>
     else if (c[i - 1] == ')') { partner[i] = open.back(); partner[open.back()] = i; open.pop_back(); }
     else if (std::strchr(unpaired, c[i - 1])) partner[i] = -1;
   }
+}
+
+// Keys of the three problems of a pair (s1 at k1[1..n1], s2 at k2[1..n2], the co-fold at k12[1..n1+n2]) from its
+// constraint strings c1, c2 (either may be null), and in con[w] whether problem w is restricted.  `cofold`: the co-fold
+// is constrained (not under --duplex, and n2 > 0).
+void pair_keys(const rp_pair& pr, const char* c1, const char* c2, bool cofold, uint16_t* k1, uint16_t* k2, uint16_t* k12,
+               int con[3]) {
+  std::vector<int> partner;
+  intra_partners(c1, pr.n1, "x[", partner);
+  con[0] = fill_keys(partner, pr.n1, k1);
+  intra_partners(c2, pr.n2, "x]", partner);
+  con[1] = fill_keys(partner, pr.n2, k2);
+  // s1&s2: the k-th '[' from the 3' end of c1 with the k-th ']' from the 5' end of c2
+  const int n12 = pr.n1 + pr.n2;
+  partner.assign(n12 + 1, 0);
+  std::vector<int> ends;
+  for (int i = pr.n1; i >= 1; i--)
+    if (c1 && c1[i - 1] == '[') ends.push_back(i);
+  size_t k = 0;
+  for (int j = 1; j <= pr.n2; j++)
+    if (c2 && c2[j - 1] == ']') { partner[ends[k]] = pr.n1 + j; partner[pr.n1 + j] = ends[k]; k++; }
+  for (int i = 1; i <= n12; i++) {
+    const char ch = i <= pr.n1 ? (c1 ? c1[i - 1] : '.') : (c2 ? c2[i - pr.n1 - 1] : '.');
+    if (ch == 'x' || ch == '(' || ch == ')') partner[i] = -1;
+  }
+  con[2] = cofold && fill_keys(partner, n12, k12);
 }
 }  // namespace
 
@@ -448,7 +495,6 @@ int plan_batch(const rp_pair* pairs, int n_pairs, const rp_opts* opts, const Dev
   seq.reserve(bytes + 16);
   std::vector<uint16_t>& key = b.key;   // (filled only for batches with constraints, then dropped if none restricts)
   bool any_constrained = false;
-  std::vector<int> partner;
   std::vector<double>& stack = b.stack;   // (the same for the stacking factors)
   bool any_stack = false;
   std::vector<double>& unp = b.unpaired;   // (and for the unpaired pseudo-energies' pair factors)
@@ -471,26 +517,10 @@ int plan_batch(const rp_pair* pairs, int n_pairs, const rp_opts* opts, const Dev
     seq.push_back(0);
     int con[3] = {0, 0, 0};   // s1, s2, s1&s2 restricted by the constraint
     if (cons && (cons[p].c1 || cons[p].c2)) {
-      const char *c1 = cons[p].c1, *c2 = cons[p].c2;
       key.resize(seq.size(), 0);
-      intra_partners(c1, pr.n1, "x[", partner);
-      con[0] = fill_keys(partner, pr.n1, &key[off1 - 1]);
-      intra_partners(c2, pr.n2, "x]", partner);
-      con[1] = fill_keys(partner, pr.n2, &key[off2 - 1]);
-      // s1&s2: the k-th '[' from the 3' end of c1 with the k-th ']' from the 5' end of c2
-      const int n12 = pr.n1 + pr.n2;
-      partner.assign(n12 + 1, 0);
-      std::vector<int> ends;
-      for (int i = pr.n1; i >= 1; i--)
-        if (c1 && c1[i - 1] == '[') ends.push_back(i);
-      size_t k = 0;
-      for (int j = 1; j <= pr.n2; j++)
-        if (c2 && c2[j - 1] == ']') { partner[ends[k]] = pr.n1 + j; partner[pr.n1 + j] = ends[k]; k++; }
-      for (int i = 1; i <= n12; i++) {
-        const char ch = i <= pr.n1 ? (c1 ? c1[i - 1] : '.') : (c2 ? c2[i - pr.n1 - 1] : '.');
-        if (ch == 'x' || ch == '(' || ch == ')') partner[i] = -1;
-      }
-      con[2] = pr.n2 > 0 && !opts->use_pf_duplex && fill_keys(partner, n12, &key[off12 - 1]);   // --duplex: unconstrained
+      // --duplex: the co-fold is unconstrained
+      pair_keys(pr, cons[p].c1, cons[p].c2, pr.n2 > 0 && !opts->use_pf_duplex, &key[off1 - 1], &key[off2 - 1],
+                &key[off12 - 1], con);
       any_constrained |= con[0] || con[1] || con[2];
     }
     // stacking pseudo-energies: s1's fold takes e1, s2's e2, the co-fold both (stack_sc, mcc_core.h, leaves out the
@@ -729,6 +759,139 @@ int plan_batch(const rp_pair* pairs, int n_pairs, const rp_opts* opts, const Dev
       b.split_fetch = !b.sect_long.empty() && !b.sect_short.empty();
     }
   }
+  return RP_OK;
+}
+
+int check_mfe(const rp_pair* pairs, int n_pairs, const rp_constraint* cons, const rp_stack_energy* se,
+              const rp_unpaired_energy* ue, int problems, std::string* msg) {
+  const rp_opts o = {15, 5, 0.5f, 0.1f, 0.003f, 0};   // rp_opts plays no part; check_pairs only needs one
+  if (check_pairs(pairs, n_pairs, &o)) {
+    if (msg) *msg = "bad pairs";
+    return RP_ERR_ARG;
+  }
+  for (int p = 0; p < n_pairs; p++)
+    if ((long long)pairs[p].n1 + pairs[p].n2 > RP_MAX_N) {
+      if (msg) *msg = "n1+n2 exceeds the 32-bit workspace indexing limit (12000 nt)";
+      return RP_ERR_TOO_LONG;
+    }
+  if (problems & ~(RP_SAMPLE_S1 | RP_SAMPLE_S2 | RP_SAMPLE_COFOLD)) {
+    char buf[96];
+    std::snprintf(buf, sizeof buf, "unknown bits 0x%x in the requested problems", problems & ~7);
+    if (msg) *msg = buf;
+    return RP_ERR_ARG;
+  }
+  int rc;
+  if ((rc = check_constraints(pairs, cons, n_pairs, msg)) != RP_OK) return rc;
+  if ((rc = check_stack_energies(pairs, se, n_pairs, msg)) != RP_OK) return rc;
+  return check_unpaired_finite(pairs, ue, n_pairs, msg);
+}
+
+int plan_mfe(const rp_pair* pairs, int n_pairs, const rp_constraint* cons, const rp_stack_energy* se,
+             const rp_unpaired_energy* ue, int problems, const DeviceFacts& dev, MfePlan* out, std::string* msg) {
+  MfePlan& m = *out;
+  m = MfePlan{};
+  rp_sample_opts so = {1, 0, problems};
+  m.layout.resize(n_pairs);
+  if (rp_sample_plan(pairs, n_pairs, &so, m.layout.data(), &m.total) != RP_OK) return RP_ERR_ARG;
+  size_t bytes = 0;
+  for (int p = 0; p < n_pairs; p++) bytes += 2 * ((size_t)pairs[p].n1 + pairs[p].n2) + 4;
+  m.seq.reserve(bytes + 16);
+  bool any_key = false, any_es = false, any_eu = false;
+  const char* names[3] = {"s1", "s2", "s1&s2"};
+  int maxn = 0;
+  for (int p = 0; p < n_pairs; p++) {
+    const rp_pair& pr = pairs[p];
+    const rp_sample_layout& L = m.layout[p];
+    m.seq.push_back(0);
+    const int off1 = (int)m.seq.size();
+    for (int i = 0; i < pr.n1; i++) m.seq.push_back(encode_base(pr.s1[i]));
+    m.seq.push_back(0);
+    const int off2 = (int)m.seq.size();
+    for (int i = 0; i < pr.n2; i++) m.seq.push_back(encode_base(pr.s2[i]));
+    m.seq.push_back(0);
+    const int off12 = (int)m.seq.size();
+    for (int i = 0; i < pr.n1; i++) m.seq.push_back(encode_base(pr.s1[i]));
+    for (int i = 0; i < pr.n2; i++) m.seq.push_back(encode_base(pr.s2[i]));
+    m.seq.push_back(0);
+    int flags[3] = {0, 0, 0};
+    if (cons && (cons[p].c1 || cons[p].c2)) {
+      m.key.resize(m.seq.size(), 0);
+      int con[3];
+      pair_keys(pr, cons[p].c1, cons[p].c2, pr.n2 > 0, &m.key[off1 - 1], &m.key[off2 - 1], &m.key[off12 - 1], con);
+      for (int w = 0; w < 3; w++) flags[w] |= con[w] ? CON_KEYS : 0;
+    }
+    // rounded pseudo-energies of s1 and s2, copied into the co-fold's concatenation; |E| summed per strand
+    double sum[2][2] = {{0., 0.}, {0., 0.}};   // [strand][stack, unpaired]
+    long long eu_sum[2] = {0, 0};
+    auto fill = [&](std::vector<int32_t>& v, const double* e1, const double* e2, int kind, bool& any) {
+      if (!e1 && !e2) return;
+      v.resize(m.seq.size(), 0);
+      const double* es[2] = {e1, e2};
+      const int ns[2] = {pr.n1, pr.n2}, offs[2] = {off1, off2}, offc[2] = {off12, off12 + pr.n1};
+      for (int s = 0; s < 2; s++)
+        for (int i = 0; es[s] && i < ns[s]; i++) {
+          const double E = cal_units(es[s][i]);
+          sum[s][kind] += std::fabs(E);
+          if (std::fabs(E) > MFE_MAX_PSEUDO) continue;   // rejected below; keeps the conversion defined
+          v[offs[s] + i] = v[offc[s] + i] = (int32_t)E;
+          if (kind) eu_sum[s] += (int32_t)E;
+          if (E != 0.) {
+            any = true;
+            flags[s] |= kind ? CON_UNPAIRED : CON_STACK;
+            flags[2] |= kind ? CON_UNPAIRED : CON_STACK;
+          }
+        }
+    };
+    if (se) fill(m.es, se[p].e1, se[p].e2, 0, any_es);
+    if (ue) fill(m.eu, ue[p].u1, ue[p].u2, 1, any_eu);
+    any_key |= (flags[0] | flags[1] | flags[2]) & CON_KEYS;
+    const long long lens[3] = {(long long)L.len_s1, (long long)L.len_s2, (long long)L.len_co};
+    const long long outs[3] = {(long long)L.s1, (long long)L.s2, (long long)L.co};
+    const int offs[3] = {off1, off2, off12}, ns[3] = {pr.n1, pr.n2, pr.n1 + pr.n2};
+    for (int w = 0; w < 3; w++) {
+      if (!lens[w]) continue;
+      const double total = w < 2 ? sum[w][0] + sum[w][1] : sum[0][0] + sum[0][1] + sum[1][0] + sum[1][1];
+      if (total > MFE_MAX_PSEUDO) {
+        char buf[200];
+        std::snprintf(buf, sizeof buf,
+                      "pair %d, problem %s: the pseudo-energies give sum |E| = %.2f kcal/mol, beyond %.2f kcal/mol, the "
+                      "range of the MFE kernel's int32 energies",
+                      p, names[w], total / 100.0, MFE_MAX_PSEUDO / 100.0);
+        if (msg) *msg = buf;
+        return RP_ERR_UNSUPPORTED;
+      }
+      MfeJob j;
+      j.seq_off = offs[w];
+      j.n = ns[w];
+      j.cp = w == 2 ? pr.n1 + 1 : 0;
+      j.flags = flags[w];
+      j.out = outs[w];
+      j.energy_at = 3 * p + w;
+      j.eu_const = (int)(w < 2 ? eu_sum[w] : eu_sum[0] + eu_sum[1]);
+      m.jobs.push_back(j);
+      maxn = std::max(maxn, j.n);
+    }
+  }
+  if (!any_key) std::vector<uint16_t>().swap(m.key);
+  else m.key.resize(m.seq.size(), 0);
+  if (!any_es) std::vector<int32_t>().swap(m.es);
+  else m.es.resize(m.seq.size(), 0);
+  if (!any_eu) std::vector<int32_t>().swap(m.eu);
+  else m.eu.resize(m.seq.size(), 0);
+  for (MfeJob& j : m.jobs) {   // a problem without nonzero data of a kind does not bind it
+    if (m.key.empty()) j.flags &= ~CON_KEYS;
+    if (m.es.empty()) j.flags &= ~CON_STACK;
+    if (m.eu.empty()) j.flags &= ~CON_UNPAIRED;
+  }
+  std::stable_sort(m.jobs.begin(), m.jobs.end(), [](const MfeJob& x, const MfeJob& y) { return x.n > y.n; });
+  if (m.jobs.empty()) return RP_OK;
+  // one workspace slot per resident CTA, within the device's memory (long problems: fewer, fatter slots)
+  m.slot_ints = mfe_slot_ints(maxn);
+  const size_t slot_bytes = m.slot_ints * sizeof(int32_t);
+  int g = dev.sm_count * std::max(1, dev.mfe_ctas_per_sm);
+  g = std::min<int>(g, (int)m.jobs.size());
+  if ((size_t)g * slot_bytes > dev.ws_bytes) g = (int)std::min<size_t>(g, std::max<size_t>(1, std::max<size_t>(1, dev.memory()) / 10 * 7 / slot_bytes));
+  m.grid = g;
   return RP_OK;
 }
 

@@ -13,6 +13,7 @@
 #include <vector>
 
 #include "mcc_core.h"
+#include "mfe_core.h"
 #include "ractip_prob.h"
 
 namespace rp {
@@ -36,6 +37,7 @@ struct DeviceFacts {
   int ctas_per_sm = 0;     // occupancy of the general kernel, 64-register build
   int ctas_per_sm1 = 0;    // ... 128-register build
   int up_ctas_per_sm = 0;  // ... of unstru_kernel
+  int mfe_ctas_per_sm = 0; // ... of mfe_kernel
   size_t ws_bytes = 0;     // workspace the context already holds
   // CTAs per SM of the band kernel with `threads` threads and `smem` bytes of dynamic shared memory
   std::function<int(int threads, size_t smem)> band_occupancy;
@@ -129,6 +131,34 @@ int check_samples(const rp_pair* pairs, int n_pairs, const rp_opts* opts, const 
 int plan_batch(const rp_pair* pairs, int n_pairs, const rp_opts* opts, const DeviceFacts& dev, const RouteSettings& rs,
                BatchPlan* plan, const rp_constraint* cons = nullptr, const rp_stack_energy* se = nullptr,
                const rp_sample_opts* so = nullptr, const rp_unpaired_energy* ue = nullptr);
+
+// Minimum free energy structures (rp_run_mfe): the inputs of mfe_kernel.  Per-base arrays are laid out like seq (per
+// pair 0 s1 0 s2 0 s1s2 0) and empty when no problem carries such data: keys as plan_batch builds them, the stacking
+// and unpaired pseudo-energies rounded to integer 0.01 kcal/mol as plan_batch rounds them.
+struct MfePlan {
+  std::vector<uint8_t> seq;
+  std::vector<uint16_t> key;
+  std::vector<int32_t> es, eu;
+  std::vector<MfeJob> jobs;              // longest first
+  std::vector<rp_sample_layout> layout;  // rp_sample_plan with num = 1
+  size_t total = 0;                      // int16 elements of the structure buffer
+  size_t slot_ints = 0;                  // workspace slot of the longest problem (mfe_slot_ints)
+  int grid = 0;                          // CTAs = workspace slots
+};
+// Largest sum of |Es| + |Eu| (0.01 kcal/mol, after rounding) over the bases of one MFE problem: RP_INF / 4.
+constexpr double MFE_MAX_PSEUDO = RP_INF / 4;
+// The pairs must pass check_pairs, the constraints check_constraints, the stacking pseudo-energies
+// check_stack_energies, the unpaired ones check_unpaired_finite, and `problems` may hold RP_SAMPLE_* bits only.  RP_OK;
+// RP_ERR_UNSUPPORTED, naming the pair and the problem, when a requested problem's pseudo-energies exceed
+// MFE_MAX_PSEUDO.
+int plan_mfe(const rp_pair* pairs, int n_pairs, const rp_constraint* cons, const rp_stack_energy* se,
+             const rp_unpaired_energy* ue, int problems, const DeviceFacts& dev, MfePlan* plan, std::string* msg);
+// Everything rp_run_mfe checks before planning, in its order: pairs (RP_ERR_ARG), lengths (RP_ERR_TOO_LONG), unknown
+// problem bits (RP_ERR_ARG), then check_constraints, check_stack_energies and check_unpaired_finite with their messages.
+int check_mfe(const rp_pair* pairs, int n_pairs, const rp_constraint* cons, const rp_stack_energy* se,
+              const rp_unpaired_energy* ue, int problems, std::string* msg);
+// The non-finite check of check_unpaired_energies alone (the same messages), without its range check.
+int check_unpaired_finite(const rp_pair* pairs, const rp_unpaired_energy* ue, int n_pairs, std::string* msg);
 
 }  // namespace rp
 #endif

@@ -22,7 +22,7 @@ import numpy as np
 from . import _lib
 from ._lib import RpIpOpts, RpModel, RpOpts
 from .ip import JointPrediction, default_ip_opts, solve_joint, solve_ss, zscore_statistic
-from .stage import ProbabilityStage, RpError, default_opts, joint_structure, shape_deigan, zscore_shuffles
+from .stage import ProbabilityStage, RpError, default_opts, dot_bracket, joint_structure, shape_deigan, zscore_shuffles
 
 
 @dataclass
@@ -144,6 +144,8 @@ class PairResult:
     e2s: Optional[float] = None
     zscore: Optional[Tuple[float, float]] = None
     samples: Optional[List[Tuple[str, str]]] = None   # co-fold samples (r1, r2) in RactIP's notation (predict(samples=))
+    # minimum free energy structures (predict(mfe=True)): {"s1", "s2", "co": (pair table, kcal/mol)}, ProbabilityStage.mfe
+    mfe: Optional[Dict[str, Tuple[np.ndarray, float]]] = None
 
 
 def _f(x: float) -> str:
@@ -162,6 +164,15 @@ def format_result(r: PairResult, show_energy: bool = False) -> str:
     if r.zscore is not None:
         out.append(f"z-score: {_f(r.zscore[0])}, {_f(r.zscore[1])}")
     out.extend(f"{r1}&{r2}" for r1, r2 in r.samples or [])
+    if r.mfe:
+        for name, label in (("s1", "s1"), ("s2", "s2")):
+            if name in r.mfe:
+                t, e = r.mfe[name]
+                out.append(f"MFE {label}: {dot_bracket(t)} ({e:.2f})")
+        if "co" in r.mfe:
+            t, e = r.mfe["co"]
+            r1, r2 = joint_structure(t, len(r.a.seq))
+            out.append(f"MFE s1&s2: {r1}&{r2} ({e:.2f})")
     return "\n".join(out)
 
 
@@ -169,7 +180,7 @@ def predict(stage: ProbabilityStage, pairs: Sequence[Tuple[FastaRecord, FastaRec
             ip_opts: Optional[RpIpOpts] = None, show_energy: bool = False, zscore: int = 0, num_shuffling: int = 1000,
             seed: int = 1, use_constraint: bool = False, shape: Optional[Dict[str, Sequence[float]]] = None,
             shape_slope: float = 1.8, shape_intercept: float = -0.6, samples: int = 0,
-            sample_seed: int = 1, shape_method: str = "D") -> List[PairResult]:
+            sample_seed: int = 1, shape_method: str = "D", mfe: bool = False) -> List[PairResult]:
     """Joint structures of all `pairs`: one GPU batch for every pair's matrices, then the integer programmes on the
     host.  zscore in (1, 2, 12): per pair one more GPU batch with all its dinucleotide shuffles (the loop of
     src/ractip.cpp:1636-1657 with the probability work hoisted out of it).  use_constraint (-c): the records'
@@ -180,7 +191,9 @@ def predict(stage: ProbabilityStage, pairs: Sequence[Tuple[FastaRecord, FastaRec
     as unpaired pseudo-energies in kcal/mol instead (RNAfold --shapeMethod=W; a missing position counts as 0, negative
     values are valid, slope and intercept do not apply).  samples > 0: that many structures
     of each pair's s1&s2 co-fold ensemble (constraints and pseudo-energies included), drawn with sample_seed in the
-    same GPU batch, on PairResult.samples; the shuffles are never sampled."""
+    same GPU batch, on PairResult.samples; the shuffles are never sampled.  mfe: each pair's minimum free energy
+    structures of s1, s2 and the s1&s2 co-fold under the same constraints and pseudo-energies as its probabilities
+    (ProbabilityStage.mfe), on PairResult.mfe; the shuffles never get one."""
     opts = opts if opts is not None else default_opts()
     ip_opts = ip_opts if ip_opts is not None else default_ip_opts()
     model: RpModel = stage.model
@@ -213,11 +226,14 @@ def predict(stage: ProbabilityStage, pairs: Sequence[Tuple[FastaRecord, FastaRec
             bt.close()
     else:
         probs = stage.run_dense(seqs, opts, constraints=cons, **kw)
+    mfes = stage.mfe(seqs, cons, kw.get("stack_energies"), kw.get("unpaired_energies")) if mfe else None
     out = []
     for k, ((a, b), p) in enumerate(zip(pairs, probs)):
         res = PairResult(a, b, solve_joint(model, a.seq, b.seq, p, ip_opts, energies=energies))
         if drawn is not None:
             res.samples = drawn[k]
+        if mfes is not None:
+            res.mfe = mfes[k]
         if energies:
             _, _, res.e1s = solve_ss(model, a.seq, p.bp1, ip_opts, energy=True)
             _, _, res.e2s = solve_ss(model, b.seq, p.bp2, ip_opts, energy=True)

@@ -447,6 +447,38 @@ class ProbabilityStage:
         except Exception:
             pass
 
+    # ------------------------------------------------------------- minimum free energy
+    def mfe(self, pairs: Sequence[Tuple[str, str]], constraints=None, stack_energies=None, unpaired_energies=None,
+            problems: Sequence[str] = ("s1", "s2", "co")) -> List[Dict[str, Tuple[np.ndarray, float]]]:
+        """rp_run_mfe: per pair {problem: (int16 pair table, MFE in kcal/mol)} for each of `problems` ("s1", "s2",
+        "co"; a pair with an empty s2 has s1 only).  constraints, stack_energies, unpaired_energies as DeviceBatch
+        takes them.  The co-fold's table runs over s1 s2 (joint_structure turns it into RactIP's notation) and its
+        energy counts DuplexInit when a pair joins the strands, as energy_of_duplex does."""
+        pairs = list(pairs)
+        n = len(pairs)
+        so = sample_opts(1, 1, problems)
+        arr, keep = _make_pairs(pairs)
+        cons, ckeep = _make_constraints(constraints, n) if constraints is not None else (None, None)
+        se, ekeep = _make_stack_energies(stack_energies, pairs) if stack_energies is not None else (None, None)
+        ue, ukeep = (_make_energies(unpaired_energies, pairs, RpUnpairedEnergy, "unpaired_energies", "u")
+                     if unpaired_energies is not None else (None, None))
+        layout = (RpSampleLayout * max(n, 1))()
+        tot = C.c_size_t()
+        self._check(self.lib.rp_sample_plan(arr, n, C.byref(so), layout, C.byref(tot)))
+        tables = np.zeros(max(tot.value, 1), dtype=np.int16)
+        energies = np.zeros(max(3 * n, 1), dtype=np.int32)
+        self._check(self.lib.rp_run_mfe(self.ctx, arr, cons, se, ue, n, so.problems, tables.ctypes.data, tot.value,
+                                        energies.ctypes.data))
+        out = []
+        for k in range(n):
+            L = layout[k]
+            d = {}
+            for w, (name, off, ln) in enumerate((("s1", L.s1, L.len_s1), ("s2", L.s2, L.len_s2), ("co", L.co, L.len_co))):
+                if ln:
+                    d[name] = (tables[off:off + ln].copy(), int(energies[3 * k + w]) / 100.0)
+            out.append(d)
+        return out
+
     # ------------------------------------------------------------- batches
     def batch(self, pairs: Sequence[Tuple[str, str]], opts: Optional[RpOpts] = None,
               constraints=None, stack_energies=None, samples: int = 0, sample_seed: int = 1,
